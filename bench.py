@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- env steps/s (and MCTS sims/s) of the B200-native Onitama self-play hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload env|mcts|playout] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload env|mcts|playout] [--impl ours|reference] [--dump-outputs DIR]
 
 One process per GPU (torchrun for N > 1, NCCL only for the barrier / max-over-ranks of the timings: games shard
 across GPUs with no data-path collective, scaling = weak). A "step" is one pass of the hot path over one batch:
@@ -11,6 +11,8 @@ across GPUs with no data-path collective, scaling = weak). A "step" is one pass 
   playout (BASELINE config 1): 4 096 random-vs-random games to terminal.
 The default run measures env as the headline and appends the mcts numbers under "mcts" in the same JSON line.
 --impl reference times the CPU restatement of the reference path (oracle/, all host threads) on the same workload.
+--dump-outputs DIR writes what the last timed step computed (env, and the mcts section or workload) as DIR/<name>.npy, for a fixed
+seeded sample of the games / trees, so that two builds can be compared output for output on identical inputs.
 """
 import argparse
 import ctypes
@@ -34,6 +36,7 @@ SELFPLAY_GAMES = 16384
 SELFPLAY_SIMS = 800
 GAMES_SLOTS = 2048     # `games` workload: slots per GPU (a step plays 2 x slots whole games)
 SEED = 20240607
+DUMP_SAMPLE = 4096     # --dump-outputs: games / trees per dumped array (env planes: 8.6 MB)
 NET_PRECISION = {"fused-f32": "f32", "fused": "f16", "fused-tf32": "tf32", "torch": "torch"}
 NET_KERNEL = {"fused-f32": "k_net_forward_x3p<true> (CTA pairs, tcgen05 cta_group::2)", "fused": "k_net_forward_f16q<true> (CTA pairs, tcgen05 cta_group::2, four accumulators)", "fused-tf32": "k_net_forward<2,tf32>",
               "torch": "library kernels"}
@@ -212,6 +215,21 @@ def cpu_selfplay(n_trees, sims):
     return done / dt, dt, torch.get_num_threads()
 
 
+def dump_sample(n):
+    """--dump-outputs: the fixed, seeded subset of the n games / trees whose outputs are written (sorted indices)"""
+    import numpy as np
+    return np.sort(np.random.default_rng(SEED).choice(n, min(n, DUMP_SAMPLE), replace=False))
+
+
+def write_dump(path, arrays):
+    import numpy as np
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20, "dump larger than 64 MB"
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def all_deals():
     return [[a, b, c, d, e] for a in range(16) for b in range(a + 1, 16) for c in range(16) if c not in (a, b)
             for d in range(c + 1, 16) if d not in (a, b) for e in range(16) if e not in (a, b, c, d)]
@@ -379,7 +397,12 @@ def main():
     ap.add_argument("--net", default="fused-f32", choices=["fused-f32", "fused", "fused-tf32", "torch"],
                     help="selfplay workload: the tensor-core network kernel -- fused-f32 = f32-faithful split-operand arithmetic (the headline: "
                          "the reference computes in f32), fused = the f16 fast mode, fused-tf32 = tf32 operands -- or the PyTorch module as a black box")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="env and mcts workloads: after the timed steps, write what the last timed step computed to DIR/<name>.npy (float32 or "
+                         "float64, a fixed seeded sample of %d games / trees; the default env run adds its mcts section as mcts_*)" % DUMP_SAMPLE)
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in ("env", "mcts")):
+        ap.error("--dump-outputs covers the env and mcts workloads of --impl ours")
     claim_stdout()
     dflt = {"env": (1000, 50), "mcts": (20, 5), "perft": (5, 3), "selfplay": (3, 3), "playout": (50, 5), "uct": (5, 3), "games": (1, 3)}[args.workload]
     if args.impl == "reference":
@@ -387,6 +410,8 @@ def main():
     args.steps_given = args.steps is not None
     args.steps = dflt[0] if args.steps is None else args.steps
     args.warmup = dflt[1] if args.warmup is None else args.warmup
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -495,6 +520,15 @@ def main():
         ms, clocks = timed(lambda i: ctx.step_random(i, auto_reset=True, out_flags=flags), warmup, steps)
         st = ctx.stats()
         assert int(st[onb.STAT_STEPS]) == n * (steps + warmup), "kernel did not step every game"
+        dump = {}
+        if args.dump_outputs and rank == 0:   # the last timed step's states, masks and planes, before the e2e runs below reset the games
+            idx = dump_sample(n)
+            sel = torch.from_numpy(idx).cuda()
+            dump = {"env_games": idx.astype(np.float64),
+                    "env_states": ctx.get_states()[idx].view("<u4").reshape(len(idx), 6).astype(np.float64),
+                    "env_masks": ctx.tensor(onb.BUF_MASKS)[sel].cpu().numpy().view(np.uint32).astype(np.float64),
+                    "env_planes": ctx.tensor(onb.BUF_PLANES)[sel].cpu().numpy(),
+                    "env_stats": st.astype(np.float64)}
         value = world * n * steps / (ms * 1e-3)
         kernel_ms = ms / steps  # one k_env_step launch per step
         achieved = ENV_BYTES_PER_STEP * n / (kernel_ms * 1e-3) / 1e9
@@ -573,7 +607,7 @@ def main():
         ctx.close()
         del host_actions
         return dict(metric="env_steps_per_sec", value=value, unit="env_steps/s", ms_per_step=ms / steps, dtype="u32", roofline=roof, e2e=e2e,
-                    gpu_launches=steps, clocks=clocks)
+                    gpu_launches=steps, clocks=clocks, dump=dump)
 
     # ---------------------------------------------------------------- mcts (config 4)
     def bench_mcts(steps, warmup):
@@ -603,6 +637,13 @@ def main():
         ms, clocks = timed(one, warmup, steps)
         nn, fl = ctx.mcts_tree_info()
         assert int((fl & 2).sum()) == 0, "node pool overflow"
+        dump = {}
+        if args.dump_outputs and rank == 0:   # the last timed search's results as onb_mcts_finish hands them to a caller
+            idx = dump_sample(n)
+            r = ctx.mcts_finish(to_host=True)
+            dump = {"mcts_trees": idx.astype(np.float64), "mcts_best": r["best"][idx].astype(np.float64),
+                    "mcts_pi": r["pi"][idx].reshape(len(idx), 50), "mcts_root_visits": r["root_visits"][idx].astype(np.float64),
+                    "mcts_root_q": r["root_q"][idx], "mcts_child_visits": r["child_visits"][idx].astype(np.float64)}
         value = world * n * sims * steps / (ms * 1e-3)
         # measured tree shape -> algorithmic bytes per simulation (DESIGN.md section 5), from the GPU's own trees:
         # mean select depth d = sum of visits of non-root nodes / sims, mean children k = (nodes - 1) / expanded nodes
@@ -653,7 +694,7 @@ def main():
         roof["train_mode_noise"] = {"value": world * n * sims * 3 / (tms * 1e-3), "unit": "sims/s", "ms_per_step": tms / 3}
         ctx.close()
         return dict(metric="mcts_sims_per_sec", value=value, unit="sims/s", ms_per_step=run_ms, dtype="u32+f64", roofline=roof, e2e=e2e,
-                    gpu_launches=3 * steps, clocks=clocks)
+                    gpu_launches=3 * steps, clocks=clocks, dump=dump)
 
     # ---------------------------------------------------------------- playout (config 1)
     def bench_playout(steps, warmup):
@@ -894,12 +935,14 @@ def main():
 
     secondary = None
     third = None
+    dumps = dict(out.get("dump", {}))
     if wl == "env" and not args.no_secondary:
         # the config-4 and config-5 sections obey --steps/--warmup too (their own defaults when the flags are absent; config 5 is
         # capped at 30 plies of 0.3 s so that an env-sized --steps cannot turn the run into minutes) and carry their own clocks
         m_steps, m_warm = (args.steps, args.warmup) if args.steps_given else (20, 5)
         m_steps = min(m_steps, 200)
         m = bench_mcts(m_steps, max(3, m_warm))
+        dumps.update(m["dump"])
         secondary = {k: m[k] for k in ("metric", "value", "unit", "ms_per_step", "roofline", "e2e", "gpu_launches", "clocks")}
         secondary["config"] = workload_config("mcts")
         secondary["steps"], secondary["warmup"] = m_steps, max(3, m_warm)
@@ -977,6 +1020,8 @@ def main():
             line["mcts"] = secondary
         if third is not None:
             line["selfplay"] = third
+        if args.dump_outputs:
+            write_dump(args.dump_outputs, dumps)
         emit_line(line)
     if world > 1:
         dist.barrier()

@@ -1,5 +1,5 @@
-"""The network stand-in: architecture restated from net.rs; loads the reference's .ot archives when they are available
-(build container only -- /root/reference does not exist on the GPU box)."""
+"""The network stand-in: architecture restated from net.rs; the reference's shipped 3-block weights come from
+tests/golden/net_golden.npz, written into .ot archives where a test needs one."""
 import os
 
 import pytest
@@ -17,16 +17,20 @@ def test_shapes_and_param_count():
     assert sum(v.numel() for k, v in ConvResNet(64, 21, 5).state_dict().items() if not k.endswith("num_batches_tracked")) == 388742
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/models/model_5e-3_3_resnet.ot"), reason="reference weights not present")
-def test_loads_reference_ot_archive():
+def test_loads_reference_ot_archive(tmp_path):
+    """The reference's 3-block weights in the archive layout VarStore::save writes load tensor for tensor and evaluate; a 5-block
+    archive loads into a 5-block module."""
     from onitama_alphazero_b200.net import ConvResNet, make_evaluator
-    m = ConvResNet(64, 21, 3).load_ot("/root/reference/models/model_5e-3_3_resnet.ot")
+    weights = golden_tensors()
+    m = ConvResNet(64, 21, 3).load_ot(golden_ot(tmp_path))
+    sd = m.state_dict()
+    assert all(torch.equal(sd[k], w) for k, w in weights.items())
     net = make_evaluator(m)
     x = torch.zeros(2, 21, 5, 5)
     x[:, 0, 4, :] = 1
     p, v = net(x)
     assert p.shape == (2, 2, 25) and v.shape == (2,) and torch.isfinite(p).all() and torch.equal(p[0], p[1])
-    m5 = ConvResNet(64, 21, 5).load_ot("/root/reference/models/model_5e-3.ot")
+    m5 = ConvResNet(64, 21, 5).load_ot(lively_model(5).save_ot(str(tmp_path / "five.ot")))
     assert m5.n_blocks == 5
 
 
@@ -94,12 +98,13 @@ def test_oracle_network_matches_the_pytorch_twin(blocks):
     assert p_ref.reshape(-1, 50).std(0).max() > 0.01 and v_ref.std() > 0.01   # the outputs do depend on the position
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/models/model_5e-3_3_resnet.ot"), reason="reference weights not present")
 def test_oracle_network_with_reference_weights():
     import numpy as np
     import oracle_lib as O
     from onitama_alphazero_b200.net import ConvResNet
-    m = ConvResNet(64, 21, 3).load_ot("/root/reference/models/model_5e-3_3_resnet.ot").eval()
+    m = ConvResNet(64, 21, 3)
+    m.load_state_dict(golden_tensors(), strict=False)
+    m.eval()
     g = O.new_games(8, seed=1)
     planes = O.encode(g).reshape(-1, 21, 5, 5)
     with torch.no_grad():
@@ -114,6 +119,19 @@ def load_net_golden():
     z = np.load(os.path.join(os.path.dirname(__file__), "golden", "net_golden.npz"))
     weights = {k[2:]: z[k] for k in z.files if k.startswith("w:")}
     return weights, z["planes"], z["policy"], z["value"]
+
+
+def golden_tensors():
+    """the reference's 3-block weights from the fixture as torch tensors (state_dict names, no num_batches_tracked)"""
+    return {k: torch.from_numpy(w) for k, w in load_net_golden()[0].items()}
+
+
+def golden_ot(tmp_path):
+    """the fixture's weights written as the reference's 3-block .ot archive; returns its path"""
+    from onitama_alphazero_b200.net import write_ot
+    path = str(tmp_path / "model_5e-3_3_resnet.ot")
+    write_ot(golden_tensors(), path)
+    return path
 
 
 def test_oracle_network_on_the_reference_trained_weights_fixture():
@@ -134,18 +152,19 @@ def test_oracle_network_on_the_reference_trained_weights_fixture():
     assert pol.std(0).max() > 0.01          # the trained policy head does depend on the position
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/models/model_5e-3.ot"), reason="reference weights not present")
-def test_ot_archives_block_count_is_inferred_and_mismatches_are_errors():
+def test_ot_archives_block_count_is_inferred_and_mismatches_are_errors(tmp_path):
     """ADVICE r01: four of the reference's five checkpoints have 5 residual blocks (ConvResNetConfig::default, net.rs:82-90); loading one
     into a 3-block module must not silently drop resnet_3 / resnet_4."""
     from onitama_alphazero_b200.net import ConvResNet
+    five = lively_model(5).save_ot(str(tmp_path / "model_5e-3.ot"))
+    three = golden_ot(tmp_path)
     assert ConvResNet().n_blocks == 5
-    assert ConvResNet.from_ot("/root/reference/models/model_5e-3.ot").n_blocks == 5
-    assert ConvResNet.from_ot("/root/reference/models/model_5e-3_3_resnet.ot").n_blocks == 3
+    assert ConvResNet.from_ot(five).n_blocks == 5
+    assert ConvResNet.from_ot(three).n_blocks == 3
     with pytest.raises(KeyError, match="unexpected"):
-        ConvResNet(64, 21, 3).load_ot("/root/reference/models/model_5e-3.ot")
+        ConvResNet(64, 21, 3).load_ot(five)
     with pytest.raises(KeyError, match="missing"):
-        ConvResNet(64, 21, 5).load_ot("/root/reference/models/model_5e-3_3_resnet.ot")
+        ConvResNet(64, 21, 5).load_ot(three)
 
 
 def test_ot_writer_round_trip(tmp_path):
@@ -164,12 +183,10 @@ def test_ot_writer_round_trip(tmp_path):
     assert "resnet_1|resnet_small_block2|small_block_bn|running_var" in names and "conv_init_1|weight" in names
     assert not any("." in n or "num_batches_tracked" in n for n in names)
     assert names["bn1|running_mean"] is False and names["bn1|weight"] is True
-    if os.path.exists("/root/reference/models/model_5e-3_3_resnet.ot"):   # same names, dtypes and shapes as an archive the reference wrote
-        ref = read_ot("/root/reference/models/model_5e-3_3_resnet.ot")
-        mine = ConvResNet(64, 21, 3)
-        p3 = mine.save_ot(str(tmp_path / "three.ot"))
-        got = read_ot(p3)
-        assert sorted(got) == sorted(ref) and all(got[k].shape == ref[k].shape and got[k].dtype == ref[k].dtype for k in ref)
+    # same names and shapes as the reference's 3-block archive (the fixture holds its tensors), all f32
+    ref = load_net_golden()[0]
+    got = read_ot(ConvResNet(64, 21, 3).save_ot(str(tmp_path / "three.ot")))
+    assert sorted(got) == sorted(ref) and all(got[k].shape == ref[k].shape and got[k].dtype == torch.float32 for k in ref)
 
 
 def test_stats_json_layout(tmp_path):
