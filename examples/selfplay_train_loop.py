@@ -7,7 +7,7 @@
 Everything game-, search- and inference-related runs in libonb.so: the current weights are handed to the library with
 onb_net_load after every update and evaluated by the tensor-core kernel between select and expand. The optimiser, the
 backward pass and the bookkeeping are plain PyTorch / Python (out of scope of the hot path).
-Usage: python examples/selfplay_train_loop.py [--slots 256] [--games 512] [--sims 64] [--iters 2] [--torch-net]
+Usage: python examples/selfplay_train_loop.py [--slots 256] [--games 512] [--sims 64] [--iters 2] [--hidden {64,128}] [--torch-net]
 """
 import argparse
 import os
@@ -35,11 +35,12 @@ def main(argv=None):
     ap.add_argument("--torch-net", action="store_true", help="evaluate with the PyTorch module as a black box instead of onb_net_load")
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--out", default=None, help="directory for the reference's on-disk artefacts: loss_stats JSON (stats.rs) and .ot checkpoints (train.rs:414-430)")
+    ap.add_argument("--hidden", type=int, default=64, choices=[64, 128], help="hidden channels of the ConvResNet (both run on the tensor cores)")
     ap.add_argument("--net-precision", default="f32", choices=["f32", "f16", "tf32"], help="arithmetic of the on-device network (f32 = the reference's)")
     args = ap.parse_args(argv)
 
     torch.manual_seed(args.seed)
-    model = ConvResNet(64, 21, 3).cuda().eval()
+    model = ConvResNet(args.hidden, 21, 3).cuda().eval()
     opt = torch.optim.SGD(model.parameters(), lr=1e-2, weight_decay=1e-4)  # train.rs:181-186
     replay = onb.ReplayBuffer(200_000, device="cuda")
     log = []

@@ -436,8 +436,9 @@ ONB_API int32_t onb_uct_run(onb_ctx* ctx, float exploration_c, uint32_t min_node
  * onb_net_load takes the parameters under the reference's VarStore names (net.rs:118-213, `|` or `.` separators),
  * e.g. "conv_init_1|weight", "bn1|running_var", "resnet_0|resnet_small_block1|small_block_conv|weight",
  * "policy_conv|bias", "ph_linear2|weight", "vh_linear1|weight": host f32 arrays in libtorch layout (OIHW, [out][in]).
- * The number of residual blocks is taken from the names; hidden_channels must be 64 and input_channels 21
- * (ConvResNetConfig of train.rs) -- anything else is rejected with ONB_E_INVALID.
+ * The number of residual blocks is taken from the names and hidden_channels from bn1|weight: 64 (ConvResNetConfig of train.rs)
+ * or 128, with input_channels 21 -- any other width, or a tensor whose size does not match the width, is rejected with
+ * ONB_E_INVALID. The two resident slots may hold networks of different widths.
  * onb_net_forward reads planes_buffer (ONB_BUF_LEAF_PLANES or ONB_BUF_PLANES, [n][21][5][5] f32) and writes
  * ONB_BUF_POLICY [n][2][25] (softmax over 50) and ONB_BUF_VALUE [n]. onb_mcts_eval / onb_mcts_run accept ONB_EVAL_NET. */
 #define ONB_NET_F16 0  /* fast mode: operands rounded to f16 (11-bit significand), f32 accumulation */

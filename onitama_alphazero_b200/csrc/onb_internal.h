@@ -77,6 +77,7 @@ struct Ctx {
         float* bias;  // folded biases
         float* head;  // head parameters
         int blocks, loaded, f16, x3;  // f16: f16 operands (else tf32); x3: split-operand f32-faithful mode (ONB_NET_F32)
+        int hid;                      // hidden channels: 64 (the k_net_forward family) or 128 (k_net_wide)
         size_t pair_off;              // x3: byte offset in w of the taps in CTA-pair order (onb_net.cu, k_net_forward_x3p<true>)
     } net[2];         // two networks can be resident (an arena pits the new model against the previous one, evaluator.rs:355-399)
     void* sp_buf[32];          // grow-only buffers of onb_self_play (slots 0-15) and onb_fight (16-31), see onb_selfplay.cu

@@ -2658,6 +2658,324 @@ __global__ void __launch_bounds__(256, 3)
     if (warp == 0) tmem_dealloc(tmem, G::TMEM_COLS);
 }
 
+// ---- 128 hidden channels (ConvResNetConfig{hidden_channels: 128}) ---------------------------------------------------------------
+// The structure of k_net_forward, widened: a cell row of the activation matrix is 2 (f16) or 4 (tf32) 128-byte blocks, a weight
+// tap is 128 B rows (N = 128) in the same swizzled K-major layout, so one block of a tap is 128 x 128 bytes. Per K step a tap costs
+// one N = 128 MMA per accumulator; ONB_NET_F32 issues a1 x [b1 ; b2] as ONE N = 256 MMA (the weight copies of a 128-byte block
+// are interleaved per block, [kb][b1 | b2][128 rows]) and a2 x b1 as N = 128, so D1 | D2 sit side by side in 256 TMEM columns.
+// Geometry (one CTA per SM in every mode; TMEM and shared memory leave no room for a second):
+//   f16:  2 accumulators x 128 cells (7 boards), TMEM 2 sets x 2 x 128 = 512 columns, activations 272 rows x 256 B, 3 slots of 32 KB
+//   tf32: 1 accumulator (3 boards), TMEM 2 x 128 = 256, activations 128 rows x 512 B, 2 slots of 64 KB
+//   f32:  1 accumulator (3 boards), TMEM 2 x 256 (D1 | D2), a1 + a2 of 128 rows x 256 B, 2 slots of 64 KB (b1, b2)
+constexpr int kHidW = 128;
+// head parameter blob of the wide network (floats): 1x1 head convolutions [128] each, their biases, ph_linear2 [50 in][50 out] + bias,
+// vh_linear1 [25 in][128 out] + bias, vh_linear2 [128] + bias
+constexpr int kWP0 = 0, kWP1 = 128, kWV = 256, kWB = 384, kWPhW = 388, kWPhB = 2888, kWV1W = 2940, kWV1B = 6140, kWV2W = 6268,
+              kWV2B = 6396, kWHeadFloats = 6400;
+template <bool F16, bool X3>
+struct GeoW {
+    static_assert(!X3 || F16, "the split-operand mode is built on f16 operands");
+    static constexpr int CPC = F16 ? 8 : 4;              // channels per 16-byte chunk
+    static constexpr int KB = kHidW / CPC / 8;           // 128-byte blocks per activation row / weight row: 2 | 4
+    static constexpr int KSTEPS = kHidW / CPC / 2;       // 32-byte K steps per tap: 8 | 16
+    static constexpr int KSTEPS0 = (F16 ? 32 : 24) / CPC / 2;  // first layer: 21 planes padded to K = 32 | 24: 2 | 3 steps
+    static constexpr int NMAT = X3 ? 2 : 1;
+    static constexpr int NACC = F16 && !X3 ? 2 : 1;      // accumulators of 128 cells
+    static constexpr int NB = NACC == 2 ? 7 : 3;         // boards per pass
+    static constexpr int CELLS = NB * kCellsPerBoard;
+    static constexpr int R = (kLead + CELLS + kTrail + 7) / 8 * 8;
+    static constexpr int WBLK = kHidW * 128;             // one 128-byte block of all 128 weight rows
+    static constexpr int TAP0_BYTES = NMAT * WBLK;       // a first-layer tap (all copies)
+    static constexpr int TAP_BYTES = NMAT * KB * WBLK;   // a tap of a 128 -> 128 layer (all copies)
+    static constexpr int NSLOT = NACC == 2 ? 3 : 2;      // single-tap ring slots
+    static constexpr int SLOT_BYTES = TAP_BYTES;
+    static constexpr int ACT_BYTES = R * KB * 128;       // a multiple of 1024
+    static constexpr int OFF_RING = NMAT * ACT_BYTES;
+    static constexpr int OFF_HEAD = OFF_RING + NSLOT * SLOT_BYTES;
+    static constexpr int SPLIT = 2 / NACC;               // threads per cell in the epilogue (each takes 128 / SPLIT channels)
+    static constexpr int HEAD_BYTES = ((SPLIT * NB * 75 * 4 + 15) / 16) * 16;
+    static constexpr int OFF_BAR = OFF_HEAD + HEAD_BYTES;
+    static constexpr int SMEM = OFF_BAR + (2 * NSLOT + 1) * 8 + 16;
+    static constexpr int ACC_COLS = X3 ? 256 : 128;      // TMEM columns per accumulator (X3: D1 | D2)
+    static constexpr int SET_COLS = NACC * ACC_COLS;
+    static constexpr int TMEM_COLS = 2 * SET_COLS;       // the plain set + the residual-preloaded set
+    static constexpr uint32_t IDESC = Op<F16>::IDESC_N128, IDESC_X3 = Op<true>::idesc(256);
+    // X3: the 9 taps x 128 channels (K = 1152) of a layer are summed in NPH phases of 3 taps: after each phase the epilogue threads
+    // add D1 + 2^-11 D2 into f32 registers and the next phase starts from zero. The tensor core's f32 accumulation error grows
+    // with the number of products it sums; in one phase the f32-faithful mode missed its 1e-5 bound (max |dv| 1.75e-5 on the
+    // 3-block test network, B200), in phases of 3 taps each accumulator sums 384 products, fewer than the 576 of the 64-wide layers
+    static constexpr int NPH = X3 ? 3 : 1;
+    static_assert(SMEM <= 227 * 1024, "shared memory");
+    static_assert(CELLS <= NACC * 128, "cells must fit the accumulators");
+    static_assert(TMEM_COLS == 256 || TMEM_COLS == 512, "power of two");
+    static_assert(ACT_BYTES % 1024 == 0 && SLOT_BYTES % 1024 == 0, "swizzle period");
+};
+
+template <bool F16, bool X3>
+__global__ void __launch_bounds__(256, 1)
+    k_net_wide(const float* __restrict__ planes, float* __restrict__ policy, float* __restrict__ value, int64_t n, NetDev net) {
+    using G = GeoW<F16, X3>;
+    constexpr int NB = G::NB, CELLS = G::CELLS, R = G::R, NSLOT = G::NSLOT, NACC = G::NACC, SPLIT = G::SPLIT;
+    extern __shared__ __align__(1024) uint8_t smem[];
+    const uint32_t s_act = smem_u32(smem), s_ring = s_act + G::OFF_RING, s_bar = s_act + G::OFF_BAR;
+    float* s_head = reinterpret_cast<float*>(smem + G::OFF_HEAD);  // [SPLIT][NB][75] partial 1x1 head sums
+    uint32_t* s_tmem = reinterpret_cast<uint32_t*>(smem + G::OFF_BAR + (2 * NSLOT + 1) * 8);
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int L = 1 + 2 * net.n_blocks;
+    const int64_t n_groups = (n + NB - 1) / NB;
+    if ((int64_t)blockIdx.x >= n_groups) return;
+    const int64_t my_groups = (n_groups - blockIdx.x + gridDim.x - 1) / gridDim.x;
+    const uint32_t total_units = (uint32_t)my_groups * (uint32_t)(9 * L);
+    auto bar_full = [&](uint32_t s) { return s_bar + s * 8u; };
+    auto bar_empty = [&](uint32_t s) { return s_bar + (NSLOT + s) * 8u; };
+    const uint32_t bar_acc = s_bar + 2 * NSLOT * 8u;
+
+    if (tid == 0) {
+        for (uint32_t s = 0; s < (uint32_t)NSLOT; ++s) {
+            mbar_init(bar_full(s), 1);
+            mbar_init(bar_empty(s), 1);
+        }
+        mbar_init(bar_acc, 1);
+        fence_barrier_init();
+    }
+    if (warp == 0) tmem_alloc(smem_u32(s_tmem), G::TMEM_COLS);
+    for (int i = tid; i < G::NMAT * G::ACT_BYTES / 16; i += 256) st_shared_v4(s_act + i * 16, 0u, 0u, 0u, 0u);  // pad cells stay zero
+    fence_proxy_async();
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem = *s_tmem;
+    constexpr uint32_t A2 = X3 ? (uint32_t)G::ACT_BYTES : 0u;
+    constexpr uint32_t ACC = (uint32_t)G::ACC_COLS, SET = (uint32_t)G::SET_COLS;
+    // epilogue ownership: TMEM lane quarter warp & 3; with two accumulators warp >> 2 picks the accumulator, with one it picks the
+    // half of the channels (both threads of a cell then write partial head sums that the head stage adds in a fixed order)
+    const int ep_acc = NACC == 2 ? (warp >> 2) : 0, ep_part = NACC == 2 ? 0 : (warp >> 2);
+    constexpr int EP_CH = kHidW / SPLIT;
+    static_assert(!X3 || EP_CH == 64, "the phase sums of the split mode are two halves of 32 channels");
+
+    uint32_t q0 = 0, q_prod = 0, acc_par = 0;
+    for (int64_t gi = 0; gi < my_groups; ++gi) {
+        const int64_t board0 = ((int64_t)blockIdx.x + gi * gridDim.x) * NB;
+        for (int cell = tid; cell < CELLS; cell += 256) {
+            const Cell c = decode_cell(cell, CELLS);
+            if (!c.real) continue;
+            const int64_t gb = board0 + c.board;
+            const float* src = planes + gb * 525 + c.pos;
+            float x[32];
+#pragma unroll
+            for (int ch = 0; ch < 32; ++ch) x[ch] = (ch < kInPlanes && gb < n) ? __ldg(src + ch * 25) : 0.f;
+            if (X3) store_channels_x3(s_act, A2, R, kLead + cell, 0, x);
+            else store_channels<F16>(s_act, R, kLead + cell, 0, x);
+        }
+        fence_proxy_async();
+        for (int l = 0; l < L; ++l) {
+            tc_fence_before();
+            __syncthreads();
+            tc_fence_after();
+            const bool use_s = l >= 2 && (l & 1) == 0;
+            const bool last = l == L - 1;
+            const uint32_t tlane = tmem + ((uint32_t)((warp & 3) * 32) << 16);
+            const uint32_t tsrc = tlane + (use_s ? SET : 0u) + ep_acc * ACC, tskip = tlane + SET + ep_acc * ACC;
+            float part[X3 ? EP_CH : 1];  // X3: the sums of the earlier phases (see GeoW::NPH); X3 has EP_CH = 64
+#pragma unroll 1
+            for (int ph = 0; ph < G::NPH; ++ph) {
+                const int t_begin = ph * 9 / G::NPH, t_end = (ph + 1) * 9 / G::NPH;
+                if (warp == 0) {
+                    const bool elected = elect_one();
+                    const uint32_t dcol = tmem + (use_s ? SET : 0u);
+                    const int ksteps = l == 0 ? G::KSTEPS0 : G::KSTEPS;
+#pragma unroll 1
+                    for (int t = t_begin; t < t_end; ++t) {
+                        const uint32_t u = q0 + t, slot = u % NSLOT, use = u / NSLOT;
+                        mbar_wait(bar_full(slot), use & 1u);
+                        tc_fence_after();
+                        const int row0 = kLead + (t / 3 - 1) * 6 + (t % 3 - 1);
+                        const uint32_t a_lo = desc_lo(s_act + (uint32_t)row0 * 128u), b_lo = desc_lo(s_ring + slot * (uint32_t)G::SLOT_BYTES);
+                        if (elected) {
+#pragma unroll 1
+                            for (int j = 0; j < ksteps; ++j) {
+                                const uint32_t kb = (uint32_t)(j >> 2), ks = (uint32_t)(j & 3) * 2u;  // 128-byte block, 32-byte step in it
+                                const uint32_t bj = b_lo + kb * (uint32_t)(G::NMAT * G::WBLK >> 4) + ks;
+                                const uint32_t acc = ((use_s && ph == 0) || t > t_begin || j > 0) ? 1u : 0u;
+#pragma unroll
+                                for (int a = 0; a < NACC; ++a) {
+                                    const uint32_t aj = a_lo + kb * (uint32_t)(R * 8) + (uint32_t)(a * 128 * 8) + ks;
+                                    if (X3) {
+                                        mma_lo<false, true>(dcol, aj, bj, acc, G::IDESC_X3);                 // a1 b1 | a1 b2
+                                        mma_lo<false, true>(dcol + 128u, aj + (A2 >> 4), bj, 1u, G::IDESC);  // a2 b1 -> D2
+                                    } else {
+                                        mma_lo<false, F16>(dcol + a * ACC, aj, bj, acc, G::IDESC);
+                                    }
+                                }
+                            }
+                            umma_commit(bar_empty(slot));
+                        }
+                        __syncwarp();
+                    }
+                    if (elected) umma_commit(bar_acc);
+                } else if (tid == 32) {
+                    // weight producer: the ring runs up to NSLOT taps past this phase (weights do not depend on the data)
+                    const uint32_t target = min(q0 + (uint32_t)(t_end + NSLOT), total_units);
+                    while (q_prod < target) {
+                        const uint32_t slot = q_prod % NSLOT, use = q_prod / NSLOT;
+                        if (use >= 1) mbar_wait(bar_empty(slot), (use - 1u) & 1u);
+                        const uint32_t ul = q_prod % (uint32_t)(9 * L), layer = ul / 9, tap = ul - layer * 9;
+                        const uint8_t* src = net.wconv + (layer == 0 ? (size_t)tap * G::TAP0_BYTES
+                                                                     : (size_t)9 * G::TAP0_BYTES + ((size_t)(layer - 1) * 9 + tap) * G::TAP_BYTES);
+                        const uint32_t bytes = layer == 0 ? (uint32_t)G::TAP0_BYTES : (uint32_t)G::TAP_BYTES;
+                        mbar_expect_tx(bar_full(slot), bytes);
+                        bulk_g2s(s_ring + slot * (uint32_t)G::SLOT_BYTES, src, bytes, bar_full(slot));
+                        ++q_prod;
+                    }
+                }
+                __syncwarp();
+                mbar_wait(bar_acc, acc_par);
+                acc_par ^= 1u;
+                tc_fence_after();
+                if constexpr (X3) {
+                    if (ph + 1 < G::NPH) {  // fold this phase into registers; the next phase restarts the accumulator from zero
+#pragma unroll
+                        for (int h = 0; h < EP_CH / 16; ++h) {
+                            uint32_t v[16], v2[16];  // 16 columns at a time: the phase sums already hold 64 registers
+                            const int ch0 = ep_part * EP_CH + h * 16;
+                            tmem_ld16_nowait(tsrc + ch0, v);
+                            tmem_ld16_nowait(tsrc + 128 + ch0, v2);
+                            tmem_wait_ld();
+#pragma unroll
+                            for (int i = 0; i < 16; ++i) {
+                                const float x = fmaf(__uint_as_float(v2[i]), kX3InvScale, __uint_as_float(v[i]));
+                                part[h * 16 + i] = ph == 0 ? x : part[h * 16 + i] + x;
+                            }
+                        }
+                        tc_fence_before();
+                        __syncthreads();
+                        tc_fence_after();
+                    }
+                }
+            }
+            // ---- epilogue: this thread owns one cell (TMEM lane) and EP_CH of its channels
+            const bool preload = (l & 1) == 0 && !last;
+            const float4* bias_l = reinterpret_cast<const float4*>(net.bias + (size_t)l * kHidW);
+            const float4* bias_n = reinterpret_cast<const float4*>(net.bias + (size_t)(preload ? l + 2 : l) * kHidW);
+            const float4* hw = reinterpret_cast<const float4*>(net.head);
+            const int cell = ep_acc * 128 + (warp & 3) * 32 + lane;
+            const Cell c = decode_cell(cell, CELLS);
+            float hp0 = 0.f, hp1 = 0.f, hv = 0.f;
+#pragma unroll 1
+            for (int h = 0; h < EP_CH / 32; ++h) {
+                const int ch0 = ep_part * EP_CH + h * 32;
+                uint32_t v[32];
+                if constexpr (X3) {  // D1 + 2^-11 D2 of the last phase + the earlier phases
+                    tmem_ld32(tsrc + ch0, v);
+#pragma unroll
+                    for (int q = 0; q < 2; ++q) {
+                        uint32_t v2[16];
+                        tmem_ld16_nowait(tsrc + 128 + ch0 + 16 * q, v2);
+                        tmem_wait_ld();
+#pragma unroll
+                        for (int i = 0; i < 16; ++i) {
+                            const int k = 16 * q + i;
+                            v[k] = __float_as_uint(fmaf(__uint_as_float(v2[i]), kX3InvScale, __uint_as_float(v[k])) + (G::NPH > 1 ? (h == 0 ? part[k] : part[32 + k]) : 0.f));
+                        }
+                    }
+                } else {
+                    tmem_ld32(tsrc + ch0, v);
+                }
+                float o[32];
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                    float4 b = make_float4(0.f, 0.f, 0.f, 0.f);
+                    if (!use_s) b = __ldg(bias_l + ch0 / 4 + i);
+                    o[4 * i + 0] = fmaxf(__uint_as_float(v[4 * i + 0]) + b.x, 0.f);
+                    o[4 * i + 1] = fmaxf(__uint_as_float(v[4 * i + 1]) + b.y, 0.f);
+                    o[4 * i + 2] = fmaxf(__uint_as_float(v[4 * i + 2]) + b.z, 0.f);
+                    o[4 * i + 3] = fmaxf(__uint_as_float(v[4 * i + 3]) + b.w, 0.f);
+                }
+                if (!last && c.real) {
+                    if (X3) store_channels_x3(s_act, A2, R, kLead + cell, ch0, o);
+                    else store_channels<F16>(s_act, R, kLead + cell, ch0, o);
+                }
+                if (preload) {
+#pragma unroll
+                    for (int i = 0; i < 8; ++i) {
+                        const float4 b = __ldg(bias_n + ch0 / 4 + i);
+                        v[4 * i + 0] = __float_as_uint(o[4 * i + 0] + b.x);
+                        v[4 * i + 1] = __float_as_uint(o[4 * i + 1] + b.y);
+                        v[4 * i + 2] = __float_as_uint(o[4 * i + 2] + b.z);
+                        v[4 * i + 3] = __float_as_uint(o[4 * i + 3] + b.w);
+                    }
+                    tmem_st32(tskip + ch0, v);
+                    if (X3) {  // the D2 half of the preloaded accumulator starts from zero
+#pragma unroll
+                        for (int i = 0; i < 32; ++i) v[i] = 0u;
+                        tmem_st32(tskip + 128 + ch0, v);
+                    }
+                }
+                if (last) {  // 1x1 convolutions of both heads (policy_conv 128 -> 2, vh_conv 128 -> 1)
+#pragma unroll
+                    for (int i = 0; i < 8; ++i) {
+                        const float4 w0 = __ldg(hw + (kWP0 + ch0) / 4 + i), w1 = __ldg(hw + (kWP1 + ch0) / 4 + i), w2 = __ldg(hw + (kWV + ch0) / 4 + i);
+                        hp0 = fmaf(o[4 * i + 0], w0.x, fmaf(o[4 * i + 1], w0.y, fmaf(o[4 * i + 2], w0.z, fmaf(o[4 * i + 3], w0.w, hp0))));
+                        hp1 = fmaf(o[4 * i + 0], w1.x, fmaf(o[4 * i + 1], w1.y, fmaf(o[4 * i + 2], w1.z, fmaf(o[4 * i + 3], w1.w, hp1))));
+                        hv = fmaf(o[4 * i + 0], w2.x, fmaf(o[4 * i + 1], w2.y, fmaf(o[4 * i + 2], w2.z, fmaf(o[4 * i + 3], w2.w, hv))));
+                    }
+                }
+            }
+            if (last && c.real) {
+                float* hb = s_head + (ep_part * NB + c.board) * 75;
+                hb[c.pos] = hp0;
+                hb[25 + c.pos] = hp1;
+                hb[50 + c.pos] = hv;
+            }
+            if (preload) tmem_wait_st();
+            fence_proxy_async();
+            q0 += 9u;
+        }
+        // ---- heads: the partial 1x1 sums are added in a fixed order (batch invariant), then one warp per board
+        __syncthreads();
+        for (int i = tid; i < NB * 75; i += 256) {
+            float s = s_head[i];
+#pragma unroll
+            for (int p = 1; p < SPLIT; ++p) s += s_head[p * NB * 75 + i];
+            s_head[i] = fmaxf(s + __ldg(net.head + kWB + (i % 75) / 25), 0.f);
+        }
+        __syncthreads();
+        for (int b = warp; b < NB; b += 8) {
+            const int64_t gb = board0 + b;
+            if (gb >= n) continue;
+            const float* hb = s_head + b * 75;
+            const bool two = lane + 32 < 50;
+            float l0 = __ldg(net.head + kWPhB + lane), l1 = two ? __ldg(net.head + kWPhB + 32 + lane) : 0.f;
+            for (int i = 0; i < 50; ++i) {
+                const float x = hb[i];
+                l0 = fmaf(x, __ldg(net.head + kWPhW + i * 50 + lane), l0);
+                if (two) l1 = fmaf(x, __ldg(net.head + kWPhW + i * 50 + 32 + lane), l1);
+            }
+            const float m = warp_max(two ? fmaxf(l0, l1) : l0);
+            const float e0 = expf(l0 - m), e1 = two ? expf(l1 - m) : 0.f;
+            const float s = warp_sum(e0 + e1);
+            policy[gb * 50 + lane] = e0 / s;
+            if (two) policy[gb * 50 + 32 + lane] = e1 / s;
+            float hj[4];  // value hidden units lane, lane + 32, lane + 64, lane + 96
+#pragma unroll
+            for (int k = 0; k < 4; ++k) hj[k] = __ldg(net.head + kWV1B + 32 * k + lane);
+            for (int i = 0; i < 25; ++i) {
+                const float x = hb[50 + i];
+#pragma unroll
+                for (int k = 0; k < 4; ++k) hj[k] = fmaf(x, __ldg(net.head + kWV1W + i * kHidW + 32 * k + lane), hj[k]);
+            }
+            float acc = 0.f;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) acc = fmaf(fmaxf(hj[k], 0.f), __ldg(net.head + kWV2W + 32 * k + lane), acc);
+            acc = warp_sum(acc);
+            if (lane == 0) value[gb] = tanhf(acc + __ldg(net.head + kWV2B));
+        }
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 0) tmem_dealloc(tmem, G::TMEM_COLS);
+}
+
 // ---- host side: fold BatchNorm, round to tf32, lay the weights out as the tensor core reads them ------------------------------
 struct Named {
     std::string name;
@@ -2702,6 +3020,121 @@ bool fold_bn(const std::vector<Named>& ts, const std::string& conv, const std::s
     return true;
 }
 
+// replaces the current slot's network with the given blobs
+int32_t upload_net(Ctx* c, const std::vector<uint8_t>& wconv, const std::vector<float>& bias, const std::vector<float>& head, int n_blocks, int hid,
+                   bool f16, bool x3, size_t pair_off, std::string& err) {
+    Ctx::NetSlot& ns = c->net[c->net_cur];
+    cudaStreamSynchronize(c->stream);  // a forward pass with the old weights may still be running
+    for (void** p : {(void**)&ns.w, (void**)&ns.bias, (void**)&ns.head})
+        if (*p) {
+            cudaFree(*p);
+            *p = nullptr;
+        }
+    ns.loaded = 0;
+    cudaError_t e = cudaMalloc(&ns.w, wconv.size());
+    if (e == cudaSuccess) e = cudaMalloc(&ns.bias, bias.size() * 4);
+    if (e == cudaSuccess) e = cudaMalloc(&ns.head, head.size() * 4);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(ns.w, wconv.data(), wconv.size(), cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(ns.bias, bias.data(), bias.size() * 4, cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(ns.head, head.data(), head.size() * 4, cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    if (e != cudaSuccess) {
+        err = std::string("CUDA: ") + cudaGetErrorString(e);
+        return e == cudaErrorMemoryAllocation ? ONB_E_NOMEM : ONB_E_CUDA;
+    }
+    ns.blocks = n_blocks;
+    ns.hid = hid;
+    ns.f16 = f16 ? 1 : 0;
+    ns.x3 = x3 ? 1 : 0;
+    ns.pair_off = pair_off;
+    ns.loaded = 1;
+    return ONB_OK;
+}
+
+// The 128-wide network (k_net_wide): BatchNorm folded in f64, taps in the swizzled K-major operand layout of GeoW,
+// [layer][tap][128-byte block kb][copy][co][128 B]; biases [L][128]; the head blob of the kW* offsets.
+int32_t net_load_wide(Ctx* c, const std::vector<Named>& ts, int n_blocks, std::string& err) {
+    constexpr int H = kHidW;
+    const double eps = 1e-5;
+    const int L = 1 + 2 * n_blocks;
+    const int mode = c->net_tf32;
+    const bool f16 = mode != ONB_NET_TF32, x3 = mode == ONB_NET_F32;
+    const int nmat = x3 ? 2 : 1, cpc = f16 ? 8 : 4, kch = H / cpc;
+    const size_t blk = (size_t)H * 128, tap0 = nmat * blk, tap = nmat * (size_t)(kch / 8) * blk;
+    std::vector<uint8_t> wconv(9 * tap0 + (size_t)(L - 1) * 9 * tap, 0);
+    std::vector<float> bias((size_t)(L + 2) * H, 0.f), head(kWHeadFloats, 0.f);
+    double w_absmax = 0.0;
+    for (int l = 0; l < L; ++l) {
+        std::string conv = "conv_init_1", bn = "bn1";
+        if (l > 0) {
+            const std::string blkname = "resnet_" + std::to_string((l - 1) / 2) + ".resnet_small_block" + std::to_string(((l - 1) & 1) + 1);
+            conv = blkname + ".small_block_conv";
+            bn = blkname + ".small_block_bn";
+        }
+        const int c_in = l == 0 ? kInPlanes : H;
+        const Named* w = find(ts, conv + ".weight", (int64_t)H * c_in * 9, err);
+        if (!w) return ONB_E_INVALID;
+        BnFold f;
+        if (!fold_bn(ts, conv, bn, H, eps, f, err)) return ONB_E_INVALID;
+        const int chunks = l == 0 ? 8 : kch;  // the first layer fills one 128-byte block (channels beyond 21 are zero)
+        const size_t tb = l == 0 ? tap0 : tap;
+        uint8_t* dst = wconv.data() + (l == 0 ? 0 : 9 * tap0 + (size_t)(l - 1) * 9 * tap);
+        for (int t = 0; t < 9; ++t)
+            for (int kc = 0; kc < chunks; ++kc)
+                for (int co = 0; co < H; ++co)
+                    for (int e = 0; e < cpc; ++e) {
+                        const int ci = kc * cpc + e;
+                        const double xd = ci < c_in ? (double)w->data[((size_t)co * c_in + ci) * 9 + t] * f.scale[co] : 0.0;
+                        const float x = (float)xd;
+                        if (std::fabs(xd) > w_absmax) w_absmax = std::fabs(xd);
+                        uint8_t* q = dst + (size_t)t * tb + (size_t)(kc >> 3) * nmat * blk + (size_t)co * 128 + (size_t)(((kc & 7) ^ (co & 7)) << 4);
+                        if (f16) {
+                            const __half hv = __float2half_rn(x);
+                            memcpy(q + e * 2, &hv, 2);
+                            if (x3) {  // w = w1 + 2^-11 w2: b2 follows b1 in the same 128-byte block (one N = 256 MMA reads both)
+                                const __half lv = __float2half_rn((float)((xd - (double)__half2float(hv)) * (double)kX3Scale));
+                                memcpy(q + blk + e * 2, &lv, 2);
+                            }
+                        } else {
+                            const float r = tf32_round_host(x);
+                            memcpy(q + e * 4, &r, 4);
+                        }
+                    }
+        for (int co = 0; co < H; ++co) bias[(size_t)l * H + co] = (float)f.shift[co];
+    }
+    const Named *pw = find(ts, "policy_conv.weight", 2 * H, err), *vw = pw ? find(ts, "vh_conv.weight", H, err) : nullptr;
+    if (!vw) return ONB_E_INVALID;
+    BnFold fp, fv;
+    if (!fold_bn(ts, "policy_conv", "policy_bn", 2, eps, fp, err) || !fold_bn(ts, "vh_conv", "vh_bn", 1, eps, fv, err)) return ONB_E_INVALID;
+    for (int ci = 0; ci < H; ++ci) {
+        head[kWP0 + ci] = (float)((double)pw->data[ci] * fp.scale[0]);
+        head[kWP1 + ci] = (float)((double)pw->data[H + ci] * fp.scale[1]);
+        head[kWV + ci] = (float)((double)vw->data[ci] * fv.scale[0]);
+    }
+    head[kWB + 0] = (float)fp.shift[0];
+    head[kWB + 1] = (float)fp.shift[1];
+    head[kWB + 2] = (float)fv.shift[0];
+    const Named *p2w = find(ts, "ph_linear2.weight", 2500, err), *p2b = p2w ? find(ts, "ph_linear2.bias", 50, err) : nullptr,
+                *v1w = p2b ? find(ts, "vh_linear1.weight", (int64_t)H * 25, err) : nullptr, *v1b = v1w ? find(ts, "vh_linear1.bias", H, err) : nullptr,
+                *v2w = v1b ? find(ts, "vh_linear2.weight", H, err) : nullptr, *v2b = v2w ? find(ts, "vh_linear2.bias", 1, err) : nullptr;
+    if (!v2b) return ONB_E_INVALID;
+    for (int j = 0; j < 50; ++j) {
+        for (int i = 0; i < 50; ++i) head[kWPhW + i * 50 + j] = p2w->data[j * 50 + i];
+        head[kWPhB + j] = p2b->data[j];
+    }
+    for (int j = 0; j < H; ++j) {
+        for (int i = 0; i < 25; ++i) head[kWV1W + i * H + j] = v1w->data[j * 25 + i];
+        head[kWV1B + j] = v1b->data[j];
+        head[kWV2W + j] = v2w->data[j];
+    }
+    head[kWV2B] = v2b->data[0];
+    if (f16 && w_absmax > 65504.0) {
+        err = "a BatchNorm-folded convolution weight has magnitude " + std::to_string(w_absmax) + " > 65504 (f16 range): load this network with ONB_NET_TF32";
+        return ONB_E_INVALID;
+    }
+    return upload_net(c, wconv, bias, head, n_blocks, H, f16, x3, 0, err);
+}
+
 }  // namespace
 
 // Parameters by the reference's VarStore names (net.rs:118-213; '|' or '.' as separator), OIHW / [out][in] f32 as libtorch stores them.
@@ -2728,6 +3161,16 @@ int32_t net_load(Ctx* c, int32_t n_tensors, const char* const* names, const floa
         err = "more residual blocks than supported";
         return ONB_E_INVALID;
     }
+    // the width (ConvResNetConfig::hidden_channels) comes from bn1; every other tensor's size is then checked against it
+    int hid = 0;
+    for (const Named& t : ts)
+        if (t.name == "bn1.weight") hid = (int)t.numel;
+    if (hid != 64 && hid != kHidW) {
+        err = hid == 0 ? "tensor bn1.weight is missing"
+                       : "bn1.weight has " + std::to_string(hid) + " channels: this build supports ConvResNetConfig{hidden_channels: 64 or 128, input_channels: 21}";
+        return ONB_E_INVALID;
+    }
+    if (hid == kHidW) return net_load_wide(c, ts, n_blocks, err);
     const double eps = 1e-5;  // nn::BatchNormConfig default of tch 0.10 / torch
     const int L = 1 + 2 * n_blocks;
     const int mode = c->net_tf32;  // ONB_NET_F16 | ONB_NET_TF32 | ONB_NET_F32 (f16 operands split in two, see Geo)
@@ -2842,31 +3285,7 @@ int32_t net_load(Ctx* c, int32_t n_tensors, const char* const* names, const floa
                 memcpy(dst + 8192, b1 + (size_t)r * 32 * 128, 4096);
             }
     }
-    Ctx::NetSlot& ns = c->net[c->net_cur];
-    cudaStreamSynchronize(c->stream);  // a forward pass with the old weights may still be running
-    for (void** p : {(void**)&ns.w, (void**)&ns.bias, (void**)&ns.head})
-        if (*p) {
-            cudaFree(*p);
-            *p = nullptr;
-        }
-    ns.loaded = 0;
-    cudaError_t e = cudaMalloc(&ns.w, wconv.size());
-    if (e == cudaSuccess) e = cudaMalloc(&ns.bias, bias.size() * 4);
-    if (e == cudaSuccess) e = cudaMalloc(&ns.head, head.size() * 4);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(ns.w, wconv.data(), wconv.size(), cudaMemcpyHostToDevice, c->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(ns.bias, bias.data(), bias.size() * 4, cudaMemcpyHostToDevice, c->stream);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(ns.head, head.data(), head.size() * 4, cudaMemcpyHostToDevice, c->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    if (e != cudaSuccess) {
-        err = std::string("CUDA: ") + cudaGetErrorString(e);
-        return e == cudaErrorMemoryAllocation ? ONB_E_NOMEM : ONB_E_CUDA;
-    }
-    ns.blocks = n_blocks;
-    ns.f16 = f16 ? 1 : 0;
-    ns.x3 = x3 ? 1 : 0;
-    ns.pair_off = pair_off;
-    ns.loaded = 1;
-    return ONB_OK;
+    return upload_net(c, wconv, bias, head, n_blocks, 64, f16, x3, pair_off, err);
 }
 
 template <int NACC, bool F16, bool X3 = false>
@@ -3047,6 +3466,23 @@ static cudaError_t launch_net_v3(Ctx* c, const float* planes, float* policy, flo
     return cudaGetLastError();
 }
 
+// the 128-wide network: one CTA per SM, each working through board groups of GeoW::NB
+template <bool F16, bool X3>
+static cudaError_t launch_net_wide(Ctx* c, const float* planes, float* policy, float* value, const NetDev& nd, int sms, int64_t count) {
+    using G = GeoW<F16, X3>;
+    static bool attr[64] = {};  // the opt-in is per device
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (dev < 0 || dev >= 64 || !attr[dev]) {
+        const cudaError_t e = cudaFuncSetAttribute(k_net_wide<F16, X3>, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM);
+        if (e != cudaSuccess) return e;
+        if (dev >= 0 && dev < 64) attr[dev] = true;
+    }
+    const int64_t groups = (count + G::NB - 1) / G::NB;
+    k_net_wide<F16, X3><<<(unsigned)(groups < sms ? groups : sms), 256, G::SMEM, c->stream>>>(planes, policy, value, count, nd);
+    return cudaGetLastError();
+}
+
 cudaError_t launch_net_forward(Ctx* c, const float* planes, float* policy, float* value, int64_t count) {
     if (count <= 0) return cudaSuccess;
     const Ctx::NetSlot& ns = c->net[c->net_cur];
@@ -3054,6 +3490,11 @@ cudaError_t launch_net_forward(Ctx* c, const float* planes, float* policy, float
     int dev = 0, sms = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (ns.hid == kHidW) {  // 128 hidden channels: k_net_wide in all three modes (the 64-wide knobs below do not apply)
+        if (ns.x3) return launch_net_wide<true, true>(c, planes, policy, value, nd, sms, count);
+        return ns.f16 ? launch_net_wide<true, false>(c, planes, policy, value, nd, sms, count)
+                      : launch_net_wide<false, false>(c, planes, policy, value, nd, sms, count);
+    }
     if (ns.x3) {
         // ONB_NET_F32: split operands, f32-faithful, one CTA per SM. Default: the warp-specialised pipeline on CTA pairs
         // (k_net_forward_x3p<true>, 0.600 ms per 16 384 positions); ONB_NET_X3_PAIR=0: the same pipeline on single CTAs (0.646 ms; also
