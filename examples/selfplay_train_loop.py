@@ -32,6 +32,7 @@ def main(argv=None):
     ap.add_argument("--sgd-steps", type=int, default=20)
     ap.add_argument("--eval-games", type=int, default=64)
     ap.add_argument("--mcts-playouts", type=int, default=200, help="playouts of the plain-UCT arena opponent")
+    ap.add_argument("--ab-depth", type=int, default=4, help="search depth in plies (1..8) of the alpha-beta arena opponent")
     ap.add_argument("--torch-net", action="store_true", help="evaluate with the PyTorch module as a black box instead of onb_net_load")
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--out", default=None, help="directory for the reference's on-disk artefacts: loss_stats JSON (stats.rs) and .ot checkpoints (train.rs:414-430)")
@@ -77,7 +78,8 @@ def main(argv=None):
             opt.step()
             losses.append((float(vl.detach()), float(pl.detach())))
         model.eval()
-        # ---- evaluation (evaluator.rs:195-353): the network-guided search against the Random and the Mcts agent, colours alternate
+        # ---- evaluation (evaluator.rs:195-353): the network-guided search against the Random, the Mcts and the AlphaBeta agent,
+        #      colours alternate
         a_is_red = (np.arange(args.eval_games) % 2) == 0
         counter = {"i": 0}
         results = {}
@@ -96,7 +98,11 @@ def main(argv=None):
                 cx.uct_search(2.0 ** 0.5, 5, args.mcts_playouts, to_host=False)
                 cx.tensor(onb.BUF_ACTIONS).copy_(cx.tensor(onb.BUF_BEST))
 
-            for name, opponent, native in (("random", rnd, ctx.agent_random()), ("mcts", plain_mcts, ctx.agent_uct(args.mcts_playouts))):
+            def alphabeta(cx):
+                cx.alphabeta(args.ab_depth, to_host=False)   # leaves the chosen actions in BUF_ACTIONS
+
+            for name, opponent, native in (("random", rnd, ctx.agent_random()), ("mcts", plain_mcts, ctx.agent_uct(args.mcts_playouts)),
+                                           ("alphabeta", alphabeta, ctx.agent_alphabeta(args.ab_depth))):
                 ctx.reset()
                 if net is None:   # the arena loop inside the library (onb_fight)
                     w, l, d, _ = ctx.fight_native(ctx.agent_puct(args.sims, 2.0, ev, 0), native, a_is_red, max_plies=150)
@@ -109,7 +115,8 @@ def main(argv=None):
         if stats_log is not None:   # what train() leaves on disk: the loss / arena log and the checkpoint of the iteration
             stats_log.push(it, losses[-1][0] + losses[-1][1], losses[-1][0], losses[-1][1])
             stats_log.push_games_played(int(data["games"]), int(data["planes"].shape[0]))
-            stats_log.push_fight(False, random_fight=results["random"]["stats"], mcts_fight=results["mcts"]["stats"])
+            stats_log.push_fight(False, random_fight=results["random"]["stats"], mcts_fight=results["mcts"]["stats"],
+                                 alphabeta_fight=results["alphabeta"]["stats"])
             stats_log.save()
             model.save_ot(os.path.join(args.out, "model_%d.ot" % it))
         for r in results.values():
@@ -117,7 +124,7 @@ def main(argv=None):
         log.append(dict(iteration=it, games=int(data["games"]), samples=int(data["planes"].shape[0]), replay=replay.size,
                         value_loss=losses[-1][0], policy_loss=losses[-1][1], wins=results["random"]["wins"],
                         losses=results["random"]["losses"], draws=results["random"]["draws"], elo=results["random"]["elo"],
-                        vs_mcts=results["mcts"]))
+                        vs_mcts=results["mcts"], vs_alphabeta=results["alphabeta"]))
         print(log[-1], flush=True)
     return log
 

@@ -330,12 +330,14 @@ ONB_API int32_t onb_copy_to_host(onb_ctx* ctx, void* host, const void* device, i
  * were played (the ply cap of evaluator.rs:386-392; such games count as draws). a_is_red_host[i] != 0: agent A plays Red in game
  * i (the reference swaps colours every game). Agents: ONB_AGENT_RANDOM = the `Random` agent (ai/random.rs, draws keyed by the
  * ply); ONB_AGENT_PUCT = AlphaZeroMcts (evaluator = ONB_EVAL_*, for ONB_EVAL_NET the resident network net_slot, sims, c);
- * ONB_AGENT_UCT = `Mcts` (sims playouts, c, min_node_visits). results (device, [n]: 0 undecided, 1 Red won, 2 Blue won) stays
+ * ONB_AGENT_UCT = `Mcts` (sims playouts, c, min_node_visits); ONB_AGENT_ALPHABETA = `AlphaBeta` (onb_alphabeta_run below, depth in
+ * plies = sims, 1 <= sims <= ONB_ALPHABETA_MAX_DEPTH; needs no search-tree pools). results (device, [n]: 0 undecided, 1 Red won, 2 Blue won) stays
  * valid until the next onb_fight; results_host (optional) receives a copy. The Elo update of evaluator.rs:58-110 is a fold over
  * these per-game results in game order: onb_fight_stats below. */
 #define ONB_AGENT_RANDOM 0
 #define ONB_AGENT_PUCT 1
 #define ONB_AGENT_UCT 2
+#define ONB_AGENT_ALPHABETA 3
 typedef struct onb_agent {
     int32_t kind;
     int32_t evaluator;
@@ -422,6 +424,25 @@ ONB_API int32_t onb_replay_indices(int64_t size, int64_t batch, uint64_t seed, i
  * reference: exploration_c = sqrt(2), min_node_visits = 5, 5000 playouts (mod.rs:21-30; its 1 s wall-clock limit is
  * not reproduced). The rollouts draw from the counter RNG keyed by (seed, global game id, playout, ply). */
 ONB_API int32_t onb_uct_run(onb_ctx* ctx, float exploration_c, uint32_t min_node_visits, uint32_t playouts);
+
+/* ---- fixed-depth alpha-beta: the `AlphaBeta` agent (onitama-game/src/ai/alpha_beta/{mod.rs,evaluation.rs}) ----------------
+ * One search per game of the context, rooted at its current state, one game per GPU thread. The search is this project's own
+ * definition (DESIGN.md §5d); its play is NOT pinned to the reference, whose evaluation tables and wall-clock limit are not
+ * reproduced: the reference deepens iteratively until a time limit, this search runs to a fixed depth in plies.
+ *   negamax with alpha-beta, fail-hard, int32 scores from the side to move's view, root window (-WIN - 1, WIN + 1), WIN = 1 000 000;
+ *   a node at ply p below the root with depth left >= 1 whose side to move has a move that wins at once (captures the enemy king or
+ *     puts the own king on the enemy temple) scores WIN - (p + 1), its best move is the first such move, no child is entered;
+ *   otherwise children in generation order (hand slot, from, to ascending), score = -search(child, -beta, -alpha, depth - 1, p + 1),
+ *     a child replaces the best move only with a strictly greater score, cut-off at alpha >= beta; a node without a legal move has
+ *     the two pass children ONB_ACTION_PASS(slot 0), then slot 1 (the reference panics there);
+ *   a leaf (depth left 0) scores eval = V(mover) - V(opponent), V = sum over pawns (100 + 4 adv + 2 ctr) + 6 (6 - manhattan(king,
+ *     enemy temple)), adv = rows advanced from the own home row, ctr = 2 - |col - 2|.
+ * best_host [n] (first maximal move in generation order), score_host [n] (exact root score), nodes_host [n] (positions entered,
+ * root and leaves included) may each be NULL; the chosen actions also stay in ONB_BUF_ACTIONS, where onb_env_step takes them.
+ * A decided game (result != 0 or State::current_state is a win) gets ONB_ACTION_NONE, score 0, 0 nodes.
+ * depth outside 1 .. ONB_ALPHABETA_MAX_DEPTH: ONB_E_INVALID. Works on a context created with mcts_max_sims = 0. */
+#define ONB_ALPHABETA_MAX_DEPTH 8
+ONB_API int32_t onb_alphabeta_run(onb_ctx* ctx, int32_t depth, onb_action* best_host, int32_t* score_host, uint64_t* nodes_host);
 
 /* ---- policy/value network on the device ---------------------------------------------------------------------
  * ConvResNet::forward (alphazero-training/src/net.rs:215-232) for every position of a plane buffer, as one fused

@@ -353,6 +353,30 @@ struct Mcts : Agent {
     uint64_t id() const override { return (uint64_t)search_time_ms * 1000000ull + (uint64_t)exploration_c + max_playouts + min_node_visits; }
 };
 
+/// ai/alpha_beta/mod.rs: the `AlphaBeta` agent as this project defines it (onb_alphabeta_run, DESIGN.md §5d): a negamax with
+/// alpha-beta pruning to a fixed depth in plies, on the GPU. The reference deepens iteratively until a wall-clock limit and scores
+/// leaves with its own tables; neither is reproduced, so this agent's play is not pinned to the reference. generate_move returns
+/// the chosen move and the root's score (side to move's view; a win in k own moves scores 1 000 000 - (2k - 1)). Like the
+/// reference (alpha_beta/mod.rs:165-167) it refuses a position without a legal move, where the search's answer is a pass.
+struct AlphaBeta : Agent {
+    int32_t depth = 4;
+    explicit AlphaBeta(int32_t depth_ = 4) : depth(depth_) {}
+    std::pair<DoneMove, double> generate_move(const GameState& gs) override {
+        Engine& e = Engine::single();
+        onb_state o = gs.state.to_onb(gs.curr_player_color);
+        e.check(onb_env_set_states(e.ctx(), &o, 0, 1));
+        onb_action best = 0;
+        int32_t score = 0;
+        e.check(onb_alphabeta_run(e.ctx(), depth, &best, &score, nullptr));
+        if (best == ONB_ACTION_NONE) throw Error(ONB_E_STATE, "AlphaBeta: the game is already decided");
+        if (best & (1u << 13)) throw Error(ONB_E_STATE, "AlphaBeta: no legal move (the search would pass)");
+        return {from_action(best), (double)score};
+    }
+    const char* name() const override { return "AlphaBeta AI"; }
+    std::unique_ptr<Agent> clone_dyn() const override { return std::make_unique<AlphaBeta>(*this); }
+    uint64_t id() const override { return (uint64_t)depth; }
+};
+
 struct AlphaZeroMctsConfig {  // alphazero_mcts/mod.rs:26-43
     double search_time_ms = 400.;  // ignored: the search always runs max_playouts simulations
     double exploration_c = 1.4142135623730951;
@@ -604,8 +628,8 @@ inline FightStatistics fight(const EvaluatorConfig& config, std::unique_ptr<Agen
 /// fight() for config.game_amnt games at once on one engine (onb_fight: the arena loop runs inside the library; each ply an agent
 /// searches only the games in which it is to move). Agent A plays Red in games 0, 2, 4, ... like the colour swap of
 /// evaluator.rs:393-397; the statistics incl. the Elo updates are folded in game order ON THE DEVICE (onb_fight_stats).
-/// Agents are described by onb_agent (ONB_AGENT_RANDOM / ONB_AGENT_PUCT / ONB_AGENT_UCT); the engine must have been created
-/// with n_games == config.game_amnt and enough mcts_max_sims.
+/// Agents are described by onb_agent (ONB_AGENT_RANDOM / ONB_AGENT_PUCT / ONB_AGENT_UCT / ONB_AGENT_ALPHABETA with the depth in
+/// sims); the engine must have been created with n_games == config.game_amnt and enough mcts_max_sims for the searching agents.
 inline FightStatistics fight_device(Engine& e, const EvaluatorConfig& config, const onb_agent& agent, const onb_agent& opponent, double rating_a = 800.,
                                     double rating_b = 800.) {
     if ((size_t)e.n() != config.game_amnt) throw Error(ONB_E_INVALID, "fight_device: the engine must hold game_amnt games");

@@ -107,6 +107,7 @@ SYMBOLS = {
     "onb_replay_sample": (C.c_int32, [_P, C.c_int64, C.c_uint64, C.POINTER(_P), C.POINTER(_P), C.POINTER(_P), C.POINTER(C.c_int64)]),
     "onb_replay_indices": (C.c_int32, [C.c_int64, C.c_int64, C.c_uint64, _P]),
     "onb_uct_run": (C.c_int32, [_P, C.c_float, C.c_uint32, C.c_uint32]),
+    "onb_alphabeta_run": (C.c_int32, [_P, C.c_int32, _P, _P, _P]),
     "onb_net_precision": (C.c_int32, [_P, C.c_int32]),
     "onb_net_select": (C.c_int32, [_P, C.c_int32]),
     "onb_net_load": (C.c_int32, [_P, C.c_int32, _P, _P, _P]),
@@ -118,11 +119,14 @@ class SelfPlayConfig(C.Structure):
                 ("train", C.c_int32), ("noise_seed", C.c_uint64), ("sample_cap", C.c_int64)]
 
 
-AGENT_RANDOM, AGENT_PUCT, AGENT_UCT = 0, 1, 2
+AGENT_RANDOM, AGENT_PUCT, AGENT_UCT, AGENT_ALPHABETA = 0, 1, 2, 3
+ALPHABETA_MAX_DEPTH = 8
+ALPHABETA_WIN = 1000000
 
 
 class Agent(C.Structure):
-    """onb_agent: kind, evaluator (PUCT), net_slot (ONB_EVAL_NET), sims / playouts, exploration constant, min_node_visits (UCT)"""
+    """onb_agent: kind, evaluator (PUCT), net_slot (ONB_EVAL_NET), sims / playouts / alpha-beta depth, exploration constant,
+    min_node_visits (UCT)"""
     _fields_ = [("kind", C.c_int32), ("evaluator", C.c_int32), ("net_slot", C.c_int32), ("sims", C.c_uint32), ("c", C.c_double),
                 ("min_node_visits", C.c_uint32), ("reserved", C.c_uint32)]
 

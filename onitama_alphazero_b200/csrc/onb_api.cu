@@ -145,7 +145,7 @@ int32_t onb_destroy(onb_ctx* ctx) {
     void* ptrs[] = {c->d_states, c->d_masks, c->d_planes, c->d_actions, c->d_stats, c->d_io_states, c->d_moves, c->d_counts, c->d_nodes,
                     c->d_tree_size, c->d_tree_flags, c->d_roots, c->d_leaf_node, c->d_leaf_state, c->d_leaf_planes, c->d_policy, c->d_value,
                     c->d_pi, c->d_best, c->d_root_visits, c->d_root_q, c->d_child_visits, c->net[0].w, c->net[0].bias, c->net[0].head, c->net[1].w,
-                    c->net[1].bias, c->net[1].head, c->d_ln_table, c->d_net_scratch};
+                    c->net[1].bias, c->net[1].head, c->d_ln_table, c->d_net_scratch, c->d_ab_score, c->d_ab_nodes};
     for (void* p : c->sp_buf)
         if (p) cudaFree(p);
     for (void* p : ptrs)
@@ -585,6 +585,10 @@ static int32_t fight_move(Ctx* c, const onb_agent* ag, uint32_t ply, const int32
         ONB_CUDA(c, cudaMemcpyAsync(d_out, c->d_actions, (size_t)c->n * 2, cudaMemcpyDeviceToDevice, c->stream));
         return ONB_OK;
     }
+    if (ag->kind == ONB_AGENT_ALPHABETA) {  // no tree: the kernel writes the actions of the listed games straight into d_out
+        ONB_CUDA(c, launch_alphabeta(c, (int)ag->sims, d_games, m, d_out, nullptr, nullptr));
+        return ONB_OK;
+    }
     int32_t rc = mcts_begin_subset(c, ag->c, ag->sims, d_games, m);
     if (rc != ONB_OK) return rc;
     if (ag->kind == ONB_AGENT_PUCT) {
@@ -605,8 +609,13 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
     if (!a || !b || !a_is_red_host || !out) return fail(c, ONB_E_INVALID, "onb_fight: null argument");
     for (const onb_agent* ag : {a, b}) {
-        if (ag->kind != ONB_AGENT_RANDOM && ag->kind != ONB_AGENT_PUCT && ag->kind != ONB_AGENT_UCT)
+        if (ag->kind != ONB_AGENT_RANDOM && ag->kind != ONB_AGENT_PUCT && ag->kind != ONB_AGENT_UCT && ag->kind != ONB_AGENT_ALPHABETA)
             return fail(c, ONB_E_INVALID, "onb_fight: unknown agent kind %d", ag->kind);
+        if (ag->kind == ONB_AGENT_ALPHABETA) {
+            if (ag->sims < 1 || ag->sims > ONB_ALPHABETA_MAX_DEPTH)
+                return fail(c, ONB_E_INVALID, "onb_fight: an alpha-beta agent needs 1 <= depth (sims) <= %d", ONB_ALPHABETA_MAX_DEPTH);
+            continue;
+        }
         if (ag->kind != ONB_AGENT_RANDOM && (!c->d_nodes || ag->sims == 0 || ag->sims > c->cfg.mcts_max_sims))
             return fail(c, ONB_E_INVALID, "onb_fight: a searching agent needs 1 <= sims <= mcts_max_sims");
     }
@@ -666,6 +675,20 @@ int32_t onb_uct_run(onb_ctx* ctx, float exploration_c, uint32_t min_node_visits,
     }
     ONB_CUDA(c, launch_uct_run(c, exploration_c, min_node_visits, playouts));
     c->sims_done += playouts;
+    return ONB_OK;
+}
+int32_t onb_alphabeta_run(onb_ctx* ctx, int32_t depth, onb_action* best_host, int32_t* score_host, uint64_t* nodes_host) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (depth < 1 || depth > ONB_ALPHABETA_MAX_DEPTH) return fail(c, ONB_E_INVALID, "onb_alphabeta_run: depth %d not in 1..%d", depth, ONB_ALPHABETA_MAX_DEPTH);
+    const size_t n = (size_t)c->n;
+    if (score_host && !c->d_ab_score) ONB_CUDA(c, dalloc(&c->d_ab_score, n));
+    if (nodes_host && !c->d_ab_nodes) ONB_CUDA(c, dalloc(&c->d_ab_nodes, n));
+    ONB_CUDA(c, launch_alphabeta(c, depth, nullptr, c->n, c->d_actions, score_host ? c->d_ab_score : nullptr, nodes_host ? c->d_ab_nodes : nullptr));
+    if (best_host) ONB_CUDA(c, cudaMemcpyAsync(best_host, c->d_actions, n * 2, cudaMemcpyDeviceToHost, c->stream));
+    if (score_host) ONB_CUDA(c, cudaMemcpyAsync(score_host, c->d_ab_score, n * 4, cudaMemcpyDeviceToHost, c->stream));
+    if (nodes_host) ONB_CUDA(c, cudaMemcpyAsync(nodes_host, c->d_ab_nodes, n * 8, cudaMemcpyDeviceToHost, c->stream));
+    if (best_host || score_host || nodes_host) ONB_CUDA(c, cudaStreamSynchronize(c->stream));
     return ONB_OK;
 }
 int32_t onb_mcts_finish(onb_ctx* ctx, onb_action* best_host, float* pi_host, uint32_t* root_visits_host, double* root_q_host, uint32_t* child_visits_host) {

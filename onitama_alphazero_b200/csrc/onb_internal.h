@@ -91,6 +91,9 @@ struct Ctx {
     // cudaMalloc/cudaFree of several hundred MB made the call time vary by +-50 %
     void* scratch[16];
     size_t scratch_cap[16];
+    // onb_alphabeta_run: per-game root score and node count (allocated on first use)
+    int32_t* d_ab_score;
+    unsigned long long* d_ab_nodes;
     char err[512];
 };
 
@@ -125,6 +128,10 @@ cudaError_t launch_mcts_scatter_best(Ctx* c, uint16_t* dst_actions);  // dst[gam
 // network (onb_net.cu)
 int32_t net_load(Ctx* c, int32_t n_tensors, const char* const* names, const float* const* data, const int64_t* numel, std::string& err);
 cudaError_t launch_net_forward(Ctx* c, const float* planes, float* policy, float* value, int64_t count);  // count positions
+
+// alpha-beta agent (onb_alphabeta.cu): searches games d_games[0 .. m) (nullptr: games 0 .. m) to `depth` plies; d_out[game] = the best
+// action (ONB_ACTION_NONE for a decided game), d_score / d_nodes [game] (optional) = root score and positions entered
+cudaError_t launch_alphabeta(Ctx* c, int depth, const int32_t* d_games, int64_t m, uint16_t* d_out, int32_t* d_score, unsigned long long* d_nodes);
 
 // native self-play driver (onb_selfplay.cu)
 int32_t run_self_play(Ctx* c, const onb_selfplay_config* cfg, onb_selfplay_result* out,

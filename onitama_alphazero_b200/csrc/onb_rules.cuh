@@ -261,6 +261,38 @@ __host__ __device__ __forceinline__ uint32_t current_state(const Game& g) {
 }
 
 // ---------------------------------------------------------------------------------------------
+// Leaf evaluation of the alpha-beta agent (project-defined, DESIGN.md §5d; restated square by square in
+// tests/alphabeta_oracle.cpp). E = V(mover) - V(opponent), for one side
+//   V = sum over pawns (100 + 4 adv(q) + 2 ctr(q)) + sum over kings 6 (6 - manhattan(king, enemy temple)),
+// q = 5 row + col, adv = 4 - row for Red and row for Blue, ctr = 2 - |col - 2|, enemy temple = 2 for Red, 22 for Blue.
+// The per-square sums are taken with popcounts over row / column masks: sum(row) = #(row >= 1) + ... + #(row >= 4),
+// sum(ctr) = #(col in 1..3) + #(col == 2); the king term is 6 (4 - row + ctr) for Red and 6 (row + ctr) for Blue.
+// ---------------------------------------------------------------------------------------------
+__host__ __device__ __forceinline__ uint32_t popc32(uint32_t x) {
+#ifdef __CUDA_ARCH__
+    return __popc(x);
+#else
+    return (uint32_t)__builtin_popcount(x);
+#endif
+}
+constexpr uint32_t each_row(uint32_t pattern5) { return pattern5 * 0x108421u; }  // the 5-bit row pattern repeated on all five rows
+constexpr uint32_t kRowGe1 = kAll25 & ~0x1Fu, kRowGe2 = kAll25 & ~0x3FFu, kRowGe3 = kAll25 & ~0x7FFFu, kRowGe4 = kAll25 & ~0xFFFFFu;
+constexpr uint32_t kColMid3 = each_row(0x0Eu), kCol2 = each_row(0x04u);
+constexpr int32_t kAlphaBetaWin = 1000000;
+__host__ __device__ __forceinline__ int32_t sum_rows(uint32_t b) {
+    return (int32_t)(popc32(b & kRowGe1) + popc32(b & kRowGe2) + popc32(b & kRowGe3) + popc32(b & kRowGe4));
+}
+__host__ __device__ __forceinline__ int32_t sum_ctr(uint32_t b) { return (int32_t)(popc32(b & kColMid3) + popc32(b & kCol2)); }
+__host__ __device__ __forceinline__ int32_t side_value(uint32_t pawns, uint32_t kings, uint32_t color) {
+    const int32_t np = (int32_t)popc32(pawns), nk = (int32_t)popc32(kings);
+    if (color == kRed) return 116 * np - 4 * sum_rows(pawns) + 2 * sum_ctr(pawns) + 24 * nk - 6 * sum_rows(kings) + 6 * sum_ctr(kings);
+    return 100 * np + 4 * sum_rows(pawns) + 2 * sum_ctr(pawns) + 6 * sum_rows(kings) + 6 * sum_ctr(kings);
+}
+__host__ __device__ __forceinline__ int32_t eval_position(const RelGame& g) {
+    return side_value(g.op, g.ok, g.side) - side_value(g.ep, g.ek, g.side ^ 1u);
+}
+
+// ---------------------------------------------------------------------------------------------
 // Move generation for one thread (State::generate_all_legal_moves, state.rs:301-378).
 // Enumeration order: hand slot ascending, from ascending, to ascending. A piece is a Pawn if the pawn
 // bit is set, else a King (state.rs:345-358). T points at the 800-word attack table (shared memory).

@@ -242,6 +242,11 @@ class Context:
     def agent_uct(playouts, exploration_c=2.0 ** 0.5, min_node_visits=5):
         return L.Agent(L.AGENT_UCT, 0, 0, playouts, exploration_c, min_node_visits, 0)
 
+    @staticmethod
+    def agent_alphabeta(depth):
+        """the `AlphaBeta` agent: fixed-depth alpha-beta search to `depth` plies (1 .. 8), see Context.alphabeta"""
+        return L.Agent(L.AGENT_ALPHABETA, 0, 0, depth, 0.0, 0, 0)
+
     def fight_native(self, agent_a, agent_b, a_is_red, max_plies=150):
         """onb_fight: the arena loop inside the library. Returns (a_wins, b_wins, draws, per-game results [n] uint8)."""
         mask = np.ascontiguousarray(np.asarray(a_is_red), dtype=np.uint8)
@@ -273,6 +278,18 @@ class Context:
         self.mcts_begin(0.0, playouts)
         self._ck(self._lib.onb_uct_run(self._h, exploration_c, min_node_visits, playouts))
         return self.mcts_finish(to_host=to_host)
+
+    def alphabeta(self, depth, to_host=True):
+        """onb_alphabeta_run: a fixed-depth alpha-beta search (negamax, fail-hard; DESIGN.md §5d) from every game's current position,
+        one game per GPU thread. The chosen actions stay in BUF_ACTIONS (ACTION_NONE for decided games), so step(None) plays them.
+        Returns dict(best [n] uint16, score [n] int32 from the side to move's view, nodes [n] uint64 positions entered), or None
+        with to_host=False."""
+        if not to_host:
+            self._ck(self._lib.onb_alphabeta_run(self._h, depth, None, None, None))
+            return None
+        out = dict(best=np.zeros(self.n, np.uint16), score=np.zeros(self.n, np.int32), nodes=np.zeros(self.n, np.uint64))
+        self._ck(self._lib.onb_alphabeta_run(self._h, depth, L.ptr(out["best"]), L.ptr(out["score"]), L.ptr(out["nodes"])))
+        return out
 
     def mcts_finish(self, to_host=True, out=None):
         """out: optional dict of preallocated arrays (e.g. views of pinned memory) with the keys below; reused across calls."""
