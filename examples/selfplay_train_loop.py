@@ -34,6 +34,8 @@ def main(argv=None):
     ap.add_argument("--mcts-playouts", type=int, default=200, help="playouts of the plain-UCT arena opponent")
     ap.add_argument("--ab-depth", type=int, default=4, help="search depth in plies (1..8) of the alpha-beta arena opponent")
     ap.add_argument("--torch-net", action="store_true", help="evaluate with the PyTorch module as a black box instead of onb_net_load")
+    ap.add_argument("--reuse", action="store_true", help="keep the played child's subtree between moves in self-play (onb_mcts_set_reuse; "
+                                                         "--sims then counts root visits, kept ones included; not with --torch-net)")
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--out", default=None, help="directory for the reference's on-disk artefacts: loss_stats JSON (stats.rs) and .ot checkpoints (train.rs:414-430)")
     ap.add_argument("--hidden", type=int, default=64, choices=[64, 128], help="hidden channels of the ConvResNet (both run on the tensor cores)")
@@ -55,13 +57,15 @@ def main(argv=None):
         ctx.net_load(model, precision=args.net_precision)   # BatchNorm folded, weights laid out for the tensor cores
         return onb.EVAL_NET, None
 
+    if args.reuse and args.torch_net:
+        ap.error("--reuse needs the on-device network (a PyTorch module drives the split phase, which tree reuse does not support)")
     for it in range(args.iters):
         # ---- self-play (train.rs:218-245): train-mode root noise, the current network as evaluator, finished slots restart at once
         with onb.Context(args.slots, seed=args.seed + it, mcts_max_sims=args.sims) as ctx:
             ev, net = evaluator_for(ctx)
             if net is None:   # the whole loop inside the library (onb_self_play)
                 data = ctx.self_play_native(2.0, args.sims, args.games, max_plies=args.max_plies, evaluator=ev, train=True,
-                                            noise_seed=args.seed + 1000 * it)
+                                            noise_seed=args.seed + 1000 * it, reuse=args.reuse)
             else:             # the same loop driven from Python, the PyTorch module between select and expand
                 data = onb.self_play_continuous(ctx, 2.0, args.sims, n_games=args.games, max_plies=args.max_plies, evaluator=ev, net=net,
                                                 train=True, noise_seed=args.seed + 1000 * it)

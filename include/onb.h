@@ -261,6 +261,32 @@ ONB_API int32_t onb_mcts_begin(onb_ctx* ctx, double c_puct, uint32_t sims);
  * keyed by (seed, global tree id, root visit count), so a run is repeatable. Reference values: epsilon 0.25, alpha 0.03.
  * Applies to the searches started after the call; enabled = 0 restores eval mode. Statistical parity only (DESIGN.md). */
 ONB_API int32_t onb_mcts_set_noise(onb_ctx* ctx, int32_t enabled, double epsilon, double alpha, uint64_t seed);
+/* Tree reuse between moves (off by default; with it off every entry point behaves exactly as without this call).
+ * On: onb_mcts_begin and every ply of onb_self_play keep, per game, the subtree of the last reuse-enabled search whose root
+ * position equals the game's current state: a child of that search's root is kept when the game is undecided and its boards,
+ * five card slots and side to move equal the position the child's action leads to (siblings always lead to different positions,
+ * so no action of the caller is needed, and onb_env_reset / onb_env_set_states / any move stay sound). No match: a fresh root.
+ * The kept subtree is the played child and all its descendants in arena order (a stable filter of the old pool; parent and
+ * first_child renumbered, the new root has no parent, every other field -- N, W, P, action, n_child, flags -- unchanged). Root W
+ * is carried over as it is: later backups keep the same alternating sign, so root Q stays consistent.
+ * `sims` becomes a visit TARGET: a tree runs max(0, sims - N_root) simulations, so a root never exceeds sims visits and the node
+ * bound 1 + 40 * mcts_max_sims still holds. onb_mcts_run after a reuse begin must be given the begin's sims. onb_mcts_finish reports
+ * over all of the root's visits, kept ones included. Outputs (finish, play_best, dump_tree, tree_info) stay in game order; the
+ * pools are laid out internally by remaining budget. Train-mode noise is keyed by (seed, game, root visit count) as before.
+ * Refused after a reuse begin (ONB_E_STATE): the caller-driven split phase (onb_mcts_select / _eval / _expand_backup) and
+ * onb_uct_run. onb_fight ignores the switch (its two agents share the pools). Remembered trees are forgotten by any search without
+ * reuse (onb_mcts_begin with reuse off, onb_fight), by onb_self_play's start and by switching reuse off.
+ * Memory: the first enabling call allocates a second node pool of n_games * node_cap * 32 bytes (the kept subtrees are compacted
+ * into it, then the pools swap), doubling node memory: 2 x 16.8 GB for 16 384 games x 800 simulations. */
+ONB_API int32_t onb_mcts_set_reuse(onb_ctx* ctx, int32_t enabled);
+/* counters of the reuse-enabled searches since the last clear: out[ONB_REUSE_TREES] trees searched, [ONB_REUSE_KEPT] trees that
+ * started with kept visits, [ONB_REUSE_KEPT_VISITS] root visits carried over (counted up to the target), [ONB_REUSE_SIMS]
+ * simulations run (= leaf evaluations). clear != 0 zeroes them after the read; out may be NULL. */
+#define ONB_REUSE_TREES 0
+#define ONB_REUSE_KEPT 1
+#define ONB_REUSE_KEPT_VISITS 2
+#define ONB_REUSE_SIMS 3
+ONB_API int32_t onb_mcts_reuse_stats(onb_ctx* ctx, uint64_t out[4], int32_t clear);
 ONB_API int32_t onb_mcts_select(onb_ctx* ctx);
 ONB_API int32_t onb_mcts_expand_backup(onb_ctx* ctx);
 ONB_API int32_t onb_mcts_eval(onb_ctx* ctx, int32_t evaluator); /* fills POLICY/VALUE from LEAF_PLANES on the device */

@@ -383,6 +383,9 @@ struct AlphaZeroMctsConfig {  // alphazero_mcts/mod.rs:26-43
     uint32_t max_playouts = 5000;
     bool train = false;  // root exploration noise, epsilon 0.25 / Dirichlet alpha 0.03 (mcts_arena.rs:186-202)
     uint64_t noise_seed = 0;
+    // keep the played child's subtree between moves (onb_mcts_set_reuse): max_playouts then counts root visits, kept ones
+    // included. Device evaluators only; false forgets the remembered trees.
+    bool reuse = false;
 };
 inline double reward(MoveResult r, PlayerColor c) {  // alphazero_mcts/mod.rs:45-53
     if (c == PlayerColor::Red) return r == MoveResult::RedWin ? 1. : r == MoveResult::BlueWin ? -1. : 0.;
@@ -396,6 +399,8 @@ using HostEvaluator = std::function<void(const float* planes, int64_t n, float* 
 namespace detail {
 inline void run_search(Engine& e, const AlphaZeroMctsConfig& cfg, int32_t device_eval, const HostEvaluator& net) {
     e.check(onb_mcts_set_noise(e.ctx(), cfg.train ? 1 : 0, 0.25, 0.03, cfg.noise_seed));
+    if (cfg.reuse && net) throw Error(ONB_E_INVALID, "AlphaZeroMctsConfig::reuse needs a device evaluator");
+    e.check(onb_mcts_set_reuse(e.ctx(), cfg.reuse ? 1 : 0));
     e.check(onb_mcts_begin(e.ctx(), cfg.exploration_c, cfg.max_playouts));
     if (!net) {
         e.check(onb_mcts_run(e.ctx(), device_eval, cfg.max_playouts));

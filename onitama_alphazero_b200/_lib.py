@@ -81,6 +81,8 @@ SYMBOLS = {
     "onb_perft": (C.c_int32, [_P, _P, C.c_int64, C.c_int32, _P, _P, _P]),
     "onb_mcts_begin": (C.c_int32, [_P, C.c_double, C.c_uint32]),
     "onb_mcts_set_noise": (C.c_int32, [_P, C.c_int32, C.c_double, C.c_double, C.c_uint64]),
+    "onb_mcts_set_reuse": (C.c_int32, [_P, C.c_int32]),
+    "onb_mcts_reuse_stats": (C.c_int32, [_P, _P, C.c_int32]),
     "onb_mcts_select": (C.c_int32, [_P]),
     "onb_mcts_expand_backup": (C.c_int32, [_P]),
     "onb_mcts_eval": (C.c_int32, [_P, C.c_int32]),

@@ -146,6 +146,7 @@ int32_t onb_destroy(onb_ctx* ctx) {
                     c->d_tree_size, c->d_tree_flags, c->d_roots, c->d_leaf_node, c->d_leaf_state, c->d_leaf_planes, c->d_policy, c->d_value,
                     c->d_pi, c->d_best, c->d_root_visits, c->d_root_q, c->d_child_visits, c->net[0].w, c->net[0].bias, c->net[0].head, c->net[1].w,
                     c->net[1].bias, c->net[1].head, c->d_ln_table, c->d_net_scratch, c->d_ab_score, c->d_ab_nodes};
+    reuse_free(c);
     for (void* p : c->sp_buf)
         if (p) cudaFree(p);
     for (void* p : ptrs)
@@ -453,9 +454,44 @@ int32_t onb_mcts_begin(onb_ctx* ctx, double c_puct, uint32_t sims) {
     c->sims_done = 0;
     c->n_act = 0;  // the public search covers every game of the context
     c->d_tree_game = nullptr;
-    ONB_CUDA(c, launch_mcts_begin(c));
+    c->mcts_phase = 0;
+    if (c->reuse_on) {  // every game, trees laid out by remaining budget; finish puts the outputs back into game order
+        ONB_CUDA(c, launch_reuse_begin(c, nullptr, c->n, sims));
+        c->ru_search = 1;
+        c->ru_public = 1;
+    } else {
+        c->ru_live = c->ru_search = c->ru_public = 0;  // a search without reuse forgets the remembered trees
+        ONB_CUDA(c, launch_mcts_begin(c));
+    }
     c->mcts_phase = 1;
     return ONB_OK;
+}
+int32_t onb_mcts_set_reuse(onb_ctx* ctx, int32_t enabled) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (enabled) {
+        if (!c->d_nodes) return fail(c, ONB_E_STATE, "onb_mcts_set_reuse: context created with mcts_max_sims = 0");
+        const cudaError_t e = reuse_alloc(c);
+        if (e == cudaErrorInvalidValue) return fail(c, ONB_E_INVALID, "onb_mcts_set_reuse: mcts_node_cap %u is too large for tree reuse", c->node_cap);
+        if (e != cudaSuccess) return e == cudaErrorMemoryAllocation ? fail(c, ONB_E_NOMEM, "onb_mcts_set_reuse: out of device memory for the second node pool")
+                                                                    : cuda_fail(c, e, "onb_mcts_set_reuse");
+        c->reuse_on = 1;
+    } else {
+        c->reuse_on = 0;
+        c->ru_live = 0;  // switching off forgets the remembered trees
+    }
+    return ONB_OK;
+}
+int32_t onb_mcts_reuse_stats(onb_ctx* ctx, uint64_t out[4], int32_t clear) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (out) memcpy(out, c->ru_stats, sizeof(c->ru_stats));
+    if (clear) memset(c->ru_stats, 0, sizeof(c->ru_stats));
+    return ONB_OK;
+}
+static int32_t refuse_after_reuse(Ctx* c, const char* what) {
+    return fail(c, ONB_E_STATE, "%s: the search was begun with tree reuse on (onb_mcts_set_reuse), which only onb_mcts_run can continue; "
+                                "switch reuse off before onb_mcts_begin for a caller-driven search", what);
 }
 int32_t onb_mcts_set_noise(onb_ctx* ctx, int32_t enabled, double epsilon, double alpha, uint64_t seed) {
     ONB_CHECK_CTX(ctx);
@@ -471,6 +507,7 @@ int32_t onb_mcts_select(onb_ctx* ctx) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
     if (c->mcts_phase != 1) return fail(c, ONB_E_STATE, "onb_mcts_select: call onb_mcts_begin / onb_mcts_expand_backup first");
+    if (c->ru_search) return refuse_after_reuse(c, "onb_mcts_select");
     ONB_CUDA(c, launch_mcts_select(c));
     c->mcts_phase = 2;
     return ONB_OK;
@@ -478,6 +515,7 @@ int32_t onb_mcts_select(onb_ctx* ctx) {
 int32_t onb_mcts_eval(onb_ctx* ctx, int32_t evaluator) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (c->ru_search) return refuse_after_reuse(c, "onb_mcts_eval");
     if (c->mcts_phase != 2) return fail(c, ONB_E_STATE, "onb_mcts_eval: no leaves selected");
     if (evaluator == ONB_EVAL_NET) {
         if (!c->net[c->net_cur].loaded) return fail(c, ONB_E_STATE, "onb_mcts_eval: no network loaded (onb_net_load)");
@@ -491,10 +529,41 @@ int32_t onb_mcts_eval(onb_ctx* ctx, int32_t evaluator) {
 int32_t onb_mcts_expand_backup(onb_ctx* ctx) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (c->ru_search) return refuse_after_reuse(c, "onb_mcts_expand_backup");
     if (c->mcts_phase != 2) return fail(c, ONB_E_STATE, "onb_mcts_expand_backup: call onb_mcts_select first");
     ONB_CUDA(c, launch_mcts_expand_backup(c));
     c->mcts_phase = 1;
     c->sims_done += 1;
+    return ONB_OK;
+}
+// onb_mcts_run after a reuse begin: slot t runs max(0, sims - N_root) simulations; the slots are ordered by that budget, so round r
+// runs the prefix [0, h_ru_off[r]) -- the network evaluates a shrinking batch, the fused kernel is launched once per run of rounds
+// with the same prefix. Splitting a tree's simulations over several launches gives the same tree: the kernels keep nothing else.
+static int32_t reuse_run(Ctx* c, int32_t evaluator, uint32_t sims) {
+    if (sims != c->sims_target || c->sims_done != 0)
+        return fail(c, ONB_E_INVALID, "onb_mcts_run: after a reuse begin, run once with the begin's visit target (%u), got %u", c->sims_target, sims);
+    if (evaluator == ONB_EVAL_NET && !c->net[c->net_cur].loaded) return fail(c, ONB_E_STATE, "onb_mcts_run: no network loaded (onb_net_load)");
+    const uint32_t* off = c->h_ru_off;
+    cudaError_t e = cudaSuccess;
+    if (evaluator == ONB_EVAL_NET) {
+        for (uint32_t r = 0; r < sims && off[r] > 0 && e == cudaSuccess; ++r) {
+            c->n_act = (int64_t)off[r];
+            e = launch_mcts_select(c);
+            if (e == cudaSuccess) e = launch_net_forward(c, c->d_leaf_planes, c->d_policy, c->d_value, (int64_t)off[r]);
+            if (e == cudaSuccess) e = launch_mcts_expand_backup(c);
+        }
+    } else {
+        for (uint32_t r = 0; r < sims && off[r] > 0 && e == cudaSuccess;) {
+            uint32_t r1 = r + 1;
+            while (r1 < sims && off[r1] == off[r]) ++r1;
+            c->n_act = (int64_t)off[r];
+            e = launch_mcts_run(c, evaluator, r1 - r);
+            r = r1;
+        }
+    }
+    c->n_act = c->ru_m;
+    if (e != cudaSuccess) return cuda_fail(c, e, "onb_mcts_run");
+    c->sims_done += sims;
     return ONB_OK;
 }
 int32_t onb_mcts_run(onb_ctx* ctx, int32_t evaluator, uint32_t sims) {
@@ -504,6 +573,7 @@ int32_t onb_mcts_run(onb_ctx* ctx, int32_t evaluator, uint32_t sims) {
     if (evaluator != ONB_EVAL_UNIFORM && evaluator != ONB_EVAL_HASH && evaluator != ONB_EVAL_NET)
         return fail(c, ONB_E_INVALID, "onb_mcts_run: unknown evaluator %d", evaluator);
     if (c->sims_done + sims > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_mcts_run: more simulations than mcts_max_sims");
+    if (c->ru_search) return reuse_run(c, evaluator, sims);
     if (evaluator == ONB_EVAL_NET) {
         // the network sits between select and expand: three launches per simulation round, all on the context's stream.
         // ONB_MCTS_STEP_FUSION=1 (exploration knob): expand_backup(s) and select(s + 1) as ONE launch (k_mcts_step_g) -- measured SLOWER
@@ -543,13 +613,27 @@ static int32_t mcts_begin_subset(Ctx* c, double c_puct, uint32_t sims, const int
     c->sims_done = 0;
     c->n_act = m;
     c->d_tree_game = d_games;
+    c->ru_live = c->ru_search = c->ru_public = 0;  // a search without reuse forgets the remembered trees
     ONB_CUDA(c, launch_mcts_begin(c));
+    c->mcts_phase = 1;
+    return ONB_OK;
+}
+// onb_self_play's search with reuse: the m games d_games (nullptr: all) in budget order; the outputs stay in slot order, the driver
+// scatters them through d_tree_game
+static int32_t reuse_begin_subset(Ctx* c, double c_puct, uint32_t sims, const int32_t* d_games, int64_t m) {
+    c->c_puct = c_puct;
+    c->sims_target = sims;
+    c->sims_done = 0;
+    c->mcts_phase = 0;
+    ONB_CUDA(c, launch_reuse_begin(c, d_games, d_games ? m : c->n, sims));
+    c->ru_search = 1;
+    c->ru_public = 0;
     c->mcts_phase = 1;
     return ONB_OK;
 }
 static int32_t self_play_search(Ctx* c, const onb_selfplay_config* cfg, const int32_t* d_games, int64_t m) {
     onb_ctx* x = reinterpret_cast<onb_ctx*>(c);
-    int32_t rc = mcts_begin_subset(c, cfg->c_puct, cfg->sims, d_games, m);
+    int32_t rc = c->reuse_on ? reuse_begin_subset(c, cfg->c_puct, cfg->sims, d_games, m) : mcts_begin_subset(c, cfg->c_puct, cfg->sims, d_games, m);
     if (rc == ONB_OK) rc = onb_mcts_run(x, cfg->evaluator, cfg->sims);
     if (rc == ONB_OK) rc = onb_mcts_finish(x, nullptr, nullptr, nullptr, nullptr, nullptr);
     return rc;
@@ -562,6 +646,7 @@ int32_t onb_self_play(onb_ctx* ctx, const onb_selfplay_config* cfg, onb_selfplay
     if (cfg->sims == 0 || cfg->sims > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_self_play: sims %u not in 1..mcts_max_sims", cfg->sims);
     if (cfg->n_games <= 0) return fail(c, ONB_E_INVALID, "onb_self_play: n_games must be positive");
     memset(out, 0, sizeof(*out));
+    c->ru_live = 0;  // self-play starts from fresh deals: nothing is kept from earlier searches
     int32_t rc = onb_mcts_set_noise(ctx, cfg->train ? 1 : 0, 0.25, 0.03, cfg->noise_seed);
     if (rc != ONB_OK) return rc;
     char err[400];
@@ -656,6 +741,7 @@ int32_t onb_uct_run(onb_ctx* ctx, float exploration_c, uint32_t min_node_visits,
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
     if (c->mcts_phase != 1) return fail(c, ONB_E_STATE, "onb_uct_run: call onb_mcts_begin first");
+    if (c->ru_search) return refuse_after_reuse(c, "onb_uct_run");
     if (c->sims_done + playouts > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_uct_run: more playouts than mcts_max_sims");
     const uint32_t need = c->sims_done + playouts + 2;
     if (c->ln_cap < need) {  // ln(parent visits) as the reference computes it: f32 logf on the host
@@ -695,7 +781,16 @@ int32_t onb_mcts_finish(onb_ctx* ctx, onb_action* best_host, float* pi_host, uin
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
     if (c->mcts_phase != 1) return fail(c, ONB_E_STATE, "onb_mcts_finish: search not in a finished-simulation state");
-    ONB_CUDA(c, launch_mcts_finish(c));
+    if (c->ru_search && c->ru_public) {  // finish in slot order into the scratch, then back into game order
+        float* pi = c->d_pi; uint16_t* best = c->d_best; uint32_t* rv = c->d_root_visits; double* q = c->d_root_q; uint32_t* cv = c->d_child_visits;
+        c->d_pi = c->d_ru_pi; c->d_best = c->d_ru_best; c->d_root_visits = c->d_ru_rv; c->d_root_q = c->d_ru_q; c->d_child_visits = c->d_ru_cv;
+        const cudaError_t e = launch_mcts_finish(c);
+        c->d_pi = pi; c->d_best = best; c->d_root_visits = rv; c->d_root_q = q; c->d_child_visits = cv;
+        ONB_CUDA(c, e);
+        ONB_CUDA(c, launch_reuse_unpermute(c));
+    } else {
+        ONB_CUDA(c, launch_mcts_finish(c));
+    }
     const size_t n = (size_t)c->n;
     bool any = false;
     if (best_host) { ONB_CUDA(c, cudaMemcpyAsync(best_host, c->d_best, n * 2, cudaMemcpyDeviceToHost, c->stream)); any = true; }
@@ -720,6 +815,16 @@ int32_t onb_mcts_dump_tree(onb_ctx* ctx, int64_t tree, int64_t cap, onb_tree_dum
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
     if (!c->d_nodes || tree < 0 || tree >= c->n || !out) return fail(c, ONB_E_INVALID, "onb_mcts_dump_tree: bad arguments");
     uint32_t size = 0;
+    if (c->ru_live) {  // trees laid out by budget: `tree` is a game; a game without a remembered tree has none (0 nodes)
+        int32_t slot = -1;
+        ONB_CUDA(c, cudaMemcpyAsync(&slot, c->d_ru_slot + tree, 4, cudaMemcpyDeviceToHost, c->stream));
+        ONB_CUDA(c, cudaStreamSynchronize(c->stream));
+        if (slot < 0) {
+            if (n_nodes) *n_nodes = 0;
+            return ONB_OK;
+        }
+        tree = slot;
+    }
     ONB_CUDA(c, cudaMemcpyAsync(&size, c->d_tree_size + tree, 4, cudaMemcpyDeviceToHost, c->stream));
     ONB_CUDA(c, cudaStreamSynchronize(c->stream));
     if (n_nodes) *n_nodes = size;
@@ -742,10 +847,33 @@ int32_t onb_mcts_dump_tree(onb_ctx* ctx, int64_t tree, int64_t cap, onb_tree_dum
     free(h);
     return ONB_OK;
 }
+// onb_mcts_tree_info with the trees laid out by budget: gathered into game order on the host (0 nodes for a game without a tree)
+static int32_t reuse_tree_info(Ctx* c, uint32_t* n_nodes_host, uint8_t* flags_host) {
+    const size_t n = (size_t)c->n;
+    uint32_t* size = static_cast<uint32_t*>(malloc(n * 4));
+    uint8_t* flags = static_cast<uint8_t*>(malloc(n));
+    int32_t* slot = static_cast<int32_t*>(malloc(n * 4));
+    cudaError_t e = (size && flags && slot) ? cudaSuccess : cudaErrorMemoryAllocation;
+    if (e == cudaSuccess) e = cudaMemcpyAsync(size, c->d_tree_size, n * 4, cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(flags, c->d_tree_flags, n, cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(slot, c->d_ru_slot, n * 4, cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    if (e == cudaSuccess)
+        for (size_t g = 0; g < n; ++g) {
+            if (n_nodes_host) n_nodes_host[g] = slot[g] >= 0 ? size[slot[g]] : 0u;
+            if (flags_host) flags_host[g] = slot[g] >= 0 ? flags[slot[g]] : (uint8_t)0;
+        }
+    free(size);
+    free(flags);
+    free(slot);
+    if (e != cudaSuccess) return cuda_fail(c, e, "onb_mcts_tree_info");
+    return ONB_OK;
+}
 int32_t onb_mcts_tree_info(onb_ctx* ctx, uint32_t* n_nodes_host, uint8_t* flags_host) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
     if (!c->d_nodes) return fail(c, ONB_E_STATE, "onb_mcts_tree_info: no search buffers");
+    if (c->ru_live) return reuse_tree_info(c, n_nodes_host, flags_host);
     if (n_nodes_host) ONB_CUDA(c, cudaMemcpyAsync(n_nodes_host, c->d_tree_size, (size_t)c->n * 4, cudaMemcpyDeviceToHost, c->stream));
     if (flags_host) ONB_CUDA(c, cudaMemcpyAsync(flags_host, c->d_tree_flags, (size_t)c->n, cudaMemcpyDeviceToHost, c->stream));
     ONB_CUDA(c, cudaStreamSynchronize(c->stream));

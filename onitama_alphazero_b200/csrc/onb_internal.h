@@ -94,6 +94,27 @@ struct Ctx {
     // onb_alphabeta_run: per-game root score and node count (allocated on first use)
     int32_t* d_ab_score;
     unsigned long long* d_ab_nodes;
+    // tree reuse (onb_reuse.cu, onb_mcts_set_reuse); buffers allocated by the first enabling call
+    int reuse_on;         // the switch
+    int ru_live;          // the pools hold the remembered trees of the last reuse search (slot layout of d_ru_game / d_ru_slot)
+    int ru_search;        // the current search was begun with reuse (split phase refused, onb_mcts_run needs sims_target)
+    int ru_public;        // ... by onb_mcts_begin: onb_mcts_finish puts its outputs back into game order
+    int64_t ru_m;         // trees of the current reuse search
+    Node* d_nodes_alt;    // second pool: the kept subtrees are compacted into it, then the pools swap
+    uint4* d_roots_alt;
+    uint32_t* d_tree_size_alt;
+    int32_t* d_ru_game;   // [n] game searched by slot t (slots ordered by remaining budget, descending)
+    int32_t* d_ru_slot;   // [n] slot holding game g's remembered tree, -1: none
+    uint4* d_ru_plan;     // [n] per searched game: old slot, kept node, budget, new slot
+    uint32_t* d_ru_mat;   // [(mcts_max_sims + 1) * blocks] counting-sort matrix
+    uint32_t* d_ru_off;   // [mcts_max_sims + 1] off[r] = trees with budget > r
+    uint32_t* h_ru_off;   // host copy (round r of the search runs trees [0, off[r]))
+    float* d_ru_pi;       // finish outputs in slot order before onb_mcts_finish puts them into game order
+    uint16_t* d_ru_best;
+    uint32_t* d_ru_rv;
+    double* d_ru_q;
+    uint32_t* d_ru_cv;
+    uint64_t ru_stats[4];
     char err[512];
 };
 
@@ -132,6 +153,14 @@ cudaError_t launch_net_forward(Ctx* c, const float* planes, float* policy, float
 // alpha-beta agent (onb_alphabeta.cu): searches games d_games[0 .. m) (nullptr: games 0 .. m) to `depth` plies; d_out[game] = the best
 // action (ONB_ACTION_NONE for a decided game), d_score / d_nodes [game] (optional) = root score and positions entered
 cudaError_t launch_alphabeta(Ctx* c, int depth, const int32_t* d_games, int64_t m, uint16_t* d_out, int32_t* d_score, unsigned long long* d_nodes);
+
+// tree reuse (onb_reuse.cu)
+cudaError_t reuse_alloc(Ctx* c);
+void reuse_free(Ctx* c);
+// reroot the remembered trees of the m games d_games (nullptr: all games) for a search to `sims` visits, swap the pools, fill
+// h_ru_off; leaves n_act = m, d_tree_game = d_ru_game
+cudaError_t launch_reuse_begin(Ctx* c, const int32_t* d_games, int64_t m, uint32_t sims);
+cudaError_t launch_reuse_unpermute(Ctx* c);  // d_ru_* (slot order) -> d_pi / d_best / ... (game order)
 
 // native self-play driver (onb_selfplay.cu)
 int32_t run_self_play(Ctx* c, const onb_selfplay_config* cfg, onb_selfplay_result* out,

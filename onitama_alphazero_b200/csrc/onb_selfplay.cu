@@ -286,10 +286,11 @@ int32_t run_self_play(Ctx* c, const onb_selfplay_config* cfg, onb_selfplay_resul
             c->d_tree_game = nullptr;
             return rc;
         }
-        if (all) {
+        if (!c->d_tree_game) {  // tree t searched game t
             SP(cudaMemcpyAsync(pi + (size_t)base * 50, c->d_pi, (size_t)n * 200, cudaMemcpyDeviceToDevice, c->stream));
-        } else {
-            k_scatter_rows50<<<(unsigned)((n_live * 50 + 255) / 256), 256, 0, c->stream>>>(c->d_pi, live_list, pi + (size_t)base * 50, n_live);
+        } else {                // the searched list (live_list, or with tree reuse that list ordered by remaining budget)
+            const int64_t nt = trees(c);
+            k_scatter_rows50<<<(unsigned)((nt * 50 + 255) / 256), 256, 0, c->stream>>>(c->d_pi, c->d_tree_game, pi + (size_t)base * 50, nt);
             SP(cudaGetLastError());
         }
         SP(cudaMemsetAsync(c->d_actions, 0xFF, (size_t)n * 2, c->stream));   // ONB_ACTION_NONE: idle slots are not stepped

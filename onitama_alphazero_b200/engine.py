@@ -193,6 +193,18 @@ class Context:
         # the select kernel's launch parameters include the noise settings: a captured simulation round is only valid for them
         self._noise = (bool(enabled), float(epsilon), float(alpha), int(seed)) if enabled else (False,)
 
+    def set_reuse(self, enabled):
+        """onb_mcts_set_reuse: keep the played child's subtree between moves (mcts_begin, self_play_native). `sims` then counts root
+        visits, kept ones included; switching off forgets the remembered trees. See include/onb.h."""
+        self._ck(self._lib.onb_mcts_set_reuse(self._h, int(bool(enabled))))
+        self.reuse = bool(enabled)
+
+    def reuse_stats(self, clear=False):
+        """onb_mcts_reuse_stats: dict(trees, kept, kept_visits, sims) summed over the reuse-enabled searches since the last clear"""
+        out = np.zeros(4, np.uint64)
+        self._ck(self._lib.onb_mcts_reuse_stats(self._h, L.ptr(out), int(bool(clear))))
+        return dict(trees=int(out[0]), kept=int(out[1]), kept_visits=int(out[2]), sims=int(out[3]))
+
     def mcts_select(self):
         self._ck(self._lib.onb_mcts_select(self._h))
 
@@ -205,11 +217,14 @@ class Context:
     def mcts_run(self, evaluator, sims):
         self._ck(self._lib.onb_mcts_run(self._h, evaluator, sims))
 
-    def self_play_native(self, c_puct, sims, n_games, max_plies=150, evaluator=L.EVAL_UNIFORM, train=False, noise_seed=0, sample_cap=None):
+    def self_play_native(self, c_puct, sims, n_games, max_plies=150, evaluator=L.EVAL_UNIFORM, train=False, noise_seed=0, sample_cap=None,
+                         reuse=None):
         """onb_self_play: the whole self-play loop inside the library (search, recording, moves, z, restart of finished slots).
         Returns torch tensors of the completed games' samples (gathered from the context's device buffers) like
-        selfplay.self_play_continuous."""
+        selfplay.self_play_continuous. reuse: True / False sets the tree-reuse switch first (set_reuse), None leaves it."""
         import torch
+        if reuse is not None:
+            self.set_reuse(reuse)
         if sample_cap is None:
             sample_cap = self.n * (max_plies + 2) * max(2, 2 * (n_games + self.n - 1) // self.n)
         cfg = L.SelfPlayConfig(c_puct, sims, evaluator, n_games, max_plies, int(bool(train)), noise_seed, sample_cap)
@@ -455,10 +470,16 @@ class Actor:
             pass
 
 
-def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_graph=False):
+def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_graph=False, reuse=None):
     """Context.search without copying the results to the host (PI / BEST stay in their device buffers).
     use_graph: capture one simulation round (select -> network -> expand/backup) in a CUDA graph on the context's stream and
-    replay it; the round is launch-bound otherwise (~40 small network kernels per round)."""
+    replay it; the round is launch-bound otherwise (~40 small network kernels per round).
+    reuse: True / False sets the tree-reuse switch first (set_reuse), None leaves it. Reuse needs a device evaluator (a torch `net`
+    drives the split phase, which a reuse search refuses)."""
+    if reuse is not None and bool(reuse) != getattr(self, "reuse", False):
+        self.set_reuse(reuse)
+    if net is not None and getattr(self, "reuse", False):
+        raise ValueError("search_device: tree reuse needs a device evaluator (EVAL_UNIFORM / EVAL_HASH / EVAL_NET), not a torch net")
     self.mcts_begin(c_puct, sims)
     if net is None:
         self.mcts_run(evaluator, sims)

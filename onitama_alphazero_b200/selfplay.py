@@ -107,12 +107,28 @@ def _self_play(ctx, c_puct, sims, max_plies, evaluator, net, decks):
     return dict(planes=planes, pi=pi, z=z, color=color, game=game)
 
 
-def self_play_continuous(ctx, c_puct, sims, n_games, max_plies=150, evaluator=L.EVAL_UNIFORM, net=None, train=False, noise_seed=0):
+def self_play_continuous(ctx, c_puct, sims, n_games, max_plies=150, evaluator=L.EVAL_UNIFORM, net=None, train=False, noise_seed=0, reuse=False):
     """self_play for at least n_games games with every slot of the context kept busy: a slot whose game ends (or hits the ply cap)
     is re-dealt at once (onb_env_reset_games), the way a worker thread of the reference starts its next game as soon as one is over
     (train.rs:218-245 around :44-98). Lockstep self_play instead searches finished slots until the longest game ends -- with game
     lengths between ~10 and 152 plies that wastes most of the work. Only completed games are returned; sample order is ply-major.
-    Extra keys: `serial` [m] (slot + n * generation: samples with the same serial belong to one game), `games` (completed games)."""
+    Extra keys: `serial` [m] (slot + n * generation: samples with the same serial belong to one game), `games` (completed games).
+    reuse=True keeps the played child's subtree between plies (Context.set_reuse; device evaluators only), as
+    onb_self_play does with the switch on; the switch is left as it was."""
+    if reuse and net is not None:
+        raise ValueError("self_play_continuous: reuse=True needs a device evaluator, not a torch net")
+    was = getattr(ctx, "reuse", False)
+    if reuse:
+        ctx.set_reuse(False)   # forget trees of earlier searches: every game starts from a fresh tree
+        ctx.set_reuse(True)
+    try:
+        return _self_play_continuous(ctx, c_puct, sims, n_games, max_plies, evaluator, net, train, noise_seed, bool(reuse))
+    finally:
+        if getattr(ctx, "reuse", False) != was:
+            ctx.set_reuse(was)
+
+
+def _self_play_continuous(ctx, c_puct, sims, n_games, max_plies, evaluator, net, train, noise_seed, reuse):
     with torch.cuda.stream(ctx.torch_stream()):
         n = ctx.n
         dev = "cuda:%d" % ctx.device
@@ -135,7 +151,7 @@ def self_play_continuous(ctx, c_puct, sims, n_games, max_plies=150, evaluator=L.
         while not bool(idle.all()):
             st = states_t.clone()
             ctx.encode(to_host=False)                       # create_tensor_from_state of the searched position (train.rs:58)
-            ctx.search_device(c_puct, sims, evaluator=evaluator, net=net)   # (this driver searches idle slots too and ignores them)
+            ctx.search_device(c_puct, sims, evaluator=evaluator, net=net, reuse=reuse)   # (this driver searches idle slots too and ignores them)
             rec["planes"].append(ctx.tensor(L.BUF_PLANES).clone())
             rec["pi"].append(ctx.tensor(L.BUF_PI).clone())
             rec["color"].append(((st[:, 1] >> 30) & 1).to(torch.int8))
