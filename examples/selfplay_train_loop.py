@@ -36,6 +36,9 @@ def main(argv=None):
     ap.add_argument("--torch-net", action="store_true", help="evaluate with the PyTorch module as a black box instead of onb_net_load")
     ap.add_argument("--reuse", action="store_true", help="keep the played child's subtree between moves in self-play (onb_mcts_set_reuse; "
                                                          "--sims then counts root visits, kept ones included; not with --torch-net)")
+    ap.add_argument("--gumbel", type=int, default=0, metavar="M",
+                    help="self-play with the Gumbel root search over M considered actions (onb_mcts_set_gumbel) and train on its improved "
+                         "policy instead of PUCT with root noise; the arena adds Gumbel(--sims) against PUCT(--sims)")
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--out", default=None, help="directory for the reference's on-disk artefacts: loss_stats JSON (stats.rs) and .ot checkpoints (train.rs:414-430)")
     ap.add_argument("--hidden", type=int, default=64, choices=[64, 128], help="hidden channels of the ConvResNet (both run on the tensor cores)")
@@ -57,6 +60,9 @@ def main(argv=None):
         ctx.net_load(model, precision=args.net_precision)   # BatchNorm folded, weights laid out for the tensor cores
         return onb.EVAL_NET, None
 
+    if args.gumbel and args.reuse:
+        ap.error("--gumbel does not combine with --reuse")
+    gumbel = dict(m=args.gumbel, seed=args.seed) if args.gumbel else None
     if args.reuse and args.torch_net:
         ap.error("--reuse needs the on-device network (a PyTorch module drives the split phase, which tree reuse does not support)")
     for it in range(args.iters):
@@ -64,11 +70,11 @@ def main(argv=None):
         with onb.Context(args.slots, seed=args.seed + it, mcts_max_sims=args.sims) as ctx:
             ev, net = evaluator_for(ctx)
             if net is None:   # the whole loop inside the library (onb_self_play)
-                data = ctx.self_play_native(2.0, args.sims, args.games, max_plies=args.max_plies, evaluator=ev, train=True,
-                                            noise_seed=args.seed + 1000 * it, reuse=args.reuse)
+                data = ctx.self_play_native(2.0, args.sims, args.games, max_plies=args.max_plies, evaluator=ev, train=not gumbel,
+                                            noise_seed=args.seed + 1000 * it, reuse=args.reuse, gumbel=gumbel)
             else:             # the same loop driven from Python, the PyTorch module between select and expand
                 data = onb.self_play_continuous(ctx, 2.0, args.sims, n_games=args.games, max_plies=args.max_plies, evaluator=ev, net=net,
-                                                train=True, noise_seed=args.seed + 1000 * it)
+                                                train=not gumbel, noise_seed=args.seed + 1000 * it, gumbel=gumbel)
         replay.add(data["planes"], data["pi"], data["z"])
         # ---- training (train.rs:264-339)
         model.train()
@@ -105,13 +111,26 @@ def main(argv=None):
             def alphabeta(cx):
                 cx.alphabeta(args.ab_depth, to_host=False)   # leaves the chosen actions in BUF_ACTIONS
 
-            for name, opponent, native in (("random", rnd, ctx.agent_random()), ("mcts", plain_mcts, ctx.agent_uct(args.mcts_playouts)),
-                                           ("alphabeta", alphabeta, ctx.agent_alphabeta(args.ab_depth))):
+            def gumbel_az(cx):   # the Gumbel agent of onb_fight: step = ply (one search per ply and agent)
+                cx.set_gumbel(True, m=args.gumbel, seed=cx.seed, step0=counter["ply"])
+                cx.search_device(2.0, args.sims, evaluator=ev, net=net)
+                cx.set_gumbel(False)
+                cx.tensor(onb.BUF_ACTIONS).copy_(cx.tensor(onb.BUF_BEST))
+                counter["ply"] += 1
+
+            fights = [("random", az, rnd, ctx.agent_puct(args.sims, 2.0, ev, 0), ctx.agent_random()),
+                      ("mcts", az, plain_mcts, ctx.agent_puct(args.sims, 2.0, ev, 0), ctx.agent_uct(args.mcts_playouts)),
+                      ("alphabeta", az, alphabeta, ctx.agent_puct(args.sims, 2.0, ev, 0), ctx.agent_alphabeta(args.ab_depth))]
+            if args.gumbel:
+                fights.append(("gumbel_vs_puct", gumbel_az, az, ctx.agent_gumbel(args.sims, args.gumbel, 0.1, ev, 0),
+                               ctx.agent_puct(args.sims, 2.0, ev, 0)))
+            for name, mine, opponent, native_a, native in fights:
                 ctx.reset()
+                counter["ply"] = 0
                 if net is None:   # the arena loop inside the library (onb_fight)
-                    w, l, d, _ = ctx.fight_native(ctx.agent_puct(args.sims, 2.0, ev, 0), native, a_is_red, max_plies=150)
+                    w, l, d, _ = ctx.fight_native(native_a, native, a_is_red, max_plies=150)
                 else:
-                    w, l, d = onb.fight(ctx, az, opponent, a_is_red, max_plies=150)
+                    w, l, d = onb.fight(ctx, mine, opponent, a_is_red, max_plies=150)
                 # FightStatistics incl. the Elo fold: on the device for the native arena (onb_fight_stats), on the host otherwise
                 stats = ctx.fight_stats(history=True) if net is None else onb.fight_statistics(ctx.last_fight_results, a_is_red)
                 elo = stats["rating_a"] if isinstance(stats, dict) else stats.rating_a
@@ -128,7 +147,8 @@ def main(argv=None):
         log.append(dict(iteration=it, games=int(data["games"]), samples=int(data["planes"].shape[0]), replay=replay.size,
                         value_loss=losses[-1][0], policy_loss=losses[-1][1], wins=results["random"]["wins"],
                         losses=results["random"]["losses"], draws=results["random"]["draws"], elo=results["random"]["elo"],
-                        vs_mcts=results["mcts"], vs_alphabeta=results["alphabeta"]))
+                        vs_mcts=results["mcts"], vs_alphabeta=results["alphabeta"],
+                        **({"gumbel_vs_puct": results["gumbel_vs_puct"]} if args.gumbel else {})))
         print(log[-1], flush=True)
     return log
 

@@ -287,6 +287,40 @@ ONB_API int32_t onb_mcts_set_reuse(onb_ctx* ctx, int32_t enabled);
 #define ONB_REUSE_KEPT_VISITS 2
 #define ONB_REUSE_SIMS 3
 ONB_API int32_t onb_mcts_reuse_stats(onb_ctx* ctx, uint64_t out[4], int32_t clear);
+/* Gumbel root search (Danihelka et al., "Policy improvement by planning with Gumbel", ICLR 2022; the root part of mctx's
+ * gumbel_muzero_policy). Off by default; with it off every entry point behaves exactly as without this call. On: the searches begun
+ * afterwards select at the ROOT by sequential halving over Gumbel-Top-k samples and report the improved policy; below the root the
+ * PUCT descent is unchanged. Definition (exact to the bit, DESIGN.md §5f), per tree, with k root children (pass pseudo-children
+ * included), P(a) the stored prior, N(a), W(a) visits and reward sum, q(a) = W(a) / N(a), r0 = the reward the root's own evaluation
+ * (simulation 0) backed up into the root and v = -r0:
+ *   logit(a) = onb_log(P(a)) (-inf for P = 0), L = max logit, p(a) = max(DBL_MIN, P(a) / sum P); if every prior is 0, every P counts as 1;
+ *   g(a) = gumbel_scale * (-onb_log(-onb_log(u))), u = (r + 0.5) 2^-32, r = onb_rand_u32(seed, global game id, step, 0x10000 + a);
+ *   v_mix = (v + sum N * (sum_{N>0} p q / sum_{N>0} p)) / (sum N + 1)  (the quotient is 0 when no child is visited);
+ *   qhat(a) = q(a) if N(a) > 0 else v_mix; sigma(a) = ((c_visit + max N) * c_scale) * ((qhat - min qhat) / max(max qhat - min qhat, 1e-8));
+ *   score(a) = max(-1e9, (g(a) + (logit(a) - L)) + sigma(a)).
+ * Descent i (i = N_root - 1) chooses the FIRST child of maximal score among those with N(a) = seq(min(m, k), sims - 1)[i] (child 0 if
+ * none), seq being mctx's sequential-halving table; onb_mcts_finish's best = the same with N(a) = max N, and pi = softmax over the
+ * children of logit + sigma (onb_exp of the difference to the maximum) summed per policy index (hand slot & 1, to) in f64, then f32.
+ * All f64 sums run in child order. onb_log / onb_exp are the project's own f64 log / exp from IEEE basic operations (fdlibm's
+ * algorithms), so the CPU and the GPU agree to the bit. root_visits, root_q and child_visits are reported as before.
+ * step: onb_mcts_begin uses a serial that this call sets to step0 and every Gumbel begin increments; onb_self_play uses step = ply,
+ * onb_fight step = ply for ONB_AGENT_GUMBEL agents (both leave the serial as they found it).
+ * Checks: 1 <= max_considered <= 40, finite c_visit, c_scale, gumbel_scale >= 0, else ONB_E_INVALID. cfg NULL or enabled = 0: off.
+ * Refused with ONB_E_STATE at onb_mcts_begin: Gumbel together with tree reuse or train-mode noise, and with the exploration knobs
+ * ONB_MCTS_WARP_PER_TREE / ONB_MCTS_STEP_FUSION / ONB_MCTS_ROOT_SMEM; after a Gumbel begin: onb_uct_run and more simulations than the
+ * begin's sims. onb_self_play while Gumbel is on: ONB_E_STATE with tree reuse on, ONB_E_INVALID with train != 0. onb_fight searches
+ * without reuse, so its Gumbel agents play whatever the reuse switch says. Every begin decides anew: a search begun with the switch
+ * off is a PUCT search. The caller-driven split phase is supported.
+ * Memory: the first enabling call allocates n_games * 1 KB of per-tree root data and a 40 x mcts_max_sims table. */
+typedef struct onb_gumbel_config {
+    int32_t enabled;
+    uint32_t max_considered; /* m, the number of root actions sampled without replacement (mctx default 16) */
+    double c_visit, c_scale, gumbel_scale; /* 50, 0.1, 1 (0: a deterministic search) */
+    uint64_t seed;
+    uint32_t step0;
+    uint32_t reserved;
+} onb_gumbel_config;
+ONB_API int32_t onb_mcts_set_gumbel(onb_ctx* ctx, const onb_gumbel_config* cfg);
 ONB_API int32_t onb_mcts_select(onb_ctx* ctx);
 ONB_API int32_t onb_mcts_expand_backup(onb_ctx* ctx);
 ONB_API int32_t onb_mcts_eval(onb_ctx* ctx, int32_t evaluator); /* fills POLICY/VALUE from LEAF_PLANES on the device */
@@ -364,6 +398,11 @@ ONB_API int32_t onb_copy_to_host(onb_ctx* ctx, void* host, const void* device, i
 #define ONB_AGENT_PUCT 1
 #define ONB_AGENT_UCT 2
 #define ONB_AGENT_ALPHABETA 3
+/* ONB_AGENT_GUMBEL: the Gumbel root search (onb_mcts_set_gumbel) with evaluator / net_slot / sims as ONB_AGENT_PUCT, m = min_node_visits
+ * (0: 16, at most 40), c_scale = c, c_visit = 50, gumbel_scale = 1, seed = onb_config.seed, step = ply, and c_puct = 2 for the PUCT
+ * descent below the root. ONB_AGENT_PUCT agents search with
+ * PUCT whatever the context's Gumbel switch says; onb_fight leaves that switch as it found it. */
+#define ONB_AGENT_GUMBEL 4
 typedef struct onb_agent {
     int32_t kind;
     int32_t evaluator;

@@ -146,6 +146,7 @@ public:
     }
     void check(int32_t rc) const { if (rc != ONB_OK) throw Error(rc, onb_last_error(ctx_)); }
     std::vector<uint8_t> last_fight_results;  ///< per-game MoveResult codes of the last fight_device (0 undecided, 1 RedWin, 2 BlueWin)
+    onb_gumbel_config gumbel_applied{};       ///< the Gumbel setting last passed to onb_mcts_set_gumbel (enabled = 0: off)
     /// one-game engine shared by the single-state methods of State / the agents (thread local: a context is single threaded)
     static Engine& single(uint32_t min_sims = 0) {
         thread_local std::unique_ptr<Engine> e;
@@ -386,6 +387,10 @@ struct AlphaZeroMctsConfig {  // alphazero_mcts/mod.rs:26-43
     // keep the played child's subtree between moves (onb_mcts_set_reuse): max_playouts then counts root visits, kept ones
     // included. Device evaluators only; false forgets the remembered trees.
     bool reuse = false;
+    // the Gumbel root search (onb_mcts_set_gumbel, DESIGN.md §5f): enabled = 1 makes every search select at the root by sequential
+    // halving and report the improved policy as the move's tensor. The setting is applied when it changes (which sets the step to
+    // step0); every search takes the next step. Does not combine with train or reuse (ONB_E_STATE).
+    onb_gumbel_config gumbel{};
 };
 inline double reward(MoveResult r, PlayerColor c) {  // alphazero_mcts/mod.rs:45-53
     if (c == PlayerColor::Red) return r == MoveResult::RedWin ? 1. : r == MoveResult::BlueWin ? -1. : 0.;
@@ -401,6 +406,13 @@ inline void run_search(Engine& e, const AlphaZeroMctsConfig& cfg, int32_t device
     e.check(onb_mcts_set_noise(e.ctx(), cfg.train ? 1 : 0, 0.25, 0.03, cfg.noise_seed));
     if (cfg.reuse && net) throw Error(ONB_E_INVALID, "AlphaZeroMctsConfig::reuse needs a device evaluator");
     e.check(onb_mcts_set_reuse(e.ctx(), cfg.reuse ? 1 : 0));
+    const onb_gumbel_config& g = cfg.gumbel;
+    const onb_gumbel_config& a = e.gumbel_applied;
+    if (g.enabled != a.enabled || (g.enabled && (g.max_considered != a.max_considered || g.c_visit != a.c_visit || g.c_scale != a.c_scale ||
+                                                 g.gumbel_scale != a.gumbel_scale || g.seed != a.seed || g.step0 != a.step0))) {
+        e.check(onb_mcts_set_gumbel(e.ctx(), &g));
+        e.gumbel_applied = g;
+    }
     e.check(onb_mcts_begin(e.ctx(), cfg.exploration_c, cfg.max_playouts));
     if (!net) {
         e.check(onb_mcts_run(e.ctx(), device_eval, cfg.max_playouts));

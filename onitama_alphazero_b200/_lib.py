@@ -83,6 +83,7 @@ SYMBOLS = {
     "onb_mcts_set_noise": (C.c_int32, [_P, C.c_int32, C.c_double, C.c_double, C.c_uint64]),
     "onb_mcts_set_reuse": (C.c_int32, [_P, C.c_int32]),
     "onb_mcts_reuse_stats": (C.c_int32, [_P, _P, C.c_int32]),
+    "onb_mcts_set_gumbel": (C.c_int32, [_P, _P]),
     "onb_mcts_select": (C.c_int32, [_P]),
     "onb_mcts_expand_backup": (C.c_int32, [_P]),
     "onb_mcts_eval": (C.c_int32, [_P, C.c_int32]),
@@ -121,9 +122,15 @@ class SelfPlayConfig(C.Structure):
                 ("train", C.c_int32), ("noise_seed", C.c_uint64), ("sample_cap", C.c_int64)]
 
 
-AGENT_RANDOM, AGENT_PUCT, AGENT_UCT, AGENT_ALPHABETA = 0, 1, 2, 3
+AGENT_RANDOM, AGENT_PUCT, AGENT_UCT, AGENT_ALPHABETA, AGENT_GUMBEL = 0, 1, 2, 3, 4
 ALPHABETA_MAX_DEPTH = 8
 ALPHABETA_WIN = 1000000
+
+
+class GumbelConfig(C.Structure):
+    """onb_gumbel_config (onb_mcts_set_gumbel)"""
+    _fields_ = [("enabled", C.c_int32), ("max_considered", C.c_uint32), ("c_visit", C.c_double), ("c_scale", C.c_double),
+                ("gumbel_scale", C.c_double), ("seed", C.c_uint64), ("step0", C.c_uint32), ("reserved", C.c_uint32)]
 
 
 class Agent(C.Structure):

@@ -7,7 +7,9 @@
 #include <exception>
 #include <new>
 #include <string>
+#include <vector>
 
+#include "onb_gumbel.cuh"
 #include "onb_internal.h"
 #include "onb_rules.cuh"
 
@@ -145,7 +147,8 @@ int32_t onb_destroy(onb_ctx* ctx) {
     void* ptrs[] = {c->d_states, c->d_masks, c->d_planes, c->d_actions, c->d_stats, c->d_io_states, c->d_moves, c->d_counts, c->d_nodes,
                     c->d_tree_size, c->d_tree_flags, c->d_roots, c->d_leaf_node, c->d_leaf_state, c->d_leaf_planes, c->d_policy, c->d_value,
                     c->d_pi, c->d_best, c->d_root_visits, c->d_root_q, c->d_child_visits, c->net[0].w, c->net[0].bias, c->net[0].head, c->net[1].w,
-                    c->net[1].bias, c->net[1].head, c->d_ln_table, c->d_net_scratch, c->d_ab_score, c->d_ab_nodes};
+                    c->net[1].bias, c->net[1].head, c->d_ln_table, c->d_net_scratch, c->d_ab_score, c->d_ab_nodes, c->d_gb,
+                    c->d_gb_tab, c->d_gb_base, c->d_gb_p, c->d_gb_r0};
     reuse_free(c);
     for (void* p : c->sp_buf)
         if (p) cudaFree(p);
@@ -444,6 +447,57 @@ int32_t onb_perft(onb_ctx* ctx, const onb_state* roots_host, int64_t n, int32_t 
 }
 
 // ---------------------------------------------------------------------------------------------- mcts
+}  // extern "C"
+namespace onb {
+static bool knob_set(const char* name, bool numeric) {
+    const char* v = getenv(name);
+    if (!v) return false;
+    return numeric ? atoi(v) != 0 : v[0] == '1';
+}
+// the combinations a Gumbel search does not support (include/onb.h, onb_mcts_set_gumbel); reuse: this begin keeps remembered trees
+// (onb_fight never does, whatever the context's reuse switch says). Every begin clears gb_search first, so a search begun after the
+// switch went off, or a refused begin, never runs the Gumbel kernels.
+static int32_t gumbel_refusals(Ctx* c, const char* what, bool reuse) {
+    c->gb_search = 0;
+    if (!c->gb_on) return ONB_OK;
+    if (reuse) return fail(c, ONB_E_STATE, "%s: the Gumbel root search does not combine with tree reuse (onb_mcts_set_reuse)", what);
+    if (c->noise_on) return fail(c, ONB_E_STATE, "%s: the Gumbel root search does not combine with train-mode noise (onb_mcts_set_noise)", what);
+    if (knob_set("ONB_MCTS_WARP_PER_TREE", false) || knob_set("ONB_MCTS_STEP_FUSION", false) || knob_set("ONB_MCTS_ROOT_SMEM", true))
+        return fail(c, ONB_E_STATE, "%s: the Gumbel root search does not run with the exploration knobs ONB_MCTS_WARP_PER_TREE / "
+                                    "ONB_MCTS_STEP_FUSION / ONB_MCTS_ROOT_SMEM", what);
+    return ONB_OK;
+}
+// after the trees are begun: the search's GumbelDev (step = the serial, which advances) and, when (m, sims) changed, the table
+static int32_t gumbel_begin(Ctx* c, uint32_t sims) {
+    c->gb_search = c->gb_on;
+    if (!c->gb_on) return ONB_OK;
+    const uint32_t m = c->gb_cfg.max_considered, nt = sims ? sims - 1u : 0u;
+    if (nt && (c->gb_tab_m != m || c->gb_tab_n != nt)) {
+        std::vector<uint32_t> tab((size_t)m * nt);
+        for (uint32_t r = 1; r <= m; ++r) onb_gumbel::seq_halving(r, nt, tab.data() + (size_t)(r - 1u) * nt);
+        // from pageable memory: the copy has taken the data when the call returns, so tab may go out of scope
+        ONB_CUDA(c, cudaMemcpyAsync(c->d_gb_tab, tab.data(), tab.size() * 4, cudaMemcpyHostToDevice, c->stream));
+        c->gb_tab_m = m;
+        c->gb_tab_n = nt;
+    }
+    GumbelDev h;
+    memset(&h, 0, sizeof(h));
+    h.c_visit = c->gb_cfg.c_visit;
+    h.c_scale = c->gb_cfg.c_scale;
+    h.scale = c->gb_cfg.gumbel_scale;
+    h.seed = c->gb_cfg.seed;
+    h.step = c->gb_serial++;
+    h.m = m;
+    h.n_tab = nt;
+    h.tab = c->d_gb_tab;
+    h.base = c->d_gb_base;
+    h.p = c->d_gb_p;
+    h.r0 = c->d_gb_r0;
+    ONB_CUDA(c, cudaMemcpyAsync(c->d_gb, &h, sizeof(h), cudaMemcpyHostToDevice, c->stream));
+    return ONB_OK;
+}
+}  // namespace onb
+extern "C" {
 int32_t onb_mcts_begin(onb_ctx* ctx, double c_puct, uint32_t sims) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
@@ -455,6 +509,8 @@ int32_t onb_mcts_begin(onb_ctx* ctx, double c_puct, uint32_t sims) {
     c->n_act = 0;  // the public search covers every game of the context
     c->d_tree_game = nullptr;
     c->mcts_phase = 0;
+    int32_t rc = gumbel_refusals(c, "onb_mcts_begin", c->reuse_on != 0);
+    if (rc != ONB_OK) return rc;
     if (c->reuse_on) {  // every game, trees laid out by remaining budget; finish puts the outputs back into game order
         ONB_CUDA(c, launch_reuse_begin(c, nullptr, c->n, sims));
         c->ru_search = 1;
@@ -463,7 +519,39 @@ int32_t onb_mcts_begin(onb_ctx* ctx, double c_puct, uint32_t sims) {
         c->ru_live = c->ru_search = c->ru_public = 0;  // a search without reuse forgets the remembered trees
         ONB_CUDA(c, launch_mcts_begin(c));
     }
+    if ((rc = gumbel_begin(c, sims)) != ONB_OK) return rc;
     c->mcts_phase = 1;
+    return ONB_OK;
+}
+int32_t onb_mcts_set_gumbel(onb_ctx* ctx, const onb_gumbel_config* cfg) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (!cfg || !cfg->enabled) {
+        c->gb_on = 0;
+        return ONB_OK;
+    }
+    if (cfg->max_considered < 1 || cfg->max_considered > 40 || !std::isfinite(cfg->c_visit) || !std::isfinite(cfg->c_scale) ||
+        !std::isfinite(cfg->gumbel_scale) || !(cfg->c_visit >= 0.0) || !(cfg->c_scale >= 0.0) || !(cfg->gumbel_scale >= 0.0))
+        return fail(c, ONB_E_INVALID, "onb_mcts_set_gumbel: need 1 <= max_considered <= 40 and finite c_visit, c_scale, gumbel_scale >= 0");
+    if (!c->d_nodes) return fail(c, ONB_E_STATE, "onb_mcts_set_gumbel: context created with mcts_max_sims = 0");
+    if (!c->d_gb) {
+        const size_t n = (size_t)c->n;
+        cudaError_t e = dalloc(&c->d_gb, 1);
+        if (e == cudaSuccess) e = dalloc(&c->d_gb_tab, (size_t)40 * c->cfg.mcts_max_sims);
+        if (e == cudaSuccess) e = dalloc(&c->d_gb_base, n * kGbStride);
+        if (e == cudaSuccess) e = dalloc(&c->d_gb_p, n * kGbStride);
+        if (e == cudaSuccess) e = dalloc(&c->d_gb_r0, n);
+        if (e != cudaSuccess) {
+            for (void* p : {(void*)c->d_gb, (void*)c->d_gb_tab, (void*)c->d_gb_base, (void*)c->d_gb_p, (void*)c->d_gb_r0})
+                if (p) cudaFree(p);
+            c->d_gb = nullptr; c->d_gb_tab = nullptr; c->d_gb_base = c->d_gb_p = c->d_gb_r0 = nullptr;
+            return e == cudaErrorMemoryAllocation ? fail(c, ONB_E_NOMEM, "onb_mcts_set_gumbel: out of device memory") : cuda_fail(c, e, "onb_mcts_set_gumbel");
+        }
+        c->gb_tab_m = c->gb_tab_n = 0;
+    }
+    c->gb_cfg = *cfg;
+    c->gb_serial = cfg->step0;
+    c->gb_on = 1;
     return ONB_OK;
 }
 int32_t onb_mcts_set_reuse(onb_ctx* ctx, int32_t enabled) {
@@ -508,6 +596,8 @@ int32_t onb_mcts_select(onb_ctx* ctx) {
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
     if (c->mcts_phase != 1) return fail(c, ONB_E_STATE, "onb_mcts_select: call onb_mcts_begin / onb_mcts_expand_backup first");
     if (c->ru_search) return refuse_after_reuse(c, "onb_mcts_select");
+    if (c->gb_search && c->sims_done >= c->sims_target)
+        return fail(c, ONB_E_STATE, "onb_mcts_select: a Gumbel search runs at most the begin's %u simulations", c->sims_target);
     ONB_CUDA(c, launch_mcts_select(c));
     c->mcts_phase = 2;
     return ONB_OK;
@@ -574,6 +664,8 @@ int32_t onb_mcts_run(onb_ctx* ctx, int32_t evaluator, uint32_t sims) {
         return fail(c, ONB_E_INVALID, "onb_mcts_run: unknown evaluator %d", evaluator);
     if (c->sims_done + sims > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_mcts_run: more simulations than mcts_max_sims");
     if (c->ru_search) return reuse_run(c, evaluator, sims);
+    if (c->gb_search && c->sims_done + sims > c->sims_target)
+        return fail(c, ONB_E_STATE, "onb_mcts_run: a Gumbel search runs at most the begin's %u simulations", c->sims_target);
     if (evaluator == ONB_EVAL_NET) {
         // the network sits between select and expand: three launches per simulation round, all on the context's stream.
         // ONB_MCTS_STEP_FUSION=1 (exploration knob): expand_backup(s) and select(s + 1) as ONE launch (k_mcts_step_g) -- measured SLOWER
@@ -614,13 +706,18 @@ static int32_t mcts_begin_subset(Ctx* c, double c_puct, uint32_t sims, const int
     c->n_act = m;
     c->d_tree_game = d_games;
     c->ru_live = c->ru_search = c->ru_public = 0;  // a search without reuse forgets the remembered trees
+    int32_t rc = gumbel_refusals(c, "search", false);
+    if (rc != ONB_OK) return rc;
     ONB_CUDA(c, launch_mcts_begin(c));
+    if ((rc = gumbel_begin(c, sims)) != ONB_OK) return rc;
     c->mcts_phase = 1;
     return ONB_OK;
 }
 // onb_self_play's search with reuse: the m games d_games (nullptr: all) in budget order; the outputs stay in slot order, the driver
 // scatters them through d_tree_game
 static int32_t reuse_begin_subset(Ctx* c, double c_puct, uint32_t sims, const int32_t* d_games, int64_t m) {
+    const int32_t rc = gumbel_refusals(c, "onb_self_play", true);
+    if (rc != ONB_OK) return rc;
     c->c_puct = c_puct;
     c->sims_target = sims;
     c->sims_done = 0;
@@ -645,10 +742,14 @@ int32_t onb_self_play(onb_ctx* ctx, const onb_selfplay_config* cfg, onb_selfplay
     if (!c->d_planes || !c->d_nodes) return fail(c, ONB_E_STATE, "onb_self_play: the context needs alloc_planes and mcts_max_sims > 0");
     if (cfg->sims == 0 || cfg->sims > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_self_play: sims %u not in 1..mcts_max_sims", cfg->sims);
     if (cfg->n_games <= 0) return fail(c, ONB_E_INVALID, "onb_self_play: n_games must be positive");
+    if (cfg->train && c->gb_on) return fail(c, ONB_E_INVALID, "onb_self_play: train-mode noise does not combine with the Gumbel root search");
+    if (c->reuse_on && c->gb_on) return fail(c, ONB_E_STATE, "onb_self_play: tree reuse does not combine with the Gumbel root search");
     memset(out, 0, sizeof(*out));
     c->ru_live = 0;  // self-play starts from fresh deals: nothing is kept from earlier searches
     int32_t rc = onb_mcts_set_noise(ctx, cfg->train ? 1 : 0, 0.25, 0.03, cfg->noise_seed);
     if (rc != ONB_OK) return rc;
+    const uint32_t serial = c->gb_serial;
+    c->gb_serial = 0;  // one search per ply: the Gumbel step of ply p is p
     char err[400];
     err[0] = 0;
     try {
@@ -657,6 +758,7 @@ int32_t onb_self_play(onb_ctx* ctx, const onb_selfplay_config* cfg, onb_selfplay
         snprintf(err, sizeof(err), "onb_self_play: %s", ex.what());
         rc = ONB_E_NOMEM;
     }
+    c->gb_serial = serial;
     onb_mcts_set_noise(ctx, 0, 0.25, 0.03, 0);
     if (rc != ONB_OK) return fail(c, rc, "%s", err);
     return ONB_OK;
@@ -674,9 +776,19 @@ static int32_t fight_move(Ctx* c, const onb_agent* ag, uint32_t ply, const int32
         ONB_CUDA(c, launch_alphabeta(c, (int)ag->sims, d_games, m, d_out, nullptr, nullptr));
         return ONB_OK;
     }
-    int32_t rc = mcts_begin_subset(c, ag->c, ag->sims, d_games, m);
+    c->gb_on = 0;  // PUCT and UCT agents search without the Gumbel root step
+    if (ag->kind == ONB_AGENT_GUMBEL) {
+        c->gb_on = 1;
+        c->gb_cfg.max_considered = ag->min_node_visits ? ag->min_node_visits : 16u;
+        c->gb_cfg.c_visit = 50.0;
+        c->gb_cfg.c_scale = ag->c;
+        c->gb_cfg.gumbel_scale = 1.0;
+        c->gb_cfg.seed = c->cfg.seed;
+        c->gb_serial = ply;
+    }
+    int32_t rc = mcts_begin_subset(c, ag->kind == ONB_AGENT_GUMBEL ? 2.0 : ag->c, ag->sims, d_games, m);
     if (rc != ONB_OK) return rc;
-    if (ag->kind == ONB_AGENT_PUCT) {
+    if (ag->kind == ONB_AGENT_PUCT || ag->kind == ONB_AGENT_GUMBEL) {
         if (ag->evaluator == ONB_EVAL_NET && (rc = onb_net_select(x, ag->net_slot)) != ONB_OK) return rc;
         rc = onb_mcts_run(x, ag->evaluator, ag->sims);
     } else {
@@ -694,8 +806,11 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
     if (!a || !b || !a_is_red_host || !out) return fail(c, ONB_E_INVALID, "onb_fight: null argument");
     for (const onb_agent* ag : {a, b}) {
-        if (ag->kind != ONB_AGENT_RANDOM && ag->kind != ONB_AGENT_PUCT && ag->kind != ONB_AGENT_UCT && ag->kind != ONB_AGENT_ALPHABETA)
+        if (ag->kind != ONB_AGENT_RANDOM && ag->kind != ONB_AGENT_PUCT && ag->kind != ONB_AGENT_UCT && ag->kind != ONB_AGENT_ALPHABETA &&
+            ag->kind != ONB_AGENT_GUMBEL)
             return fail(c, ONB_E_INVALID, "onb_fight: unknown agent kind %d", ag->kind);
+        if (ag->kind == ONB_AGENT_GUMBEL && (ag->min_node_visits > 40 || !std::isfinite(ag->c) || !(ag->c >= 0.0)))
+            return fail(c, ONB_E_INVALID, "onb_fight: a Gumbel agent needs min_node_visits (m) <= 40 and a finite c (c_scale) >= 0");
         if (ag->kind == ONB_AGENT_ALPHABETA) {
             if (ag->sims < 1 || ag->sims > ONB_ALPHABETA_MAX_DEPTH)
                 return fail(c, ONB_E_INVALID, "onb_fight: an alpha-beta agent needs 1 <= depth (sims) <= %d", ONB_ALPHABETA_MAX_DEPTH);
@@ -707,9 +822,25 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
     memset(out, 0, sizeof(*out));
     int32_t rc = onb_mcts_set_noise(ctx, 0, 0.25, 0.03, 0);  // arenas search in eval mode (AlphaZeroMcts, not TrainingAlphaZeroMcts)
     if (rc != ONB_OK) return rc;
+    const int gb_on = c->gb_on;  // the agents set the Gumbel switch per move; the context's own setting comes back afterwards
+    const onb_gumbel_config gb_cfg = c->gb_cfg;
+    const uint32_t gb_serial = c->gb_serial;
+    if (a->kind == ONB_AGENT_GUMBEL || b->kind == ONB_AGENT_GUMBEL) {
+        onb_gumbel_config on;
+        memset(&on, 0, sizeof(on));
+        on.enabled = 1;
+        on.max_considered = 16;
+        if ((rc = onb_mcts_set_gumbel(ctx, &on)) != ONB_OK) return rc;  // allocates the Gumbel buffers; the context's setting is restored below
+        c->gb_on = gb_on;
+        c->gb_cfg = gb_cfg;
+        c->gb_serial = gb_serial;
+    }
     char err[400];
     err[0] = 0;
     rc = run_fight(c, a, b, a_is_red_host, max_plies, out, fight_move, err, sizeof(err));
+    c->gb_on = gb_on;
+    c->gb_cfg = gb_cfg;
+    c->gb_serial = gb_serial;
     if (rc != ONB_OK) return fail(c, rc, "%s", err);
     if (results_host) {
         ONB_CUDA(c, cudaMemcpyAsync(results_host, out->results, (size_t)c->n, cudaMemcpyDeviceToHost, c->stream));
@@ -742,6 +873,7 @@ int32_t onb_uct_run(onb_ctx* ctx, float exploration_c, uint32_t min_node_visits,
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
     if (c->mcts_phase != 1) return fail(c, ONB_E_STATE, "onb_uct_run: call onb_mcts_begin first");
     if (c->ru_search) return refuse_after_reuse(c, "onb_uct_run");
+    if (c->gb_search) return fail(c, ONB_E_STATE, "onb_uct_run: the search was begun with the Gumbel root search on (onb_mcts_set_gumbel)");
     if (c->sims_done + playouts > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_uct_run: more playouts than mcts_max_sims");
     const uint32_t need = c->sims_done + playouts + 2;
     if (c->ln_cap < need) {  // ln(parent visits) as the reference computes it: f32 logf on the host

@@ -27,6 +27,19 @@ constexpr uint8_t kNodeExpanded = 1, kNodeTerminal = 2, kNodePass = 4;
 constexpr uint8_t kTreePassSeen = 1, kTreeOverflow = 2;
 constexpr int kMaxDepth = 32;  // path entries kept in registers (lane l <-> level l); deeper paths spill to the parent chain
 
+// Gumbel root search (onb_mcts_set_gumbel, DESIGN.md §5f). Every onb_mcts_begin with the switch on rewrites this device struct, so
+// a captured simulation round (CUDA graph) reads the current search's step and table instead of baking them into its launches.
+constexpr int kGbStride = 64;  // per-tree root-child slots: 8 pieces x 2 cards x 4 moves, the most the lane-group expansion writes
+struct GumbelDev {
+    double c_visit, c_scale, scale;
+    uint64_t seed;
+    uint32_t step, m, n_tab, reserved;  // n_tab = sims - 1 descents
+    const uint32_t* tab;                // [m][n_tab]: row m_eff - 1 = seq_halving(m_eff, n_tab)
+    double* base;                       // [n][kGbStride] g(a) + (logit(a) - L), written by the root's first descent
+    double* p;                          // [n][kGbStride] max(DBL_MIN, P(a) / sum P)
+    double* r0;                         // [n] the reward the root's own evaluation backed up into the root
+};
+
 struct Ctx {
     onb_config cfg;
     cudaStream_t stream;
@@ -115,6 +128,17 @@ struct Ctx {
     double* d_ru_q;
     uint32_t* d_ru_cv;
     uint64_t ru_stats[4];
+    // Gumbel root search (onb_mcts_set_gumbel); buffers allocated by the first enabling call
+    int gb_on;                // the switch
+    onb_gumbel_config gb_cfg;
+    uint32_t gb_serial;       // step of the next Gumbel onb_mcts_begin
+    int gb_search;            // the current search was begun with Gumbel
+    GumbelDev* d_gb;          // the device struct every Gumbel begin rewrites
+    uint32_t* d_gb_tab;       // [40][mcts_max_sims]
+    double* d_gb_base;
+    double* d_gb_p;
+    double* d_gb_r0;
+    uint32_t gb_tab_m, gb_tab_n;  // the table d_gb_tab holds (gb_tab_m = 0: none)
     char err[512];
 };
 
@@ -145,6 +169,7 @@ cudaError_t launch_uct_run(Ctx* c, float exploration_c, uint32_t min_node_visits
 cudaError_t launch_mcts_finish(Ctx* c);
 cudaError_t launch_mcts_play_best(Ctx* c, uint32_t out_flags);
 cudaError_t launch_mcts_scatter_best(Ctx* c, uint16_t* dst_actions);  // dst[game of tree t] = best[t]
+// with c->gb_search the three launchers above that select at the root (select, run, finish) run the Gumbel variants
 
 // network (onb_net.cu)
 int32_t net_load(Ctx* c, int32_t n_tensors, const char* const* names, const float* const* data, const int64_t* numel, std::string& err);

@@ -186,6 +186,8 @@ class Context:
     # ------------------------------------------------------------------ mcts
     def mcts_begin(self, c_puct, sims):
         self._ck(self._lib.onb_mcts_begin(self._h, float(c_puct), sims))
+        if getattr(self, "gumbel", None) is not None:
+            self.gumbel_step += 1  # the library's serial: the step of the next Gumbel search
 
     def mcts_set_noise(self, enabled, epsilon=0.25, alpha=0.03, seed=0):
         """train mode: root exploration noise (AlphaZeroMctsConfig::train); statistical parity only."""
@@ -205,6 +207,30 @@ class Context:
         self._ck(self._lib.onb_mcts_reuse_stats(self._h, L.ptr(out), int(bool(clear))))
         return dict(trees=int(out[0]), kept=int(out[1]), kept_visits=int(out[2]), sims=int(out[3]))
 
+    def set_gumbel(self, enabled, m=16, c_visit=50.0, c_scale=0.1, gumbel_scale=1.0, seed=0, step0=0):
+        """onb_mcts_set_gumbel: the Gumbel root search (sequential halving over m Gumbel-Top-k samples at the root, improved-policy
+        targets in mcts_finish's pi). The step of the next search becomes step0; every search begun afterwards takes the next step.
+        See include/onb.h and DESIGN.md §5f."""
+        cfg = L.GumbelConfig(int(bool(enabled)), int(m), float(c_visit), float(c_scale), float(gumbel_scale), int(seed), int(step0), 0)
+        self._ck(self._lib.onb_mcts_set_gumbel(self._h, C.byref(cfg)))
+        self.gumbel = (int(m), float(c_visit), float(c_scale), float(gumbel_scale), int(seed)) if enabled else None
+        self.gumbel_step = int(step0)  # self_play_native and fight_native leave the library's serial as they found it
+
+    def _use_gumbel(self, gumbel):
+        """the gumbel= argument of the search drivers: None leaves the switch, False switches it off, True (the defaults) or a dict of
+        set_gumbel keywords switches it on unless that setting is already on (so consecutive searches keep advancing the step)"""
+        if gumbel is None:
+            return
+        if not gumbel:
+            if getattr(self, "gumbel", None) is not None:
+                self.set_gumbel(False)
+            return
+        kw = dict(gumbel) if isinstance(gumbel, dict) else {}
+        want = (int(kw.get("m", 16)), float(kw.get("c_visit", 50.0)), float(kw.get("c_scale", 0.1)), float(kw.get("gumbel_scale", 1.0)),
+                int(kw.get("seed", 0)))
+        if getattr(self, "gumbel", None) != want or "step0" in kw:
+            self.set_gumbel(True, **kw)
+
     def mcts_select(self):
         self._ck(self._lib.onb_mcts_select(self._h))
 
@@ -218,13 +244,15 @@ class Context:
         self._ck(self._lib.onb_mcts_run(self._h, evaluator, sims))
 
     def self_play_native(self, c_puct, sims, n_games, max_plies=150, evaluator=L.EVAL_UNIFORM, train=False, noise_seed=0, sample_cap=None,
-                         reuse=None):
+                         reuse=None, gumbel=None):
         """onb_self_play: the whole self-play loop inside the library (search, recording, moves, z, restart of finished slots).
         Returns torch tensors of the completed games' samples (gathered from the context's device buffers) like
-        selfplay.self_play_continuous. reuse: True / False sets the tree-reuse switch first (set_reuse), None leaves it."""
+        selfplay.self_play_continuous. reuse: True / False sets the tree-reuse switch first (set_reuse), None leaves it. gumbel: as for
+        search_device (the Gumbel step of ply p is p; pi is then the improved policy)."""
         import torch
         if reuse is not None:
             self.set_reuse(reuse)
+        self._use_gumbel(gumbel)
         if sample_cap is None:
             sample_cap = self.n * (max_plies + 2) * max(2, 2 * (n_games + self.n - 1) // self.n)
         cfg = L.SelfPlayConfig(c_puct, sims, evaluator, n_games, max_plies, int(bool(train)), noise_seed, sample_cap)
@@ -256,6 +284,11 @@ class Context:
     @staticmethod
     def agent_uct(playouts, exploration_c=2.0 ** 0.5, min_node_visits=5):
         return L.Agent(L.AGENT_UCT, 0, 0, playouts, exploration_c, min_node_visits, 0)
+
+    @staticmethod
+    def agent_gumbel(sims, m=16, c_scale=0.1, evaluator=L.EVAL_UNIFORM, net_slot=0):
+        """the Gumbel root search as an arena agent (c_visit 50, gumbel_scale 1, seed = the context's seed, step = ply)"""
+        return L.Agent(L.AGENT_GUMBEL, evaluator, net_slot, sims, c_scale, m, 0)
 
     @staticmethod
     def agent_alphabeta(depth):
@@ -470,14 +503,17 @@ class Actor:
             pass
 
 
-def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_graph=False, reuse=None):
+def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_graph=False, reuse=None, gumbel=None):
     """Context.search without copying the results to the host (PI / BEST stay in their device buffers).
     use_graph: capture one simulation round (select -> network -> expand/backup) in a CUDA graph on the context's stream and
     replay it; the round is launch-bound otherwise (~40 small network kernels per round).
     reuse: True / False sets the tree-reuse switch first (set_reuse), None leaves it. Reuse needs a device evaluator (a torch `net`
-    drives the split phase, which a reuse search refuses)."""
+    drives the split phase, which a reuse search refuses).
+    gumbel: None leaves the Gumbel switch as it is, False switches it off, True or a dict of set_gumbel keywords switches it on (only
+    when that setting is not on already, so that consecutive searches take consecutive steps)."""
     if reuse is not None and bool(reuse) != getattr(self, "reuse", False):
         self.set_reuse(reuse)
+    self._use_gumbel(gumbel)
     if net is not None and getattr(self, "reuse", False):
         raise ValueError("search_device: tree reuse needs a device evaluator (EVAL_UNIFORM / EVAL_HASH / EVAL_NET), not a torch net")
     self.mcts_begin(c_puct, sims)
@@ -503,7 +539,7 @@ def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_g
                 # a captured round bakes in everything the launches were given: the evaluator, c_puct AND the root-noise settings
                 # (ADVICE r01: switching train mode after a capture must not replay the old setting). The cache holds a strong
                 # reference to `net`, so its id cannot be recycled for another module while the graph lives; close() drops it.
-                key = (id(net), float(c_puct), getattr(self, "_noise", (False,)))
+                key = (id(net), float(c_puct), getattr(self, "_noise", (False,)), getattr(self, "gumbel", None))
                 cache = self.__dict__.setdefault("_graphs", {})
                 done = 0
                 if key not in cache:

@@ -107,25 +107,37 @@ def _self_play(ctx, c_puct, sims, max_plies, evaluator, net, decks):
     return dict(planes=planes, pi=pi, z=z, color=color, game=game)
 
 
-def self_play_continuous(ctx, c_puct, sims, n_games, max_plies=150, evaluator=L.EVAL_UNIFORM, net=None, train=False, noise_seed=0, reuse=False):
+def self_play_continuous(ctx, c_puct, sims, n_games, max_plies=150, evaluator=L.EVAL_UNIFORM, net=None, train=False, noise_seed=0, reuse=False,
+                         gumbel=None):
     """self_play for at least n_games games with every slot of the context kept busy: a slot whose game ends (or hits the ply cap)
     is re-dealt at once (onb_env_reset_games), the way a worker thread of the reference starts its next game as soon as one is over
     (train.rs:218-245 around :44-98). Lockstep self_play instead searches finished slots until the longest game ends -- with game
     lengths between ~10 and 152 plies that wastes most of the work. Only completed games are returned; sample order is ply-major.
     Extra keys: `serial` [m] (slot + n * generation: samples with the same serial belong to one game), `games` (completed games).
     reuse=True keeps the played child's subtree between plies (Context.set_reuse; device evaluators only), as
-    onb_self_play does with the switch on; the switch is left as it was."""
+    onb_self_play does with the switch on; the switch is left as it was.
+    gumbel=True or a dict of Context.set_gumbel keywords: the Gumbel root search with step = ply (set_gumbel(step0=0) at the start, one
+    search per ply), pi = its improved policy, as onb_self_play does with the switch on; the switch is left as it was."""
     if reuse and net is not None:
         raise ValueError("self_play_continuous: reuse=True needs a device evaluator, not a torch net")
     was = getattr(ctx, "reuse", False)
+    gb_was, step_was = getattr(ctx, "gumbel", None), getattr(ctx, "gumbel_step", 0)
     if reuse:
         ctx.set_reuse(False)   # forget trees of earlier searches: every game starts from a fresh tree
         ctx.set_reuse(True)
+    if gumbel:
+        ctx.set_gumbel(True, **dict(dict(gumbel) if isinstance(gumbel, dict) else {}, step0=0))
     try:
         return _self_play_continuous(ctx, c_puct, sims, n_games, max_plies, evaluator, net, train, noise_seed, bool(reuse))
     finally:
         if getattr(ctx, "reuse", False) != was:
             ctx.set_reuse(was)
+        if gumbel:
+            if gb_was is None:
+                ctx.set_gumbel(False)
+            else:
+                m, c_visit, c_scale, scale, seed = gb_was
+                ctx.set_gumbel(True, m, c_visit, c_scale, scale, seed, step0=step_was)  # the setting and its step as they were
 
 
 def _self_play_continuous(ctx, c_puct, sims, n_games, max_plies, evaluator, net, train, noise_seed, reuse):
