@@ -509,6 +509,60 @@ ONB_API int32_t onb_uct_run(onb_ctx* ctx, float exploration_c, uint32_t min_node
 #define ONB_ALPHABETA_MAX_DEPTH 8
 ONB_API int32_t onb_alphabeta_run(onb_ctx* ctx, int32_t depth, onb_action* best_host, int32_t* score_host, uint64_t* nodes_host);
 
+/* ---- endgame tablebases (DESIGN.md §5g; the reference has none, so this definition is the project's own) ---------------------
+ * Position: the four boards, the red hand and the blue hand as unordered pairs of cards, the neutral card and the side to move
+ * (result, flags and the order within a hand are not part of it; that order only changes the generation order of the moves).
+ * Game value, from the side to move's view, with unbounded play (no ply cap). The children of a position are its legal moves in
+ * generation order (hand slot, from, to ascending); a position without a legal move has the two pass children ONB_ACTION_PASS of
+ * its hand slot 0, then slot 1 (as in §5d). A move that captures the enemy king or puts the own king on the enemy temple wins at once.
+ *   +n (n odd): win in n plies (the winning move is ply n; the winner minimises n, the loser maximises it; passes count as plies);
+ *   -n (n even, >= 2): loss in n plies;  0: draw (neither side can force a win);  ONB_TB_NONE: not a position of the table.
+ *   A position is +1 iff it has an immediately winning move; +n iff its smallest child loss is -(n-1); -n iff every child is a win
+ *   and the largest is +(n-1); every other position is a draw. A value that does not fit in int16 makes the solve fail with
+ *   ONB_E_OVERFLOW.
+ * Index (public: part of the ABI). Card set: five distinct ids, s0 < ... < s4 sorted. Card configuration cfg = 6 j + r (0..29):
+ * j = the neutral card's position in the sorted set, r = the colex rank of the red pair among the four remaining cards renumbered
+ * 0..3; the blue hand is the other two. Class (p, q): p red and q blue pawns, p + q <= max_pawns <= ONB_TB_MAX_PAWNS, class id
+ * 5 p + q, E(p, q) = 36 000 C(23, p) C(23 - p, q) entries. With squares n = 5 row + col (a5 = 0), entry
+ *   ((cfg 2 + side) 600 + 24 kr + kb - [kb > kr]) C(23,p) C(23-p,q) + rank_r C(23-p,q) + rank_b,
+ * rank_r = the colex rank of the red pawns' squares among the 23 squares without a king, rank_b = that of the blue pawns' squares
+ * among the 23 - p squares left (a square's position among the free squares is s - popc(occupied below s)). Entries with the red
+ * king on square 2 or the blue king on 22 (47 of the 600 king pairs) are decided positions and hold ONB_TB_NONE.
+ *
+ * onb_tb_solve: solves the classes with p + q <= max_pawns of the set cards5 (any order) on the device, replacing any table the
+ *   context holds; out[5 p + q] receives the per-class counts (solved = 0 for the classes not in the table). Duplicate ids, ids
+ *   above 15 or max_pawns outside 0..4: ONB_E_INVALID; a failed allocation: ONB_E_NOMEM (the message gives the bytes needed).
+ *   Works on a context created with mcts_max_sims = 0. The table stays resident until onb_tb_free, the next solve or onb_destroy.
+ * onb_tb_table: the device table of class (red_pawns, blue_pawns), borrowed, E(p, q) int16 entries.
+ * onb_tb_probe: the value of every game of the context; ONB_TB_NONE for a decided game (result != 0 or State::current_state is a
+ *   win), a game whose five card slots are another set, or whose class is not solved.
+ * onb_tb_best: per game, in generation order of the game's actual slots (passes included), in a win in n the first move that wins
+ *   at once (n = 1) or the first whose child holds -(n-1); in a loss in n the first whose child holds +(n-1); in a draw the first
+ *   whose child holds 0. ONB_ACTION_NONE for a game outside the table. The moves also stay in ONB_BUF_ACTIONS.
+ * Probe, best and the table pointer return ONB_E_STATE when no table is resident.
+ * onb_tb_index (pure host): class and entry of each state; cls = idx = -1 for a state that is no position of the set's classes.
+ * onb_tb_state (pure host): the states of entries of one class, each hand in ascending card order, then the neutral card,
+ *   result = flags = 0; ONB_E_INVALID for an entry out of range.
+ * ONB_AGENT_TABLEBASE in onb_fight plays onb_tb_best in the games in which it is to move (sims and c are ignored). onb_fight checks at
+ * its start that every undecided game is in the table (ONB_E_INVALID otherwise; ONB_E_STATE without a table); a game cannot leave the
+ * table by moving, because material only decreases. */
+#define ONB_TB_MAX_PAWNS 4
+#define ONB_TB_NONE ((int16_t)-32768)
+#define ONB_AGENT_TABLEBASE 5
+typedef struct onb_tb_class {
+    int64_t entries, wins, losses, draws, invalid;
+    int32_t max_win, max_loss;  /* longest win / loss in plies */
+    int32_t iterations, solved; /* solved = 0: class not in the table */
+    int64_t examined;           /* work-list entries examined over all iterations */
+} onb_tb_class;
+ONB_API int32_t onb_tb_solve(onb_ctx* ctx, const uint8_t cards5[5], int32_t max_pawns, onb_tb_class out[25]);
+ONB_API int32_t onb_tb_free(onb_ctx* ctx);
+ONB_API int32_t onb_tb_table(onb_ctx* ctx, int32_t red_pawns, int32_t blue_pawns, int16_t** dev_ptr, int64_t* entries);
+ONB_API int32_t onb_tb_probe(onb_ctx* ctx, int16_t* values_host); /* [n] */
+ONB_API int32_t onb_tb_best(onb_ctx* ctx, onb_action* best_host); /* [n], also left in ONB_BUF_ACTIONS */
+ONB_API int32_t onb_tb_index(const uint8_t cards5[5], const onb_state* s, int64_t n, int32_t* cls, int64_t* idx);
+ONB_API int32_t onb_tb_state(const uint8_t cards5[5], int32_t cls, const int64_t* idx, int64_t n, onb_state* out);
+
 /* ---- policy/value network on the device ---------------------------------------------------------------------
  * ConvResNet::forward (alphazero-training/src/net.rs:215-232) for every position of a plane buffer, as one fused
  * tensor-core kernel (BatchNorm in eval mode folded into the convolutions; f32 accumulation; heads in f32). Arithmetic of the

@@ -378,6 +378,37 @@ struct AlphaBeta : Agent {
     uint64_t id() const override { return (uint64_t)depth; }
 };
 
+/// The perfect endgame agent (onb_tb_solve / onb_tb_best, DESIGN.md §5g): plays the tablebase's move for one five-card set with at
+/// most max_pawns pawns. The table is solved on first use on a one-game context of the agent's own (copies share it). generate_move
+/// returns the move and the position's value (+n: win in n plies, -n: loss in n plies, 0: draw); it refuses a decided position and
+/// one outside the table. A position without a legal move is answered with a pass, which DoneMove cannot carry: refused as well.
+struct Tablebase : Agent {
+    std::array<uint8_t, 5> cards;
+    int32_t max_pawns = 3;
+    explicit Tablebase(std::array<uint8_t, 5> cards_, int32_t max_pawns_ = 3) : cards(cards_), max_pawns(max_pawns_) {}
+    std::pair<DoneMove, double> generate_move(const GameState& gs) override {
+        if (!engine) {
+            auto e = std::make_shared<Engine>(1, 0, 0, 0, false);
+            e->check(onb_tb_solve(e->ctx(), cards.data(), max_pawns, nullptr));
+            engine = e;
+        }
+        onb_state o = gs.state.to_onb(gs.curr_player_color);
+        engine->check(onb_env_set_states(engine->ctx(), &o, 0, 1));
+        int16_t value = 0;
+        onb_action best = 0;
+        engine->check(onb_tb_probe(engine->ctx(), &value));
+        engine->check(onb_tb_best(engine->ctx(), &best));
+        if (best == ONB_ACTION_NONE) throw Error(ONB_E_STATE, "Tablebase: the game is decided or not a position of the table");
+        if (best & (1u << 13)) throw Error(ONB_E_STATE, "Tablebase: no legal move (the table's answer is a pass)");
+        return {from_action(best), (double)value};
+    }
+    const char* name() const override { return "Tablebase AI"; }
+    std::unique_ptr<Agent> clone_dyn() const override { return std::make_unique<Tablebase>(*this); }
+    uint64_t id() const override { return (uint64_t)max_pawns; }
+private:
+    std::shared_ptr<Engine> engine;
+};
+
 struct AlphaZeroMctsConfig {  // alphazero_mcts/mod.rs:26-43
     double search_time_ms = 400.;  // ignored: the search always runs max_playouts simulations
     double exploration_c = 1.4142135623730951;

@@ -111,6 +111,13 @@ SYMBOLS = {
     "onb_replay_indices": (C.c_int32, [C.c_int64, C.c_int64, C.c_uint64, _P]),
     "onb_uct_run": (C.c_int32, [_P, C.c_float, C.c_uint32, C.c_uint32]),
     "onb_alphabeta_run": (C.c_int32, [_P, C.c_int32, _P, _P, _P]),
+    "onb_tb_solve": (C.c_int32, [_P, _P, C.c_int32, _P]),
+    "onb_tb_free": (C.c_int32, [_P]),
+    "onb_tb_table": (C.c_int32, [_P, C.c_int32, C.c_int32, C.POINTER(_P), C.POINTER(C.c_int64)]),
+    "onb_tb_probe": (C.c_int32, [_P, _P]),
+    "onb_tb_best": (C.c_int32, [_P, _P]),
+    "onb_tb_index": (C.c_int32, [_P, _P, C.c_int64, _P, _P]),
+    "onb_tb_state": (C.c_int32, [_P, C.c_int32, _P, C.c_int64, _P]),
     "onb_net_precision": (C.c_int32, [_P, C.c_int32]),
     "onb_net_select": (C.c_int32, [_P, C.c_int32]),
     "onb_net_load": (C.c_int32, [_P, C.c_int32, _P, _P, _P]),
@@ -122,9 +129,17 @@ class SelfPlayConfig(C.Structure):
                 ("train", C.c_int32), ("noise_seed", C.c_uint64), ("sample_cap", C.c_int64)]
 
 
-AGENT_RANDOM, AGENT_PUCT, AGENT_UCT, AGENT_ALPHABETA, AGENT_GUMBEL = 0, 1, 2, 3, 4
+AGENT_RANDOM, AGENT_PUCT, AGENT_UCT, AGENT_ALPHABETA, AGENT_GUMBEL, AGENT_TABLEBASE = 0, 1, 2, 3, 4, 5
 ALPHABETA_MAX_DEPTH = 8
 ALPHABETA_WIN = 1000000
+TB_MAX_PAWNS = 4
+TB_NONE = -32768
+
+
+class TbClass(C.Structure):
+    """onb_tb_class (onb_tb_solve): per-class counts of a solved tablebase"""
+    _fields_ = [("entries", C.c_int64), ("wins", C.c_int64), ("losses", C.c_int64), ("draws", C.c_int64), ("invalid", C.c_int64),
+                ("max_win", C.c_int32), ("max_loss", C.c_int32), ("iterations", C.c_int32), ("solved", C.c_int32), ("examined", C.c_int64)]
 
 
 class GumbelConfig(C.Structure):

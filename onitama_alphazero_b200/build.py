@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libonb.so")
-SOURCES = ["onb_api.cu", "onb_env.cu", "onb_perft.cu", "onb_mcts.cu", "onb_net.cu", "onb_selfplay.cu", "onb_actor.cu", "onb_comm.cu", "onb_replay.cu", "onb_alphabeta.cu", "onb_reuse.cu"]
+SOURCES = ["onb_api.cu", "onb_env.cu", "onb_perft.cu", "onb_mcts.cu", "onb_net.cu", "onb_selfplay.cu", "onb_actor.cu", "onb_comm.cu", "onb_replay.cu", "onb_alphabeta.cu", "onb_reuse.cu", "onb_tablebase.cu"]
 HEADERS = ["onb_rules.cuh", "onb_internal.h", "onb_gumbel.cuh", os.path.join("..", "..", "include", "onb.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC",
               "-Xcompiler", "-fvisibility=hidden", "--fmad=false", "-Xptxas", "-v"]

@@ -148,8 +148,9 @@ int32_t onb_destroy(onb_ctx* ctx) {
                     c->d_tree_size, c->d_tree_flags, c->d_roots, c->d_leaf_node, c->d_leaf_state, c->d_leaf_planes, c->d_policy, c->d_value,
                     c->d_pi, c->d_best, c->d_root_visits, c->d_root_q, c->d_child_visits, c->net[0].w, c->net[0].bias, c->net[0].head, c->net[1].w,
                     c->net[1].bias, c->net[1].head, c->d_ln_table, c->d_net_scratch, c->d_ab_score, c->d_ab_nodes, c->d_gb,
-                    c->d_gb_tab, c->d_gb_base, c->d_gb_p, c->d_gb_r0};
+                    c->d_gb_tab, c->d_gb_base, c->d_gb_p, c->d_gb_r0, c->d_tb_values};
     reuse_free(c);
+    tb_free(c);
     for (void* p : c->sp_buf)
         if (p) cudaFree(p);
     for (void* p : ptrs)
@@ -776,6 +777,10 @@ static int32_t fight_move(Ctx* c, const onb_agent* ag, uint32_t ply, const int32
         ONB_CUDA(c, launch_alphabeta(c, (int)ag->sims, d_games, m, d_out, nullptr, nullptr));
         return ONB_OK;
     }
+    if (ag->kind == ONB_AGENT_TABLEBASE) {
+        ONB_CUDA(c, launch_tb_best(c, d_games, m, d_out));
+        return ONB_OK;
+    }
     c->gb_on = 0;  // PUCT and UCT agents search without the Gumbel root step
     if (ag->kind == ONB_AGENT_GUMBEL) {
         c->gb_on = 1;
@@ -807,8 +812,12 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
     if (!a || !b || !a_is_red_host || !out) return fail(c, ONB_E_INVALID, "onb_fight: null argument");
     for (const onb_agent* ag : {a, b}) {
         if (ag->kind != ONB_AGENT_RANDOM && ag->kind != ONB_AGENT_PUCT && ag->kind != ONB_AGENT_UCT && ag->kind != ONB_AGENT_ALPHABETA &&
-            ag->kind != ONB_AGENT_GUMBEL)
+            ag->kind != ONB_AGENT_GUMBEL && ag->kind != ONB_AGENT_TABLEBASE)
             return fail(c, ONB_E_INVALID, "onb_fight: unknown agent kind %d", ag->kind);
+        if (ag->kind == ONB_AGENT_TABLEBASE) {
+            if (!c->tb_live) return fail(c, ONB_E_STATE, "onb_fight: a tablebase agent needs a solved table (onb_tb_solve)");
+            continue;
+        }
         if (ag->kind == ONB_AGENT_GUMBEL && (ag->min_node_visits > 40 || !std::isfinite(ag->c) || !(ag->c >= 0.0)))
             return fail(c, ONB_E_INVALID, "onb_fight: a Gumbel agent needs min_node_visits (m) <= 40 and a finite c (c_scale) >= 0");
         if (ag->kind == ONB_AGENT_ALPHABETA) {
@@ -818,6 +827,19 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
         }
         if (ag->kind != ONB_AGENT_RANDOM && (!c->d_nodes || ag->sims == 0 || ag->sims > c->cfg.mcts_max_sims))
             return fail(c, ONB_E_INVALID, "onb_fight: a searching agent needs 1 <= sims <= mcts_max_sims");
+    }
+    if (a->kind == ONB_AGENT_TABLEBASE || b->kind == ONB_AGENT_TABLEBASE) {  // games stay in the table once they start in it
+        unsigned long long* d_missing = nullptr;
+        unsigned long long missing = 0;
+        ONB_CUDA(c, dalloc(&d_missing, 1));
+        cudaError_t e = cudaMemsetAsync(d_missing, 0, 8, c->stream);
+        if (e == cudaSuccess) e = launch_tb_probe(c, nullptr, d_missing);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(&missing, d_missing, 8, cudaMemcpyDeviceToHost, c->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+        cudaFree(d_missing);
+        ONB_CUDA(c, e);
+        if (missing)
+            return fail(c, ONB_E_INVALID, "onb_fight: %llu undecided games are not positions of the tablebase (card set or material)", missing);
     }
     memset(out, 0, sizeof(*out));
     int32_t rc = onb_mcts_set_noise(ctx, 0, 0.25, 0.03, 0);  // arenas search in eval mode (AlphaZeroMcts, not TrainingAlphaZeroMcts)
@@ -907,6 +929,56 @@ int32_t onb_alphabeta_run(onb_ctx* ctx, int32_t depth, onb_action* best_host, in
     if (score_host) ONB_CUDA(c, cudaMemcpyAsync(score_host, c->d_ab_score, n * 4, cudaMemcpyDeviceToHost, c->stream));
     if (nodes_host) ONB_CUDA(c, cudaMemcpyAsync(nodes_host, c->d_ab_nodes, n * 8, cudaMemcpyDeviceToHost, c->stream));
     if (best_host || score_host || nodes_host) ONB_CUDA(c, cudaStreamSynchronize(c->stream));
+    return ONB_OK;
+}
+int32_t onb_tb_solve(onb_ctx* ctx, const uint8_t cards5[5], int32_t max_pawns, onb_tb_class out[25]) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    char err[400];
+    err[0] = 0;
+    const int32_t rc = tb_solve(c, cards5, max_pawns, out, err, sizeof(err));
+    if (rc != ONB_OK) return fail(c, rc, "%s", err);
+    return ONB_OK;
+}
+int32_t onb_tb_free(onb_ctx* ctx) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    ONB_CUDA(c, cudaStreamSynchronize(c->stream));
+    tb_free(c);
+    return ONB_OK;
+}
+int32_t onb_tb_table(onb_ctx* ctx, int32_t red_pawns, int32_t blue_pawns, int16_t** dev_ptr, int64_t* entries) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (!c->tb_live) return fail(c, ONB_E_STATE, "onb_tb_table: no tablebase is resident (onb_tb_solve)");
+    if (!dev_ptr || red_pawns < 0 || blue_pawns < 0 || red_pawns + blue_pawns > c->tb_max_pawns)
+        return fail(c, ONB_E_INVALID, "onb_tb_table: class (%d,%d) is not in the table (max_pawns %d)", red_pawns, blue_pawns, c->tb_max_pawns);
+    const int k = 5 * red_pawns + blue_pawns;
+    *dev_ptr = c->d_tb + c->tb_off[k];
+    if (entries) *entries = c->tb_len[k];
+    return ONB_OK;
+}
+int32_t onb_tb_probe(onb_ctx* ctx, int16_t* values_host) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (!c->tb_live) return fail(c, ONB_E_STATE, "onb_tb_probe: no tablebase is resident (onb_tb_solve)");
+    if (!values_host) return fail(c, ONB_E_INVALID, "onb_tb_probe: null output");
+    const size_t n = (size_t)c->n;
+    if (!c->d_tb_values) ONB_CUDA(c, dalloc(&c->d_tb_values, n));
+    ONB_CUDA(c, launch_tb_probe(c, c->d_tb_values, nullptr));
+    ONB_CUDA(c, cudaMemcpyAsync(values_host, c->d_tb_values, n * 2, cudaMemcpyDeviceToHost, c->stream));
+    ONB_CUDA(c, cudaStreamSynchronize(c->stream));
+    return ONB_OK;
+}
+int32_t onb_tb_best(onb_ctx* ctx, onb_action* best_host) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (!c->tb_live) return fail(c, ONB_E_STATE, "onb_tb_best: no tablebase is resident (onb_tb_solve)");
+    ONB_CUDA(c, launch_tb_best(c, nullptr, c->n, c->d_actions));
+    if (best_host) {
+        ONB_CUDA(c, cudaMemcpyAsync(best_host, c->d_actions, (size_t)c->n * 2, cudaMemcpyDeviceToHost, c->stream));
+        ONB_CUDA(c, cudaStreamSynchronize(c->stream));
+    }
     return ONB_OK;
 }
 int32_t onb_mcts_finish(onb_ctx* ctx, onb_action* best_host, float* pi_host, uint32_t* root_visits_host, double* root_q_host, uint32_t* child_visits_host) {

@@ -139,6 +139,13 @@ struct Ctx {
     double* d_gb_p;
     double* d_gb_r0;
     uint32_t gb_tab_m, gb_tab_n;  // the table d_gb_tab holds (gb_tab_m = 0: none)
+    // endgame tablebase (onb_tablebase.cu, onb_tb_solve)
+    int16_t* d_tb;            // every solved class, class 5 p + q at d_tb + tb_off[5 p + q]
+    int64_t tb_off[25], tb_len[25];  // tb_len = 0: class not in the table
+    uint32_t tb_setmask;      // bit id set for the five cards of the set
+    int32_t tb_max_pawns;
+    int tb_live;              // a solved table is resident
+    int16_t* d_tb_values;     // [n] onb_tb_probe's output (allocated on first use)
     char err[512];
 };
 
@@ -178,6 +185,14 @@ cudaError_t launch_net_forward(Ctx* c, const float* planes, float* policy, float
 // alpha-beta agent (onb_alphabeta.cu): searches games d_games[0 .. m) (nullptr: games 0 .. m) to `depth` plies; d_out[game] = the best
 // action (ONB_ACTION_NONE for a decided game), d_score / d_nodes [game] (optional) = root score and positions entered
 cudaError_t launch_alphabeta(Ctx* c, int depth, const int32_t* d_games, int64_t m, uint16_t* d_out, int32_t* d_score, unsigned long long* d_nodes);
+
+// endgame tablebase (onb_tablebase.cu)
+int32_t tb_solve(Ctx* c, const uint8_t cards5[5], int32_t max_pawns, onb_tb_class out[25], char* err, size_t err_len);
+void tb_free(Ctx* c);
+// values [n] of every game (optional) and the number of undecided games outside the table (optional, accumulated)
+cudaError_t launch_tb_probe(Ctx* c, int16_t* d_values, unsigned long long* d_missing);
+// d_out[game] = onb_tb_best's move for the games d_games[0 .. m) (nullptr: games 0 .. m)
+cudaError_t launch_tb_best(Ctx* c, const int32_t* d_games, int64_t m, uint16_t* d_out);
 
 // tree reuse (onb_reuse.cu)
 cudaError_t reuse_alloc(Ctx* c);

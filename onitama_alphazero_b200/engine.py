@@ -295,6 +295,12 @@ class Context:
         """the `AlphaBeta` agent: fixed-depth alpha-beta search to `depth` plies (1 .. 8), see Context.alphabeta"""
         return L.Agent(L.AGENT_ALPHABETA, 0, 0, depth, 0.0, 0, 0)
 
+    @staticmethod
+    def agent_tablebase():
+        """the perfect endgame agent: plays Context.tb_best in the games in which it is to move (needs a solved table that holds every
+        undecided game)"""
+        return L.Agent(L.AGENT_TABLEBASE, 0, 0, 0, 0.0, 0, 0)
+
     def fight_native(self, agent_a, agent_b, a_is_red, max_plies=150):
         """onb_fight: the arena loop inside the library. Returns (a_wins, b_wins, draws, per-game results [n] uint8)."""
         mask = np.ascontiguousarray(np.asarray(a_is_red), dtype=np.uint8)
@@ -337,6 +343,38 @@ class Context:
             return None
         out = dict(best=np.zeros(self.n, np.uint16), score=np.zeros(self.n, np.int32), nodes=np.zeros(self.n, np.uint64))
         self._ck(self._lib.onb_alphabeta_run(self._h, depth, L.ptr(out["best"]), L.ptr(out["score"]), L.ptr(out["nodes"])))
+        return out
+
+    # ------------------------------------------------------------------ endgame tablebase (DESIGN.md §5g)
+    def tb_solve(self, cards, max_pawns=3):
+        """onb_tb_solve: solves every class with p + q <= max_pawns of the five-card set `cards` on the device; the table stays in the
+        context. Returns {(p, q): dict(entries, wins, losses, draws, invalid, max_win, max_loss, iterations, examined)}."""
+        c = np.ascontiguousarray(cards, dtype=np.uint8).reshape(5)
+        out = (L.TbClass * 25)()
+        self._ck(self._lib.onb_tb_solve(self._h, L.ptr(c), int(max_pawns), out))
+        return {(k // 5, k % 5): {f: int(getattr(out[k], f)) for f, _ in L.TbClass._fields_ if f != "solved"}
+                for k in range(25) if out[k].solved}
+
+    def tb_free(self):
+        self._ck(self._lib.onb_tb_free(self._h))
+
+    def tb_table(self, p, q):
+        """zero-copy torch int16 view of the solved class (p, q) on the device (valid until the next solve / tb_free)"""
+        import torch
+        ptr, n = C.c_void_p(), C.c_int64()
+        self._ck(self._lib.onb_tb_table(self._h, int(p), int(q), C.byref(ptr), C.byref(n)))
+        return torch.as_tensor(_DevBuf(ptr.value, (n.value,), "<i2"), device="cuda:%d" % self.device)
+
+    def tb_probe(self):
+        """onb_tb_probe: the game value of every game [n] np.int16 (TB_NONE outside the table)"""
+        out = np.zeros(self.n, dtype=np.int16)
+        self._ck(self._lib.onb_tb_probe(self._h, L.ptr(out)))
+        return out
+
+    def tb_best(self, to_host=True):
+        """onb_tb_best: the table's move for every game (ACTION_NONE outside it); the moves also stay in BUF_ACTIONS"""
+        out = np.zeros(self.n, dtype=np.uint16) if to_host else None
+        self._ck(self._lib.onb_tb_best(self._h, L.ptr(out)))
         return out
 
     def mcts_finish(self, to_host=True, out=None):
@@ -557,6 +595,28 @@ def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_g
 
 
 Context.search_device = _search_device
+
+
+def tb_index(cards, states):
+    """onb_tb_index: (class id 5 p + q, entry) of each state for the card set `cards`; -1, -1 for states outside the classes"""
+    c = np.ascontiguousarray(cards, dtype=np.uint8).reshape(5)
+    s = np.ascontiguousarray(states, dtype=STATE_DTYPE).reshape(-1)
+    cls, idx = np.zeros(len(s), np.int32), np.zeros(len(s), np.int64)
+    rc = L.load().onb_tb_index(L.ptr(c), L.ptr(s), len(s), L.ptr(cls), L.ptr(idx))
+    if rc != 0:
+        raise OnbError(rc, "onb_tb_index: invalid card set")
+    return cls, idx
+
+
+def tb_states(cards, cls, idx):
+    """onb_tb_state: the states of entries idx of class cls (hands in ascending card order, then the neutral card)"""
+    c = np.ascontiguousarray(cards, dtype=np.uint8).reshape(5)
+    i = np.ascontiguousarray(idx, dtype=np.int64).reshape(-1)
+    out = np.zeros(len(i), dtype=STATE_DTYPE)
+    rc = L.load().onb_tb_state(L.ptr(c), int(cls), L.ptr(i), len(i), L.ptr(out))
+    if rc != 0:
+        raise OnbError(rc, "onb_tb_state: invalid card set, class or entry")
+    return out
 
 
 def start_states(decks):

@@ -11,8 +11,8 @@ TMAP = {'int32_t': 'i32', 'uint32_t': 'u32', 'int64_t': 'i64', 'uint64_t': 'u64'
         'onb_state': 'onb_state', 'onb_tree_dump': 'onb_tree_dump', 'onb_selfplay_config': 'onb_selfplay_config',
         'onb_selfplay_result': 'onb_selfplay_result', 'onb_agent': 'onb_agent', 'onb_fight_result': 'onb_fight_result',
         'onb_actor': 'onb_actor', 'onb_actor_view': 'onb_actor_view', 'onb_fight_statistics': 'onb_fight_statistics', 'onb_comm': 'onb_comm', 'onb_replay': 'onb_replay',
-        'onb_gumbel_config': 'onb_gumbel_config'}
-I32_PREFIXES = ('ONB_E_', 'ONB_BUF', 'ONB_STAT', 'ONB_RESULT', 'ONB_POLICY', 'ONB_EVAL', 'ONB_AGENT', 'ONB_NET_', 'ONB_SELFTEST', 'ONB_ALPHABETA')
+        'onb_gumbel_config': 'onb_gumbel_config', 'int16_t': 'i16', 'onb_tb_class': 'onb_tb_class'}
+I32_PREFIXES = ('ONB_E_', 'ONB_BUF', 'ONB_STAT', 'ONB_RESULT', 'ONB_POLICY', 'ONB_EVAL', 'ONB_AGENT', 'ONB_NET_', 'ONB_SELFTEST', 'ONB_ALPHABETA', 'ONB_TB_MAX')
 I32_NAMES = ('ONB_VERSION', 'ONB_OK', 'ONB_RED', 'ONB_BLUE', 'ONB_PAWN', 'ONB_KING')
 STRUCTS = '''#[repr(C)]
 pub struct onb_ctx { _private: [u8; 0] }
@@ -93,6 +93,21 @@ pub struct onb_gumbel_config {
     pub seed: u64,
     pub step0: u32,
     pub reserved: u32,
+}
+
+#[repr(C)]
+#[derive(Clone, Copy, Default, Debug)]
+pub struct onb_tb_class {
+    pub entries: i64,
+    pub wins: i64,
+    pub losses: i64,
+    pub draws: i64,
+    pub invalid: i64,
+    pub max_win: i32,
+    pub max_loss: i32,
+    pub iterations: i32,
+    pub solved: i32,
+    pub examined: i64,
 }
 
 #[repr(C)]
@@ -190,7 +205,7 @@ def main():
             lines.append("pub const %s: i32 = %s;" % (k, v))
         elif k.startswith(('ONB_OUT', 'ONB_HOST')):
             lines.append("pub const %s: u32 = %s;" % (k, v))
-    lines += ['pub const ONB_ACTION_NONE: u16 = 0xFFFF;', '',
+    lines += ['pub const ONB_ACTION_NONE: u16 = 0xFFFF;', 'pub const ONB_TB_NONE: i16 = -32768;', '',
               '/// action code: to | from << 5 | used_card_idx << 10 | piece << 12 | pass << 13',
               'pub const fn onb_action(card_idx: u16, from: u16, to: u16, piece: u16) -> u16 { to | (from << 5) | (card_idx << 10) | (piece << 12) }',
               'pub const fn onb_action_pass(card_idx: u16) -> u16 { (card_idx << 10) | (1 << 13) }', '', STRUCTS,
