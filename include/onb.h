@@ -306,9 +306,8 @@ ONB_API int32_t onb_mcts_reuse_stats(onb_ctx* ctx, uint64_t out[4], int32_t clea
  * step: onb_mcts_begin uses a serial that this call sets to step0 and every Gumbel begin increments; onb_self_play uses step = ply,
  * onb_fight step = ply for ONB_AGENT_GUMBEL agents (both leave the serial as they found it).
  * Checks: 1 <= max_considered <= 40, finite c_visit, c_scale, gumbel_scale >= 0, else ONB_E_INVALID. cfg NULL or enabled = 0: off.
- * Refused with ONB_E_STATE at onb_mcts_begin: Gumbel together with tree reuse or train-mode noise, and with the exploration knobs
- * ONB_MCTS_WARP_PER_TREE / ONB_MCTS_STEP_FUSION / ONB_MCTS_ROOT_SMEM; after a Gumbel begin: onb_uct_run and more simulations than the
- * begin's sims. onb_self_play while Gumbel is on: ONB_E_STATE with tree reuse on, ONB_E_INVALID with train != 0. onb_fight searches
+ * Refused with ONB_E_STATE at onb_mcts_begin: Gumbel together with tree reuse or train-mode noise; after a Gumbel begin: onb_uct_run
+ * and more simulations than the begin's sims. onb_self_play while Gumbel is on: ONB_E_STATE with tree reuse on, ONB_E_INVALID with train != 0. onb_fight searches
  * without reuse, so its Gumbel agents play whatever the reuse switch says. Every begin decides anew: a search begun with the switch
  * off is a PUCT search. The caller-driven split phase is supported.
  * Memory: the first enabling call allocates n_games * 1 KB of per-tree root data and a 40 x mcts_max_sims table. */

@@ -147,7 +147,7 @@ int32_t onb_destroy(onb_ctx* ctx) {
     void* ptrs[] = {c->d_states, c->d_masks, c->d_planes, c->d_actions, c->d_stats, c->d_io_states, c->d_moves, c->d_counts, c->d_nodes,
                     c->d_tree_size, c->d_tree_flags, c->d_roots, c->d_leaf_node, c->d_leaf_state, c->d_leaf_planes, c->d_policy, c->d_value,
                     c->d_pi, c->d_best, c->d_root_visits, c->d_root_q, c->d_child_visits, c->net[0].w, c->net[0].bias, c->net[0].head, c->net[1].w,
-                    c->net[1].bias, c->net[1].head, c->d_ln_table, c->d_net_scratch, c->d_ab_score, c->d_ab_nodes, c->d_gb,
+                    c->net[1].bias, c->net[1].head, c->d_ln_table, c->d_ab_score, c->d_ab_nodes, c->d_gb,
                     c->d_gb_tab, c->d_gb_base, c->d_gb_p, c->d_gb_r0, c->d_tb_values};
     reuse_free(c);
     tb_free(c);
@@ -450,11 +450,6 @@ int32_t onb_perft(onb_ctx* ctx, const onb_state* roots_host, int64_t n, int32_t 
 // ---------------------------------------------------------------------------------------------- mcts
 }  // extern "C"
 namespace onb {
-static bool knob_set(const char* name, bool numeric) {
-    const char* v = getenv(name);
-    if (!v) return false;
-    return numeric ? atoi(v) != 0 : v[0] == '1';
-}
 // the combinations a Gumbel search does not support (include/onb.h, onb_mcts_set_gumbel); reuse: this begin keeps remembered trees
 // (onb_fight never does, whatever the context's reuse switch says). Every begin clears gb_search first, so a search begun after the
 // switch went off, or a refused begin, never runs the Gumbel kernels.
@@ -463,9 +458,6 @@ static int32_t gumbel_refusals(Ctx* c, const char* what, bool reuse) {
     if (!c->gb_on) return ONB_OK;
     if (reuse) return fail(c, ONB_E_STATE, "%s: the Gumbel root search does not combine with tree reuse (onb_mcts_set_reuse)", what);
     if (c->noise_on) return fail(c, ONB_E_STATE, "%s: the Gumbel root search does not combine with train-mode noise (onb_mcts_set_noise)", what);
-    if (knob_set("ONB_MCTS_WARP_PER_TREE", false) || knob_set("ONB_MCTS_STEP_FUSION", false) || knob_set("ONB_MCTS_ROOT_SMEM", true))
-        return fail(c, ONB_E_STATE, "%s: the Gumbel root search does not run with the exploration knobs ONB_MCTS_WARP_PER_TREE / "
-                                    "ONB_MCTS_STEP_FUSION / ONB_MCTS_ROOT_SMEM", what);
     return ONB_OK;
 }
 // after the trees are begun: the search's GumbelDev (step = the serial, which advances) and, when (m, sims) changed, the table
@@ -668,24 +660,14 @@ int32_t onb_mcts_run(onb_ctx* ctx, int32_t evaluator, uint32_t sims) {
     if (c->gb_search && c->sims_done + sims > c->sims_target)
         return fail(c, ONB_E_STATE, "onb_mcts_run: a Gumbel search runs at most the begin's %u simulations", c->sims_target);
     if (evaluator == ONB_EVAL_NET) {
-        // the network sits between select and expand: three launches per simulation round, all on the context's stream.
-        // ONB_MCTS_STEP_FUSION=1 (exploration knob): expand_backup(s) and select(s + 1) as ONE launch (k_mcts_step_g) -- measured SLOWER
-        // on B200 (config 5, f16 network: 304.8 vs 293.9 ms per ply): the fused kernel carries both halves' shared tables (36.6 KB, one
-        // CTA fewer per SM) and a block barrier between them, which costs more than the saved launch boundary
+        // the network sits between select and expand: three launches per simulation round, all on the context's stream
+        // (one launch for expand_backup(s) + select(s + 1) was measured slower, DESIGN.md section 8)
         if (!c->net[c->net_cur].loaded) return fail(c, ONB_E_STATE, "onb_mcts_run: no network loaded (onb_net_load)");
-        const char* fuse_env = getenv("ONB_MCTS_STEP_FUSION");
-        const bool fuse = fuse_env && fuse_env[0] == '1';
         if (sims > 0) ONB_CUDA(c, launch_mcts_select(c));
         for (uint32_t s = 0; s < sims; ++s) {
             ONB_CUDA(c, launch_net_forward(c, c->d_leaf_planes, c->d_policy, c->d_value, trees(c)));
-            if (s + 1 == sims) {
-                ONB_CUDA(c, launch_mcts_expand_backup(c));
-            } else if (fuse) {
-                ONB_CUDA(c, launch_mcts_step(c));
-            } else {
-                ONB_CUDA(c, launch_mcts_expand_backup(c));
-                ONB_CUDA(c, launch_mcts_select(c));
-            }
+            ONB_CUDA(c, launch_mcts_expand_backup(c));
+            if (s + 1 < sims) ONB_CUDA(c, launch_mcts_select(c));
         }
         c->sims_done += sims;
         return ONB_OK;

@@ -96,8 +96,6 @@ struct Ctx {
     void* sp_buf[32];          // grow-only buffers of onb_self_play (slots 0-15) and onb_fight (16-31), see onb_selfplay.cu
     size_t sp_cap[32];
     int fight_valid;           // an onb_fight has left its per-game results on the device (onb_fight_statistics)
-    void* d_net_scratch;       // residual scratch of the three-CTAs-per-SM network kernel
-    size_t net_scratch_bytes;
     int net_cur;      // slot used by onb_net_load / onb_net_forward / ONB_EVAL_NET (onb_net_select)
     int net_tf32;     // requested arithmetic for the next onb_net_load: ONB_NET_F16 (default) | ONB_NET_TF32 | ONB_NET_F32
     // grow-only device scratch reused across onb_perft calls (counters, cursor, two ping-pong frontiers): repeated
@@ -169,7 +167,6 @@ cudaError_t launch_selftest_div(Ctx* c, unsigned long long* d_mismatches);
 cudaError_t launch_mcts_begin(Ctx* c);
 cudaError_t launch_mcts_select(Ctx* c);
 cudaError_t launch_mcts_expand_backup(Ctx* c);
-cudaError_t launch_mcts_step(Ctx* c);  // expand_backup of this simulation + select of the next one, one launch
 cudaError_t launch_mcts_eval(Ctx* c, int evaluator);
 cudaError_t launch_mcts_run(Ctx* c, int evaluator, uint32_t sims);
 cudaError_t launch_uct_run(Ctx* c, float exploration_c, uint32_t min_node_visits, uint32_t sims);

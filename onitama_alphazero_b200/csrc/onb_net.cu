@@ -13,7 +13,7 @@
 // but a ROW SHIFT of the activation matrix by dy*6+dx cells. The activations live in shared memory in the tensor core's K-major
 // operand layout, one 128-byte swizzled row per cell: a shifted window is just a different start address in the shared-memory
 // descriptor -- no im2col copy is ever made.
-// One CTA keeps NB boards (NACC accumulators of 128 cells x 64 channels in TMEM) on chip through ALL layers; only the input planes
+// One CTA keeps NB boards (two accumulators of 128 cells x 64 channels in TMEM) on chip through ALL layers; only the input planes
 // are read from and only policy/value are written to global memory. The residual input of a block is parked in TMEM (pre-loaded
 // into the accumulator of the block's second convolution together with that layer's bias), so the skip connection costs nothing.
 // Weights (rounded, BN folded, already in the swizzled operand layout) are streamed through a small ring by one producer thread
@@ -61,19 +61,20 @@ constexpr int kHP0 = 0, kHP1 = 64, kHV = 128, kHB = 192, kPhW = 196, kPhB = 2696
 // (22+ significand bits; the scaling keeps x2 in f16's normal range however small x is). A product a b is then
 // a1 b1 + 2^-11 (a1 b2 + a2 b1) up to 2^-23 relative: three MMAs per step, the first into accumulator D1, the other two into a
 // second accumulator D2 that the epilogue adds as D1 + 2^-11 D2. Two activation matrices (a1, a2), weights streamed as (b1, b2)
-// pairs per tap, TMEM = {D1, D2} x {plain, residual-preloaded} x NACC x 64 columns = 512: one CTA per SM.
+// pairs per tap, TMEM = {D1, D2} x {plain, residual-preloaded} x 2 x 64 columns = 512: one CTA per SM.
 constexpr float kX3Scale = 2048.f, kX3InvScale = 1.f / 2048.f;
-template <int NACC, bool F16, bool X3 = false>
+template <bool F16, bool X3 = false>
 struct Geo {
-    static_assert(!X3 || (F16 && NACC == 2), "the split-operand mode is built on the f16 operand path with two accumulators");
-    static constexpr int NMAT = X3 ? 2 : 1;                    // activation matrices / weight copies per tap
-    static constexpr int NB = NACC == 2 ? (F16 ? 7 : 6) : 14;  // boards per pass (two CTAs per SM when NACC == 2)
+    static_assert(!X3 || F16, "the split-operand mode is built on the f16 operand path");
+    static constexpr int NACC = 2;           // accumulators of 128 cells
+    static constexpr int NMAT = X3 ? 2 : 1;  // activation matrices / weight copies per tap
+    static constexpr int NB = F16 ? 7 : 6;   // boards per pass (two CTAs per SM)
     static constexpr int CELLS = NB * kCellsPerBoard;
     static constexpr int R = (kLead + CELLS + kTrail + 7) / 8 * 8;  // rows of the activation matrix (whole swizzle periods)
     // weight ring: NSLOT slots of TPS taps, one full/empty barrier round trip and one bulk copy per slot. f16: 3 slots x 3 taps =
     // one whole layer in flight, so the producer runs a layer ahead of the MMAs (with 4 single-tap slots the MMA thread waited for
     // weights, and per-tap slots cost a try_wait + fence + commit for every 8 MMAs); tf32 taps are twice as large: single taps
-    static constexpr int NSLOT = F16 ? 3 : (NACC == 2 ? 3 : 4);
+    static constexpr int NSLOT = 3;
     static constexpr int TPS = F16 ? 3 : 1;
     static constexpr int UPL = 9 / TPS;  // slots per layer
     static constexpr int TAP_STRIDE = NMAT * Op<F16>::TAP_BYTES;  // X3: [b1 tap][b2 tap]
@@ -86,7 +87,7 @@ struct Geo {
     static constexpr int OFF_BAR = OFF_HEAD + HEAD_BYTES;
     static constexpr int SMEM_USED = OFF_BAR + (2 * NSLOT + 1) * 8 + 16;
     // TMEM holds two CTAs of 256 columns: ask for enough shared memory that a third CTA can never become resident and block in tcgen05.alloc
-    static constexpr int SMEM = NACC == 2 && SMEM_USED < 78 * 1024 ? 78 * 1024 : SMEM_USED;
+    static constexpr int SMEM = SMEM_USED < 78 * 1024 ? 78 * 1024 : SMEM_USED;
     static constexpr int SET_COLS = NMAT * NACC * 64;  // one accumulator set: D1 (and D2) of NACC x 64 columns
     static constexpr int TMEM_COLS = 2 * SET_COLS;     // the plain set + the residual-preloaded set
     static_assert(SMEM_USED <= 227 * 1024, "shared memory");
@@ -229,13 +230,13 @@ __device__ __forceinline__ void mma_lo(uint32_t d_tmem, uint32_t a_lo, uint32_t 
             "r"(a_lo), "r"(b_lo), "r"(hi), "r"(idesc), "r"(accumulate)
             : "memory");
 }
-// all MMAs of one tap: K steps of 32 bytes (4 per 128-byte block) x NACC accumulators of 128 rows
+// all MMAs of one tap: K steps of 32 bytes (4 per 128-byte block) x 2 accumulators of 128 rows
 // X3: per step TWO instructions instead of three: a1 x [b1 ; b2] as ONE N = 128 MMA (the tap's two weight copies are adjacent in
 // the ring, so they are simply 128 consecutive B rows; its 128 result columns are D1 | D2 of the accumulator, which therefore sit
 // side by side in TMEM), then a2 x b1 (N = 64) onto D2. a1 is fetched from shared memory once for both of its products: 14 KB of
 // operands per step instead of 18 KB -- the operand fetch is what bounds this kernel. a2_off = byte distance of the second
 // activation matrix. D2 must hold zeros when D1 was preloaded with the residual (the epilogue that parks the residual writes them).
-template <bool F16, int NACC, bool X3 = false>
+template <bool F16, bool X3 = false>
 __device__ __forceinline__ void issue_tap_mmas(bool elected, uint32_t dcol, uint32_t s_act, int R, int row0, uint32_t b_slot, int ksteps,
                                                bool accumulate_first, uint32_t a2_off = 0) {
     using O = Op<F16>;
@@ -250,7 +251,7 @@ __device__ __forceinline__ void issue_tap_mmas(bool elected, uint32_t dcol, uint
                 const uint32_t kb = (uint32_t)(j / 4), ks = (uint32_t)(j % 4) * 2u;  // 128-byte block of the row, 32-byte step inside it
                 const uint32_t bj = b_lo + kb * (64u * 128u >> 4) + ks;
 #pragma unroll
-                for (int a = 0; a < NACC; ++a) {
+                for (int a = 0; a < 2; ++a) {
                     const uint32_t aj = a_lo + kb * (uint32_t)(R * 8) + (uint32_t)(a * 128 * 8) + ks;
                     if (X3) {
                         mma_lo<false, F16>(dcol + a * ACC_COLS, aj, bj, (accumulate_first || j > 0) ? 1u : 0u, O::IDESC_N128);  // a1 b1 | a1 b2
@@ -372,7 +373,6 @@ __device__ __forceinline__ void store_packed_x3(uint32_t s_act, uint32_t a2_off,
         st_shared_v4(addr + a2_off, lo[4 * i], lo[4 * i + 1], lo[4 * i + 2], lo[4 * i + 3]);
     }
 }
-__device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t count) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory"); }
 __device__ __forceinline__ float warp_max(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xFFFFFFFFu, v, o));
@@ -399,10 +399,10 @@ __device__ __forceinline__ Cell decode_cell(int cell, int n_cells) {
     return c;
 }
 
-template <int NACC, bool F16, bool X3 = false>
-__global__ void __launch_bounds__(256, (NACC == 2 && !X3) ? 2 : 1)
+template <bool F16, bool X3 = false>
+__global__ void __launch_bounds__(256, X3 ? 1 : 2)
     k_net_forward(const float* __restrict__ planes, float* __restrict__ policy, float* __restrict__ value, int64_t n, NetDev net) {
-    using G = Geo<NACC, F16, X3>;
+    using G = Geo<F16, X3>;
     using O = Op<F16>;
     constexpr int NB = G::NB, CELLS = G::CELLS, R = G::R, NSLOT = G::NSLOT;
     extern __shared__ __align__(1024) uint8_t smem[];
@@ -472,7 +472,7 @@ __global__ void __launch_bounds__(256, (NACC == 2 && !X3) ? 2 : 1)
             const bool use_s = l >= 2 && (l & 1) == 0;  // second convolution of a block accumulates onto the parked residual
             const bool last = l == L - 1;
             if (warp == 0) {
-                // ---- MMA issue: 9 taps x K steps x NACC accumulators (the whole warp runs the loop, one lane issues)
+                // ---- MMA issue: 9 taps x K steps x 2 accumulators (the whole warp runs the loop, one lane issues)
                 const bool elected = elect_one();
                 const uint32_t dcol = tmem + (use_s ? SET : 0u);
                 auto issue_unit = [&](int g, int ksteps) {
@@ -487,7 +487,7 @@ __global__ void __launch_bounds__(256, (NACC == 2 && !X3) ? 2 : 1)
 #pragma unroll
                     for (int tt = 0; tt < TPS; ++tt) {
                         const int t = g * TPS + tt;
-                        issue_tap_mmas<F16, NACC, X3>(elected, dcol, s_act, R, kLead + (t / 3 - 1) * 6 + (t % 3 - 1),
+                        issue_tap_mmas<F16, X3>(elected, dcol, s_act, R, kLead + (t / 3 - 1) * 6 + (t % 3 - 1),
                                                       s_ring + slot * (uint32_t)G::SLOT_BYTES + (uint32_t)tt * (uint32_t)G::TAP_STRIDE, ksteps,
                                                       use_s || t > 0, A2);
                     }
@@ -528,7 +528,7 @@ __global__ void __launch_bounds__(256, (NACC == 2 && !X3) ? 2 : 1)
             acc_par ^= 1u;
             tc_fence_after();
             PF(4);  // waiting for the accumulators
-            // ---- epilogue: this thread owns one cell (TMEM lane) of accumulator(s) warp/4 (+2)
+            // ---- epilogue: this thread owns one cell (TMEM lane) of accumulator warp/4
             const bool preload = (l & 1) == 0 && !last;  // this layer's output is a block input: park it (+ next bias) in TMEM
             const float4* bias_l = reinterpret_cast<const float4*>(net.bias + (size_t)l * 64);
             const float4* bias_n = reinterpret_cast<const float4*>(net.bias + (size_t)(preload ? l + 2 : l) * 64);
@@ -536,75 +536,72 @@ __global__ void __launch_bounds__(256, (NACC == 2 && !X3) ? 2 : 1)
 #ifdef ONB_NET_DBG_NOEPI
             if (l >= 0 && !last) { fence_proxy_async(); q0 += (uint32_t)UPL; continue; }
 #endif
+            const int a = warp >> 2;
+            const int cell = a * 128 + (warp & 3) * 32 + lane;
+            const Cell c = decode_cell(cell, CELLS);
+            const uint32_t tlane = tmem + ((uint32_t)((warp & 3) * 32) << 16);
+            const uint32_t tsrc = tlane + (use_s ? SET : 0u) + a * ACC;
+            const uint32_t tskip = tlane + SET + a * ACC;
+            float hp0 = 0.f, hp1 = 0.f, hv = 0.f;
 #pragma unroll
-            for (int ai = 0; ai < NACC / 2; ++ai) {
-                const int a = (warp >> 2) + 2 * ai;
-                const int cell = a * 128 + (warp & 3) * 32 + lane;
-                const Cell c = decode_cell(cell, CELLS);
-                const uint32_t tlane = tmem + ((uint32_t)((warp & 3) * 32) << 16);
-                const uint32_t tsrc = tlane + (use_s ? SET : 0u) + a * ACC;
-                const uint32_t tskip = tlane + SET + a * ACC;
-                float hp0 = 0.f, hp1 = 0.f, hv = 0.f;
+            for (int h = 0; h < 2; ++h) {
+                uint32_t v[32];
+                if (X3) {  // D1 + 2^-11 D2: both loads in flight, one wait
+                    uint32_t v2[32];
+                    tmem_ld32_nowait(tsrc + h * 32, v);
+                    tmem_ld32_nowait(tsrc + 64 + h * 32, v2);
+                    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 #pragma unroll
-                for (int h = 0; h < 2; ++h) {
-                    uint32_t v[32];
-                    if (X3) {  // D1 + 2^-11 D2: both loads in flight, one wait
-                        uint32_t v2[32];
-                        tmem_ld32_nowait(tsrc + h * 32, v);
-                        tmem_ld32_nowait(tsrc + 64 + h * 32, v2);
-                        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                    for (int i = 0; i < 32; ++i) v[i] = __float_as_uint(fmaf(__uint_as_float(v2[i]), kX3InvScale, __uint_as_float(v[i])));
+                } else {
+                    tmem_ld32(tsrc + h * 32, v);
+                }
+                float o[32];
 #pragma unroll
-                        for (int i = 0; i < 32; ++i) v[i] = __float_as_uint(fmaf(__uint_as_float(v2[i]), kX3InvScale, __uint_as_float(v[i])));
-                    } else {
-                        tmem_ld32(tsrc + h * 32, v);
-                    }
-                    float o[32];
+                for (int i = 0; i < 8; ++i) {
+                    float4 b = make_float4(0.f, 0.f, 0.f, 0.f);
+                    if (!use_s) b = __ldg(bias_l + h * 8 + i);
+                    o[4 * i + 0] = fmaxf(__uint_as_float(v[4 * i + 0]) + b.x, 0.f);
+                    o[4 * i + 1] = fmaxf(__uint_as_float(v[4 * i + 1]) + b.y, 0.f);
+                    o[4 * i + 2] = fmaxf(__uint_as_float(v[4 * i + 2]) + b.z, 0.f);
+                    o[4 * i + 3] = fmaxf(__uint_as_float(v[4 * i + 3]) + b.w, 0.f);
+                }
+                if (!last && c.real) {
+                    if (X3) store_channels_x3(s_act, A2, R, kLead + cell, h * 32, o);
+                    else store_channels<F16>(s_act, R, kLead + cell, h * 32, o);
+                }
+                if (preload) {
 #pragma unroll
                     for (int i = 0; i < 8; ++i) {
-                        float4 b = make_float4(0.f, 0.f, 0.f, 0.f);
-                        if (!use_s) b = __ldg(bias_l + h * 8 + i);
-                        o[4 * i + 0] = fmaxf(__uint_as_float(v[4 * i + 0]) + b.x, 0.f);
-                        o[4 * i + 1] = fmaxf(__uint_as_float(v[4 * i + 1]) + b.y, 0.f);
-                        o[4 * i + 2] = fmaxf(__uint_as_float(v[4 * i + 2]) + b.z, 0.f);
-                        o[4 * i + 3] = fmaxf(__uint_as_float(v[4 * i + 3]) + b.w, 0.f);
+                        const float4 b = __ldg(bias_n + h * 8 + i);
+                        v[4 * i + 0] = __float_as_uint(o[4 * i + 0] + b.x);
+                        v[4 * i + 1] = __float_as_uint(o[4 * i + 1] + b.y);
+                        v[4 * i + 2] = __float_as_uint(o[4 * i + 2] + b.z);
+                        v[4 * i + 3] = __float_as_uint(o[4 * i + 3] + b.w);
                     }
-                    if (!last && c.real) {
-                        if (X3) store_channels_x3(s_act, A2, R, kLead + cell, h * 32, o);
-                        else store_channels<F16>(s_act, R, kLead + cell, h * 32, o);
-                    }
-                    if (preload) {
+                    tmem_st32(tskip + h * 32, v);
+                    if (X3) {  // the D2 half of the preloaded accumulator starts the next-but-one layer from zero
 #pragma unroll
-                        for (int i = 0; i < 8; ++i) {
-                            const float4 b = __ldg(bias_n + h * 8 + i);
-                            v[4 * i + 0] = __float_as_uint(o[4 * i + 0] + b.x);
-                            v[4 * i + 1] = __float_as_uint(o[4 * i + 1] + b.y);
-                            v[4 * i + 2] = __float_as_uint(o[4 * i + 2] + b.z);
-                            v[4 * i + 3] = __float_as_uint(o[4 * i + 3] + b.w);
-                        }
-                        tmem_st32(tskip + h * 32, v);
-                        if (X3) {  // the D2 half of the preloaded accumulator starts the next-but-one layer from zero
-#pragma unroll
-                            for (int i = 0; i < 32; ++i) v[i] = 0u;
-                            tmem_st32(tskip + 64 + h * 32, v);
-                        }
-                    }
-                    if (last) {  // 1x1 convolutions of both heads (net.rs: policy_conv 64 -> 2, vh_conv 64 -> 1)
-#pragma unroll
-                        for (int i = 0; i < 8; ++i) {
-                            const float4 w0 = __ldg(hw + (kHP0 / 4) + h * 8 + i), w1 = __ldg(hw + (kHP1 / 4) + h * 8 + i),
-                                         w2 = __ldg(hw + (kHV / 4) + h * 8 + i);
-                            hp0 = fmaf(o[4 * i + 0], w0.x, fmaf(o[4 * i + 1], w0.y, fmaf(o[4 * i + 2], w0.z, fmaf(o[4 * i + 3], w0.w, hp0))));
-                            hp1 = fmaf(o[4 * i + 0], w1.x, fmaf(o[4 * i + 1], w1.y, fmaf(o[4 * i + 2], w1.z, fmaf(o[4 * i + 3], w1.w, hp1))));
-                            hv = fmaf(o[4 * i + 0], w2.x, fmaf(o[4 * i + 1], w2.y, fmaf(o[4 * i + 2], w2.z, fmaf(o[4 * i + 3], w2.w, hv))));
-                        }
+                        for (int i = 0; i < 32; ++i) v[i] = 0u;
+                        tmem_st32(tskip + 64 + h * 32, v);
                     }
                 }
-                if (last && c.real) {
-                    float* hb = s_head + c.board * 75;
-                    hb[c.pos] = fmaxf(hp0 + __ldg(net.head + kHB + 0), 0.f);
-                    hb[25 + c.pos] = fmaxf(hp1 + __ldg(net.head + kHB + 1), 0.f);
-                    hb[50 + c.pos] = fmaxf(hv + __ldg(net.head + kHB + 2), 0.f);
+                if (last) {  // 1x1 convolutions of both heads (net.rs: policy_conv 64 -> 2, vh_conv 64 -> 1)
+#pragma unroll
+                    for (int i = 0; i < 8; ++i) {
+                        const float4 w0 = __ldg(hw + (kHP0 / 4) + h * 8 + i), w1 = __ldg(hw + (kHP1 / 4) + h * 8 + i),
+                                     w2 = __ldg(hw + (kHV / 4) + h * 8 + i);
+                        hp0 = fmaf(o[4 * i + 0], w0.x, fmaf(o[4 * i + 1], w0.y, fmaf(o[4 * i + 2], w0.z, fmaf(o[4 * i + 3], w0.w, hp0))));
+                        hp1 = fmaf(o[4 * i + 0], w1.x, fmaf(o[4 * i + 1], w1.y, fmaf(o[4 * i + 2], w1.z, fmaf(o[4 * i + 3], w1.w, hp1))));
+                        hv = fmaf(o[4 * i + 0], w2.x, fmaf(o[4 * i + 1], w2.y, fmaf(o[4 * i + 2], w2.z, fmaf(o[4 * i + 3], w2.w, hv))));
+                    }
                 }
+            }
+            if (last && c.real) {
+                float* hb = s_head + c.board * 75;
+                hb[c.pos] = fmaxf(hp0 + __ldg(net.head + kHB + 0), 0.f);
+                hb[25 + c.pos] = fmaxf(hp1 + __ldg(net.head + kHB + 1), 0.f);
+                hb[50 + c.pos] = fmaxf(hv + __ldg(net.head + kHB + 2), 0.f);
             }
             if (preload) tmem_wait_st();
             fence_proxy_async();
@@ -651,7 +648,7 @@ __global__ void __launch_bounds__(256, (NACC == 2 && !X3) ? 2 : 1)
     if (warp == 0) tmem_dealloc(tmem, G::TMEM_COLS);
 }
 
-// 16-column TMEM access and split-operand stores shared by the many-warp epilogues below
+// 16-column TMEM access and f16 operand stores of the many-warp epilogues below
 __device__ __forceinline__ void tmem_ld16_nowait(uint32_t taddr, uint32_t (&v)[16]) {
     asm volatile(
         "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
@@ -668,22 +665,12 @@ __device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&v)[16
         "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
         : "memory");
 }
-// 16 consecutive channels [c0, c0 + 16) of one cell as split operand chunks (two 16-byte chunks in each activation matrix)
-__device__ __forceinline__ void store_channels_x3_16(uint32_t s_act, uint32_t a2_off, int R, int row, int c0, const float (&o)[16]) {
+// 16 consecutive channels [c0, c0 + 16) of one cell as f16 operand chunks
+__device__ __forceinline__ void store_channels_f16_16(uint32_t s_act, int R, int row, int c0, const float (&o)[16]) {
 #pragma unroll
-    for (int i = 0; i < 2; ++i) {
-        uint32_t hi[4], lo[4];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const float x0 = o[8 * i + 2 * q], x1 = o[8 * i + 2 * q + 1];
-            hi[q] = to_f16x2(x0, x1);  // saturating
-            const float2 hf = f16x2_to_float2(hi[q]);
-            lo[q] = to_f16x2((x0 - hf.x) * kX3Scale, (x1 - hf.y) * kX3Scale);
-        }
-        const uint32_t addr = act_addr(s_act, R, row, c0 / 8 + i);
-        st_shared_v4(addr, hi[0], hi[1], hi[2], hi[3]);
-        st_shared_v4(addr + a2_off, lo[0], lo[1], lo[2], lo[3]);
-    }
+    for (int i = 0; i < 2; ++i)
+        st_shared_v4(act_addr(s_act, R, row, c0 / 8 + i), to_f16x2(o[8 * i + 0], o[8 * i + 1]), to_f16x2(o[8 * i + 2], o[8 * i + 3]),
+                     to_f16x2(o[8 * i + 4], o[8 * i + 5]), to_f16x2(o[8 * i + 6], o[8 * i + 7]));
 }
 
 // ---- CTA-pair (cta_group::2) helpers: cluster-scope barrier traffic and the paired MMA / commit -------------------------------------
@@ -764,7 +751,7 @@ __device__ __forceinline__ void issue_tap_mmas_pair(bool elected, uint32_t dcol,
 }
 
 // ---- the split-operand (f32-faithful) network, warp-specialised and software-pipelined over the two accumulators ------------------
-// k_net_forward<2, f16, X3> issues a layer's MMAs, waits, runs the epilogue with the tensor pipe idle, synchronises the CTA and
+// k_net_forward<f16, X3> issues a layer's MMAs, waits, runs the epilogue with the tensor pipe idle, synchronises the CTA and
 // starts over: 63 % of its time is MMA issue (at the operand-fetch / tensor floor), the rest is exposed epilogue, barriers and
 // waits, and neither TMEM (512 columns) nor shared memory (219 KB) leaves room for a second CTA to fill the gaps. Here the SAME
 // geometry (7 boards, two 128-row accumulators, a1/a2 activation matrices, 3 x 3-tap weight ring) runs as a pipeline of roles:
@@ -777,10 +764,10 @@ __device__ __forceinline__ void issue_tap_mmas_pair(bool elected, uint32_t dcol,
 // the write-after-read hazard of updating the activations in place) and wait for warp 4's rows only in front of their sixth tap.
 // The history of the kernel -- what a per-layer timeline (-DONB_X3P_PROFILE) showed at each step and what each change bought, from
 // 0.745 ms (plain build) to 0.514 ms -- is in DESIGN.md section 5b. Same products, same accumulation order, same results as
-// k_net_forward<2, f16, X3>.
+// k_net_forward<f16, X3>.
 template <bool CL>
 struct GeoX3PT {
-    using G = Geo<2, true, true>;
+    using G = Geo<true, true>;
     static constexpr int THREADS = 11 * 32;  // 8 epilogue warps, warp 8: helper of warp 4 (see the kernel), warp 9: MMA issue, warp 10: weights
     // CL (CTA pair, see below): a tap is [this CTA's 64 B rows of the N = 128 MMA][its 32 B rows of the N = 64 MMA]
     static constexpr int TAP_STRIDE = CL ? 12 * 1024 : G::TAP_STRIDE;
@@ -821,7 +808,7 @@ __device__ long long s_t2[2][8];   // layer 4 of that group, per accumulator: wa
 template <bool CL>
 __global__ void __launch_bounds__(GeoX3P::THREADS, 1)
     k_net_forward_x3p(const float* __restrict__ planes, float* __restrict__ policy, float* __restrict__ value, int64_t n, NetDev net) {
-    using G = Geo<2, true, true>;
+    using G = Geo<true, true>;
     using GP = GeoX3PT<CL>;
     using O = Op<true>;
     constexpr int NACC = 2;
@@ -1280,255 +1267,6 @@ __global__ void __launch_bounds__(GeoX3P::THREADS, 1)
     }
 }
 
-// ---- the f16 fast mode with the same role pipeline, TWO CTAs per SM -------------------------------------------------------------
-// k_net_forward<2, f16> already overlaps one CTA's epilogue with the other CTA's MMAs, but each CTA still serialises issue ->
-// wait -> epilogue -> CTA barrier, and the tensor pipe is busy 46 % of the time (2 x 4 032 MMAs x 33.5 cycles of 581 k). Here
-// each of the two co-resident CTAs is the warp-specialised pipeline of k_net_forward_x3p (8 epilogue warps, one MMA warp, one
-// weight warp, mbarriers only), so an SM always has two MMA streams whose bubbles (the halo dependency between accumulators) fall
-// into each other's issue phases. The epilogue works 16 channels at a time to fit 96 registers (2 x 320 threads per SM).
-// Same products, accumulation order and head sums as k_net_forward<2, f16>: bit-identical results.
-constexpr int kF16PThreads = 10 * 32;  // k_net_forward_f16p: 8 epilogue warps, MMA issue, weights
-__device__ __forceinline__ void store_channels_f16_16(uint32_t s_act, int R, int row, int c0, const float (&o)[16]) {
-#pragma unroll
-    for (int i = 0; i < 2; ++i)
-        st_shared_v4(act_addr(s_act, R, row, c0 / 8 + i), to_f16x2(o[8 * i + 0], o[8 * i + 1]), to_f16x2(o[8 * i + 2], o[8 * i + 3]),
-                     to_f16x2(o[8 * i + 4], o[8 * i + 5]), to_f16x2(o[8 * i + 6], o[8 * i + 7]));
-}
-__global__ void __launch_bounds__(kF16PThreads, 2)
-    k_net_forward_f16p(const float* __restrict__ planes, float* __restrict__ policy, float* __restrict__ value, int64_t n, NetDev net) {
-    using G = Geo<2, true, false>;
-    using O = Op<true>;
-    constexpr int NACC = 2;
-    constexpr int NB = G::NB, CELLS = G::CELLS, R = G::R, NSLOT = G::NSLOT, TPS = G::TPS, UPL = G::UPL;
-    constexpr uint32_t ACC = 64u, SET = (uint32_t)G::SET_COLS;
-    extern __shared__ __align__(1024) uint8_t smem[];
-    const uint32_t s_act = smem_u32(smem), s_ring = s_act + G::OFF_RING, s_bar = s_act + G::OFF_BAR;
-    float* s_head = reinterpret_cast<float*>(smem + G::OFF_HEAD);
-    uint32_t* s_tmem = reinterpret_cast<uint32_t*>(smem + G::OFF_BAR + GeoX3P::N_BARS * 8);
-    static_assert(2 * (G::OFF_BAR + GeoX3P::N_BARS * 8 + 16 + 1024) <= 227 * 1024, "two CTAs per SM");
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int L = 1 + 2 * net.n_blocks;
-    const int64_t n_groups = (n + NB - 1) / NB;
-    if ((int64_t)blockIdx.x >= n_groups) return;  // whole CTA, before any allocation
-    const int64_t my_groups = (n_groups - blockIdx.x + gridDim.x - 1) / gridDim.x;
-    const uint32_t total_units = (uint32_t)my_groups * (uint32_t)(UPL * L);
-    auto bar_full = [&](uint32_t s) { return s_bar + s * 8u; };
-    auto bar_empty = [&](uint32_t s) { return s_bar + (NSLOT + s) * 8u; };
-    auto bar_acc = [&](uint32_t a) { return s_bar + (2 * NSLOT + a) * 8u; };
-    auto bar_rows = [&](uint32_t k) { return s_bar + (2 * NSLOT + 2 + k) * 8u; };  // 0: group 0, 1: warp 4, 2: warps 5-7
-
-    if (tid == 0) {
-        for (uint32_t s = 0; s < (uint32_t)NSLOT; ++s) {
-            mbar_init(bar_full(s), 1);
-            mbar_init(bar_empty(s), 1);
-        }
-        mbar_init(bar_acc(0), 1);
-        mbar_init(bar_acc(1), 1);
-        mbar_init(bar_rows(0), 128);
-        mbar_init(bar_rows(1), 32);
-        mbar_init(bar_rows(2), 96);
-        fence_barrier_init();
-    }
-    if (warp == 0) tmem_alloc(smem_u32(s_tmem), G::TMEM_COLS);
-    for (int i = tid; i < G::NMAT * G::ACT_BYTES / 16; i += kF16PThreads) st_shared_v4(s_act + i * 16, 0u, 0u, 0u, 0u);  // pad cells stay zero
-    fence_proxy_async();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = *s_tmem;
-    auto arrive = [&](uint32_t bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory"); };
-
-    if (warp == 9) {
-        // ---- weight producer: the ring is filled strictly in tap order, as far ahead as it has free slots
-        if (lane == 0) {
-            for (uint32_t u = 0; u < total_units; ++u) {
-                const uint32_t slot = u % NSLOT, use = u / NSLOT;
-                if (use >= 1) mbar_wait(bar_empty(slot), (use - 1u) & 1u);
-                const uint32_t ul = u % (uint32_t)(UPL * L), layer = ul / UPL, tap = (ul - layer * UPL) * TPS;
-                const uint8_t* src = net.wconv + (size_t)G::NMAT * (layer == 0 ? (size_t)tap * O::TAP_BYTES0
-                                                                              : (size_t)9 * O::TAP_BYTES0 + ((size_t)(layer - 1) * 9 + tap) * O::TAP_BYTES);
-                const uint32_t bytes = (uint32_t)(TPS * G::NMAT) * (layer == 0 ? O::TAP_BYTES0 : O::TAP_BYTES);
-                mbar_expect_tx(bar_full(slot), bytes);
-                bulk_g2s(s_ring + slot * (uint32_t)G::SLOT_BYTES, src, bytes, bar_full(slot));
-            }
-        }
-    } else if (warp == 8) {
-        // ---- MMA issue (the whole warp runs the loop so that descriptors stay in uniform registers; one elected lane issues)
-        const bool elected = elect_one();
-        uint32_t q0 = 0, stage = 0;  // stage = number of "rows ready" rounds consumed so far (input stage + epilogues)
-        for (int64_t gi = 0; gi < my_groups; ++gi) {
-            for (int l = 0; l < L; ++l) {
-                const bool use_s = l >= 2 && (l & 1) == 0;
-                const uint32_t dcol = tmem + (use_s ? SET : 0u);
-                const int ksteps = l == 0 ? O::KCH0 / 2 : O::KCH / 2;
-#pragma unroll 1
-                for (int a = 0; a < NACC; ++a) {
-                    // accumulator 0 needs its own rows and the first rows of accumulator 1 (its windows reach 7 rows further);
-                    // accumulator 1 needs the rest as well
-                    if (a == 0) {
-                        mbar_wait(bar_rows(0), stage & 1u);
-                        mbar_wait(bar_rows(1), stage & 1u);
-                    } else {
-                        mbar_wait(bar_rows(2), stage & 1u);
-                    }
-                    tc_fence_after();
-#pragma unroll 1
-                    for (int g = 0; g < UPL; ++g) {
-                        const uint32_t u = q0 + g, slot = u % NSLOT, use = u / NSLOT;
-                        mbar_wait(bar_full(slot), use & 1u);
-                        tc_fence_after();
-#pragma unroll
-                        for (int tt = 0; tt < TPS; ++tt) {
-                            const int t = g * TPS + tt;
-                            // one accumulator per pass: issue_tap_mmas<.., NACC = 1> on this accumulator's rows and columns
-                            issue_tap_mmas<true, 1, false>(elected, dcol + (uint32_t)a * ACC, s_act, R, kLead + (t / 3 - 1) * 6 + (t % 3 - 1) + a * 128,
-                                                           s_ring + slot * (uint32_t)G::SLOT_BYTES + (uint32_t)tt * (uint32_t)G::TAP_STRIDE, ksteps,
-                                                           use_s || t > 0);
-                        }
-                        if (a == NACC - 1 && elected) umma_commit(bar_empty(slot));  // both accumulators' MMAs have read the slot
-                    }
-                    if (elected) umma_commit(bar_acc(a));
-                }
-                q0 += (uint32_t)UPL;
-                stage += 1;
-            }
-        }
-    } else {
-        // ---- epilogue warps: group a = warp >> 2 owns accumulator a; this thread owns one cell (TMEM lane) and its 64 channels
-        const int a = warp >> 2;
-        const int cell = a * 128 + (warp & 3) * 32 + lane;
-        const Cell c = decode_cell(cell, CELLS);
-        const uint32_t my_rows = a == 0 ? bar_rows(0) : (warp == 4 ? bar_rows(1) : bar_rows(2));
-        const bool halo = a == 0 && cell >= 128 - 7;  // rows accumulator 1's MMAs of the SAME layer still read
-        const uint32_t tlane = tmem + ((uint32_t)((warp & 3) * 32) << 16);
-        uint32_t acc_par = 0;  // parity of the layer counter (both accumulator barriers complete once per layer)
-        for (int64_t gi = 0; gi < my_groups; ++gi) {
-            const int64_t board0 = ((int64_t)blockIdx.x + gi * gridDim.x) * NB;
-            // ---- input planes -> channel chunks of both activation matrices (create_tensor_from_state layout [21][5][5]).
-            // The previous group's last MMAs have completed (every thread waited for both accumulators before its heads).
-            if (c.real) {
-                const int64_t gb = board0 + c.board;
-                const float* src = planes + gb * 525 + c.pos;
-#pragma unroll
-                for (int part = 0; part < 2; ++part) {
-                    float x[16];  // the planes are 0 / 1: exact in f16
-#pragma unroll
-                    for (int ch = 0; ch < 16; ++ch) x[ch] = (part * 16 + ch < kInPlanes && gb < n) ? __ldg(src + (part * 16 + ch) * 25) : 0.f;
-                    store_channels_f16_16(s_act, R, kLead + cell, part * 16, x);  // 32 channels: planes 21..31 are zero
-                }
-            }
-            fence_proxy_async();
-            arrive(my_rows);
-            for (int l = 0; l < L; ++l) {
-                const bool use_s = l >= 2 && (l & 1) == 0;  // second convolution of a block accumulates onto the parked residual
-                const bool last = l == L - 1;
-                mbar_wait(bar_acc(a), acc_par);
-                tc_fence_after();
-                const bool preload = (l & 1) == 0 && !last;  // this layer's output is a block input: park it (+ next bias) in TMEM
-                const float4* bias_l = reinterpret_cast<const float4*>(net.bias + (size_t)l * 64);
-                const float4* bias_n = reinterpret_cast<const float4*>(net.bias + (size_t)(preload ? l + 2 : l) * 64);
-                const float4* hw = reinterpret_cast<const float4*>(net.head);
-                const uint32_t tsrc = tlane + (use_s ? SET : 0u) + a * ACC;
-                const uint32_t tskip = tlane + SET + a * ACC;
-                float hp0 = 0.f, hp1 = 0.f, hv = 0.f;
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {  // 16 channels at a time: the kernel must fit 96 registers for two CTAs per SM
-                    const int c0 = q * 16;
-                    uint32_t v[16];
-                    tmem_ld16_nowait(tsrc + c0, v);
-                    tmem_wait_ld();
-                    float o[16];
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        float4 b = make_float4(0.f, 0.f, 0.f, 0.f);
-                        if (!use_s) b = __ldg(bias_l + c0 / 4 + i);
-                        o[4 * i + 0] = fmaxf(__uint_as_float(v[4 * i + 0]) + b.x, 0.f);
-                        o[4 * i + 1] = fmaxf(__uint_as_float(v[4 * i + 1]) + b.y, 0.f);
-                        o[4 * i + 2] = fmaxf(__uint_as_float(v[4 * i + 2]) + b.z, 0.f);
-                        o[4 * i + 3] = fmaxf(__uint_as_float(v[4 * i + 3]) + b.w, 0.f);
-                    }
-                    if (!last && c.real) {
-                        // accumulator 1's MMAs of this layer read rows 121..127 through their negatively shifted windows: wait for them
-                        if (halo && q == 0) mbar_wait(bar_acc(1), acc_par);
-                        store_channels_f16_16(s_act, R, kLead + cell, c0, o);
-                    }
-                    if (preload) {
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            const float4 b = __ldg(bias_n + c0 / 4 + i);
-                            v[4 * i + 0] = __float_as_uint(o[4 * i + 0] + b.x);
-                            v[4 * i + 1] = __float_as_uint(o[4 * i + 1] + b.y);
-                            v[4 * i + 2] = __float_as_uint(o[4 * i + 2] + b.z);
-                            v[4 * i + 3] = __float_as_uint(o[4 * i + 3] + b.w);
-                        }
-                        tmem_st16(tskip + c0, v);
-                    }
-                    if (last) {  // 1x1 convolutions of both heads (net.rs: policy_conv 64 -> 2, vh_conv 64 -> 1)
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            const float4 w0 = __ldg(hw + (kHP0 / 4) + c0 / 4 + i), w1 = __ldg(hw + (kHP1 / 4) + c0 / 4 + i),
-                                         w2 = __ldg(hw + (kHV / 4) + c0 / 4 + i);
-                            hp0 = fmaf(o[4 * i + 0], w0.x, fmaf(o[4 * i + 1], w0.y, fmaf(o[4 * i + 2], w0.z, fmaf(o[4 * i + 3], w0.w, hp0))));
-                            hp1 = fmaf(o[4 * i + 0], w1.x, fmaf(o[4 * i + 1], w1.y, fmaf(o[4 * i + 2], w1.z, fmaf(o[4 * i + 3], w1.w, hp1))));
-                            hv = fmaf(o[4 * i + 0], w2.x, fmaf(o[4 * i + 1], w2.y, fmaf(o[4 * i + 2], w2.z, fmaf(o[4 * i + 3], w2.w, hv))));
-                        }
-                    }
-                }
-                if (last && c.real) {
-                    float* hb = s_head + c.board * 75;
-                    hb[c.pos] = fmaxf(hp0 + __ldg(net.head + kHB + 0), 0.f);
-                    hb[25 + c.pos] = fmaxf(hp1 + __ldg(net.head + kHB + 1), 0.f);
-                    hb[50 + c.pos] = fmaxf(hv + __ldg(net.head + kHB + 2), 0.f);
-                }
-                if (preload) tmem_wait_st();
-                if (last) {
-                    // the next group's input stage overwrites rows the OTHER accumulator's last MMAs may still read: wait for both
-                    mbar_wait(bar_acc(a ^ 1), acc_par);
-                } else {
-                    fence_proxy_async();
-                    tc_fence_before();
-                    arrive(my_rows);  // this thread's rows (and its TMEM reads) of the layer are done
-                }
-                acc_par ^= 1u;
-            }
-            // ---- heads: one warp per board (ph_linear2 + softmax, vh_linear1 + ReLU + vh_linear2 + tanh)
-            named_bar_sync(1, 256);
-            for (int b = warp; b < NB; b += 8) {
-                const int64_t gb = board0 + b;
-                if (gb >= n) continue;
-                const float* hb = s_head + b * 75;
-                const bool two = lane + 32 < 50;
-                float l0 = __ldg(net.head + kPhB + lane), l1 = two ? __ldg(net.head + kPhB + 32 + lane) : 0.f;
-#pragma unroll 10
-                for (int i = 0; i < 50; ++i) {
-                    const float x = hb[i];
-                    l0 = fmaf(x, __ldg(net.head + kPhW + i * 50 + lane), l0);
-                    if (two) l1 = fmaf(x, __ldg(net.head + kPhW + i * 50 + 32 + lane), l1);
-                }
-                const float m = warp_max(two ? fmaxf(l0, l1) : l0);
-                const float e0 = expf(l0 - m), e1 = two ? expf(l1 - m) : 0.f;
-                const float s = warp_sum(e0 + e1);
-                policy[gb * 50 + lane] = e0 / s;
-                if (two) policy[gb * 50 + 32 + lane] = e1 / s;
-                float h0 = __ldg(net.head + kV1B + lane), h1 = __ldg(net.head + kV1B + 32 + lane);
-#pragma unroll 5
-                for (int i = 0; i < 25; ++i) {
-                    const float x = hb[50 + i];
-                    h0 = fmaf(x, __ldg(net.head + kV1W + i * 64 + lane), h0);
-                    h1 = fmaf(x, __ldg(net.head + kV1W + i * 64 + 32 + lane), h1);
-                }
-                float acc = fmaf(fmaxf(h0, 0.f), __ldg(net.head + kV2W + lane), fmaxf(h1, 0.f) * __ldg(net.head + kV2W + 32 + lane));
-                acc = warp_sum(acc);
-                if (lane == 0) value[gb] = tanhf(acc + __ldg(net.head + kV2B));
-            }
-            named_bar_sync(1, 256);  // s_head is free again before anybody's next last-layer epilogue
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc(tmem, G::TMEM_COLS);
-}
-
 // ---- the f16 fast mode as ONE CTA per SM with FOUR accumulators: the pipeline of k_net_forward_x3p with everything it learned ------
 // 14 boards (504 cells) per pass in four 128-row accumulators (TMEM: 4 x 64 columns x {plain, residual-preloaded} = 512), sixteen
 // epilogue warps (four per accumulator, 16 channels at a time: 576 threads leave 113 registers), one MMA warp, one weight warp.
@@ -1538,7 +1276,7 @@ __global__ void __launch_bounds__(kF16PThreads, 2)
 // the next group's input stored from the last layer's epilogue, heads computed in the next group's slack, and CL = CTA pairs
 // (tcgen05 cta_group::2: each SM keeps rows 32 r .. 32 r + 31 of every tap, 4 KB instead of 8 KB). Twice the boards per weight pass
 // of the two-CTAs-per-SM builds (and a quarter of their weight bytes per SM with CL): the L2 -> SM weight stream was 55 % of their
-// time. Same products, accumulation order and head sums as k_net_forward<2, f16>: bit-identical results.
+// time. Same products, accumulation order and head sums as k_net_forward<f16>: bit-identical results.
 #ifdef ONB_F16Q_PROFILE
 __device__ long long q_tl[8][4][4];  // [layer][accumulator][issue start, issue end, accumulator done (first warp of its group), that warp arrives]
 #define QTL(l_, a_, e_) do { if (blockIdx.x == 2 && gi == 3 && (l_) < 8) q_tl[l_][a_][e_] = clock64(); } while (0)
@@ -1922,740 +1660,6 @@ __global__ void __launch_bounds__(GeoF16Q<CL>::THREADS, 1)
     } else if (warp == 0) {
         tmem_dealloc(tmem, GP::TMEM_COLS);
     }
-}
-
-// ---- version 2: ONE CTA per SM, two independent halves that share one weight stream ---------------------------------------------
-// Measured on version 1 (two CTAs per SM, each streaming its own weights): with MMAs and epilogues disabled the kernel still took
-// 55 % of its time -- 2 341 board groups x 451 KB of weights = 1.06 GB through L2 per call (5.6 TB/s). TMEM (512 columns = accumulators
-// + parked residuals of 14 boards) fixes how many boards an SM can hold, so the only way to halve that traffic is to let both groups
-// of an SM consume the SAME ring. Layout: 16 worker warps = 2 halves x 8 warps, each half exactly the version-1 CTA (its own 7 boards,
-// activation matrix, 256 TMEM columns, MMA-issuing thread, named barrier), running out of phase so one half's MMAs overlap the other
-// half's epilogue; warp 16 is the producer (lane 0 streams taps into a 16-slot ring; a slot is refilled when BOTH halves' MMAs have
-// read it: empty barriers count 2).
-template <bool F16>
-struct Geo2 {
-    static constexpr int NB = 7;  // boards per half
-    static constexpr int CELLS = NB * kCellsPerBoard;
-    static constexpr int R = (kLead + CELLS + kTrail + 7) / 8 * 8;
-    // ring granularity: f16 keeps two WHOLE LAYERS (9 taps, 72 KB each) -- one full/empty barrier round trip and one bulk copy per layer
-    // instead of per tap (the per-tap try_wait + fence + commit cost ~480 cycles, more than the 8 MMAs between them); tf32 taps are
-    // twice as large, so that variant keeps a 5-slot ring of single taps
-    static constexpr int TPS = F16 ? 9 : 1;   // taps per slot
-    static constexpr int UPL = 9 / TPS;       // slots ("units") per layer
-    static constexpr int NSLOT = F16 ? 2 : 5;
-    static constexpr int SLOT_BYTES = TPS * Op<F16>::TAP_BYTES;
-    static constexpr int ACT_BYTES = R * Op<F16>::KCH * 16;  // per half
-    static constexpr int OFF_RING = 2 * ACT_BYTES;
-    static constexpr int RING_BYTES = NSLOT * SLOT_BYTES;
-    static constexpr int OFF_HEAD = OFF_RING + RING_BYTES;
-    static constexpr int HEAD_BYTES = ((NB * 75 * 4 + 15) / 16) * 16;  // per half
-    static constexpr int OFF_BAR = OFF_HEAD + 2 * HEAD_BYTES;
-    static constexpr int SMEM = OFF_BAR + (2 * NSLOT + 2) * 8 + 16;
-    static constexpr int THREADS = 17 * 32;
-    static_assert(CELLS <= 256, "two accumulators of 128 cells per half");
-    static_assert(SMEM <= 227 * 1024, "shared memory");
-};
-
-template <bool F16>
-__global__ void __launch_bounds__(Geo2<F16>::THREADS, 1)
-    k_net_forward2(const float* __restrict__ planes, float* __restrict__ policy, float* __restrict__ value, int64_t n, NetDev net) {
-    using G = Geo2<F16>;
-    using O = Op<F16>;
-    constexpr int NB = G::NB, CELLS = G::CELLS, R = G::R, NSLOT = G::NSLOT, NACC = 2;
-    extern __shared__ __align__(1024) uint8_t smem[];
-    const uint32_t s_base = smem_u32(smem), s_ring = s_base + G::OFF_RING, s_bar = s_base + G::OFF_BAR;
-    uint32_t* s_tmem = reinterpret_cast<uint32_t*>(smem + G::OFF_BAR + (2 * NSLOT + 2) * 8);
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int L = 1 + 2 * net.n_blocks;
-    const int64_t n_groups = (n + NB - 1) / NB;
-    // iteration i of this CTA: half h works on group (blockIdx.x + i * gridDim.x) * 2 + h (possibly past the end: computed, not stored)
-    const int64_t n_pairs = (n_groups + 1) / 2;
-    if ((int64_t)blockIdx.x >= n_pairs) return;
-    const int64_t my_iters = (n_pairs - blockIdx.x + gridDim.x - 1) / gridDim.x;
-    constexpr int TPS = G::TPS, UPL = G::UPL;
-    const uint32_t total_units = (uint32_t)my_iters * (uint32_t)(UPL * L);
-    auto bar_full = [&](uint32_t s) { return s_bar + s * 8u; };
-    auto bar_empty = [&](uint32_t s) { return s_bar + (NSLOT + s) * 8u; };
-
-    if (tid == 0) {
-        for (uint32_t s = 0; s < (uint32_t)NSLOT; ++s) {
-            mbar_init(bar_full(s), 1);
-            mbar_init(bar_empty(s), 2);  // both halves' MMAs must have read the slot
-        }
-        mbar_init(s_bar + 2 * NSLOT * 8u, 1);
-        mbar_init(s_bar + (2 * NSLOT + 1) * 8u, 1);
-        fence_barrier_init();
-    }
-    if (warp == 0) tmem_alloc(smem_u32(s_tmem), 512);
-    for (int i = tid; i < 2 * G::ACT_BYTES / 16; i += G::THREADS) st_shared_v4(s_base + i * 16, 0u, 0u, 0u, 0u);  // pad cells stay zero
-    fence_proxy_async();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-
-    if (warp == 16) {
-        // ---- weight producer (one lane): the ring is filled strictly in tap order, as far ahead as it has free slots
-        if (lane == 0) {
-            for (uint32_t u = 0; u < total_units; ++u) {
-                const uint32_t slot = u % NSLOT, use = u / NSLOT;
-                if (use >= 1) mbar_wait(bar_empty(slot), (use - 1u) & 1u);
-                const uint32_t ul = u % (uint32_t)(UPL * L), layer = ul / UPL, tap = (ul - layer * UPL) * TPS;
-                const uint8_t* src = net.wconv + (layer == 0 ? (size_t)tap * O::TAP_BYTES0
-                                                              : (size_t)9 * O::TAP_BYTES0 + ((size_t)(layer - 1) * 9 + tap) * O::TAP_BYTES);
-                const uint32_t bytes = (uint32_t)TPS * (layer == 0 ? O::TAP_BYTES0 : O::TAP_BYTES);
-                mbar_expect_tx(bar_full(slot), bytes);
-                bulk_g2s(s_ring + slot * (uint32_t)G::SLOT_BYTES, src, bytes, bar_full(slot));
-            }
-        }
-        return;  // the workers only use named barriers from here on
-    }
-
-    const int half = warp >> 3, hwarp = warp & 7, htid = tid & 255;
-    const uint32_t s_act = s_base + (uint32_t)half * G::ACT_BYTES;
-    float* s_head = reinterpret_cast<float*>(smem + G::OFF_HEAD + half * G::HEAD_BYTES);
-    const uint32_t bar_acc = s_bar + (2 * NSLOT + half) * 8u;
-    const uint32_t tmem = *s_tmem + (uint32_t)half * 256u;
-    const uint32_t bar_id = 1u + (uint32_t)half;
-
-#ifdef ONB_NET_PROFILE
-    long long pf[8] = {0, 0, 0, 0, 0, 0, 0, 0}, pt = clock64();
-#endif
-    uint32_t q0 = 0, acc_par = 0;
-    for (int64_t gi = 0; gi < my_iters; ++gi) {
-        const int64_t board0 = (((int64_t)blockIdx.x + gi * gridDim.x) * 2 + half) * NB;
-        // ---- input planes -> the first channel chunks of the activation matrix (create_tensor_from_state layout [21][5][5])
-        {
-            const int cell = htid;
-            const Cell c = decode_cell(cell, CELLS);
-            if (c.real) {
-                const int64_t gb = board0 + c.board;
-                const float* src = planes + gb * 525 + c.pos;
-                float x[32];  // the planes are 0 / 1: exact in either operand format
-#pragma unroll
-                for (int ch = 0; ch < 32; ++ch) x[ch] = (ch < kInPlanes && gb < n) ? __ldg(src + ch * 25) : 0.f;
-                store_channels<F16>(s_act, R, kLead + cell, 0, x);  // 32 channels: planes 21..31 are zero
-            }
-        }
-        fence_proxy_async();
-        PF(0);
-        for (int l = 0; l < L; ++l) {
-            tc_fence_before();
-            named_bar_sync(bar_id, 256);
-            tc_fence_after();
-            PF(1);
-            const bool use_s = l >= 2 && (l & 1) == 0;  // second convolution of a block accumulates onto the parked residual
-            const bool last = l == L - 1;
-            if (hwarp == 0) {
-                // ---- MMA issue: 9 taps x K steps x 2 accumulators (the whole warp runs the loop, one lane issues)
-                const bool elected = elect_one();
-                const uint32_t dcol = tmem + (use_s ? NACC * 64 : 0);
-                auto issue_unit = [&](int g, int ksteps) {
-                    const uint32_t u = q0 + g, slot = u % NSLOT, use = u / NSLOT;
-                    mbar_wait(bar_full(slot), use & 1u);
-                    tc_fence_after();
-                    PF(2);
-#pragma unroll
-                    for (int tt = 0; tt < TPS; ++tt) {
-                        const int t = g * TPS + tt;
-                        issue_tap_mmas<F16, NACC>(elected, dcol, s_act, R, kLead + (t / 3 - 1) * 6 + (t % 3 - 1),
-                                                  s_ring + slot * (uint32_t)G::SLOT_BYTES + (uint32_t)tt * O::TAP_BYTES, ksteps, use_s || t > 0);
-                    }
-                    PF(3);
-                    if (elected) umma_commit(bar_empty(slot));  // the slot is free again once these MMAs have read it
-                    PF(7);
-                };
-                if (l == 0) {
-#pragma unroll 1
-                    for (int g = 0; g < UPL; ++g) issue_unit(g, O::KCH0 / 2);
-                } else {
-#pragma unroll 1
-                    for (int g = 0; g < UPL; ++g) issue_unit(g, O::KCH / 2);
-                }
-                if (elected) umma_commit(bar_acc);
-            }
-            __syncwarp();
-            mbar_wait(bar_acc, acc_par);
-            acc_par ^= 1u;
-            tc_fence_after();
-            PF(4);
-            // ---- epilogue: this thread owns one cell (TMEM lane) of accumulator hwarp / 4
-            const bool preload = (l & 1) == 0 && !last;  // this layer's output is a block input: park it (+ next bias) in TMEM
-            const float4* bias_l = reinterpret_cast<const float4*>(net.bias + (size_t)l * 64);
-            const float4* bias_n = reinterpret_cast<const float4*>(net.bias + (size_t)(preload ? l + 2 : l) * 64);
-            const float4* hw = reinterpret_cast<const float4*>(net.head);
-#ifdef ONB_NET_DBG_NOEPI
-            if (!last) { fence_proxy_async(); q0 += (uint32_t)UPL; continue; }
-#endif
-            {
-                const int a = hwarp >> 2;
-                const int cell = a * 128 + (hwarp & 3) * 32 + lane;
-                const Cell c = decode_cell(cell, CELLS);
-                const uint32_t tlane = tmem + ((uint32_t)((hwarp & 3) * 32) << 16);
-                const uint32_t tsrc = tlane + (use_s ? NACC * 64 : 0) + a * 64;
-                const uint32_t tskip = tlane + NACC * 64 + a * 64;
-                float hp0 = 0.f, hp1 = 0.f, hv = 0.f;
-#pragma unroll
-                for (int h = 0; h < 2; ++h) {
-                    uint32_t v[32];
-                    tmem_ld32(tsrc + h * 32, v);
-                    float o[32];
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        float4 b = make_float4(0.f, 0.f, 0.f, 0.f);
-                        if (!use_s) b = __ldg(bias_l + h * 8 + i);
-                        o[4 * i + 0] = fmaxf(__uint_as_float(v[4 * i + 0]) + b.x, 0.f);
-                        o[4 * i + 1] = fmaxf(__uint_as_float(v[4 * i + 1]) + b.y, 0.f);
-                        o[4 * i + 2] = fmaxf(__uint_as_float(v[4 * i + 2]) + b.z, 0.f);
-                        o[4 * i + 3] = fmaxf(__uint_as_float(v[4 * i + 3]) + b.w, 0.f);
-                    }
-                    if (!last && c.real) store_channels<F16>(s_act, R, kLead + cell, h * 32, o);
-                    if (preload) {
-#pragma unroll
-                        for (int i = 0; i < 8; ++i) {
-                            const float4 b = __ldg(bias_n + h * 8 + i);
-                            v[4 * i + 0] = __float_as_uint(o[4 * i + 0] + b.x);
-                            v[4 * i + 1] = __float_as_uint(o[4 * i + 1] + b.y);
-                            v[4 * i + 2] = __float_as_uint(o[4 * i + 2] + b.z);
-                            v[4 * i + 3] = __float_as_uint(o[4 * i + 3] + b.w);
-                        }
-                        tmem_st32(tskip + h * 32, v);
-                    }
-                    if (last) {  // 1x1 convolutions of both heads (net.rs: policy_conv 64 -> 2, vh_conv 64 -> 1)
-#pragma unroll
-                        for (int i = 0; i < 8; ++i) {
-                            const float4 w0 = __ldg(hw + (kHP0 / 4) + h * 8 + i), w1 = __ldg(hw + (kHP1 / 4) + h * 8 + i),
-                                         w2 = __ldg(hw + (kHV / 4) + h * 8 + i);
-                            hp0 = fmaf(o[4 * i + 0], w0.x, fmaf(o[4 * i + 1], w0.y, fmaf(o[4 * i + 2], w0.z, fmaf(o[4 * i + 3], w0.w, hp0))));
-                            hp1 = fmaf(o[4 * i + 0], w1.x, fmaf(o[4 * i + 1], w1.y, fmaf(o[4 * i + 2], w1.z, fmaf(o[4 * i + 3], w1.w, hp1))));
-                            hv = fmaf(o[4 * i + 0], w2.x, fmaf(o[4 * i + 1], w2.y, fmaf(o[4 * i + 2], w2.z, fmaf(o[4 * i + 3], w2.w, hv))));
-                        }
-                    }
-                }
-                if (last && c.real) {
-                    float* hb = s_head + c.board * 75;
-                    hb[c.pos] = fmaxf(hp0 + __ldg(net.head + kHB + 0), 0.f);
-                    hb[25 + c.pos] = fmaxf(hp1 + __ldg(net.head + kHB + 1), 0.f);
-                    hb[50 + c.pos] = fmaxf(hv + __ldg(net.head + kHB + 2), 0.f);
-                }
-            }
-            if (preload) tmem_wait_st();
-            fence_proxy_async();
-            q0 += (uint32_t)UPL;
-            PF(5);
-        }
-        // ---- heads: one warp per board (ph_linear2 + softmax, vh_linear1 + ReLU + vh_linear2 + tanh)
-        named_bar_sync(bar_id, 256);
-        for (int b = hwarp; b < NB; b += 8) {
-            const int64_t gb = board0 + b;
-            if (gb >= n) continue;
-            const float* hb = s_head + b * 75;
-            const bool two = lane + 32 < 50;
-            float l0 = __ldg(net.head + kPhB + lane), l1 = two ? __ldg(net.head + kPhB + 32 + lane) : 0.f;
-#pragma unroll 10
-            for (int i = 0; i < 50; ++i) {  // unrolled: ten independent weight loads in flight instead of one
-                const float x = hb[i];
-                l0 = fmaf(x, __ldg(net.head + kPhW + i * 50 + lane), l0);
-                if (two) l1 = fmaf(x, __ldg(net.head + kPhW + i * 50 + 32 + lane), l1);
-            }
-            const float m = warp_max(two ? fmaxf(l0, l1) : l0);
-            const float e0 = expf(l0 - m), e1 = two ? expf(l1 - m) : 0.f;
-            const float s = warp_sum(e0 + e1);
-            policy[gb * 50 + lane] = e0 / s;
-            if (two) policy[gb * 50 + 32 + lane] = e1 / s;
-            float h0 = __ldg(net.head + kV1B + lane), h1 = __ldg(net.head + kV1B + 32 + lane);
-#pragma unroll 5
-            for (int i = 0; i < 25; ++i) {
-                const float x = hb[50 + i];
-                h0 = fmaf(x, __ldg(net.head + kV1W + i * 64 + lane), h0);
-                h1 = fmaf(x, __ldg(net.head + kV1W + i * 64 + 32 + lane), h1);
-            }
-            float acc = fmaf(fmaxf(h0, 0.f), __ldg(net.head + kV2W + lane), fmaxf(h1, 0.f) * __ldg(net.head + kV2W + 32 + lane));
-            acc = warp_sum(acc);
-            if (lane == 0) value[gb] = tanhf(acc + __ldg(net.head + kV2B));
-        }
-        PF(6);
-    }
-#ifdef ONB_NET_PROFILE
-    if (blockIdx.x == (CL ? 2 : 3) && (htid == 0 || htid == 64))
-        printf("net2 profile tid %d iters %lld: input %lld barrier %lld weights %lld issue %lld commit %lld acc %lld epilogue %lld heads %lld\n", tid,
-               (long long)my_iters, pf[0], pf[1], pf[2], pf[3], pf[7], pf[4], pf[5], pf[6]);
-#endif
-    tc_fence_before();
-    named_bar_sync(3, 512);  // both halves are done with TMEM
-    if (warp == 0) tmem_dealloc(*s_tmem, 512);
-}
-
-// ---- the split-operand (f32-faithful) network as TWO independent halves of one CTA that share one weight stream ----------------------
-// The one-CTA-per-SM split kernel above (k_net_forward<2, f16, X3>) spends 63 % of its time issuing MMAs and the rest with the tensor
-// pipe idle (epilogue, barriers, heads): TMEM (512 columns) and shared memory (219 KB) leave no room for a second CTA to fill the gaps.
-// Here a CTA is two halves of 8 warps, each with ONE 128-row accumulator = 3 boards whose cells never straddle an accumulator (so the
-// halves share nothing but the weights), its own activation matrices (a1, a2: 2 x 16 KB), 256 TMEM columns ({D1|D2} x {plain,
-// residual-preloaded}) and its own MMA-issuing lane; they run out of phase, so one half's MMAs cover the other's epilogue. Warp 16
-// streams the (b1, b2) weight copies into a ring of 3 slots x 3 taps that is refilled when BOTH halves' MMAs have read a slot. The 8
-// warps of a half split the epilogue by channels (warps 0-3: channels 0-31, warps 4-7: channels 32-63 of the same 128 cells), 16
-// columns at a time to stay within 120 registers. Same products and accumulation order per accumulator as the one-CTA kernel (the
-// heads add the two channel halves in a different order: last-bit differences). MEASURED (B200, 16 384 positions, 3 blocks): 0.876 ms
-// when the halves run freely (they fall into step: both issue, then both run epilogues), 0.794 ms when they take turns issuing a
-// layer -- against 0.745 ms for the one-CTA kernel, which wastes no accumulator rows (252 of 256 vs 108 of 128) and streams the
-// weights once per 7 boards instead of 6. Kept behind ONB_NET_X3_HALVES=1; not the default.
-struct Geo2X {
-    static constexpr int NB = 3;  // boards per half: 108 cells in one 128-row accumulator
-    static constexpr int CELLS = NB * kCellsPerBoard;
-    static constexpr int R = (kLead + 128 + kTrail + 7) / 8 * 8;  // 144: an MMA reads 128 rows from any of the 15 shifted windows
-    static constexpr int TPS = 3, UPL = 3, NSLOT = 3;
-    static constexpr int TAP_STRIDE = 2 * Op<true>::TAP_BYTES;  // [b1 tap][b2 tap]
-    static constexpr int SLOT_BYTES = TPS * TAP_STRIDE;
-    static constexpr int ACT_BYTES = R * Op<true>::KCH * 16;  // one activation matrix
-    static constexpr int HALF_ACT = 2 * ACT_BYTES;              // a1 + a2
-    static constexpr int OFF_RING = 2 * HALF_ACT;
-    static constexpr int RING_BYTES = NSLOT * SLOT_BYTES;
-    static constexpr int OFF_HEAD = OFF_RING + RING_BYTES;
-    static constexpr int HEAD_BYTES = ((2 * NB * 75 * 4 + 15) / 16) * 16;  // per half: two partial sums (channels 0-31 / 32-63) per head input
-    static constexpr int OFF_BAR = OFF_HEAD + 2 * HEAD_BYTES;
-    static constexpr int SMEM = OFF_BAR + (2 * NSLOT + 4) * 8 + 16;
-    static constexpr int THREADS = 17 * 32;
-    static_assert(CELLS <= 128 && R >= kLead + 128 + kTrail - 1, "one accumulator per half; shifted windows stay inside the matrix");
-    static_assert(ACT_BYTES % 1024 == 0 && OFF_RING % 1024 == 0, "swizzle period");
-    static_assert(SMEM <= 227 * 1024, "shared memory");
-};
-__global__ void __launch_bounds__(Geo2X::THREADS, 1)
-    k_net_forward2x(const float* __restrict__ planes, float* __restrict__ policy, float* __restrict__ value, int64_t n, NetDev net) {
-    using G = Geo2X;
-    using O = Op<true>;
-    constexpr int NB = G::NB, CELLS = G::CELLS, R = G::R, NSLOT = G::NSLOT;
-    constexpr uint32_t A2 = (uint32_t)G::ACT_BYTES, SET = 128u;
-    extern __shared__ __align__(1024) uint8_t smem[];
-    const uint32_t s_base = smem_u32(smem), s_ring = s_base + G::OFF_RING, s_bar = s_base + G::OFF_BAR;
-    uint32_t* s_tmem = reinterpret_cast<uint32_t*>(smem + G::OFF_BAR + (2 * NSLOT + 4) * 8);
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int L = 1 + 2 * net.n_blocks;
-    const int64_t n_groups = (n + NB - 1) / NB;
-    // iteration i of this CTA: half h works on group (blockIdx.x + i * gridDim.x) * 2 + h (possibly past the end: computed, not stored)
-    const int64_t n_pairs = (n_groups + 1) / 2;
-    if ((int64_t)blockIdx.x >= n_pairs) return;
-    const int64_t my_iters = (n_pairs - blockIdx.x + gridDim.x - 1) / gridDim.x;
-    constexpr int TPS = G::TPS, UPL = G::UPL;
-    const uint32_t total_units = (uint32_t)my_iters * (uint32_t)(UPL * L);
-    auto bar_full = [&](uint32_t s) { return s_bar + s * 8u; };
-    auto bar_empty = [&](uint32_t s) { return s_bar + (NSLOT + s) * 8u; };
-
-    if (tid == 0) {
-        for (uint32_t s = 0; s < (uint32_t)NSLOT; ++s) {
-            mbar_init(bar_full(s), 1);
-            mbar_init(bar_empty(s), 2);  // both halves' MMAs must have read the slot
-        }
-        mbar_init(s_bar + 2 * NSLOT * 8u, 1);
-        mbar_init(s_bar + (2 * NSLOT + 1) * 8u, 1);
-        // the halves take turns issuing a layer's MMAs (half 0 first): left alone they fall into step -- both issue, then both run
-        // their epilogues with the tensor pipe idle -- and the kernel is slower than the one-CTA version (measured 0.876 vs 0.745 ms)
-        mbar_init(s_bar + (2 * NSLOT + 2) * 8u, 1);
-        mbar_init(s_bar + (2 * NSLOT + 3) * 8u, 1);
-        fence_barrier_init();
-        asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(s_bar + (2 * NSLOT + 2) * 8u) : "memory");  // half 0 may start
-    }
-    if (warp == 0) tmem_alloc(smem_u32(s_tmem), 512);
-    for (int i = tid; i < 2 * G::HALF_ACT / 16; i += G::THREADS) st_shared_v4(s_base + i * 16, 0u, 0u, 0u, 0u);  // pad cells stay zero
-    fence_proxy_async();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-
-    if (warp == 16) {
-        // ---- weight producer (one lane): the ring is filled strictly in tap order, as far ahead as it has free slots
-        if (lane == 0) {
-            for (uint32_t u = 0; u < total_units; ++u) {
-                const uint32_t slot = u % NSLOT, use = u / NSLOT;
-                if (use >= 1) mbar_wait(bar_empty(slot), (use - 1u) & 1u);
-                const uint32_t ul = u % (uint32_t)(UPL * L), layer = ul / UPL, tap = (ul - layer * UPL) * TPS;
-                const uint8_t* src = net.wconv + (size_t)2 * (layer == 0 ? (size_t)tap * O::TAP_BYTES0
-                                                                          : (size_t)9 * O::TAP_BYTES0 + ((size_t)(layer - 1) * 9 + tap) * O::TAP_BYTES);
-                const uint32_t bytes = (uint32_t)(2 * TPS) * (layer == 0 ? O::TAP_BYTES0 : O::TAP_BYTES);
-                mbar_expect_tx(bar_full(slot), bytes);
-                bulk_g2s(s_ring + slot * (uint32_t)G::SLOT_BYTES, src, bytes, bar_full(slot));
-            }
-        }
-        return;  // the workers only use named barriers from here on
-    }
-
-    const int half = warp >> 3, hwarp = warp & 7, htid = tid & 255;
-    const uint32_t s_act = s_base + (uint32_t)half * G::HALF_ACT;
-    float* s_head = reinterpret_cast<float*>(smem + G::OFF_HEAD + half * G::HEAD_BYTES);  // [2 channel halves][NB][75] partial sums
-    const uint32_t bar_acc = s_bar + (2 * NSLOT + half) * 8u;
-    const uint32_t bar_turn_mine = s_bar + (2 * NSLOT + 2 + half) * 8u, bar_turn_other = s_bar + (2 * NSLOT + 2 + (half ^ 1)) * 8u;
-    uint32_t turn_par = 0;
-    const uint32_t tmem = *s_tmem + (uint32_t)half * 256u;
-    const uint32_t bar_id = 1u + (uint32_t)half;
-
-    uint32_t q0 = 0, acc_par = 0;
-    for (int64_t gi = 0; gi < my_iters; ++gi) {
-        const int64_t board0 = (((int64_t)blockIdx.x + gi * gridDim.x) * 2 + half) * NB;
-        // ---- input planes -> the first channel chunks of both activation matrices (create_tensor_from_state layout [21][5][5])
-        if (htid < 128) {
-            const int cell = htid;
-            const Cell c = decode_cell(cell, CELLS);
-            if (c.real) {
-                const int64_t gb = board0 + c.board;
-                const float* src = planes + gb * 525 + c.pos;
-#pragma unroll
-                for (int part = 0; part < 2; ++part) {
-                    float x[16];  // the planes are 0 / 1: exact, the second operand part is zero
-#pragma unroll
-                    for (int ch = 0; ch < 16; ++ch) x[ch] = (part * 16 + ch < kInPlanes && gb < n) ? __ldg(src + (part * 16 + ch) * 25) : 0.f;
-                    store_channels_x3_16(s_act, A2, R, kLead + cell, part * 16, x);  // 32 channels: planes 21..31 are zero
-                }
-            }
-        }
-        fence_proxy_async();
-        for (int l = 0; l < L; ++l) {
-            tc_fence_before();
-            named_bar_sync(bar_id, 256);
-            tc_fence_after();
-            const bool use_s = l >= 2 && (l & 1) == 0;  // second convolution of a block accumulates onto the parked residual
-            const bool last = l == L - 1;
-            if (hwarp == 0) {
-                // ---- MMA issue: 9 taps x K steps x {a1 x [b1;b2] (N = 128), a2 x b1 (N = 64)} (the whole warp runs the loop, one lane issues)
-                const bool elected = elect_one();
-                const uint32_t dcol = tmem + (use_s ? SET : 0u);
-                mbar_wait(bar_turn_mine, turn_par);  // the other half has issued its layer: ours queues behind it while it runs its epilogue
-                turn_par ^= 1u;
-                auto issue_unit = [&](int g, int ksteps) {
-                    const uint32_t u = q0 + g, slot = u % NSLOT, use = u / NSLOT;
-                    mbar_wait(bar_full(slot), use & 1u);
-                    tc_fence_after();
-#pragma unroll
-                    for (int tt = 0; tt < TPS; ++tt) {
-                        const int t = g * TPS + tt;
-                        issue_tap_mmas<true, 1, true>(elected, dcol, s_act, R, kLead + (t / 3 - 1) * 6 + (t % 3 - 1),
-                                                      s_ring + slot * (uint32_t)G::SLOT_BYTES + (uint32_t)tt * (uint32_t)G::TAP_STRIDE, ksteps,
-                                                      use_s || t > 0, A2);
-                    }
-                    if (elected) umma_commit(bar_empty(slot));  // the slot is free again once BOTH halves' MMAs have read it
-                };
-                if (l == 0) {
-#pragma unroll 1
-                    for (int g = 0; g < UPL; ++g) issue_unit(g, O::KCH0 / 2);
-                } else {
-#pragma unroll 1
-                    for (int g = 0; g < UPL; ++g) issue_unit(g, O::KCH / 2);
-                }
-                if (elected) {
-                    umma_commit(bar_acc);
-                    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar_turn_other) : "memory");
-                }
-            }
-            __syncwarp();
-            mbar_wait(bar_acc, acc_par);
-            acc_par ^= 1u;
-            tc_fence_after();
-            // ---- epilogue: this thread owns one cell (TMEM lane) and 32 of its 64 channels, 16 at a time
-            const bool preload = (l & 1) == 0 && !last;  // this layer's output is a block input: park it (+ next bias) in TMEM
-            const float4* bias_l = reinterpret_cast<const float4*>(net.bias + (size_t)l * 64);
-            const float4* bias_n = reinterpret_cast<const float4*>(net.bias + (size_t)(preload ? l + 2 : l) * 64);
-            const float4* hw = reinterpret_cast<const float4*>(net.head);
-            {
-                const int ch_half = hwarp >> 2;  // 0: channels 0-31, 1: channels 32-63
-                const int cell = (hwarp & 3) * 32 + lane;
-                const Cell c = decode_cell(cell, CELLS);
-                const uint32_t tlane = tmem + ((uint32_t)((hwarp & 3) * 32) << 16);
-                const uint32_t tsrc = tlane + (use_s ? SET : 0u);
-                const uint32_t tskip = tlane + SET;
-                float hp0 = 0.f, hp1 = 0.f, hv = 0.f;
-#pragma unroll
-                for (int q = 0; q < 2; ++q) {
-                    const int c0 = ch_half * 32 + q * 16;  // first channel of this piece
-                    uint32_t v[16], v2[16];
-                    tmem_ld16_nowait(tsrc + c0, v);
-                    tmem_ld16_nowait(tsrc + 64 + c0, v2);
-                    tmem_wait_ld();
-                    float o[16];
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        float4 b = make_float4(0.f, 0.f, 0.f, 0.f);
-                        if (!use_s) b = __ldg(bias_l + c0 / 4 + i);
-                        o[4 * i + 0] = fmaxf(fmaf(__uint_as_float(v2[4 * i + 0]), kX3InvScale, __uint_as_float(v[4 * i + 0])) + b.x, 0.f);
-                        o[4 * i + 1] = fmaxf(fmaf(__uint_as_float(v2[4 * i + 1]), kX3InvScale, __uint_as_float(v[4 * i + 1])) + b.y, 0.f);
-                        o[4 * i + 2] = fmaxf(fmaf(__uint_as_float(v2[4 * i + 2]), kX3InvScale, __uint_as_float(v[4 * i + 2])) + b.z, 0.f);
-                        o[4 * i + 3] = fmaxf(fmaf(__uint_as_float(v2[4 * i + 3]), kX3InvScale, __uint_as_float(v[4 * i + 3])) + b.w, 0.f);
-                    }
-                    if (!last && c.real) store_channels_x3_16(s_act, A2, R, kLead + cell, c0, o);
-                    if (preload) {
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            const float4 b = __ldg(bias_n + c0 / 4 + i);
-                            v[4 * i + 0] = __float_as_uint(o[4 * i + 0] + b.x);
-                            v[4 * i + 1] = __float_as_uint(o[4 * i + 1] + b.y);
-                            v[4 * i + 2] = __float_as_uint(o[4 * i + 2] + b.z);
-                            v[4 * i + 3] = __float_as_uint(o[4 * i + 3] + b.w);
-                        }
-                        tmem_st16(tskip + c0, v);
-#pragma unroll
-                        for (int i = 0; i < 16; ++i) v2[i] = 0u;  // the D2 half of the preloaded accumulator starts from zero
-                        tmem_st16(tskip + 64 + c0, v2);
-                    }
-                    if (last) {  // 1x1 convolutions of both heads (net.rs: policy_conv 64 -> 2, vh_conv 64 -> 1), this thread's channels
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            const float4 w0 = __ldg(hw + (kHP0 / 4) + c0 / 4 + i), w1 = __ldg(hw + (kHP1 / 4) + c0 / 4 + i),
-                                         w2 = __ldg(hw + (kHV / 4) + c0 / 4 + i);
-                            hp0 = fmaf(o[4 * i + 0], w0.x, fmaf(o[4 * i + 1], w0.y, fmaf(o[4 * i + 2], w0.z, fmaf(o[4 * i + 3], w0.w, hp0))));
-                            hp1 = fmaf(o[4 * i + 0], w1.x, fmaf(o[4 * i + 1], w1.y, fmaf(o[4 * i + 2], w1.z, fmaf(o[4 * i + 3], w1.w, hp1))));
-                            hv = fmaf(o[4 * i + 0], w2.x, fmaf(o[4 * i + 1], w2.y, fmaf(o[4 * i + 2], w2.z, fmaf(o[4 * i + 3], w2.w, hv))));
-                        }
-                    }
-                }
-                if (last && c.real) {  // partial sums over this thread's 32 channels; the heads add the two halves, the bias and the ReLU
-                    float* hb = s_head + (ch_half * NB + c.board) * 75;
-                    hb[c.pos] = hp0;
-                    hb[25 + c.pos] = hp1;
-                    hb[50 + c.pos] = hv;
-                }
-            }
-            if (preload) tmem_wait_st();
-            fence_proxy_async();
-            q0 += (uint32_t)UPL;
-        }
-        // ---- heads: one warp per board (ph_linear2 + softmax, vh_linear1 + ReLU + vh_linear2 + tanh)
-        named_bar_sync(bar_id, 256);
-        for (int b = hwarp; b < NB; b += 8) {
-            const int64_t gb = board0 + b;
-            if (gb >= n) continue;
-            const float *h0p = s_head + b * 75, *h1p = s_head + (NB + b) * 75;
-            const float bp0 = __ldg(net.head + kHB + 0), bp1 = __ldg(net.head + kHB + 1), bv = __ldg(net.head + kHB + 2);
-            const bool two = lane + 32 < 50;
-            float l0 = __ldg(net.head + kPhB + lane), l1 = two ? __ldg(net.head + kPhB + 32 + lane) : 0.f;
-#pragma unroll 10
-            for (int i = 0; i < 50; ++i) {
-                const float x = fmaxf(h0p[i] + h1p[i] + (i < 25 ? bp0 : bp1), 0.f);
-                l0 = fmaf(x, __ldg(net.head + kPhW + i * 50 + lane), l0);
-                if (two) l1 = fmaf(x, __ldg(net.head + kPhW + i * 50 + 32 + lane), l1);
-            }
-            const float m = warp_max(two ? fmaxf(l0, l1) : l0);
-            const float e0 = expf(l0 - m), e1 = two ? expf(l1 - m) : 0.f;
-            const float s = warp_sum(e0 + e1);
-            policy[gb * 50 + lane] = e0 / s;
-            if (two) policy[gb * 50 + 32 + lane] = e1 / s;
-            float h0 = __ldg(net.head + kV1B + lane), h1 = __ldg(net.head + kV1B + 32 + lane);
-#pragma unroll 5
-            for (int i = 0; i < 25; ++i) {
-                const float x = fmaxf(h0p[50 + i] + h1p[50 + i] + bv, 0.f);
-                h0 = fmaf(x, __ldg(net.head + kV1W + i * 64 + lane), h0);
-                h1 = fmaf(x, __ldg(net.head + kV1W + i * 64 + 32 + lane), h1);
-            }
-            float acc = fmaf(fmaxf(h0, 0.f), __ldg(net.head + kV2W + lane), fmaxf(h1, 0.f) * __ldg(net.head + kV2W + 32 + lane));
-            acc = warp_sum(acc);
-            if (lane == 0) value[gb] = tanhf(acc + __ldg(net.head + kV2B));
-        }
-    }
-    tc_fence_before();
-    named_bar_sync(3, 512);  // both halves are done with TMEM
-    if (warp == 0) tmem_dealloc(*s_tmem, 512);
-}
-
-// ---- version 3: three CTAs per SM ---------------------------------------------------------------------------------------------
-// The phase timers of version 1 show ~4.2 k cycles per layer and CTA with no MMA in flight against 4.8 k of MMA issue, and TMEM (two
-// accumulators + two parked residuals = 256 columns per CTA) is what limits an SM to two CTAs. Here the residual lives in an
-// L2-resident global scratch instead (f32, written by the epilogue that produces a block input, read back by the epilogue of the
-// block's second convolution -- 64 KB per CTA, coalesced 16-byte accesses), a CTA needs only its two accumulators (128 columns),
-// the weight ring holds single taps (4 x 8 KB), and the epilogue works on 16 channels at a time to fit 80 registers: three CTAs of
-// 7 boards per SM, so that a third group's MMAs fill the gaps of the other two. f16 operands only.
-struct Geo3 {
-    static constexpr int NB = 7, CELLS = NB * kCellsPerBoard, R = (kLead + CELLS + kTrail + 7) / 8 * 8;
-    static constexpr int NSLOT = 4;
-    static constexpr int ACT_BYTES = R * 128;
-    static constexpr int OFF_RING = ACT_BYTES;
-    static constexpr int RING_BYTES = NSLOT * Op<true>::TAP_BYTES;
-    static constexpr int OFF_HEAD = OFF_RING + RING_BYTES;
-    static constexpr int HEAD_BYTES = ((NB * 75 * 4 + 15) / 16) * 16;
-    static constexpr int OFF_BAR = OFF_HEAD + HEAD_BYTES;
-    static constexpr int SMEM = OFF_BAR + (2 * NSLOT + 1) * 8 + 16;
-    static constexpr int TMEM_COLS = 128;
-    static constexpr int SCRATCH_FLOAT4 = 16 * 256;  // residual scratch per CTA: [16 chunks of 4 channels][256 cells]
-    static_assert(SMEM * 3 <= 227 * 1024, "three CTAs per SM");
-};
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]), "=r"(v[10]),
-          "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-        : "r"(taddr)
-        : "memory");
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-}
-
-__global__ void __launch_bounds__(256, 3)
-    k_net_forward3(const float* __restrict__ planes, float* __restrict__ policy, float* __restrict__ value, int64_t n, NetDev net,
-                   float4* __restrict__ scratch) {
-    using G = Geo3;
-    using O = Op<true>;
-    constexpr int NB = G::NB, CELLS = G::CELLS, R = G::R, NSLOT = G::NSLOT, NACC = 2;
-    extern __shared__ __align__(1024) uint8_t smem[];
-    const uint32_t s_act = smem_u32(smem), s_ring = s_act + G::OFF_RING, s_bar = s_act + G::OFF_BAR;
-    float* s_head = reinterpret_cast<float*>(smem + G::OFF_HEAD);
-    uint32_t* s_tmem = reinterpret_cast<uint32_t*>(smem + G::OFF_BAR + (2 * NSLOT + 1) * 8);
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int L = 1 + 2 * net.n_blocks;
-    const int64_t n_groups = (n + NB - 1) / NB;
-    if ((int64_t)blockIdx.x >= n_groups) return;  // whole CTA, before any allocation
-    const int64_t my_groups = (n_groups - blockIdx.x + gridDim.x - 1) / gridDim.x;
-    const uint32_t total_taps = (uint32_t)my_groups * 9u * (uint32_t)L;
-    auto bar_full = [&](uint32_t s) { return s_bar + s * 8u; };
-    auto bar_empty = [&](uint32_t s) { return s_bar + (NSLOT + s) * 8u; };
-    const uint32_t bar_acc = s_bar + 2 * NSLOT * 8u;
-    float4* skip = scratch + (size_t)blockIdx.x * G::SCRATCH_FLOAT4 + tid;  // + chunk * 256
-
-    if (tid == 0) {
-        for (uint32_t s = 0; s < (uint32_t)NSLOT; ++s) {
-            mbar_init(bar_full(s), 1);
-            mbar_init(bar_empty(s), 1);
-        }
-        mbar_init(bar_acc, 1);
-        fence_barrier_init();
-    }
-    if (warp == 0) tmem_alloc(smem_u32(s_tmem), G::TMEM_COLS);
-    for (int i = tid; i < G::ACT_BYTES / 16; i += 256) st_shared_v4(s_act + i * 16, 0u, 0u, 0u, 0u);  // pad cells stay zero for good
-    fence_proxy_async();
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = *s_tmem;
-
-    uint32_t q0 = 0, q_prod = 0, acc_par = 0;
-    const int a = warp >> 2;                               // this thread's accumulator and cell
-    const int cell = a * 128 + (warp & 3) * 32 + lane;
-    const Cell c = decode_cell(cell, CELLS);
-    const uint32_t tsrc = tmem + ((uint32_t)((warp & 3) * 32) << 16) + a * 64;
-    for (int64_t gi = 0; gi < my_groups; ++gi) {
-        const int64_t board0 = ((int64_t)blockIdx.x + gi * gridDim.x) * NB;
-        // ---- input planes -> the first channel chunks of the activation matrix
-        if (c.real) {
-            const int64_t gb = board0 + c.board;
-            const float* src = planes + gb * 525 + c.pos;
-#pragma unroll
-            for (int q = 0; q < 2; ++q) {  // 32 channels (planes 21..31 are zero), 16 at a time
-                float x[16];
-#pragma unroll
-                for (int ch = 0; ch < 16; ++ch) x[ch] = (q * 16 + ch < kInPlanes && gb < n) ? __ldg(src + (q * 16 + ch) * 25) : 0.f;
-#pragma unroll
-                for (int i = 0; i < 2; ++i)
-                    st_shared_v4(act_addr(s_act, R, kLead + cell, q * 2 + i), to_f16x2(x[8 * i + 0], x[8 * i + 1]), to_f16x2(x[8 * i + 2], x[8 * i + 3]),
-                                 to_f16x2(x[8 * i + 4], x[8 * i + 5]), to_f16x2(x[8 * i + 6], x[8 * i + 7]));
-            }
-        }
-        fence_proxy_async();
-        for (int l = 0; l < L; ++l) {
-            tc_fence_before();
-            __syncthreads();
-            tc_fence_after();
-            const bool second = l >= 2 && (l & 1) == 0;  // second convolution of a block: the residual is added in the epilogue
-            const bool last = l == L - 1;
-            if (warp == 0) {
-                // ---- MMA issue (the whole warp runs the loop, one lane issues)
-                const bool elected = elect_one();
-                const int ksteps = (l == 0 ? O::KCH0 : O::KCH) / 2;
-#pragma unroll 1
-                for (int t = 0; t < 9; ++t) {
-                    const uint32_t q = q0 + t, slot = q % NSLOT, use = q / NSLOT;
-                    mbar_wait(bar_full(slot), use & 1u);
-                    tc_fence_after();
-                    issue_tap_mmas<true, NACC>(elected, tmem, s_act, R, kLead + (t / 3 - 1) * 6 + (t % 3 - 1), s_ring + slot * (uint32_t)O::TAP_BYTES,
-                                               ksteps, t > 0);
-                    if (elected) umma_commit(bar_empty(slot));
-                }
-                if (elected) umma_commit(bar_acc);
-            } else if (tid == 32) {
-                // ---- weight producer: keeps the ring NSLOT taps ahead of the MMAs
-                const uint32_t target = min(q0 + 9u + (uint32_t)NSLOT, total_taps);
-                while (q_prod < target) {
-                    const uint32_t slot = q_prod % NSLOT, use = q_prod / NSLOT;
-                    if (use >= 1) mbar_wait(bar_empty(slot), (use - 1u) & 1u);
-                    const uint32_t ql = q_prod % (9u * (uint32_t)L);
-                    mbar_expect_tx(bar_full(slot), O::TAP_BYTES);
-                    bulk_g2s(s_ring + slot * (uint32_t)O::TAP_BYTES, net.wconv + (size_t)ql * O::TAP_BYTES, O::TAP_BYTES, bar_full(slot));
-                    ++q_prod;
-                }
-            }
-            __syncwarp();
-            mbar_wait(bar_acc, acc_par);
-            acc_par ^= 1u;
-            tc_fence_after();
-            // ---- epilogue: 16 channels at a time
-            const bool park = (l & 1) == 0 && !last;  // this layer's output is a block input: keep it for the residual add
-            const float4* bias_l = reinterpret_cast<const float4*>(net.bias + (size_t)l * 64);
-            const float4* hw = reinterpret_cast<const float4*>(net.head);
-            float hp0 = 0.f, hp1 = 0.f, hv = 0.f;
-#pragma unroll 1
-            for (int h = 0; h < 4; ++h) {
-                uint32_t v[16];
-                tmem_ld16(tsrc + h * 16, v);
-                float o[16];
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    const float4 b = __ldg(bias_l + h * 4 + i);
-                    float4 r = make_float4(0.f, 0.f, 0.f, 0.f);
-                    if (second) r = __ldcg(skip + (h * 4 + i) * 256);
-                    o[4 * i + 0] = fmaxf(__uint_as_float(v[4 * i + 0]) + b.x + r.x, 0.f);
-                    o[4 * i + 1] = fmaxf(__uint_as_float(v[4 * i + 1]) + b.y + r.y, 0.f);
-                    o[4 * i + 2] = fmaxf(__uint_as_float(v[4 * i + 2]) + b.z + r.z, 0.f);
-                    o[4 * i + 3] = fmaxf(__uint_as_float(v[4 * i + 3]) + b.w + r.w, 0.f);
-                    if (park) __stcg(skip + (h * 4 + i) * 256, make_float4(o[4 * i + 0], o[4 * i + 1], o[4 * i + 2], o[4 * i + 3]));
-                }
-                if (!last && c.real) {
-#pragma unroll
-                    for (int i = 0; i < 2; ++i)
-                        st_shared_v4(act_addr(s_act, R, kLead + cell, h * 2 + i), to_f16x2(o[8 * i + 0], o[8 * i + 1]), to_f16x2(o[8 * i + 2], o[8 * i + 3]),
-                                     to_f16x2(o[8 * i + 4], o[8 * i + 5]), to_f16x2(o[8 * i + 6], o[8 * i + 7]));
-                }
-                if (last) {  // 1x1 convolutions of both heads
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const float4 w0 = __ldg(hw + (kHP0 / 4) + h * 4 + i), w1 = __ldg(hw + (kHP1 / 4) + h * 4 + i), w2 = __ldg(hw + (kHV / 4) + h * 4 + i);
-                        hp0 = fmaf(o[4 * i + 0], w0.x, fmaf(o[4 * i + 1], w0.y, fmaf(o[4 * i + 2], w0.z, fmaf(o[4 * i + 3], w0.w, hp0))));
-                        hp1 = fmaf(o[4 * i + 0], w1.x, fmaf(o[4 * i + 1], w1.y, fmaf(o[4 * i + 2], w1.z, fmaf(o[4 * i + 3], w1.w, hp1))));
-                        hv = fmaf(o[4 * i + 0], w2.x, fmaf(o[4 * i + 1], w2.y, fmaf(o[4 * i + 2], w2.z, fmaf(o[4 * i + 3], w2.w, hv))));
-                    }
-                }
-            }
-            if (last && c.real) {
-                float* hb = s_head + c.board * 75;
-                hb[c.pos] = fmaxf(hp0 + __ldg(net.head + kHB + 0), 0.f);
-                hb[25 + c.pos] = fmaxf(hp1 + __ldg(net.head + kHB + 1), 0.f);
-                hb[50 + c.pos] = fmaxf(hv + __ldg(net.head + kHB + 2), 0.f);
-            }
-            fence_proxy_async();
-            q0 += 9u;
-        }
-        // ---- heads: one warp per board
-        __syncthreads();
-        for (int b = warp; b < NB; b += 8) {
-            const int64_t gb = board0 + b;
-            if (gb >= n) continue;
-            const float* hb = s_head + b * 75;
-            const bool two = lane + 32 < 50;
-            float l0 = __ldg(net.head + kPhB + lane), l1 = two ? __ldg(net.head + kPhB + 32 + lane) : 0.f;
-            for (int i = 0; i < 50; ++i) {
-                const float x = hb[i];
-                l0 = fmaf(x, __ldg(net.head + kPhW + i * 50 + lane), l0);
-                if (two) l1 = fmaf(x, __ldg(net.head + kPhW + i * 50 + 32 + lane), l1);
-            }
-            const float m = warp_max(two ? fmaxf(l0, l1) : l0);
-            const float e0 = expf(l0 - m), e1 = two ? expf(l1 - m) : 0.f;
-            const float s = warp_sum(e0 + e1);
-            policy[gb * 50 + lane] = e0 / s;
-            if (two) policy[gb * 50 + 32 + lane] = e1 / s;
-            float h0 = __ldg(net.head + kV1B + lane), h1 = __ldg(net.head + kV1B + 32 + lane);
-            for (int i = 0; i < 25; ++i) {
-                const float x = hb[50 + i];
-                h0 = fmaf(x, __ldg(net.head + kV1W + i * 64 + lane), h0);
-                h1 = fmaf(x, __ldg(net.head + kV1W + i * 64 + 32 + lane), h1);
-            }
-            float acc = fmaf(fmaxf(h0, 0.f), __ldg(net.head + kV2W + lane), fmaxf(h1, 0.f) * __ldg(net.head + kV2W + 32 + lane));
-            acc = warp_sum(acc);
-            if (lane == 0) value[gb] = tanhf(acc + __ldg(net.head + kV2B));
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc(tmem, G::TMEM_COLS);
 }
 
 // ---- 128 hidden channels (ConvResNetConfig{hidden_channels: 128}) ---------------------------------------------------------------
@@ -3288,57 +2292,24 @@ int32_t net_load(Ctx* c, int32_t n_tensors, const char* const* names, const floa
     return upload_net(c, wconv, bias, head, n_blocks, 64, f16, x3, pair_off, err);
 }
 
-template <int NACC, bool F16, bool X3 = false>
+template <bool F16, bool X3 = false>
 static cudaError_t launch_net_variant(Ctx* c, const float* planes, float* policy, float* value, const NetDev& nd, int sms, int64_t count) {
-    using G = Geo<NACC, F16, X3>;
+    using G = Geo<F16, X3>;
     static bool attr[64] = {};  // the opt-in is per device
     int dev = 0;
     cudaGetDevice(&dev);
     if (dev < 0 || dev >= 64 || !attr[dev]) {
-        const cudaError_t e = cudaFuncSetAttribute(k_net_forward<NACC, F16, X3>, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM);
+        const cudaError_t e = cudaFuncSetAttribute(k_net_forward<F16, X3>, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM);
         if (e != cudaSuccess) return e;
         if (dev >= 0 && dev < 64) attr[dev] = true;
     }
-    const char* one = getenv("ONB_NET_ONE_CTA");  // experiment: a single CTA per SM (is the MMA issue time contention or a per-thread limit?)
-    const int64_t groups = (count + G::NB - 1) / G::NB, slots = (int64_t)sms * ((NACC == 2 && !X3 && !(one && one[0] == '1')) ? 2 : 1);
-    k_net_forward<NACC, F16, X3><<<(unsigned)(groups < slots ? groups : slots), 256, G::SMEM, c->stream>>>(planes, policy, value, count, nd);
-    return cudaGetLastError();
-}
-
-template <bool F16>
-static cudaError_t launch_net_v2(Ctx* c, const float* planes, float* policy, float* value, const NetDev& nd, int sms, int64_t count) {
-    using G = Geo2<F16>;
-    static bool attr[64] = {};  // the opt-in is per device
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr[dev]) {
-        const cudaError_t e = cudaFuncSetAttribute(k_net_forward2<F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM);
-        if (e != cudaSuccess) return e;
-        if (dev >= 0 && dev < 64) attr[dev] = true;
-    }
-    const int64_t pairs = ((count + G::NB - 1) / G::NB + 1) / 2;
-    k_net_forward2<F16><<<(unsigned)(pairs < sms ? pairs : sms), G::THREADS, G::SMEM, c->stream>>>(planes, policy, value, count, nd);
-    return cudaGetLastError();
-}
-
-static cudaError_t launch_net_f16p(Ctx* c, const float* planes, float* policy, float* value, const NetDev& nd, int sms, int64_t count) {
-    using G = Geo<2, true, false>;
-    constexpr int kSmemF16P = G::OFF_BAR + GeoX3P::N_BARS * 8 + 16;
-    static bool attr[64] = {};  // the opt-in is per device
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr[dev]) {
-        const cudaError_t e = cudaFuncSetAttribute(k_net_forward_f16p, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemF16P);
-        if (e != cudaSuccess) return e;
-        if (dev >= 0 && dev < 64) attr[dev] = true;
-    }
-    const int64_t groups = (count + G::NB - 1) / G::NB, slots = (int64_t)sms * 2;
-    k_net_forward_f16p<<<(unsigned)(groups < slots ? groups : slots), kF16PThreads, kSmemF16P, c->stream>>>(planes, policy, value, count, nd);
+    const int64_t groups = (count + G::NB - 1) / G::NB, slots = (int64_t)sms * (X3 ? 1 : 2);
+    k_net_forward<F16, X3><<<(unsigned)(groups < slots ? groups : slots), 256, G::SMEM, c->stream>>>(planes, policy, value, count, nd);
     return cudaGetLastError();
 }
 
 static cudaError_t launch_net_x3p(Ctx* c, const float* planes, float* policy, float* value, const NetDev& nd, int sms, int64_t count) {
-    using G = Geo<2, true, true>;
+    using G = Geo<true, true>;
     static bool attr[64] = {};  // the opt-in is per device
     int dev = 0;
     cudaGetDevice(&dev);
@@ -3354,7 +2325,7 @@ static cudaError_t launch_net_x3p(Ctx* c, const float* planes, float* policy, fl
 
 // the CTA-pair build: clusters of two CTAs, as many as the device can hold at once (one CTA per SM)
 static cudaError_t launch_net_x3pair(Ctx* c, const float* planes, float* policy, float* value, const NetDev& nd, int sms, int64_t count) {
-    using G = Geo<2, true, true>;
+    using G = Geo<true, true>;
     using GP = GeoX3PT<true>;
     static int max_clusters[64] = {};  // per device; 0 = not asked yet
     int dev = 0;
@@ -3425,47 +2396,6 @@ static cudaError_t launch_net_f16q(Ctx* c, const float* planes, float* policy, f
     return cudaLaunchKernelEx(&cfg, k_net_forward_f16q<CL>, planes, (float*)policy, (float*)value, (int64_t)count, nd);
 }
 
-static cudaError_t launch_net_v2x(Ctx* c, const float* planes, float* policy, float* value, const NetDev& nd, int sms, int64_t count) {
-    using G = Geo2X;
-    static bool attr[64] = {};  // the opt-in is per device
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr[dev]) {
-        const cudaError_t e = cudaFuncSetAttribute(k_net_forward2x, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM);
-        if (e != cudaSuccess) return e;
-        if (dev >= 0 && dev < 64) attr[dev] = true;
-    }
-    const int64_t pairs = ((count + G::NB - 1) / G::NB + 1) / 2;
-    k_net_forward2x<<<(unsigned)(pairs < sms ? pairs : sms), G::THREADS, G::SMEM, c->stream>>>(planes, policy, value, count, nd);
-    return cudaGetLastError();
-}
-
-static cudaError_t launch_net_v3(Ctx* c, const float* planes, float* policy, float* value, const NetDev& nd, int sms, int64_t count) {
-    using G = Geo3;
-    static bool attr[64] = {};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64 || !attr[dev]) {
-        const cudaError_t e = cudaFuncSetAttribute(k_net_forward3, cudaFuncAttributeMaxDynamicSharedMemorySize, G::SMEM);
-        if (e != cudaSuccess) return e;
-        if (dev >= 0 && dev < 64) attr[dev] = true;
-    }
-    const int64_t groups = (count + G::NB - 1) / G::NB, slots = (int64_t)sms * 3;
-    const unsigned grid = (unsigned)(groups < slots ? groups : slots);
-    const size_t need = (size_t)grid * G::SCRATCH_FLOAT4 * sizeof(float4);
-    if (c->net_scratch_bytes < need) {
-        cudaStreamSynchronize(c->stream);
-        if (c->d_net_scratch) cudaFree(c->d_net_scratch);
-        c->d_net_scratch = nullptr;
-        c->net_scratch_bytes = 0;
-        const cudaError_t e = cudaMalloc(&c->d_net_scratch, need);
-        if (e != cudaSuccess) return e;
-        c->net_scratch_bytes = need;
-    }
-    k_net_forward3<<<grid, 256, G::SMEM, c->stream>>>(planes, policy, value, count, nd, reinterpret_cast<float4*>(c->d_net_scratch));
-    return cudaGetLastError();
-}
-
 // the 128-wide network: one CTA per SM, each working through board groups of GeoW::NB
 template <bool F16, bool X3>
 static cudaError_t launch_net_wide(Ctx* c, const float* planes, float* policy, float* value, const NetDev& nd, int sms, int64_t count) {
@@ -3499,12 +2429,8 @@ cudaError_t launch_net_forward(Ctx* c, const float* planes, float* policy, float
         // ONB_NET_F32: split operands, f32-faithful, one CTA per SM. Default: the warp-specialised pipeline on CTA pairs
         // (k_net_forward_x3p<true>, 0.600 ms per 16 384 positions); ONB_NET_X3_PAIR=0: the same pipeline on single CTAs (0.646 ms; also
         // the fallback when the device cannot co-schedule the clusters); ONB_NET_X3_PIPE=0: the plain kernel (0.745 ms).
-        // Exploration knob ONB_NET_X3_HALVES=1: two halves of 3 boards that share the weight stream and take turns issuing (0.794 ms:
-        // the overlap of one half's epilogue with the other's MMAs does not pay for 6 instead of 7 boards per weight pass)
-        const char* halves = getenv("ONB_NET_X3_HALVES");
-        if (halves && halves[0] == '1') return launch_net_v2x(c, planes, policy, value, nd, sms, count);
         const char* pipe = getenv("ONB_NET_X3_PIPE");
-        if (pipe && pipe[0] == '0') return launch_net_variant<2, true, true>(c, planes, policy, value, nd, sms, count);
+        if (pipe && pipe[0] == '0') return launch_net_variant<true, true>(c, planes, policy, value, nd, sms, count);
         const char* pair = getenv("ONB_NET_X3_PAIR");
         if (!(pair && pair[0] == '0')) {
             const cudaError_t e = launch_net_x3pair(c, planes, policy, value, nd, sms, count);
@@ -3513,33 +2439,18 @@ cudaError_t launch_net_forward(Ctx* c, const float* planes, float* policy, float
         }
         return launch_net_x3p(c, planes, policy, value, nd, sms, count);
     }
-    const char* v3 = getenv("ONB_NET_V3");  // three CTAs per SM, residual in an L2-resident scratch (f16 operands only)
-    if (v3 && v3[0] == '1' && c->net[c->net_cur].f16) return launch_net_v3(c, planes, policy, value, nd, sms, count);
-    const char* v2 = getenv("ONB_NET_V2");  // exploration knob: one CTA per SM whose two halves share the weight stream (0.392 vs 0.343 ms)
-    if (v2 && v2[0] == '1') return ns.f16 ? launch_net_v2<true>(c, planes, policy, value, nd, sms, count) : launch_net_v2<false>(c, planes, policy, value, nd, sms, count);
+    if (!ns.f16) return launch_net_variant<false>(c, planes, policy, value, nd, sms, count);  // ONB_NET_TF32: two plain CTAs per SM
     // ONB_NET_F16 default: one CTA per SM with four accumulators (14 boards), the pipeline of k_net_forward_x3p, on CTA pairs
     // (k_net_forward_f16q<true>, 0.226 ms per 16 384 positions); ONB_NET_F16_QUAD=2: on single CTAs (0.269 ms; also the fallback when
     // the clusters cannot be co-scheduled); ONB_NET_F16_QUAD=0: the round-1 build, two plain CTAs per SM (0.322 ms)
     const char* quad = getenv("ONB_NET_F16_QUAD");
-    const char* any_old = nullptr;
-    for (const char* knob : {"ONB_NET_V3", "ONB_NET_V2", "ONB_NET_F16_PIPE", "ONB_NET_WIDE", "ONB_NET_ONE_CTA"}) {
-        const char* v = getenv(knob);
-        if (v && v[0] == '1') any_old = v;  // an exploration knob of the older builds asks for them
+    if (quad && quad[0] == '0') return launch_net_variant<true>(c, planes, policy, value, nd, sms, count);
+    if (!(quad && quad[0] == '2')) {
+        const cudaError_t e = launch_net_f16q<true>(c, planes, policy, value, nd, sms, count);
+        if (e != cudaErrorLaunchOutOfResources) return e;
+        (void)cudaGetLastError();
     }
-    if (ns.f16 && !any_old && !(quad && quad[0] == '0')) {
-        if (!(quad && quad[0] == '2')) {
-            const cudaError_t e = launch_net_f16q<true>(c, planes, policy, value, nd, sms, count);
-            if (e != cudaErrorLaunchOutOfResources) return e;
-            (void)cudaGetLastError();
-        }
-        return launch_net_f16q<false>(c, planes, policy, value, nd, sms, count);
-    }
-    const char* f16p = getenv("ONB_NET_F16_PIPE");  // exploration knob: the warp-specialised pipeline for the f16 fast mode
-    if (f16p && f16p[0] == '1' && ns.f16) return launch_net_f16p(c, planes, policy, value, nd, sms, count);
-    const char* wide = getenv("ONB_NET_WIDE");  // exploration knob: 14 boards per CTA, one CTA per SM
-    const bool w = wide && wide[0] == '1';
-    if (ns.f16) return w ? launch_net_variant<4, true>(c, planes, policy, value, nd, sms, count) : launch_net_variant<2, true>(c, planes, policy, value, nd, sms, count);
-    return w ? launch_net_variant<4, false>(c, planes, policy, value, nd, sms, count) : launch_net_variant<2, false>(c, planes, policy, value, nd, sms, count);
+    return launch_net_f16q<false>(c, planes, policy, value, nd, sms, count);
 }
 
 }  // namespace onb

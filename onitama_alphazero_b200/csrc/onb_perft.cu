@@ -2,9 +2,8 @@
 //
 // Two phases: (1) lockstep breadth-first frontier expansion in HBM (32 B per node: read parent, write child)
 // until there are enough independent subtrees to fill the machine; (2) every frontier node is finished by one
-// thread's depth-first search with bulk counting at the last ply: k_perft_flat (flat state machine, stack in shared
-// memory, the shipped path) or k_perft_dfs (nested loops in registers, kept for comparison). Phase 2 moves ~0 bytes
-// per node and is issue-bound; see DESIGN.md.
+// thread's depth-first search with bulk counting at the last ply (k_perft_flat: a flat state machine, stack in shared
+// memory). Phase 2 moves ~0 bytes per node and is issue-bound; see DESIGN.md.
 #include <cstdlib>
 #include <cstring>
 #include <vector>
@@ -115,78 +114,9 @@ __global__ void __launch_bounds__(128) k_perft_expand(const uint4* __restrict__ 
     }
 }
 
-// ---- phase 2: register DFS ---------------------------------------------------------------------------------
-template <int REM>
-struct Dfs {
-    __device__ __forceinline__ static void run(const uint32_t* T, const Game& g, unsigned long long* nodes, unsigned long long* wins, uint32_t* zero) {
-        const uint32_t side = g.side;
-        const uint32_t own_p = side ? g.pawn_b : g.pawn_r, own_k = side ? g.king_b : g.king_r;
-        const uint32_t en_p = side ? g.pawn_r : g.pawn_b, en_k = side ? g.king_r : g.king_b;
-        const uint32_t own = own_p | own_k;
-        const uint32_t win_t = en_k & ~en_p;
-        const uint32_t temple = 1u << (side ? kRedTemple : kBlueTemple);
-        uint32_t total = 0, nwin = 0;
-#pragma unroll 1
-        for (uint32_t s = 0; s < 2; ++s) {
-            const uint32_t idx = side * 2u + s;
-            const uint32_t* Ts = T + (side * 16u + card_at(g.cards, idx)) * 25u;
-            uint32_t rem = own;
-#pragma unroll 1
-            while (rem) {
-                const int f = __ffs(rem) - 1;
-                rem &= rem - 1;
-                const uint32_t king = ((own_p >> f) & 1u) ^ 1u;
-                const uint32_t a = Ts[f] & ~own;
-                const uint32_t wm = a & (win_t | (king ? temple : 0u));
-                total += __popc(a);
-                nwin += __popc(wm);
-                if constexpr (REM > 1) {
-                    uint32_t b = a & ~wm;
-#pragma unroll 1
-                    while (b) {
-                        const uint32_t to = __ffs(b) - 1;
-                        b &= b - 1;
-                        Game ch = g;
-                        apply_move(ch, make_action(idx, (uint32_t)f, to, king));
-                        Dfs<REM - 1>::run(T, ch, nodes, wins, zero);
-                    }
-                }
-            }
-        }
-        nodes[REM - 1] += total;
-        wins[REM - 1] += nwin;
-        zero[REM - 1] += total == 0 ? 1u : 0u;
-    }
-};
-
-template <int REM>
-__global__ void __launch_bounds__(128) k_perft_dfs(const uint4* __restrict__ states, const uint32_t* __restrict__ roots, int64_t n_items,
-                                                   unsigned long long* __restrict__ nodes, unsigned long long* __restrict__ wins,
-                                                   unsigned long long* __restrict__ zero, int depth_total) {
-    __shared__ uint32_t s_att[800];
-    load_attack_table_to_smem(s_att);
-    __syncthreads();
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n_items) return;
-    const Game g = unpack(states[i]);
-    unsigned long long ln[REM], lw[REM];
-    uint32_t lz[REM];
-#pragma unroll
-    for (int k = 0; k < REM; ++k) { ln[k] = 0; lw[k] = 0; lz[k] = 0; }
-    Dfs<REM>::run(s_att, g, ln, lw, lz);
-    const int64_t row = (int64_t)roots[i] * depth_total;
-#pragma unroll
-    for (int k = 0; k < REM; ++k) {
-        const int d = depth_total - 1 - k;  // REM-1 == k levels from the bottom
-        if (ln[k]) atomicAdd(&nodes[row + d], ln[k]);
-        if (lw[k]) atomicAdd(&wins[row + d], lw[k]);
-        if (lz[k]) atomicAdd(&zero[row + d], (unsigned long long)lz[k]);
-    }
-}
-
-// ---- phase 2, flattened: one move per loop iteration -----------------------------------------------------------------------
-// The nested-loop DFS above keeps everything in registers but its lanes drift apart (each lane sits at a different nesting
-// level with a different trip count): ~14 % SIMT efficiency. This variant runs the same search as a state machine whose
+// ---- phase 2: depth-first search, one move per loop iteration ---------------------------------------------------------------
+// A nested-loop DFS keeps everything in registers but its lanes drift apart (each lane sits at a different nesting level with a
+// different trip count): ~14 % SIMT efficiency (DESIGN.md). This kernel runs the search as a state machine whose
 // iteration either advances the (slot, piece) iterator of the current node or plays ONE move; positions at the last interior
 // level are bulk-counted immediately. The per-level stack lives in shared memory ([level][word][thread], conflict free), the
 // current level in registers, so every lane executes the same short instruction stream in every iteration.
@@ -316,12 +246,8 @@ __global__ void __launch_bounds__(kFlatThreads, ONB_PERFT_MINB) k_perft_flat(con
 template <int REM>
 static cudaError_t launch_dfs(Ctx* c, const uint4* st, const uint32_t* rt, int64_t n_items, unsigned long long* nodes, unsigned long long* wins,
                               unsigned long long* zero, int depth) {
-    const char* legacy = getenv("ONB_PERFT_NESTED");  // exploration knob: the nested-loop register DFS
-    if (legacy && legacy[0] == '1')
-        k_perft_dfs<REM><<<(unsigned)((n_items + 127) / 128), 128, 0, c->stream>>>(st, rt, n_items, nodes, wins, zero, depth);
-    else
-        k_perft_flat<REM><<<(unsigned)((n_items + kFlatThreads - 1) / kFlatThreads), kFlatThreads, 0, c->stream>>>(st, rt, n_items, nodes, wins, zero,
-                                                                                                                 depth);
+    k_perft_flat<REM><<<(unsigned)((n_items + kFlatThreads - 1) / kFlatThreads), kFlatThreads, 0, c->stream>>>(st, rt, n_items, nodes, wins, zero,
+                                                                                                             depth);
     return cudaGetLastError();
 }
 
@@ -590,8 +516,7 @@ int32_t run_perft(Ctx* c, const onb_state* roots_host, int64_t n, int depth, uin
             PF(cudaStreamSynchronize(c->stream), "sync");
             int level = 0;
             // breadth-first while the frontier is too small to fill 148 SMs or the remaining depth exceeds the DFS template range
-            int64_t bfs_nodes = 1 << 21;
-            if (const char* env = getenv("ONB_PERFT_BFS_NODES")) bfs_nodes = atoll(env);  // experiment: deeper frontier, shallower DFS
+            const int64_t bfs_nodes = 1 << 21;
             while (n_cur > 0 && ((depth - level) > kMaxDfs || ((depth - level) > 1 && n_cur < bfs_nodes))) {
                 unsigned long long total = 0;
                 PF(cudaMemsetAsync(d_cursor, 0, 8, c->stream), "memset");

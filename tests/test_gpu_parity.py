@@ -1618,17 +1618,15 @@ def test_cuda_graph_cache_follows_the_noise_setting(onb):
 def test_network_split_mode_variants_agree(onb, monkeypatch):
     """The builds of the f32-faithful network compute the same products in the same order per accumulator: the warp-specialised
     pipelined kernel on CTA pairs (the default) and on single CTAs (ONB_NET_X3_PAIR=0) are bit-identical to the plain one-CTA kernel
-    (ONB_NET_X3_PIPE=0), the two-halves build (ONB_NET_X3_HALVES=1, an exploration knob) agrees to a few ulps (its heads add the two
-    channel halves in a different order); all meet the 1e-5 tolerance."""
+    (ONB_NET_X3_PIPE=0); all meet the 1e-5 tolerance."""
     from test_net_cpu import lively_model
     for blocks, n in ((3, 100), (0, 33), (5, 250)):   # n not a multiple of 3, 6 or 7
         model = lively_model(blocks, seed=9)
         planes = O.encode(_positions(n, 5)).reshape(n, 21, 5, 5)
         want_p, want_v = O.net_forward(model.state_dict(), planes)
         outs = {}
-        for name, env in (("plain", {"ONB_NET_X3_PIPE": "0"}), ("pipe", {}), ("halves", {"ONB_NET_X3_HALVES": "1"}),
-                          ("single", {"ONB_NET_X3_PAIR": "0"})):
-            for k in ("ONB_NET_X3_PIPE", "ONB_NET_X3_HALVES", "ONB_NET_X3_PAIR"):
+        for name, env in (("plain", {"ONB_NET_X3_PIPE": "0"}), ("pipe", {}), ("single", {"ONB_NET_X3_PAIR": "0"})):
+            for k in ("ONB_NET_X3_PIPE", "ONB_NET_X3_PAIR"):
                 monkeypatch.delenv(k, raising=False)
             for k, v in env.items():
                 monkeypatch.setenv(k, v)
@@ -1641,14 +1639,11 @@ def test_network_split_mode_variants_agree(onb, monkeypatch):
             assert np.abs(outs[name][0] - want_p).max() <= 1e-5 and np.abs(outs[name][1] - want_v).max() <= 1e-5, (name, blocks)
         assert np.array_equal(outs["plain"][0], outs["pipe"][0]) and np.array_equal(outs["plain"][1], outs["pipe"][1]), blocks
         assert np.array_equal(outs["plain"][0], outs["single"][0]) and np.array_equal(outs["plain"][1], outs["single"][1]), blocks
-        for other in ("halves",):   # its heads add the two channel halves' partial sums: a few ulps
-            assert np.abs(outs["plain"][0] - outs[other][0]).max() <= 1e-6 and np.abs(outs["plain"][1] - outs[other][1]).max() <= 2e-6, other
-        # the f16 fast mode: the warp-specialised two-CTAs-per-SM build against the plain one, bit for bit
-        for k in ("ONB_NET_X3_PIPE", "ONB_NET_X3_HALVES", "ONB_NET_X3_PAIR"):
+        # the f16 fast mode: the four-accumulator pipeline on CTA pairs and on single CTAs against the plain build, bit for bit
+        for k in ("ONB_NET_X3_PIPE", "ONB_NET_X3_PAIR"):
             monkeypatch.delenv(k, raising=False)
         f16 = {}
-        for name, env in (("plain", {"ONB_NET_F16_PIPE": "0", "ONB_NET_F16_QUAD": "0"}), ("pipe", {"ONB_NET_F16_PIPE": "1", "ONB_NET_F16_QUAD": "0"}),
-                          ("quad_pair", {"ONB_NET_F16_PIPE": "0", "ONB_NET_F16_QUAD": "1"}), ("quad_single", {"ONB_NET_F16_PIPE": "0", "ONB_NET_F16_QUAD": "2"})):
+        for name, env in (("plain", {"ONB_NET_F16_QUAD": "0"}), ("quad_pair", {"ONB_NET_F16_QUAD": "1"}), ("quad_single", {"ONB_NET_F16_QUAD": "2"})):
             for k, v in env.items():
                 monkeypatch.setenv(k, v)
             with onb.Context(n, mcts_max_sims=2, planes=False) as ctx:
@@ -1657,9 +1652,8 @@ def test_network_split_mode_variants_agree(onb, monkeypatch):
                 ctx.net_forward(onb.BUF_LEAF_PLANES)
                 ctx.net_forward(onb.BUF_LEAF_PLANES)
                 f16[name] = (ctx.read(onb.BUF_POLICY, np.float32, (n, 50)), ctx.read(onb.BUF_VALUE, np.float32, (n,)))
-        monkeypatch.delenv("ONB_NET_F16_PIPE", raising=False)
         monkeypatch.delenv("ONB_NET_F16_QUAD", raising=False)
-        for other in ("pipe", "quad_pair", "quad_single"):
+        for other in ("quad_pair", "quad_single"):
             assert np.array_equal(f16["plain"][0], f16[other][0]) and np.array_equal(f16["plain"][1], f16[other][1]), (blocks, other)
 
 
@@ -1674,7 +1668,7 @@ def test_network_drifting_window_wraps(onb, monkeypatch):
     planes = O.encode(_positions(n, 11)).reshape(n, 21, 5, 5)
     outs = {}
     for name, env in (("plain", {"ONB_NET_X3_PIPE": "0"}), ("pair", {}), ("single", {"ONB_NET_X3_PAIR": "0"})):
-        for k in ("ONB_NET_X3_PIPE", "ONB_NET_X3_HALVES", "ONB_NET_X3_PAIR"):
+        for k in ("ONB_NET_X3_PIPE", "ONB_NET_X3_PAIR"):
             monkeypatch.delenv(k, raising=False)
         for k, v in env.items():
             monkeypatch.setenv(k, v)
@@ -1689,7 +1683,7 @@ def test_network_drifting_window_wraps(onb, monkeypatch):
     # the f16 pipeline (four accumulators, window wraps after 12 / 8 layers) against the round-1 build
     f16 = {}
     for name, env in (("plain", {"ONB_NET_F16_QUAD": "0"}), ("pair", {}), ("single", {"ONB_NET_F16_QUAD": "2"})):
-        for k in ("ONB_NET_X3_PIPE", "ONB_NET_X3_HALVES", "ONB_NET_X3_PAIR", "ONB_NET_F16_QUAD", "ONB_NET_F16_PIPE"):
+        for k in ("ONB_NET_X3_PIPE", "ONB_NET_X3_PAIR", "ONB_NET_F16_QUAD"):
             monkeypatch.delenv(k, raising=False)
         for k, v in env.items():
             monkeypatch.setenv(k, v)
@@ -1710,7 +1704,7 @@ def test_network_pipelines_match_plain_builds_on_ragged_sizes(onb, monkeypatch):
     groups (the peer CTA of the last pair computes on zeros), more groups than one round of clusters, and 0 / 1 / 3 blocks (0 blocks:
     the only layer is the last one, heads run at once)."""
     from test_net_cpu import lively_model
-    knobs = ("ONB_NET_X3_PIPE", "ONB_NET_X3_PAIR", "ONB_NET_X3_HALVES", "ONB_NET_F16_QUAD", "ONB_NET_F16_PIPE")
+    knobs = ("ONB_NET_X3_PIPE", "ONB_NET_X3_PAIR", "ONB_NET_F16_QUAD")
     sizes = (1, 6, 7, 8, 13, 14, 15, 27, 28, 29, 43, 148 * 7 + 3, 148 * 14 + 1, 4099)
     for blocks in (0, 1, 3):
         model = lively_model(blocks, seed=21 + blocks)
@@ -1731,28 +1725,6 @@ def test_network_pipelines_match_plain_builds_on_ragged_sizes(onb, monkeypatch):
                 assert np.array_equal(outs[0][0], outs[1][0]) and np.array_equal(outs[0][1], outs[1][1]), (blocks, precision, n)
     for k in knobs:
         monkeypatch.delenv(k, raising=False)
-
-
-@pytest.mark.gpu
-def test_step_fusion_knob_builds_the_same_trees(onb, monkeypatch):
-    """ONB_MCTS_STEP_FUSION=1 (expand_backup(s) + select(s+1) in one launch, an exploration knob) must not change a single tree: eval
-    and train mode, network evaluator, against the default three-launch rounds."""
-    from test_net_cpu import lively_model
-    n, sims = 96, 40
-    roots = _cfg4_roots(n, 9)
-    with onb.Context(n, seed=3, mcts_max_sims=sims, planes=False) as ctx:
-        ctx.net_load(lively_model(1, seed=6))
-        got = {}
-        for noise in (False, True):
-            ctx.mcts_set_noise(noise, 0.25, 0.03, 11)
-            for fuse in ("0", "1"):
-                monkeypatch.setenv("ONB_MCTS_STEP_FUSION", fuse)
-                ctx.set_states(roots)
-                res = ctx.search(2.0, sims, evaluator=onb.EVAL_NET)
-                got[(noise, fuse)] = (res["child_visits"].copy(), res["root_q"].copy(), ctx.mcts_tree_info()[0].copy())
-            for a, b in zip(got[(noise, "0")], got[(noise, "1")]):
-                assert np.array_equal(a, b)
-        assert not np.array_equal(got[(False, "0")][0], got[(True, "0")][0])
 
 
 @pytest.mark.gpu

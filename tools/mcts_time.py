@@ -1,6 +1,6 @@
-"""Times the fused PUCT search (BASELINE config 4: 16 384 trees x 400 simulations, uniform evaluator) under the exploration knobs of
-onb_mcts.cu and checks that every variant builds the same trees:   python tools/mcts_time.py [VAR=a,b,c ...]
-e.g.  python tools/mcts_time.py ONB_MCTS_ROOT_SMEM=0,24,32"""
+"""Times the fused PUCT search (BASELINE config 4: 16 384 trees x 400 simulations, uniform and hash evaluators), by default as built,
+or once per value of environment variables, and checks that every variant builds the same trees:
+python tools/mcts_time.py [VAR=a,b,c ...]"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -37,13 +37,14 @@ def run(label, evaluator=onb.EVAL_UNIFORM, reps=8):
     return out["child_visits"].copy(), out["root_q"].copy()
 
 
-specs = [a.split("=") for a in sys.argv[1:]] or [["ONB_MCTS_ROOT_SMEM", "0"]]
+specs = [a.split("=") for a in sys.argv[1:]] or [[None, "default"]]
 ref = None
 for var, vals in specs:
     for v in vals.split(","):
-        os.environ[var] = v
+        if var is not None:
+            os.environ[var] = v
         for ev, name in ((onb.EVAL_UNIFORM, "uniform"), (onb.EVAL_HASH, "hash")):
-            got = run("%s=%s %s" % (var, v, name), ev)
+            got = run("%s %s" % (v if var is None else "%s=%s" % (var, v), name), ev)
             key = name
             if ref is None:
                 ref = {}
@@ -51,5 +52,6 @@ for var, vals in specs:
                 ref[key] = got
             else:
                 assert np.array_equal(ref[key][0], got[0]) and np.array_equal(ref[key][1].view(np.uint64), got[1].view(np.uint64)), "variant changed the trees"
-    os.environ.pop(var, None)
+    if var is not None:
+        os.environ.pop(var, None)
 print("all variants built identical trees")

@@ -8,7 +8,7 @@ $B > $OUT/r2_plain_bench.log 2>&1 &&
 ncu --metrics gpu__time_duration.sum --clock-control none -c 600 --csv --log-file $OUT/r2_launches_bench.csv $B > $OUT/r2_ncu_launch.log 2>&1
 $B > $OUT/r2_plain_bench2.log 2>&1 &&
 ncu --set full --clock-control none --import-source on -k regex:k_env_step -s 4 -c 1 -o $OUT/r2_env_step -f $B > $OUT/r2_ncu_env.log 2>&1
-M="python tools/mcts_time.py ONB_MCTS_ROOT_SMEM=0"
+M="python tools/mcts_time.py"
 $M > $OUT/r2_plain_mcts.log 2>&1 &&
 ncu --set full --clock-control none --import-source on -k regex:k_mcts_run_g -s 3 -c 1 -o $OUT/r2_mcts_run_g -f $M > $OUT/r2_ncu_mcts.log 2>&1
 for P in f32 f16; do

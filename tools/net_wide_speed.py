@@ -99,7 +99,7 @@ def main(argv=None):
             if width == 128:
                 per_pass, nb = wide_weight_bytes(mode, blocks)
                 wbytes = per_pass * -(-B // nb)
-            elif quad is not None:  # round-1 k_net_forward<2, true>: 7 boards per pass, 8 KB per tap
+            elif quad is not None:  # round-1 k_net_forward<true>: 7 boards per pass, 8 KB per tap
                 wbytes = 9 * (1 + 2 * blocks) * 8 * KB * -(-B // 7)
             else:
                 wbytes = None

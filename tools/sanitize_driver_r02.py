@@ -1,6 +1,6 @@
 """Round-2 code paths for compute-sanitizer memcheck, sized to finish quickly: the pipelined actor (slices, done words), the
 deterministic compaction + subset searches of onb_self_play / onb_fight, the device Elo fold, the split-operand network kernels
-(pipelined, plain, two-halves), onb_selfplay_pack and the single-rank gather."""
+(pipelined, plain), onb_selfplay_pack and the single-rank gather."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests"))
@@ -26,16 +26,14 @@ with onb.Context(n, seed=3, mcts_max_sims=24) as ctx:
         for j in range(act.n_sub):
             act.wait(j)
         act.join()
-    for prec, env in (("f32", {}), ("f32", {"ONB_NET_X3_PIPE": "0"}), ("f32", {"ONB_NET_X3_HALVES": "1"}), ("f16", {})):
-        for k in ("ONB_NET_X3_PIPE", "ONB_NET_X3_HALVES"):
-            os.environ.pop(k, None)
+    for prec, env in (("f32", {}), ("f32", {"ONB_NET_X3_PIPE": "0"}), ("f16", {})):
+        os.environ.pop("ONB_NET_X3_PIPE", None)
         os.environ.update(env)
         ctx.net_load(model, precision=prec)
         ctx.encode(to_host=False)
         ctx.net_forward(onb.BUF_PLANES)
         ctx.sync()
-    for k in ("ONB_NET_X3_PIPE", "ONB_NET_X3_HALVES"):
-        os.environ.pop(k, None)
+    os.environ.pop("ONB_NET_X3_PIPE", None)
     res = ctx.self_play_native(2.0, 12, 400, max_plies=6, evaluator=onb.EVAL_NET, train=True, noise_seed=4)
     assert res["games"] == 400
     import ctypes as C
@@ -48,11 +46,7 @@ with onb.Context(n, seed=3, mcts_max_sims=24) as ctx:
     ctx.fight_native(ctx.agent_puct(12, 2.0), ctx.agent_uct(24), a_is_red, max_plies=8)
     st = ctx.fight_stats(history=True)
     assert st["n_games"] == n
-    os.environ["ONB_MCTS_STEP_FUSION"] = "1"
     ctx.reset()
     ctx.search(2.0, 8, evaluator=onb.EVAL_NET)
-    os.environ.pop("ONB_MCTS_STEP_FUSION")
-    os.environ["ONB_MCTS_ROOT_SMEM"] = "24"
     ctx.search(2.0, 20)
-    os.environ.pop("ONB_MCTS_ROOT_SMEM")
 print("sanitize driver r02 ok")

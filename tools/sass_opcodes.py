@@ -34,7 +34,7 @@ for line in out.split("\n"):
 print("# SASS opcode histogram of the network kernels (python tools/sass_opcodes.py: cuobjdump -sass %s, sm_100a)" % OBJ)
 print("# tcgen05.mma -> UTC*MMA, tcgen05.ld/st -> LDTM/STTM, cp.async.bulk -> UBLKCP, tcgen05.commit -> UTCBAR, tcgen05.alloc -> UTCATOMSWS,")
 print("# mbarrier -> SYNCS. Shipped: k_net_forward_x3p<true> (ONB_NET_F32: CTA pairs, tcgen05 cta_group::2), k_net_forward_x3p<false> (its")
-print("# single-CTA fallback), k_net_forward<2, true, false> (ONB_NET_F16), k_net_forward<2, false, false> (ONB_NET_TF32); the others are knobs")
+print("# single-CTA fallback), k_net_forward_f16q<true|false> (ONB_NET_F16), k_net_forward<false, false> (ONB_NET_TF32); the others are plain builds")
 print()
 print("%-44s" % "kernel" + "".join("%13s" % c for c in COLS) + "%9s" % "total")
 for k in order:
