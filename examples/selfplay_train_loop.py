@@ -39,6 +39,8 @@ def main(argv=None):
     ap.add_argument("--gumbel", type=int, default=0, metavar="M",
                     help="self-play with the Gumbel root search over M considered actions (onb_mcts_set_gumbel) and train on its improved "
                          "policy instead of PUCT with root noise; the arena adds Gumbel(--sims) against PUCT(--sims)")
+    ap.add_argument("--gumbel-interior", action="store_true",
+                    help="with --gumbel: Gumbel MuZero, interior selection below the root instead of PUCT (onb_gumbel_config.interior)")
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--out", default=None, help="directory for the reference's on-disk artefacts: loss_stats JSON (stats.rs) and .ot checkpoints (train.rs:414-430)")
     ap.add_argument("--hidden", type=int, default=64, choices=[64, 128], help="hidden channels of the ConvResNet (both run on the tensor cores)")
@@ -62,7 +64,9 @@ def main(argv=None):
 
     if args.gumbel and args.reuse:
         ap.error("--gumbel does not combine with --reuse")
-    gumbel = dict(m=args.gumbel, seed=args.seed) if args.gumbel else None
+    if args.gumbel_interior and not args.gumbel:
+        ap.error("--gumbel-interior needs --gumbel M")
+    gumbel = dict(m=args.gumbel, seed=args.seed, interior=args.gumbel_interior) if args.gumbel else None
     if args.reuse and args.torch_net:
         ap.error("--reuse needs the on-device network (a PyTorch module drives the split phase, which tree reuse does not support)")
     for it in range(args.iters):
@@ -112,7 +116,7 @@ def main(argv=None):
                 cx.alphabeta(args.ab_depth, to_host=False)   # leaves the chosen actions in BUF_ACTIONS
 
             def gumbel_az(cx):   # the Gumbel agent of onb_fight: step = ply (one search per ply and agent)
-                cx.set_gumbel(True, m=args.gumbel, seed=cx.seed, step0=counter["ply"])
+                cx.set_gumbel(True, m=args.gumbel, seed=cx.seed, step0=counter["ply"], interior=args.gumbel_interior)
                 cx.search_device(2.0, args.sims, evaluator=ev, net=net)
                 cx.set_gumbel(False)
                 cx.tensor(onb.BUF_ACTIONS).copy_(cx.tensor(onb.BUF_BEST))
@@ -122,7 +126,7 @@ def main(argv=None):
                       ("mcts", az, plain_mcts, ctx.agent_puct(args.sims, 2.0, ev, 0), ctx.agent_uct(args.mcts_playouts)),
                       ("alphabeta", az, alphabeta, ctx.agent_puct(args.sims, 2.0, ev, 0), ctx.agent_alphabeta(args.ab_depth))]
             if args.gumbel:
-                fights.append(("gumbel_vs_puct", gumbel_az, az, ctx.agent_gumbel(args.sims, args.gumbel, 0.1, ev, 0),
+                fights.append(("gumbel_vs_puct", gumbel_az, az, ctx.agent_gumbel(args.sims, args.gumbel, 0.1, ev, 0, args.gumbel_interior),
                                ctx.agent_puct(args.sims, 2.0, ev, 0)))
             for name, mine, opponent, native_a, native in fights:
                 ctx.reset()

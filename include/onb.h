@@ -290,7 +290,7 @@ ONB_API int32_t onb_mcts_reuse_stats(onb_ctx* ctx, uint64_t out[4], int32_t clea
 /* Gumbel root search (Danihelka et al., "Policy improvement by planning with Gumbel", ICLR 2022; the root part of mctx's
  * gumbel_muzero_policy). Off by default; with it off every entry point behaves exactly as without this call. On: the searches begun
  * afterwards select at the ROOT by sequential halving over Gumbel-Top-k samples and report the improved policy; below the root the
- * PUCT descent is unchanged. Definition (exact to the bit, DESIGN.md §5f), per tree, with k root children (pass pseudo-children
+ * PUCT descent is unchanged unless interior = 1 (interior selection, below). Definition (exact to the bit, DESIGN.md §5f), per tree, with k root children (pass pseudo-children
  * included), P(a) the stored prior, N(a), W(a) visits and reward sum, q(a) = W(a) / N(a), r0 = the reward the root's own evaluation
  * (simulation 0) backed up into the root and v = -r0:
  *   logit(a) = onb_log(P(a)) (-inf for P = 0), L = max logit, p(a) = max(DBL_MIN, P(a) / sum P); if every prior is 0, every P counts as 1;
@@ -304,20 +304,36 @@ ONB_API int32_t onb_mcts_reuse_stats(onb_ctx* ctx, uint64_t out[4], int32_t clea
  * All f64 sums run in child order. onb_log / onb_exp are the project's own f64 log / exp from IEEE basic operations (fdlibm's
  * algorithms), so the CPU and the GPU agree to the bit. root_visits, root_q and child_visits are reported as before.
  * step: onb_mcts_begin uses a serial that this call sets to step0 and every Gumbel begin increments; onb_self_play uses step = ply,
- * onb_fight step = ply for ONB_AGENT_GUMBEL agents (both leave the serial as they found it).
+ * onb_fight step = ply for ONB_AGENT_GUMBEL and ONB_AGENT_GUMBEL_MUZERO agents (both leave the serial as they found it).
  * Checks: 1 <= max_considered <= 40, finite c_visit, c_scale, gumbel_scale >= 0, else ONB_E_INVALID. cfg NULL or enabled = 0: off.
  * Refused with ONB_E_STATE at onb_mcts_begin: Gumbel together with tree reuse or train-mode noise; after a Gumbel begin: onb_uct_run
  * and more simulations than the begin's sims. onb_self_play while Gumbel is on: ONB_E_STATE with tree reuse on, ONB_E_INVALID with train != 0. onb_fight searches
  * without reuse, so its Gumbel agents play whatever the reuse switch says. Every begin decides anew: a search begun with the switch
  * off is a PUCT search. The caller-driven split phase is supported.
- * Memory: the first enabling call allocates n_games * 1 KB of per-tree root data and a 40 x mcts_max_sims table. */
+ * Memory: the first enabling call allocates n_games * 1 KB of per-tree root data and a 40 x mcts_max_sims table; the first call with
+ * interior = 1 also n_games * mcts_node_cap * 4 B for r_x (16 384 games x 800 simulations: 2.1 GB).
+ *
+ * Interior selection (interior = 1; the rest of mctx's gumbel_muzero_policy, gumbel_muzero_interior_action_selection): every descent
+ * step at depth >= 1 at an expanded, non-terminal node x chooses by the rule below instead of the PUCT argmax. The root keeps the
+ * sequential halving above, and onb_mcts_finish's best and pi are unchanged. With k children of x, P(a) the stored prior (the
+ * per-card renormalised prior, as at the root; mctx's raw network logits differ from its log by a constant per card), N(a), W(a),
+ * q(a) = W(a) / N(a):
+ *   r_x = the reward the expanding simulation backed up into x (stored when the expansion succeeds), v = -r_x;
+ *   p(a), v_mix, sigma(a) exactly as at the root with r_x in place of r0 (the all-priors-0 rule, the sums in child order, c_visit,
+ *     c_scale, the 1e-8 floor: mctx's qtransform_completed_by_mix_value with the node's raw value);
+ *   z(a) = logit(a) + sigma(a), logit(a) = onb_log(P(a)) (-inf for P = 0; P counts as 1 when every prior of x is 0);
+ *   e(a) = onb_exp(z(a) - max z), pi'(a) = e(a) / sum e (the sum in child order);
+ *   choice = the FIRST child maximising pi'(a) - N(a) / (1 + sum N), sum N over x's children (mctx's _prepare_argmax_input + argmax).
+ * All f64 with IEEE basic operations (no FMA contraction), so the CPU oracle gives the same bits. It needs no c_puct. interior = 0
+ * keeps PUCT below the root; any other value than 0 or 1: ONB_E_INVALID. The refusals above hold unchanged. If allocating r_x fails the
+ * call returns ONB_E_NOMEM and leaves the switch as it was. */
 typedef struct onb_gumbel_config {
     int32_t enabled;
     uint32_t max_considered; /* m, the number of root actions sampled without replacement (mctx default 16) */
     double c_visit, c_scale, gumbel_scale; /* 50, 0.1, 1 (0: a deterministic search) */
     uint64_t seed;
     uint32_t step0;
-    uint32_t reserved;
+    uint32_t interior; /* 0: PUCT below the root, 1: interior selection below the root (Gumbel MuZero) */
 } onb_gumbel_config;
 ONB_API int32_t onb_mcts_set_gumbel(onb_ctx* ctx, const onb_gumbel_config* cfg);
 ONB_API int32_t onb_mcts_select(onb_ctx* ctx);
@@ -402,6 +418,9 @@ ONB_API int32_t onb_copy_to_host(onb_ctx* ctx, void* host, const void* device, i
  * descent below the root. ONB_AGENT_PUCT agents search with
  * PUCT whatever the context's Gumbel switch says; onb_fight leaves that switch as it found it. */
 #define ONB_AGENT_GUMBEL 4
+/* ONB_AGENT_GUMBEL_MUZERO: as ONB_AGENT_GUMBEL (the same fields and defaults) with interior = 1: Gumbel MuZero, interior selection
+ * below the root instead of PUCT. ONB_AGENT_GUMBEL agents search with interior = 0 whatever the context's setting says. */
+#define ONB_AGENT_GUMBEL_MUZERO 6
 typedef struct onb_agent {
     int32_t kind;
     int32_t evaluator;

@@ -420,7 +420,8 @@ struct AlphaZeroMctsConfig {  // alphazero_mcts/mod.rs:26-43
     bool reuse = false;
     // the Gumbel root search (onb_mcts_set_gumbel, DESIGN.md §5f): enabled = 1 makes every search select at the root by sequential
     // halving and report the improved policy as the move's tensor. The setting is applied when it changes (which sets the step to
-    // step0); every search takes the next step. Does not combine with train or reuse (ONB_E_STATE).
+    // step0); every search takes the next step. Does not combine with train or reuse (ONB_E_STATE). interior = 1: Gumbel MuZero's
+    // interior selection below the root instead of PUCT.
     onb_gumbel_config gumbel{};
 };
 inline double reward(MoveResult r, PlayerColor c) {  // alphazero_mcts/mod.rs:45-53
@@ -440,7 +441,8 @@ inline void run_search(Engine& e, const AlphaZeroMctsConfig& cfg, int32_t device
     const onb_gumbel_config& g = cfg.gumbel;
     const onb_gumbel_config& a = e.gumbel_applied;
     if (g.enabled != a.enabled || (g.enabled && (g.max_considered != a.max_considered || g.c_visit != a.c_visit || g.c_scale != a.c_scale ||
-                                                 g.gumbel_scale != a.gumbel_scale || g.seed != a.seed || g.step0 != a.step0))) {
+                                                 g.gumbel_scale != a.gumbel_scale || g.seed != a.seed || g.step0 != a.step0 ||
+                                                 g.interior != a.interior))) {
         e.check(onb_mcts_set_gumbel(e.ctx(), &g));
         e.gumbel_applied = g;
     }
@@ -507,6 +509,22 @@ struct AlphaZeroMcts : Agent {  // alphazero_mcts/mod.rs:81-161
     const char* name() const override { return "AlphaZero MCTS AI"; }
     std::unique_ptr<Agent> clone_dyn() const override { return std::make_unique<AlphaZeroMcts>(*this); }
     uint64_t id() const override { return (uint64_t)config.exploration_c + config.max_playouts + (uint64_t)config.train; }
+};
+
+/// Gumbel MuZero (onb_gumbel_config.interior = 1, DESIGN.md §5f): AlphaZeroMcts with the Gumbel root search over m considered actions
+/// and interior selection below the root (c_visit 50, gumbel_scale 1). The project's own agent; the reference has none.
+struct GumbelMuZero : AlphaZeroMcts {
+    explicit GumbelMuZero(uint32_t m = 16, double c_scale = 0.1, uint64_t seed = 0) {
+        config.gumbel.enabled = 1;
+        config.gumbel.max_considered = m;
+        config.gumbel.c_visit = 50.0;
+        config.gumbel.c_scale = c_scale;
+        config.gumbel.gumbel_scale = 1.0;
+        config.gumbel.seed = seed;
+        config.gumbel.interior = 1;
+    }
+    const char* name() const override { return "Gumbel MuZero AI"; }
+    std::unique_ptr<Agent> clone_dyn() const override { return std::make_unique<GumbelMuZero>(*this); }
 };
 
 // ---------------------------------------------------------------------------------------------- self_play (train.rs:27-98)

@@ -129,7 +129,7 @@ class SelfPlayConfig(C.Structure):
                 ("train", C.c_int32), ("noise_seed", C.c_uint64), ("sample_cap", C.c_int64)]
 
 
-AGENT_RANDOM, AGENT_PUCT, AGENT_UCT, AGENT_ALPHABETA, AGENT_GUMBEL, AGENT_TABLEBASE = 0, 1, 2, 3, 4, 5
+AGENT_RANDOM, AGENT_PUCT, AGENT_UCT, AGENT_ALPHABETA, AGENT_GUMBEL, AGENT_TABLEBASE, AGENT_GUMBEL_MUZERO = 0, 1, 2, 3, 4, 5, 6
 ALPHABETA_MAX_DEPTH = 8
 ALPHABETA_WIN = 1000000
 TB_MAX_PAWNS = 4
@@ -145,7 +145,7 @@ class TbClass(C.Structure):
 class GumbelConfig(C.Structure):
     """onb_gumbel_config (onb_mcts_set_gumbel)"""
     _fields_ = [("enabled", C.c_int32), ("max_considered", C.c_uint32), ("c_visit", C.c_double), ("c_scale", C.c_double),
-                ("gumbel_scale", C.c_double), ("seed", C.c_uint64), ("step0", C.c_uint32), ("reserved", C.c_uint32)]
+                ("gumbel_scale", C.c_double), ("seed", C.c_uint64), ("step0", C.c_uint32), ("interior", C.c_uint32)]
 
 
 class Agent(C.Structure):

@@ -148,7 +148,7 @@ int32_t onb_destroy(onb_ctx* ctx) {
                     c->d_tree_size, c->d_tree_flags, c->d_roots, c->d_leaf_node, c->d_leaf_state, c->d_leaf_planes, c->d_policy, c->d_value,
                     c->d_pi, c->d_best, c->d_root_visits, c->d_root_q, c->d_child_visits, c->net[0].w, c->net[0].bias, c->net[0].head, c->net[1].w,
                     c->net[1].bias, c->net[1].head, c->d_ln_table, c->d_ab_score, c->d_ab_nodes, c->d_gb,
-                    c->d_gb_tab, c->d_gb_base, c->d_gb_p, c->d_gb_r0, c->d_tb_values};
+                    c->d_gb_tab, c->d_gb_base, c->d_gb_p, c->d_gb_r0, c->d_gb_rx, c->d_tb_values};
     reuse_free(c);
     tb_free(c);
     for (void* p : c->sp_buf)
@@ -454,7 +454,7 @@ namespace onb {
 // (onb_fight never does, whatever the context's reuse switch says). Every begin clears gb_search first, so a search begun after the
 // switch went off, or a refused begin, never runs the Gumbel kernels.
 static int32_t gumbel_refusals(Ctx* c, const char* what, bool reuse) {
-    c->gb_search = 0;
+    c->gb_search = c->gi_search = 0;
     if (!c->gb_on) return ONB_OK;
     if (reuse) return fail(c, ONB_E_STATE, "%s: the Gumbel root search does not combine with tree reuse (onb_mcts_set_reuse)", what);
     if (c->noise_on) return fail(c, ONB_E_STATE, "%s: the Gumbel root search does not combine with train-mode noise (onb_mcts_set_noise)", what);
@@ -463,6 +463,7 @@ static int32_t gumbel_refusals(Ctx* c, const char* what, bool reuse) {
 // after the trees are begun: the search's GumbelDev (step = the serial, which advances) and, when (m, sims) changed, the table
 static int32_t gumbel_begin(Ctx* c, uint32_t sims) {
     c->gb_search = c->gb_on;
+    c->gi_search = c->gb_on && c->gb_cfg.interior;
     if (!c->gb_on) return ONB_OK;
     const uint32_t m = c->gb_cfg.max_considered, nt = sims ? sims - 1u : 0u;
     if (nt && (c->gb_tab_m != m || c->gb_tab_n != nt)) {
@@ -486,6 +487,8 @@ static int32_t gumbel_begin(Ctx* c, uint32_t sims) {
     h.base = c->d_gb_base;
     h.p = c->d_gb_p;
     h.r0 = c->d_gb_r0;
+    h.interior = c->gi_search ? 1u : 0u;
+    h.rx = c->d_gb_rx;
     ONB_CUDA(c, cudaMemcpyAsync(c->d_gb, &h, sizeof(h), cudaMemcpyHostToDevice, c->stream));
     return ONB_OK;
 }
@@ -526,6 +529,7 @@ int32_t onb_mcts_set_gumbel(onb_ctx* ctx, const onb_gumbel_config* cfg) {
     if (cfg->max_considered < 1 || cfg->max_considered > 40 || !std::isfinite(cfg->c_visit) || !std::isfinite(cfg->c_scale) ||
         !std::isfinite(cfg->gumbel_scale) || !(cfg->c_visit >= 0.0) || !(cfg->c_scale >= 0.0) || !(cfg->gumbel_scale >= 0.0))
         return fail(c, ONB_E_INVALID, "onb_mcts_set_gumbel: need 1 <= max_considered <= 40 and finite c_visit, c_scale, gumbel_scale >= 0");
+    if (cfg->interior > 1) return fail(c, ONB_E_INVALID, "onb_mcts_set_gumbel: interior must be 0 or 1");
     if (!c->d_nodes) return fail(c, ONB_E_STATE, "onb_mcts_set_gumbel: context created with mcts_max_sims = 0");
     if (!c->d_gb) {
         const size_t n = (size_t)c->n;
@@ -541,6 +545,14 @@ int32_t onb_mcts_set_gumbel(onb_ctx* ctx, const onb_gumbel_config* cfg) {
             return e == cudaErrorMemoryAllocation ? fail(c, ONB_E_NOMEM, "onb_mcts_set_gumbel: out of device memory") : cuda_fail(c, e, "onb_mcts_set_gumbel");
         }
         c->gb_tab_m = c->gb_tab_n = 0;
+    }
+    if (cfg->interior && !c->d_gb_rx) {  // r_x of every node of every tree
+        const cudaError_t e = dalloc(&c->d_gb_rx, (size_t)c->n * c->node_cap);
+        if (e != cudaSuccess) {
+            c->d_gb_rx = nullptr;
+            return e == cudaErrorMemoryAllocation ? fail(c, ONB_E_NOMEM, "onb_mcts_set_gumbel: out of device memory for interior selection")
+                                                  : cuda_fail(c, e, "onb_mcts_set_gumbel");
+        }
     }
     c->gb_cfg = *cfg;
     c->gb_serial = cfg->step0;
@@ -764,8 +776,10 @@ static int32_t fight_move(Ctx* c, const onb_agent* ag, uint32_t ply, const int32
         return ONB_OK;
     }
     c->gb_on = 0;  // PUCT and UCT agents search without the Gumbel root step
-    if (ag->kind == ONB_AGENT_GUMBEL) {
+    const bool gumbel = ag->kind == ONB_AGENT_GUMBEL || ag->kind == ONB_AGENT_GUMBEL_MUZERO;
+    if (gumbel) {
         c->gb_on = 1;
+        c->gb_cfg.interior = ag->kind == ONB_AGENT_GUMBEL_MUZERO ? 1u : 0u;
         c->gb_cfg.max_considered = ag->min_node_visits ? ag->min_node_visits : 16u;
         c->gb_cfg.c_visit = 50.0;
         c->gb_cfg.c_scale = ag->c;
@@ -773,9 +787,9 @@ static int32_t fight_move(Ctx* c, const onb_agent* ag, uint32_t ply, const int32
         c->gb_cfg.seed = c->cfg.seed;
         c->gb_serial = ply;
     }
-    int32_t rc = mcts_begin_subset(c, ag->kind == ONB_AGENT_GUMBEL ? 2.0 : ag->c, ag->sims, d_games, m);
+    int32_t rc = mcts_begin_subset(c, gumbel ? 2.0 : ag->c, ag->sims, d_games, m);
     if (rc != ONB_OK) return rc;
-    if (ag->kind == ONB_AGENT_PUCT || ag->kind == ONB_AGENT_GUMBEL) {
+    if (ag->kind == ONB_AGENT_PUCT || gumbel) {
         if (ag->evaluator == ONB_EVAL_NET && (rc = onb_net_select(x, ag->net_slot)) != ONB_OK) return rc;
         rc = onb_mcts_run(x, ag->evaluator, ag->sims);
     } else {
@@ -794,13 +808,13 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
     if (!a || !b || !a_is_red_host || !out) return fail(c, ONB_E_INVALID, "onb_fight: null argument");
     for (const onb_agent* ag : {a, b}) {
         if (ag->kind != ONB_AGENT_RANDOM && ag->kind != ONB_AGENT_PUCT && ag->kind != ONB_AGENT_UCT && ag->kind != ONB_AGENT_ALPHABETA &&
-            ag->kind != ONB_AGENT_GUMBEL && ag->kind != ONB_AGENT_TABLEBASE)
+            ag->kind != ONB_AGENT_GUMBEL && ag->kind != ONB_AGENT_TABLEBASE && ag->kind != ONB_AGENT_GUMBEL_MUZERO)
             return fail(c, ONB_E_INVALID, "onb_fight: unknown agent kind %d", ag->kind);
         if (ag->kind == ONB_AGENT_TABLEBASE) {
             if (!c->tb_live) return fail(c, ONB_E_STATE, "onb_fight: a tablebase agent needs a solved table (onb_tb_solve)");
             continue;
         }
-        if (ag->kind == ONB_AGENT_GUMBEL && (ag->min_node_visits > 40 || !std::isfinite(ag->c) || !(ag->c >= 0.0)))
+        if ((ag->kind == ONB_AGENT_GUMBEL || ag->kind == ONB_AGENT_GUMBEL_MUZERO) && (ag->min_node_visits > 40 || !std::isfinite(ag->c) || !(ag->c >= 0.0)))
             return fail(c, ONB_E_INVALID, "onb_fight: a Gumbel agent needs min_node_visits (m) <= 40 and a finite c (c_scale) >= 0");
         if (ag->kind == ONB_AGENT_ALPHABETA) {
             if (ag->sims < 1 || ag->sims > ONB_ALPHABETA_MAX_DEPTH)
@@ -829,11 +843,13 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
     const int gb_on = c->gb_on;  // the agents set the Gumbel switch per move; the context's own setting comes back afterwards
     const onb_gumbel_config gb_cfg = c->gb_cfg;
     const uint32_t gb_serial = c->gb_serial;
-    if (a->kind == ONB_AGENT_GUMBEL || b->kind == ONB_AGENT_GUMBEL) {
+    const bool muzero = a->kind == ONB_AGENT_GUMBEL_MUZERO || b->kind == ONB_AGENT_GUMBEL_MUZERO;
+    if (a->kind == ONB_AGENT_GUMBEL || b->kind == ONB_AGENT_GUMBEL || muzero) {
         onb_gumbel_config on;
         memset(&on, 0, sizeof(on));
         on.enabled = 1;
         on.max_considered = 16;
+        on.interior = muzero ? 1u : 0u;  // allocates r_x too
         if ((rc = onb_mcts_set_gumbel(ctx, &on)) != ONB_OK) return rc;  // allocates the Gumbel buffers; the context's setting is restored below
         c->gb_on = gb_on;
         c->gb_cfg = gb_cfg;

@@ -33,11 +33,12 @@ constexpr int kGbStride = 64;  // per-tree root-child slots: 8 pieces x 2 cards 
 struct GumbelDev {
     double c_visit, c_scale, scale;
     uint64_t seed;
-    uint32_t step, m, n_tab, reserved;  // n_tab = sims - 1 descents
+    uint32_t step, m, n_tab, interior;  // n_tab = sims - 1 descents; interior: the search runs the interior-selection kernels
     const uint32_t* tab;                // [m][n_tab]: row m_eff - 1 = seq_halving(m_eff, n_tab)
     double* base;                       // [n][kGbStride] g(a) + (logit(a) - L), written by the root's first descent
     double* p;                          // [n][kGbStride] max(DBL_MIN, P(a) / sum P)
     double* r0;                         // [n] the reward the root's own evaluation backed up into the root
+    float* rx;                          // [n][node_cap] r_x: the reward the expanding simulation backed up into node x (interior only)
 };
 
 struct Ctx {
@@ -131,11 +132,13 @@ struct Ctx {
     onb_gumbel_config gb_cfg;
     uint32_t gb_serial;       // step of the next Gumbel onb_mcts_begin
     int gb_search;            // the current search was begun with Gumbel
+    int gi_search;            // ... with Gumbel and interior selection (gb_cfg.interior)
     GumbelDev* d_gb;          // the device struct every Gumbel begin rewrites
     uint32_t* d_gb_tab;       // [40][mcts_max_sims]
     double* d_gb_base;
     double* d_gb_p;
     double* d_gb_r0;
+    float* d_gb_rx;           // [n][node_cap], allocated by the first call that turns interior selection on
     uint32_t gb_tab_m, gb_tab_n;  // the table d_gb_tab holds (gb_tab_m = 0: none)
     // endgame tablebase (onb_tablebase.cu, onb_tb_solve)
     int16_t* d_tb;            // every solved class, class 5 p + q at d_tb + tb_off[5 p + q]
@@ -173,7 +176,8 @@ cudaError_t launch_uct_run(Ctx* c, float exploration_c, uint32_t min_node_visits
 cudaError_t launch_mcts_finish(Ctx* c);
 cudaError_t launch_mcts_play_best(Ctx* c, uint32_t out_flags);
 cudaError_t launch_mcts_scatter_best(Ctx* c, uint16_t* dst_actions);  // dst[game of tree t] = best[t]
-// with c->gb_search the three launchers above that select at the root (select, run, finish) run the Gumbel variants
+// with c->gb_search the three launchers above that select at the root (select, run, finish) run the Gumbel variants; with
+// c->gi_search select, run and expand_backup run the interior-selection variants
 
 // network (onb_net.cu)
 int32_t net_load(Ctx* c, int32_t n_tensors, const char* const* names, const float* const* data, const int64_t* numel, std::string& err);

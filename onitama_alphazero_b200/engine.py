@@ -207,13 +207,15 @@ class Context:
         self._ck(self._lib.onb_mcts_reuse_stats(self._h, L.ptr(out), int(bool(clear))))
         return dict(trees=int(out[0]), kept=int(out[1]), kept_visits=int(out[2]), sims=int(out[3]))
 
-    def set_gumbel(self, enabled, m=16, c_visit=50.0, c_scale=0.1, gumbel_scale=1.0, seed=0, step0=0):
+    def set_gumbel(self, enabled, m=16, c_visit=50.0, c_scale=0.1, gumbel_scale=1.0, seed=0, step0=0, interior=False):
         """onb_mcts_set_gumbel: the Gumbel root search (sequential halving over m Gumbel-Top-k samples at the root, improved-policy
         targets in mcts_finish's pi). The step of the next search becomes step0; every search begun afterwards takes the next step.
-        See include/onb.h and DESIGN.md §5f."""
-        cfg = L.GumbelConfig(int(bool(enabled)), int(m), float(c_visit), float(c_scale), float(gumbel_scale), int(seed), int(step0), 0)
+        interior=True: Gumbel MuZero's interior selection below the root instead of PUCT. See include/onb.h and DESIGN.md §5f."""
+        cfg = L.GumbelConfig(int(bool(enabled)), int(m), float(c_visit), float(c_scale), float(gumbel_scale), int(seed), int(step0),
+                             int(bool(interior)))
         self._ck(self._lib.onb_mcts_set_gumbel(self._h, C.byref(cfg)))
-        self.gumbel = (int(m), float(c_visit), float(c_scale), float(gumbel_scale), int(seed)) if enabled else None
+        # interior appends a sixth entry, so that a root-only setting keeps its five-entry tuple
+        self.gumbel = (int(m), float(c_visit), float(c_scale), float(gumbel_scale), int(seed)) + ((True,) if interior else ()) if enabled else None
         self.gumbel_step = int(step0)  # self_play_native and fight_native leave the library's serial as they found it
 
     def _use_gumbel(self, gumbel):
@@ -227,7 +229,7 @@ class Context:
             return
         kw = dict(gumbel) if isinstance(gumbel, dict) else {}
         want = (int(kw.get("m", 16)), float(kw.get("c_visit", 50.0)), float(kw.get("c_scale", 0.1)), float(kw.get("gumbel_scale", 1.0)),
-                int(kw.get("seed", 0)))
+                int(kw.get("seed", 0))) + ((True,) if kw.get("interior", False) else ())
         if getattr(self, "gumbel", None) != want or "step0" in kw:
             self.set_gumbel(True, **kw)
 
@@ -286,9 +288,10 @@ class Context:
         return L.Agent(L.AGENT_UCT, 0, 0, playouts, exploration_c, min_node_visits, 0)
 
     @staticmethod
-    def agent_gumbel(sims, m=16, c_scale=0.1, evaluator=L.EVAL_UNIFORM, net_slot=0):
-        """the Gumbel root search as an arena agent (c_visit 50, gumbel_scale 1, seed = the context's seed, step = ply)"""
-        return L.Agent(L.AGENT_GUMBEL, evaluator, net_slot, sims, c_scale, m, 0)
+    def agent_gumbel(sims, m=16, c_scale=0.1, evaluator=L.EVAL_UNIFORM, net_slot=0, interior=False):
+        """the Gumbel root search as an arena agent (c_visit 50, gumbel_scale 1, seed = the context's seed, step = ply);
+        interior=True: Gumbel MuZero (ONB_AGENT_GUMBEL_MUZERO, interior selection below the root)"""
+        return L.Agent(L.AGENT_GUMBEL_MUZERO if interior else L.AGENT_GUMBEL, evaluator, net_slot, sims, c_scale, m, 0)
 
     @staticmethod
     def agent_alphabeta(depth):

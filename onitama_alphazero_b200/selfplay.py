@@ -136,8 +136,8 @@ def self_play_continuous(ctx, c_puct, sims, n_games, max_plies=150, evaluator=L.
             if gb_was is None:
                 ctx.set_gumbel(False)
             else:
-                m, c_visit, c_scale, scale, seed = gb_was
-                ctx.set_gumbel(True, m, c_visit, c_scale, scale, seed, step0=step_was)  # the setting and its step as they were
+                m, c_visit, c_scale, scale, seed = gb_was[:5]
+                ctx.set_gumbel(True, m, c_visit, c_scale, scale, seed, step0=step_was, interior=len(gb_was) > 5)  # the setting and its step as they were
 
 
 def _self_play_continuous(ctx, c_puct, sims, n_games, max_plies, evaluator, net, train, noise_seed, reuse):

@@ -92,7 +92,7 @@ pub struct onb_gumbel_config {
     pub gumbel_scale: f64,
     pub seed: u64,
     pub step0: u32,
-    pub reserved: u32,
+    pub interior: u32,
 }
 
 #[repr(C)]
