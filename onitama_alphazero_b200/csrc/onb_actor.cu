@@ -184,7 +184,7 @@ int32_t onb_actor_submit(onb_actor* actor, int32_t sub, const onb_action* action
     if (a->host_flags & ONB_HOST_STATS) ACT_CUDA(c, cudaMemcpyAsync(s.h_stats, c->d_stats, ONB_STAT_COUNT * 8, cudaMemcpyDeviceToHost, s.stream));
     ACT_CUDA(c, cudaEventRecord(s.done, s.stream));
     s.in_flight = true;
-    c->mcts_phase = 0;
+    c->search.phase = 0;
     return ONB_OK;
 }
 

@@ -288,7 +288,7 @@ int32_t onb_env_reset(onb_ctx* ctx, const uint8_t* decks5_host, int64_t n_decks,
         const uint8_t* d = decks5_host;
         c->fixed_cards = (int32_t)((d[0]) | (d[1] << 4) | (d[2] << 8) | (d[3] << 12) | (d[4] << 16));
     }
-    c->mcts_phase = 0;
+    c->search.phase = 0;
     return ONB_OK;
 }
 
@@ -321,7 +321,7 @@ int32_t onb_env_set_states(onb_ctx* ctx, const onb_state* states_host, int64_t f
     ONB_CUDA(c, cudaMemcpyAsync(c->d_io_states, states_host, (size_t)n * sizeof(onb_state), cudaMemcpyHostToDevice, c->stream));
     ONB_CUDA(c, launch_states_import(c, c->d_io_states, first, n));
     ONB_CUDA(c, cudaStreamSynchronize(c->stream));
-    c->mcts_phase = 0;
+    c->search.phase = 0;
     return ONB_OK;
 }
 
@@ -381,7 +381,7 @@ int32_t onb_env_step(onb_ctx* ctx, const onb_action* actions_host, uint32_t step
     if ((out_flags & ONB_OUT_PLANES) && !c->d_planes) return fail(c, ONB_E_STATE, "onb_env_step: plane buffer not allocated");
     if (actions_host) ONB_CUDA(c, cudaMemcpyAsync(c->d_actions, actions_host, (size_t)c->n * sizeof(uint16_t), cudaMemcpyHostToDevice, c->stream));
     ONB_CUDA(c, launch_env_step(c, kModeActions, step, auto_reset, out_flags));
-    c->mcts_phase = 0;
+    c->search.phase = 0;
     return ONB_OK;
 }
 
@@ -391,7 +391,7 @@ int32_t onb_env_step_random(onb_ctx* ctx, uint32_t step, int32_t policy, int32_t
     if (policy != ONB_POLICY_UNIFORM && policy != ONB_POLICY_AGENT) return fail(c, ONB_E_INVALID, "onb_env_step_random: unknown policy %d", policy);
     if ((out_flags & ONB_OUT_PLANES) && !c->d_planes) return fail(c, ONB_E_STATE, "onb_env_step_random: plane buffer not allocated");
     ONB_CUDA(c, launch_env_step(c, policy, step, auto_reset, out_flags));
-    c->mcts_phase = 0;
+    c->search.phase = 0;
     return ONB_OK;
 }
 
@@ -426,7 +426,7 @@ int32_t onb_env_playout(onb_ctx* ctx, uint32_t step0, uint32_t max_plies, int32_
     if (d_plies) cudaFree(d_plies);
     if (d_trace) cudaFree(d_trace);
     if (e != cudaSuccess) return cuda_fail(c, e, "onb_env_playout");
-    c->mcts_phase = 0;
+    c->search.phase = 0;
     return ONB_OK;
 }
 
@@ -450,87 +450,59 @@ int32_t onb_perft(onb_ctx* ctx, const onb_state* roots_host, int64_t n, int32_t 
 // ---------------------------------------------------------------------------------------------- mcts
 }  // extern "C"
 namespace onb {
-// the combinations a Gumbel search does not support (include/onb.h, onb_mcts_set_gumbel); reuse: this begin keeps remembered trees
-// (onb_fight never does, whatever the context's reuse switch says). Every begin clears gb_search first, so a search begun after the
-// switch went off, or a refused begin, never runs the Gumbel kernels.
-static int32_t gumbel_refusals(Ctx* c, const char* what, bool reuse) {
-    c->gb_search = c->gi_search = 0;
-    if (!c->gb_on) return ONB_OK;
-    if (reuse) return fail(c, ONB_E_STATE, "%s: the Gumbel root search does not combine with tree reuse (onb_mcts_set_reuse)", what);
-    if (c->noise_on) return fail(c, ONB_E_STATE, "%s: the Gumbel root search does not combine with train-mode noise (onb_mcts_set_noise)", what);
-    return ONB_OK;
-}
-// after the trees are begun: the search's GumbelDev (step = the serial, which advances) and, when (m, sims) changed, the table
-static int32_t gumbel_begin(Ctx* c, uint32_t sims) {
-    c->gb_search = c->gb_on;
-    c->gi_search = c->gb_on && c->gb_cfg.interior;
-    if (!c->gb_on) return ONB_OK;
-    const uint32_t m = c->gb_cfg.max_considered, nt = sims ? sims - 1u : 0u;
-    if (nt && (c->gb_tab_m != m || c->gb_tab_n != nt)) {
-        std::vector<uint32_t> tab((size_t)m * nt);
-        for (uint32_t r = 1; r <= m; ++r) onb_gumbel::seq_halving(r, nt, tab.data() + (size_t)(r - 1u) * nt);
-        // from pageable memory: the copy has taken the data when the call returns, so tab may go out of scope
-        ONB_CUDA(c, cudaMemcpyAsync(c->d_gb_tab, tab.data(), tab.size() * 4, cudaMemcpyHostToDevice, c->stream));
-        c->gb_tab_m = m;
-        c->gb_tab_n = nt;
-    }
-    GumbelDev h;
-    memset(&h, 0, sizeof(h));
-    h.c_visit = c->gb_cfg.c_visit;
-    h.c_scale = c->gb_cfg.c_scale;
-    h.scale = c->gb_cfg.gumbel_scale;
-    h.seed = c->gb_cfg.seed;
-    h.step = c->gb_serial++;
-    h.m = m;
-    h.n_tab = nt;
-    h.tab = c->d_gb_tab;
-    h.base = c->d_gb_base;
-    h.p = c->d_gb_p;
-    h.r0 = c->d_gb_r0;
-    h.interior = c->gi_search ? 1u : 0u;
-    h.rx = c->d_gb_rx;
-    ONB_CUDA(c, cudaMemcpyAsync(c->d_gb, &h, sizeof(h), cudaMemcpyHostToDevice, c->stream));
-    return ONB_OK;
-}
-}  // namespace onb
-extern "C" {
-int32_t onb_mcts_begin(onb_ctx* ctx, double c_puct, uint32_t sims) {
-    ONB_CHECK_CTX(ctx);
-    Ctx* c = reinterpret_cast<Ctx*>(ctx);
-    if (!c->d_nodes) return fail(c, ONB_E_STATE, "onb_mcts_begin: context created with mcts_max_sims = 0");
-    if (sims > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_mcts_begin: sims %u > mcts_max_sims %u", sims, c->cfg.mcts_max_sims);
-    c->c_puct = c_puct;
-    c->sims_target = sims;
-    c->sims_done = 0;
-    c->n_act = 0;  // the public search covers every game of the context
-    c->d_tree_game = nullptr;
-    c->mcts_phase = 0;
-    int32_t rc = gumbel_refusals(c, "onb_mcts_begin", c->reuse_on != 0);
-    if (rc != ONB_OK) return rc;
-    if (c->reuse_on) {  // every game, trees laid out by remaining budget; finish puts the outputs back into game order
-        ONB_CUDA(c, launch_reuse_begin(c, nullptr, c->n, sims));
-        c->ru_search = 1;
-        c->ru_public = 1;
+// Begins every search: checks the plan, replaces the active search with it, builds the trees (fresh, or rerooted from the remembered
+// ones with reuse) and, for a Gumbel plan, writes the search's GumbelDev and, when (m, sims) changed, the halving table. A begin
+// refused after the argument checks leaves no search to continue.
+static int32_t begin_search(Ctx* c, const SearchPlan& p, const char* who) {
+    if (!c->d_nodes) return fail(c, ONB_E_STATE, "%s: context created with mcts_max_sims = 0", who);
+    if (p.sims > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "%s: sims %u > mcts_max_sims %u", who, p.sims, c->cfg.mcts_max_sims);
+    if (p.d_games && (p.m <= 0 || p.m > c->n)) return fail(c, ONB_E_INVALID, "%s: bad subset size", who);
+    c->search = ActiveSearch();
+    // the combinations a Gumbel search does not support (include/onb.h, onb_mcts_set_gumbel)
+    if (p.gumbel && p.reuse) return fail(c, ONB_E_STATE, "%s: the Gumbel root search does not combine with tree reuse (onb_mcts_set_reuse)", who);
+    if (p.gumbel && p.noise) return fail(c, ONB_E_STATE, "%s: the Gumbel root search does not combine with train-mode noise (onb_mcts_set_noise)", who);
+    c->search.plan = p;
+    if (p.reuse) {
+        ONB_CUDA(c, launch_reuse_begin(c, p.d_games, p.d_games ? p.m : c->n, p.sims));
     } else {
-        c->ru_live = c->ru_search = c->ru_public = 0;  // a search without reuse forgets the remembered trees
+        c->ru_live = 0;  // a search without reuse forgets the remembered trees
+        c->search.n_act = p.d_games ? p.m : 0;
+        c->search.d_tree_game = p.d_games;
         ONB_CUDA(c, launch_mcts_begin(c));
     }
-    if ((rc = gumbel_begin(c, sims)) != ONB_OK) return rc;
-    c->mcts_phase = 1;
+    if (p.gumbel) {
+        const uint32_t m = p.gb_cfg.max_considered, nt = p.sims ? p.sims - 1u : 0u;
+        if (nt && (c->gb_tab_m != m || c->gb_tab_n != nt)) {
+            std::vector<uint32_t> tab((size_t)m * nt);
+            for (uint32_t r = 1; r <= m; ++r) onb_gumbel::seq_halving(r, nt, tab.data() + (size_t)(r - 1u) * nt);
+            // from pageable memory: the copy has taken the data when the call returns, so tab may go out of scope
+            ONB_CUDA(c, cudaMemcpyAsync(c->d_gb_tab, tab.data(), tab.size() * 4, cudaMemcpyHostToDevice, c->stream));
+            c->gb_tab_m = m;
+            c->gb_tab_n = nt;
+        }
+        GumbelDev h;
+        memset(&h, 0, sizeof(h));
+        h.c_visit = p.gb_cfg.c_visit;
+        h.c_scale = p.gb_cfg.c_scale;
+        h.scale = p.gb_cfg.gumbel_scale;
+        h.seed = p.gb_cfg.seed;
+        h.step = p.gb_step;
+        h.m = m;
+        h.n_tab = nt;
+        h.tab = c->d_gb_tab;
+        h.base = c->d_gb_base;
+        h.p = c->d_gb_p;
+        h.r0 = c->d_gb_r0;
+        h.interior = p.gb_cfg.interior ? 1u : 0u;
+        h.rx = c->d_gb_rx;
+        ONB_CUDA(c, cudaMemcpyAsync(c->d_gb, &h, sizeof(h), cudaMemcpyHostToDevice, c->stream));
+    }
+    c->search.phase = 1;
     return ONB_OK;
 }
-int32_t onb_mcts_set_gumbel(onb_ctx* ctx, const onb_gumbel_config* cfg) {
-    ONB_CHECK_CTX(ctx);
-    Ctx* c = reinterpret_cast<Ctx*>(ctx);
-    if (!cfg || !cfg->enabled) {
-        c->gb_on = 0;
-        return ONB_OK;
-    }
-    if (cfg->max_considered < 1 || cfg->max_considered > 40 || !std::isfinite(cfg->c_visit) || !std::isfinite(cfg->c_scale) ||
-        !std::isfinite(cfg->gumbel_scale) || !(cfg->c_visit >= 0.0) || !(cfg->c_scale >= 0.0) || !(cfg->gumbel_scale >= 0.0))
-        return fail(c, ONB_E_INVALID, "onb_mcts_set_gumbel: need 1 <= max_considered <= 40 and finite c_visit, c_scale, gumbel_scale >= 0");
-    if (cfg->interior > 1) return fail(c, ONB_E_INVALID, "onb_mcts_set_gumbel: interior must be 0 or 1");
-    if (!c->d_nodes) return fail(c, ONB_E_STATE, "onb_mcts_set_gumbel: context created with mcts_max_sims = 0");
+// the Gumbel search's buffers, allocated by the first call (r_x by the first with interior): onb_mcts_set_gumbel and onb_fight's
+// Gumbel agents. A failed allocation frees what this call allocated.
+static int32_t gumbel_alloc(Ctx* c, bool interior) {
     if (!c->d_gb) {
         const size_t n = (size_t)c->n;
         cudaError_t e = dalloc(&c->d_gb, 1);
@@ -546,7 +518,7 @@ int32_t onb_mcts_set_gumbel(onb_ctx* ctx, const onb_gumbel_config* cfg) {
         }
         c->gb_tab_m = c->gb_tab_n = 0;
     }
-    if (cfg->interior && !c->d_gb_rx) {  // r_x of every node of every tree
+    if (interior && !c->d_gb_rx) {  // r_x of every node of every tree
         const cudaError_t e = dalloc(&c->d_gb_rx, (size_t)c->n * c->node_cap);
         if (e != cudaSuccess) {
             c->d_gb_rx = nullptr;
@@ -554,6 +526,42 @@ int32_t onb_mcts_set_gumbel(onb_ctx* ctx, const onb_gumbel_config* cfg) {
                                                   : cuda_fail(c, e, "onb_mcts_set_gumbel");
         }
     }
+    return ONB_OK;
+}
+}  // namespace onb
+extern "C" {
+int32_t onb_mcts_begin(onb_ctx* ctx, double c_puct, uint32_t sims) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    SearchPlan p = {};
+    p.c_puct = c_puct;
+    p.sims = sims;
+    p.reuse = p.game_order = c->reuse_on != 0;  // with reuse: every game, trees laid out by remaining budget
+    p.noise = c->noise_on != 0;
+    p.noise_eps = c->noise_eps;
+    p.noise_alpha = c->noise_alpha;
+    p.noise_seed = c->noise_seed;
+    p.gumbel = c->gb_on != 0;
+    p.gb_cfg = c->gb_cfg;
+    p.gb_step = c->gb_serial;
+    const int32_t rc = begin_search(c, p, "onb_mcts_begin");
+    if (rc == ONB_OK && p.gumbel) c->gb_serial += 1;
+    return rc;
+}
+int32_t onb_mcts_set_gumbel(onb_ctx* ctx, const onb_gumbel_config* cfg) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (!cfg || !cfg->enabled) {
+        c->gb_on = 0;
+        return ONB_OK;
+    }
+    if (cfg->max_considered < 1 || cfg->max_considered > 40 || !std::isfinite(cfg->c_visit) || !std::isfinite(cfg->c_scale) ||
+        !std::isfinite(cfg->gumbel_scale) || !(cfg->c_visit >= 0.0) || !(cfg->c_scale >= 0.0) || !(cfg->gumbel_scale >= 0.0))
+        return fail(c, ONB_E_INVALID, "onb_mcts_set_gumbel: need 1 <= max_considered <= 40 and finite c_visit, c_scale, gumbel_scale >= 0");
+    if (cfg->interior > 1) return fail(c, ONB_E_INVALID, "onb_mcts_set_gumbel: interior must be 0 or 1");
+    if (!c->d_nodes) return fail(c, ONB_E_STATE, "onb_mcts_set_gumbel: context created with mcts_max_sims = 0");
+    const int32_t rc = gumbel_alloc(c, cfg->interior != 0);
+    if (rc != ONB_OK) return rc;
     c->gb_cfg = *cfg;
     c->gb_serial = cfg->step0;
     c->gb_on = 1;
@@ -599,19 +607,20 @@ int32_t onb_mcts_set_noise(onb_ctx* ctx, int32_t enabled, double epsilon, double
 int32_t onb_mcts_select(onb_ctx* ctx) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
-    if (c->mcts_phase != 1) return fail(c, ONB_E_STATE, "onb_mcts_select: call onb_mcts_begin / onb_mcts_expand_backup first");
-    if (c->ru_search) return refuse_after_reuse(c, "onb_mcts_select");
-    if (c->gb_search && c->sims_done >= c->sims_target)
-        return fail(c, ONB_E_STATE, "onb_mcts_select: a Gumbel search runs at most the begin's %u simulations", c->sims_target);
+    ActiveSearch& a = c->search;
+    if (a.phase != 1) return fail(c, ONB_E_STATE, "onb_mcts_select: call onb_mcts_begin / onb_mcts_expand_backup first");
+    if (a.plan.reuse) return refuse_after_reuse(c, "onb_mcts_select");
+    if (a.plan.gumbel && a.sims_done >= a.plan.sims)
+        return fail(c, ONB_E_STATE, "onb_mcts_select: a Gumbel search runs at most the begin's %u simulations", a.plan.sims);
     ONB_CUDA(c, launch_mcts_select(c));
-    c->mcts_phase = 2;
+    a.phase = 2;
     return ONB_OK;
 }
 int32_t onb_mcts_eval(onb_ctx* ctx, int32_t evaluator) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
-    if (c->ru_search) return refuse_after_reuse(c, "onb_mcts_eval");
-    if (c->mcts_phase != 2) return fail(c, ONB_E_STATE, "onb_mcts_eval: no leaves selected");
+    if (c->search.plan.reuse) return refuse_after_reuse(c, "onb_mcts_eval");
+    if (c->search.phase != 2) return fail(c, ONB_E_STATE, "onb_mcts_eval: no leaves selected");
     if (evaluator == ONB_EVAL_NET) {
         if (!c->net[c->net_cur].loaded) return fail(c, ONB_E_STATE, "onb_mcts_eval: no network loaded (onb_net_load)");
         ONB_CUDA(c, launch_net_forward(c, c->d_leaf_planes, c->d_policy, c->d_value, trees(c)));
@@ -624,25 +633,26 @@ int32_t onb_mcts_eval(onb_ctx* ctx, int32_t evaluator) {
 int32_t onb_mcts_expand_backup(onb_ctx* ctx) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
-    if (c->ru_search) return refuse_after_reuse(c, "onb_mcts_expand_backup");
-    if (c->mcts_phase != 2) return fail(c, ONB_E_STATE, "onb_mcts_expand_backup: call onb_mcts_select first");
+    if (c->search.plan.reuse) return refuse_after_reuse(c, "onb_mcts_expand_backup");
+    if (c->search.phase != 2) return fail(c, ONB_E_STATE, "onb_mcts_expand_backup: call onb_mcts_select first");
     ONB_CUDA(c, launch_mcts_expand_backup(c));
-    c->mcts_phase = 1;
-    c->sims_done += 1;
+    c->search.phase = 1;
+    c->search.sims_done += 1;
     return ONB_OK;
 }
 // onb_mcts_run after a reuse begin: slot t runs max(0, sims - N_root) simulations; the slots are ordered by that budget, so round r
 // runs the prefix [0, h_ru_off[r]) -- the network evaluates a shrinking batch, the fused kernel is launched once per run of rounds
 // with the same prefix. Splitting a tree's simulations over several launches gives the same tree: the kernels keep nothing else.
 static int32_t reuse_run(Ctx* c, int32_t evaluator, uint32_t sims) {
-    if (sims != c->sims_target || c->sims_done != 0)
-        return fail(c, ONB_E_INVALID, "onb_mcts_run: after a reuse begin, run once with the begin's visit target (%u), got %u", c->sims_target, sims);
+    ActiveSearch& a = c->search;
+    if (sims != a.plan.sims || a.sims_done != 0)
+        return fail(c, ONB_E_INVALID, "onb_mcts_run: after a reuse begin, run once with the begin's visit target (%u), got %u", a.plan.sims, sims);
     if (evaluator == ONB_EVAL_NET && !c->net[c->net_cur].loaded) return fail(c, ONB_E_STATE, "onb_mcts_run: no network loaded (onb_net_load)");
     const uint32_t* off = c->h_ru_off;
     cudaError_t e = cudaSuccess;
     if (evaluator == ONB_EVAL_NET) {
         for (uint32_t r = 0; r < sims && off[r] > 0 && e == cudaSuccess; ++r) {
-            c->n_act = (int64_t)off[r];
+            a.n_act = (int64_t)off[r];
             e = launch_mcts_select(c);
             if (e == cudaSuccess) e = launch_net_forward(c, c->d_leaf_planes, c->d_policy, c->d_value, (int64_t)off[r]);
             if (e == cudaSuccess) e = launch_mcts_expand_backup(c);
@@ -651,26 +661,27 @@ static int32_t reuse_run(Ctx* c, int32_t evaluator, uint32_t sims) {
         for (uint32_t r = 0; r < sims && off[r] > 0 && e == cudaSuccess;) {
             uint32_t r1 = r + 1;
             while (r1 < sims && off[r1] == off[r]) ++r1;
-            c->n_act = (int64_t)off[r];
+            a.n_act = (int64_t)off[r];
             e = launch_mcts_run(c, evaluator, r1 - r);
             r = r1;
         }
     }
-    c->n_act = c->ru_m;
+    a.n_act = c->ru_m;
     if (e != cudaSuccess) return cuda_fail(c, e, "onb_mcts_run");
-    c->sims_done += sims;
+    a.sims_done += sims;
     return ONB_OK;
 }
 int32_t onb_mcts_run(onb_ctx* ctx, int32_t evaluator, uint32_t sims) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
-    if (c->mcts_phase != 1) return fail(c, ONB_E_STATE, "onb_mcts_run: call onb_mcts_begin first");
+    ActiveSearch& a = c->search;
+    if (a.phase != 1) return fail(c, ONB_E_STATE, "onb_mcts_run: call onb_mcts_begin first");
     if (evaluator != ONB_EVAL_UNIFORM && evaluator != ONB_EVAL_HASH && evaluator != ONB_EVAL_NET)
         return fail(c, ONB_E_INVALID, "onb_mcts_run: unknown evaluator %d", evaluator);
-    if (c->sims_done + sims > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_mcts_run: more simulations than mcts_max_sims");
-    if (c->ru_search) return reuse_run(c, evaluator, sims);
-    if (c->gb_search && c->sims_done + sims > c->sims_target)
-        return fail(c, ONB_E_STATE, "onb_mcts_run: a Gumbel search runs at most the begin's %u simulations", c->sims_target);
+    if (a.sims_done + sims > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_mcts_run: more simulations than mcts_max_sims");
+    if (a.plan.reuse) return reuse_run(c, evaluator, sims);
+    if (a.plan.gumbel && a.sims_done + sims > a.plan.sims)
+        return fail(c, ONB_E_STATE, "onb_mcts_run: a Gumbel search runs at most the begin's %u simulations", a.plan.sims);
     if (evaluator == ONB_EVAL_NET) {
         // the network sits between select and expand: three launches per simulation round, all on the context's stream
         // (one launch for expand_backup(s) + select(s + 1) was measured slower, DESIGN.md section 8)
@@ -681,51 +692,31 @@ int32_t onb_mcts_run(onb_ctx* ctx, int32_t evaluator, uint32_t sims) {
             ONB_CUDA(c, launch_mcts_expand_backup(c));
             if (s + 1 < sims) ONB_CUDA(c, launch_mcts_select(c));
         }
-        c->sims_done += sims;
+        a.sims_done += sims;
         return ONB_OK;
     }
     ONB_CUDA(c, launch_mcts_run(c, evaluator, sims));
-    c->sims_done += sims;
+    a.sims_done += sims;
     return ONB_OK;
 }
-// onb_mcts_begin for a SUBSET of the games: tree t searches game d_games[t] (device list, ascending), t < m. d_games == nullptr: all games.
-static int32_t mcts_begin_subset(Ctx* c, double c_puct, uint32_t sims, const int32_t* d_games, int64_t m) {
+// onb_self_play's search of ply `ply` over the m games d_games (nullptr: all): noise from the config, Gumbel (step = ply) and reuse
+// from the context's switches. With reuse the outputs stay in slot order; the driver scatters them through search.d_tree_game.
+static int32_t self_play_search(Ctx* c, const onb_selfplay_config* cfg, uint32_t ply, const int32_t* d_games, int64_t m) {
     onb_ctx* x = reinterpret_cast<onb_ctx*>(c);
-    if (!d_games) return onb_mcts_begin(x, c_puct, sims);
-    if (!c->d_nodes) return fail(c, ONB_E_STATE, "search: context created with mcts_max_sims = 0");
-    if (sims > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "search: sims %u > mcts_max_sims %u", sims, c->cfg.mcts_max_sims);
-    if (m <= 0 || m > c->n) return fail(c, ONB_E_INVALID, "search: bad subset size");
-    c->c_puct = c_puct;
-    c->sims_target = sims;
-    c->sims_done = 0;
-    c->n_act = m;
-    c->d_tree_game = d_games;
-    c->ru_live = c->ru_search = c->ru_public = 0;  // a search without reuse forgets the remembered trees
-    int32_t rc = gumbel_refusals(c, "search", false);
-    if (rc != ONB_OK) return rc;
-    ONB_CUDA(c, launch_mcts_begin(c));
-    if ((rc = gumbel_begin(c, sims)) != ONB_OK) return rc;
-    c->mcts_phase = 1;
-    return ONB_OK;
-}
-// onb_self_play's search with reuse: the m games d_games (nullptr: all) in budget order; the outputs stay in slot order, the driver
-// scatters them through d_tree_game
-static int32_t reuse_begin_subset(Ctx* c, double c_puct, uint32_t sims, const int32_t* d_games, int64_t m) {
-    const int32_t rc = gumbel_refusals(c, "onb_self_play", true);
-    if (rc != ONB_OK) return rc;
-    c->c_puct = c_puct;
-    c->sims_target = sims;
-    c->sims_done = 0;
-    c->mcts_phase = 0;
-    ONB_CUDA(c, launch_reuse_begin(c, d_games, d_games ? m : c->n, sims));
-    c->ru_search = 1;
-    c->ru_public = 0;
-    c->mcts_phase = 1;
-    return ONB_OK;
-}
-static int32_t self_play_search(Ctx* c, const onb_selfplay_config* cfg, const int32_t* d_games, int64_t m) {
-    onb_ctx* x = reinterpret_cast<onb_ctx*>(c);
-    int32_t rc = c->reuse_on ? reuse_begin_subset(c, cfg->c_puct, cfg->sims, d_games, m) : mcts_begin_subset(c, cfg->c_puct, cfg->sims, d_games, m);
+    SearchPlan p = {};
+    p.c_puct = cfg->c_puct;
+    p.sims = cfg->sims;
+    p.d_games = d_games;
+    p.m = m;
+    p.reuse = c->reuse_on != 0;
+    p.noise = cfg->train != 0;
+    p.noise_eps = 0.25;
+    p.noise_alpha = 0.03;
+    p.noise_seed = cfg->noise_seed;
+    p.gumbel = c->gb_on != 0;
+    p.gb_cfg = c->gb_cfg;
+    p.gb_step = ply;
+    int32_t rc = begin_search(c, p, "search");
     if (rc == ONB_OK) rc = onb_mcts_run(x, cfg->evaluator, cfg->sims);
     if (rc == ONB_OK) rc = onb_mcts_finish(x, nullptr, nullptr, nullptr, nullptr, nullptr);
     return rc;
@@ -741,20 +732,18 @@ int32_t onb_self_play(onb_ctx* ctx, const onb_selfplay_config* cfg, onb_selfplay
     if (c->reuse_on && c->gb_on) return fail(c, ONB_E_STATE, "onb_self_play: tree reuse does not combine with the Gumbel root search");
     memset(out, 0, sizeof(*out));
     c->ru_live = 0;  // self-play starts from fresh deals: nothing is kept from earlier searches
-    int32_t rc = onb_mcts_set_noise(ctx, cfg->train ? 1 : 0, 0.25, 0.03, cfg->noise_seed);
-    if (rc != ONB_OK) return rc;
-    const uint32_t serial = c->gb_serial;
-    c->gb_serial = 0;  // one search per ply: the Gumbel step of ply p is p
     char err[400];
     err[0] = 0;
+    int32_t rc;
     try {
         rc = run_self_play(c, cfg, out, self_play_search, err, sizeof(err));
     } catch (const std::exception& ex) {
         snprintf(err, sizeof(err), "onb_self_play: %s", ex.what());
         rc = ONB_E_NOMEM;
     }
-    c->gb_serial = serial;
-    onb_mcts_set_noise(ctx, 0, 0.25, 0.03, 0);
+    c->search.n_act = 0;  // the driver's last search may have covered a subset; later calls see every game
+    c->search.d_tree_game = nullptr;
+    onb_mcts_set_noise(ctx, 0, 0.25, 0.03, 0);  // onb_self_play has always left train-mode noise off; its searches take noise from cfg
     if (rc != ONB_OK) return fail(c, rc, "%s", err);
     return ONB_OK;
 }
@@ -775,21 +764,27 @@ static int32_t fight_move(Ctx* c, const onb_agent* ag, uint32_t ply, const int32
         ONB_CUDA(c, launch_tb_best(c, d_games, m, d_out));
         return ONB_OK;
     }
-    c->gb_on = 0;  // PUCT and UCT agents search without the Gumbel root step
-    const bool gumbel = ag->kind == ONB_AGENT_GUMBEL || ag->kind == ONB_AGENT_GUMBEL_MUZERO;
-    if (gumbel) {
-        c->gb_on = 1;
-        c->gb_cfg.interior = ag->kind == ONB_AGENT_GUMBEL_MUZERO ? 1u : 0u;
-        c->gb_cfg.max_considered = ag->min_node_visits ? ag->min_node_visits : 16u;
-        c->gb_cfg.c_visit = 50.0;
-        c->gb_cfg.c_scale = ag->c;
-        c->gb_cfg.gumbel_scale = 1.0;
-        c->gb_cfg.seed = c->cfg.seed;
-        c->gb_serial = ply;
+    // eval mode (AlphaZeroMcts, not TrainingAlphaZeroMcts) and no reuse; PUCT and UCT agents search without the Gumbel root step
+    SearchPlan p = {};
+    p.c_puct = ag->c;
+    p.sims = ag->sims;
+    p.d_games = d_games;
+    p.m = m;
+    p.gumbel = ag->kind == ONB_AGENT_GUMBEL || ag->kind == ONB_AGENT_GUMBEL_MUZERO;
+    if (p.gumbel) {  // PUCT with c_puct 2 below the root, or Gumbel MuZero's interior selection
+        p.c_puct = 2.0;
+        p.gb_cfg.enabled = 1;
+        p.gb_cfg.max_considered = ag->min_node_visits ? ag->min_node_visits : 16u;
+        p.gb_cfg.c_visit = 50.0;
+        p.gb_cfg.c_scale = ag->c;
+        p.gb_cfg.gumbel_scale = 1.0;
+        p.gb_cfg.seed = c->cfg.seed;
+        p.gb_cfg.interior = ag->kind == ONB_AGENT_GUMBEL_MUZERO ? 1u : 0u;
+        p.gb_step = ply;
     }
-    int32_t rc = mcts_begin_subset(c, gumbel ? 2.0 : ag->c, ag->sims, d_games, m);
+    int32_t rc = begin_search(c, p, "search");
     if (rc != ONB_OK) return rc;
-    if (ag->kind == ONB_AGENT_PUCT || gumbel) {
+    if (ag->kind == ONB_AGENT_PUCT || p.gumbel) {
         if (ag->evaluator == ONB_EVAL_NET && (rc = onb_net_select(x, ag->net_slot)) != ONB_OK) return rc;
         rc = onb_mcts_run(x, ag->evaluator, ag->sims);
     } else {
@@ -838,29 +833,15 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
             return fail(c, ONB_E_INVALID, "onb_fight: %llu undecided games are not positions of the tablebase (card set or material)", missing);
     }
     memset(out, 0, sizeof(*out));
-    int32_t rc = onb_mcts_set_noise(ctx, 0, 0.25, 0.03, 0);  // arenas search in eval mode (AlphaZeroMcts, not TrainingAlphaZeroMcts)
-    if (rc != ONB_OK) return rc;
-    const int gb_on = c->gb_on;  // the agents set the Gumbel switch per move; the context's own setting comes back afterwards
-    const onb_gumbel_config gb_cfg = c->gb_cfg;
-    const uint32_t gb_serial = c->gb_serial;
+    onb_mcts_set_noise(ctx, 0, 0.25, 0.03, 0);  // onb_fight has always left train-mode noise off; its plans search in eval mode anyway
     const bool muzero = a->kind == ONB_AGENT_GUMBEL_MUZERO || b->kind == ONB_AGENT_GUMBEL_MUZERO;
-    if (a->kind == ONB_AGENT_GUMBEL || b->kind == ONB_AGENT_GUMBEL || muzero) {
-        onb_gumbel_config on;
-        memset(&on, 0, sizeof(on));
-        on.enabled = 1;
-        on.max_considered = 16;
-        on.interior = muzero ? 1u : 0u;  // allocates r_x too
-        if ((rc = onb_mcts_set_gumbel(ctx, &on)) != ONB_OK) return rc;  // allocates the Gumbel buffers; the context's setting is restored below
-        c->gb_on = gb_on;
-        c->gb_cfg = gb_cfg;
-        c->gb_serial = gb_serial;
-    }
+    int32_t rc;
+    if ((a->kind == ONB_AGENT_GUMBEL || b->kind == ONB_AGENT_GUMBEL || muzero) && (rc = gumbel_alloc(c, muzero)) != ONB_OK) return rc;
     char err[400];
     err[0] = 0;
     rc = run_fight(c, a, b, a_is_red_host, max_plies, out, fight_move, err, sizeof(err));
-    c->gb_on = gb_on;
-    c->gb_cfg = gb_cfg;
-    c->gb_serial = gb_serial;
+    c->search.n_act = 0;  // the agents searched subsets; later calls see every game
+    c->search.d_tree_game = nullptr;
     if (rc != ONB_OK) return fail(c, rc, "%s", err);
     if (results_host) {
         ONB_CUDA(c, cudaMemcpyAsync(results_host, out->results, (size_t)c->n, cudaMemcpyDeviceToHost, c->stream));
@@ -891,11 +872,12 @@ int32_t onb_copy_to_host(onb_ctx* ctx, void* host, const void* device, int64_t b
 int32_t onb_uct_run(onb_ctx* ctx, float exploration_c, uint32_t min_node_visits, uint32_t playouts) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
-    if (c->mcts_phase != 1) return fail(c, ONB_E_STATE, "onb_uct_run: call onb_mcts_begin first");
-    if (c->ru_search) return refuse_after_reuse(c, "onb_uct_run");
-    if (c->gb_search) return fail(c, ONB_E_STATE, "onb_uct_run: the search was begun with the Gumbel root search on (onb_mcts_set_gumbel)");
-    if (c->sims_done + playouts > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_uct_run: more playouts than mcts_max_sims");
-    const uint32_t need = c->sims_done + playouts + 2;
+    ActiveSearch& a = c->search;
+    if (a.phase != 1) return fail(c, ONB_E_STATE, "onb_uct_run: call onb_mcts_begin first");
+    if (a.plan.reuse) return refuse_after_reuse(c, "onb_uct_run");
+    if (a.plan.gumbel) return fail(c, ONB_E_STATE, "onb_uct_run: the search was begun with the Gumbel root search on (onb_mcts_set_gumbel)");
+    if (a.sims_done + playouts > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_uct_run: more playouts than mcts_max_sims");
+    const uint32_t need = a.sims_done + playouts + 2;
     if (c->ln_cap < need) {  // ln(parent visits) as the reference computes it: f32 logf on the host
         ONB_CUDA(c, cudaStreamSynchronize(c->stream));
         if (c->d_ln_table) cudaFree(c->d_ln_table);
@@ -912,7 +894,7 @@ int32_t onb_uct_run(onb_ctx* ctx, float exploration_c, uint32_t min_node_visits,
         c->ln_cap = cap;
     }
     ONB_CUDA(c, launch_uct_run(c, exploration_c, min_node_visits, playouts));
-    c->sims_done += playouts;
+    a.sims_done += playouts;
     return ONB_OK;
 }
 int32_t onb_alphabeta_run(onb_ctx* ctx, int32_t depth, onb_action* best_host, int32_t* score_host, uint64_t* nodes_host) {
@@ -982,16 +964,12 @@ int32_t onb_tb_best(onb_ctx* ctx, onb_action* best_host) {
 int32_t onb_mcts_finish(onb_ctx* ctx, onb_action* best_host, float* pi_host, uint32_t* root_visits_host, double* root_q_host, uint32_t* child_visits_host) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
-    if (c->mcts_phase != 1) return fail(c, ONB_E_STATE, "onb_mcts_finish: search not in a finished-simulation state");
-    if (c->ru_search && c->ru_public) {  // finish in slot order into the scratch, then back into game order
-        float* pi = c->d_pi; uint16_t* best = c->d_best; uint32_t* rv = c->d_root_visits; double* q = c->d_root_q; uint32_t* cv = c->d_child_visits;
-        c->d_pi = c->d_ru_pi; c->d_best = c->d_ru_best; c->d_root_visits = c->d_ru_rv; c->d_root_q = c->d_ru_q; c->d_child_visits = c->d_ru_cv;
-        const cudaError_t e = launch_mcts_finish(c);
-        c->d_pi = pi; c->d_best = best; c->d_root_visits = rv; c->d_root_q = q; c->d_child_visits = cv;
-        ONB_CUDA(c, e);
+    if (c->search.phase != 1) return fail(c, ONB_E_STATE, "onb_mcts_finish: search not in a finished-simulation state");
+    if (c->search.plan.reuse && c->search.plan.game_order) {  // finish in slot order into the scratch, then back into game order
+        ONB_CUDA(c, launch_mcts_finish(c, c->d_ru_pi, c->d_ru_best, c->d_ru_rv, c->d_ru_q, c->d_ru_cv));
         ONB_CUDA(c, launch_reuse_unpermute(c));
     } else {
-        ONB_CUDA(c, launch_mcts_finish(c));
+        ONB_CUDA(c, launch_mcts_finish(c, c->d_pi, c->d_best, c->d_root_visits, c->d_root_q, c->d_child_visits));
     }
     const size_t n = (size_t)c->n;
     bool any = false;
@@ -1009,7 +987,7 @@ int32_t onb_mcts_play_best(onb_ctx* ctx, uint32_t out_flags) {
     if (!c->d_best) return fail(c, ONB_E_STATE, "onb_mcts_play_best: no search buffers");
     if ((out_flags & ONB_OUT_PLANES) && !c->d_planes) return fail(c, ONB_E_STATE, "onb_mcts_play_best: plane buffer not allocated");
     ONB_CUDA(c, launch_mcts_play_best(c, out_flags));
-    c->mcts_phase = 0;
+    c->search.phase = 0;
     return ONB_OK;
 }
 int32_t onb_mcts_dump_tree(onb_ctx* ctx, int64_t tree, int64_t cap, onb_tree_dump* out, int64_t* n_nodes) {

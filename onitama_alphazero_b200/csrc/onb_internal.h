@@ -41,6 +41,34 @@ struct GumbelDev {
     float* rx;                          // [n][node_cap] r_x: the reward the expanding simulation backed up into node x (interior only)
 };
 
+// Everything a search is begun with (begin_search). onb_mcts_begin builds it from the context's switches, onb_self_play from its
+// config, onb_fight from the agent; the launchers read only the copy in Ctx::search, so a switch changed after the begin does not
+// reach the search already running.
+struct SearchPlan {
+    double c_puct;
+    uint32_t sims;
+    const int32_t* d_games;  // tree t searches game d_games[t] (device, ascending), t < m; nullptr: every game
+    int64_t m;
+    bool reuse;              // keep the remembered trees (onb_reuse.cu): the trees are laid out by remaining budget
+    bool game_order;         // ... and onb_mcts_finish puts its outputs back into game order (the public onb_mcts_begin)
+    bool noise;              // train-mode root noise (onb_mcts_set_noise)
+    double noise_eps, noise_alpha;
+    uint64_t noise_seed;
+    bool gumbel;             // the Gumbel root search (onb_mcts_set_gumbel); gb_cfg.interior: Gumbel MuZero below the root
+    onb_gumbel_config gb_cfg;
+    uint32_t gb_step;
+};
+// the search begun last
+struct ActiveSearch {
+    SearchPlan plan;
+    uint32_t sims_done;
+    int phase;  // 0 idle, 1 begun/after expand, 2 after select
+    // the first n_act trees search the games listed in d_tree_game (device, ascending); n_act == 0: every game is searched by the
+    // tree of the same index. A subset plan sets them, launch_reuse_begin fills them for a reuse begin.
+    int64_t n_act;
+    const int32_t* d_tree_game;
+};
+
 struct Ctx {
     onb_config cfg;
     cudaStream_t stream;
@@ -73,16 +101,10 @@ struct Ctx {
     uint32_t* d_root_visits;
     double* d_root_q;
     uint32_t* d_child_visits;  // [n][40]
-    double c_puct;
-    int noise_on;           // train mode: Dirichlet-like exploration noise at the root (mcts_arena.rs:186-202)
+    ActiveSearch search;
+    int noise_on;           // the switch of onb_mcts_set_noise: Dirichlet-like exploration noise at the root (mcts_arena.rs:186-202)
     double noise_eps, noise_alpha;
     uint64_t noise_seed;
-    uint32_t sims_target, sims_done;
-    int mcts_phase;  // 0 idle, 1 begun/after expand, 2 after select
-    // subset search (onb_fight / onb_self_play): the first n_act trees search the games listed in d_tree_game (device, ascending);
-    // n_act == 0: every game is searched by the tree of the same index (the public onb_mcts_begin always selects this)
-    int64_t n_act;
-    const int32_t* d_tree_game;
     float* d_ln_table;  // logf(i) for the plain UCT search (filled by the host: the libm call behind Rust's f32::ln)
     uint32_t ln_cap;
     // policy/value network (onb_net.cu): weights in tensor-core operand layout, folded biases, head parameters
@@ -109,8 +131,6 @@ struct Ctx {
     // tree reuse (onb_reuse.cu, onb_mcts_set_reuse); buffers allocated by the first enabling call
     int reuse_on;         // the switch
     int ru_live;          // the pools hold the remembered trees of the last reuse search (slot layout of d_ru_game / d_ru_slot)
-    int ru_search;        // the current search was begun with reuse (split phase refused, onb_mcts_run needs sims_target)
-    int ru_public;        // ... by onb_mcts_begin: onb_mcts_finish puts its outputs back into game order
     int64_t ru_m;         // trees of the current reuse search
     Node* d_nodes_alt;    // second pool: the kept subtrees are compacted into it, then the pools swap
     uint4* d_roots_alt;
@@ -131,8 +151,6 @@ struct Ctx {
     int gb_on;                // the switch
     onb_gumbel_config gb_cfg;
     uint32_t gb_serial;       // step of the next Gumbel onb_mcts_begin
-    int gb_search;            // the current search was begun with Gumbel
-    int gi_search;            // ... with Gumbel and interior selection (gb_cfg.interior)
     GumbelDev* d_gb;          // the device struct every Gumbel begin rewrites
     uint32_t* d_gb_tab;       // [40][mcts_max_sims]
     double* d_gb_base;
@@ -150,7 +168,7 @@ struct Ctx {
     char err[512];
 };
 
-inline int64_t trees(const Ctx* c) { return c->n_act > 0 ? c->n_act : c->n; }
+inline int64_t trees(const Ctx* c) { return c->search.n_act > 0 ? c->search.n_act : c->n; }
 
 // env (onb_env.cu)
 cudaError_t launch_env_reset(Ctx* c, const uint8_t* d_decks5, int64_t n_decks, uint32_t epoch);
@@ -173,11 +191,11 @@ cudaError_t launch_mcts_expand_backup(Ctx* c);
 cudaError_t launch_mcts_eval(Ctx* c, int evaluator);
 cudaError_t launch_mcts_run(Ctx* c, int evaluator, uint32_t sims);
 cudaError_t launch_uct_run(Ctx* c, float exploration_c, uint32_t min_node_visits, uint32_t sims);
-cudaError_t launch_mcts_finish(Ctx* c);
+cudaError_t launch_mcts_finish(Ctx* c, float* pi, uint16_t* best, uint32_t* root_visits, double* root_q, uint32_t* child_visits);
 cudaError_t launch_mcts_play_best(Ctx* c, uint32_t out_flags);
 cudaError_t launch_mcts_scatter_best(Ctx* c, uint16_t* dst_actions);  // dst[game of tree t] = best[t]
-// with c->gb_search the three launchers above that select at the root (select, run, finish) run the Gumbel variants; with
-// c->gi_search select, run and expand_backup run the interior-selection variants
+// the search launchers take their kernel from c->search.plan: noise, Gumbel at the root (select, run, finish) and Gumbel MuZero
+// below it (select, run, expand_backup)
 
 // network (onb_net.cu)
 int32_t net_load(Ctx* c, int32_t n_tensors, const char* const* names, const float* const* data, const int64_t* numel, std::string& err);
@@ -199,13 +217,14 @@ cudaError_t launch_tb_best(Ctx* c, const int32_t* d_games, int64_t m, uint16_t* 
 cudaError_t reuse_alloc(Ctx* c);
 void reuse_free(Ctx* c);
 // reroot the remembered trees of the m games d_games (nullptr: all games) for a search to `sims` visits, swap the pools, fill
-// h_ru_off; leaves n_act = m, d_tree_game = d_ru_game
+// h_ru_off; leaves search.n_act = m, search.d_tree_game = d_ru_game
 cudaError_t launch_reuse_begin(Ctx* c, const int32_t* d_games, int64_t m, uint32_t sims);
 cudaError_t launch_reuse_unpermute(Ctx* c);  // d_ru_* (slot order) -> d_pi / d_best / ... (game order)
 
 // native self-play driver (onb_selfplay.cu)
 int32_t run_self_play(Ctx* c, const onb_selfplay_config* cfg, onb_selfplay_result* out,
-                      int32_t (*search)(Ctx*, const onb_selfplay_config*, const int32_t* d_games, int64_t m), char* err, size_t err_len);
+                      int32_t (*search)(Ctx*, const onb_selfplay_config*, uint32_t ply, const int32_t* d_games, int64_t m), char* err,
+                      size_t err_len);
 
 int32_t run_fight(Ctx* c, const onb_agent* a, const onb_agent* b, const uint8_t* a_is_red_host, uint32_t max_plies, onb_fight_result* out,
                   int32_t (*move)(Ctx*, const onb_agent*, uint32_t ply, const int32_t* d_games, int64_t m, uint16_t* d_out), char* err, size_t err_len);

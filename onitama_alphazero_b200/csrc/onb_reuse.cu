@@ -278,8 +278,8 @@ cudaError_t launch_reuse_begin(Ctx* c, const int32_t* d_games, int64_t m, uint32
     uint32_t* ts = c->d_tree_size; c->d_tree_size = c->d_tree_size_alt; c->d_tree_size_alt = ts;
     if ((e = cudaMemcpyAsync(c->h_ru_off, c->d_ru_off, (size_t)(sims + 1) * 4, cudaMemcpyDeviceToHost, c->stream)) != cudaSuccess) return e;
     if ((e = cudaStreamSynchronize(c->stream)) != cudaSuccess) return e;
-    c->n_act = m;
-    c->d_tree_game = c->d_ru_game;
+    c->search.n_act = m;
+    c->search.d_tree_game = c->d_ru_game;
     c->ru_live = 1;
     c->ru_m = m;
     // counters: sum over rounds of the active trees = simulations; kept = trees whose budget is below the target

@@ -211,10 +211,10 @@ enum : int {
 };
 static_assert(kFtHistory < 32, "Ctx::sp_buf has 32 slots");
 
-// Returns ONB_OK, or an ONB_E_* code with `err` filled. `search` runs one search (begin / run / finish) over the m games listed in
-// d_games (device, ascending; nullptr = all games of the context).
+// Returns ONB_OK, or an ONB_E_* code with `err` filled. `search` runs one search (begin / run / finish) for ply `ply` over the m games
+// listed in d_games (device, ascending; nullptr = all games of the context).
 int32_t run_self_play(Ctx* c, const onb_selfplay_config* cfg, onb_selfplay_result* out,
-                      int32_t (*search)(Ctx*, const onb_selfplay_config*, const int32_t*, int64_t), char* err, size_t err_len) {
+                      int32_t (*search)(Ctx*, const onb_selfplay_config*, uint32_t, const int32_t*, int64_t), char* err, size_t err_len) {
     const int64_t n = c->n;
     const int64_t cap_ticks = cfg->sample_cap / n;
     if (cap_ticks < 1) {
@@ -234,8 +234,6 @@ int32_t run_self_play(Ctx* c, const onb_selfplay_config* cfg, onb_selfplay_resul
         e = (call);                                                                    \
         if (e != cudaSuccess) {                                                        \
             snprintf(err, err_len, "onb_self_play: %s: %s", #call, cudaGetErrorString(e)); \
-            c->n_act = 0;                                                              \
-            c->d_tree_game = nullptr;                                                  \
             return e == cudaErrorMemoryAllocation ? ONB_E_NOMEM : ONB_E_CUDA;          \
         }                                                                              \
     } while (0)
@@ -279,18 +277,16 @@ int32_t run_self_play(Ctx* c, const onb_selfplay_config* cfg, onb_selfplay_resul
         SP(cudaMemcpyAsync(planes + (size_t)base * 525, c->d_planes, (size_t)n * 2100, cudaMemcpyDeviceToDevice, c->stream));
         k_sp_record<<<grid, 256, 0, c->stream>>>(c->d_states, n, generation, base, color, serial, valid, z);
         SP(cudaGetLastError());
-        const int32_t rc = search(c, cfg, all ? nullptr : live_list, all ? 0 : n_live);   // only the slots with a game in progress
+        const int32_t rc = search(c, cfg, (uint32_t)tick, all ? nullptr : live_list, all ? 0 : n_live);  // only the slots with a game in progress
         if (rc != ONB_OK) {
             snprintf(err, err_len, "%s", c->err);
-            c->n_act = 0;
-            c->d_tree_game = nullptr;
             return rc;
         }
-        if (!c->d_tree_game) {  // tree t searched game t
+        if (!c->search.d_tree_game) {  // tree t searched game t
             SP(cudaMemcpyAsync(pi + (size_t)base * 50, c->d_pi, (size_t)n * 200, cudaMemcpyDeviceToDevice, c->stream));
         } else {                // the searched list (live_list, or with tree reuse that list ordered by remaining budget)
             const int64_t nt = trees(c);
-            k_scatter_rows50<<<(unsigned)((nt * 50 + 255) / 256), 256, 0, c->stream>>>(c->d_pi, c->d_tree_game, pi + (size_t)base * 50, nt);
+            k_scatter_rows50<<<(unsigned)((nt * 50 + 255) / 256), 256, 0, c->stream>>>(c->d_pi, c->search.d_tree_game, pi + (size_t)base * 50, nt);
             SP(cudaGetLastError());
         }
         SP(cudaMemsetAsync(c->d_actions, 0xFF, (size_t)n * 2, c->stream));   // ONB_ACTION_NONE: idle slots are not stepped
@@ -311,8 +307,6 @@ int32_t run_self_play(Ctx* c, const onb_selfplay_config* cfg, onb_selfplay_resul
         n_live = (int64_t)h[1];
         ++tick;
     }
-    c->n_act = 0;
-    c->d_tree_game = nullptr;
     // index list of the valid samples (ascending): flags to the host, indices back
     const size_t total = (size_t)tick * (size_t)n;
     std::vector<uint8_t> flags(total);
@@ -335,7 +329,7 @@ int32_t run_self_play(Ctx* c, const onb_selfplay_config* cfg, onb_selfplay_resul
     out->color = color;
     out->serial = serial;
     out->valid_idx = idx;
-    c->mcts_phase = 0;
+    c->search.phase = 0;
     return ONB_OK;
 }
 
@@ -357,8 +351,6 @@ int32_t run_fight(Ctx* c, const onb_agent* a, const onb_agent* b, const uint8_t*
         e = (call);                                                                 \
         if (e != cudaSuccess) {                                                     \
             snprintf(err, err_len, "onb_fight: %s: %s", #call, cudaGetErrorString(e)); \
-            c->n_act = 0;                                                           \
-            c->d_tree_game = nullptr;                                               \
             return e == cudaErrorMemoryAllocation ? ONB_E_NOMEM : ONB_E_CUDA;       \
         }                                                                           \
     } while (0)
@@ -389,8 +381,6 @@ int32_t run_fight(Ctx* c, const onb_agent* a, const onb_agent* b, const uint8_t*
             const int32_t rc = move(c, who ? b : a, (uint32_t)tick, who ? list_b : list_a, (int64_t)m[who], who ? act_b : act_a);
             if (rc != ONB_OK) {
                 snprintf(err, err_len, "%s", c->err);
-                c->n_act = 0;
-                c->d_tree_game = nullptr;
                 return rc;
             }
         }
@@ -402,8 +392,6 @@ int32_t run_fight(Ctx* c, const onb_agent* a, const onb_agent* b, const uint8_t*
         if (plies_left < 0) break;                  // evaluator.rs:386-392: checked after the move, then decremented (max_plies + 2 plies)
         plies_left -= 1;
     }
-    c->n_act = 0;
-    c->d_tree_game = nullptr;
     FT(cudaMemsetAsync(counters + 2, 0, 24, c->stream));
     k_fight_tally<<<grid, 256, 0, c->stream>>>(c->d_states, n, mask, results, counters + 2);
     FT(cudaGetLastError());
@@ -418,7 +406,7 @@ int32_t run_fight(Ctx* c, const onb_agent* a, const onb_agent* b, const uint8_t*
     out->results = results;
     out->moves_chosen = searched;
     c->fight_valid = 1;
-    c->mcts_phase = 0;
+    c->search.phase = 0;
     return ONB_OK;
 }
 
