@@ -96,6 +96,12 @@ typedef struct onb_state {
 #define ONB_BUF_PI 7          /* float[n][2][25]      written by onb_mcts_finish */
 #define ONB_BUF_BEST 8        /* uint16[n]            written by onb_mcts_finish */
 #define ONB_BUF_STATS 9       /* uint64[ONB_STAT_COUNT] */
+/* the rows of a search with virtual loss (onb_mcts_set_virtual_loss), row t * K + j = descent j of tree t, n_games * K' rows with K'
+ * the largest K enabled so far (a search with K uses the first n_games * K rows). They exist after the first enabling call (before:
+ * ONB_E_STATE); an enabling call with a larger K reallocates them, which invalidates pointers taken earlier (and captured graphs). */
+#define ONB_BUF_VL_PLANES 10  /* float[n K'][21][5][5] written by onb_mcts_select */
+#define ONB_BUF_VL_POLICY 11  /* float[n K'][2][25]    read by onb_mcts_expand_backup */
+#define ONB_BUF_VL_VALUE 12   /* float[n K']           read by onb_mcts_expand_backup */
 
 #define ONB_STAT_STEPS 0     /* transitions applied */
 #define ONB_STAT_RED_WINS 1
@@ -336,6 +342,33 @@ typedef struct onb_gumbel_config {
     uint32_t interior; /* 0: PUCT below the root, 1: interior selection below the root (Gumbel MuZero) */
 } onb_gumbel_config;
 ONB_API int32_t onb_mcts_set_gumbel(onb_ctx* ctx, const onb_gumbel_config* cfg);
+/* Leaf parallelism with virtual loss (the remedy of AlphaGo Zero, Leela and KataGo for searches over few trees; DESIGN.md §5h). Off by
+ * default; leaves <= 1 switches it off, and every entry point then computes what it computes without this call. 2 <= leaves <= 32
+ * with a finite virtual_loss >= 0 switches it on for the searches begun afterwards; any other value: ONB_E_INVALID. With K = leaves,
+ * vl = virtual_loss, a search begun with the switch on runs in ROUNDS (exact to the bit):
+ *   descents: round 0 has b = 1 descent (it evaluates the root), every later round b = min(K, descents left), counted against the
+ *     current onb_mcts_run call's sims or, in the split phase, against the begin's sims; the search never runs more than the begin's
+ *     sims (beyond: ONB_E_STATE). Every descent is a visit, so the root ends with exactly sims visits and at most 1 + 40 sims nodes.
+ *   descent j (0 <= j < b) of a tree starts at the root and goes on while the node is expanded and not terminal. At node x it
+ *     chooses the LAST child c maximising u = q' + (c_puct P) (sqrt(Np') / (N' + 1)), q' = W' / N' (0 if N' = 0), with
+ *     v(c) = the earlier descents 0 .. j-1 of this round whose path contains c (the leaf included; v = j at the root),
+ *     N' = N(c) + v(c), W' = W(c) if v(c) = 0, else W(c) - vl v(c) (W is kept from the view of the side that moved into c, so a
+ *     pending descent counts as a lost visit for the chooser), Np' = N(x) + v(x); f64, IEEE basic operations, no FMA contraction.
+ *     With v = 0 this is the PUCT selection bit for bit. Terminal marking during the descent is unchanged.
+ *   leaves: the leaf of descent j of tree t is row t K + j of ONB_BUF_VL_PLANES / _POLICY / _VALUE. The evaluator runs over
+ *     trees x K rows (rows j >= b are no descents, their output is ignored; the rows are zeroed at allocation, so they are finite).
+ *   expand/backup: per tree, for j = 0 .. b-1 in order: a leaf still unexpanded and not terminal is expanded with row j's policy
+ *     (a leaf an earlier descent of the round expanded is not expanded again); then row j's reward is backed up along the parent
+ *     chain as without virtual loss. All virtual counts are zero after every round.
+ * onb_mcts_select fills the rows, onb_mcts_eval evaluates them (ONB_EVAL_NET included), onb_mcts_expand_backup consumes them; every
+ * onb_mcts_select / _eval / _expand_backup triple is one round. onb_mcts_run runs the same rounds (device evaluators too). Outputs
+ * (onb_mcts_finish, play_best, dump_tree, tree_info) read the tree as before.
+ * Refused with ONB_E_STATE: a begin with the switch on together with train-mode noise, the Gumbel root search or tree reuse;
+ * onb_uct_run after such a begin; onb_self_play while the switch is on. onb_fight searches with virtual loss only for
+ * ONB_AGENT_PUCT_VL agents, whatever the switch says, and leaves the switch as it found it.
+ * Memory: the first enabling call allocates n_games * mcts_node_cap bytes of virtual counts and n_games * K rows of about 2.3 KB;
+ * a later call with a larger K reallocates the rows. A failed allocation returns ONB_E_NOMEM and leaves the switch as it was. */
+ONB_API int32_t onb_mcts_set_virtual_loss(onb_ctx* ctx, uint32_t leaves, double virtual_loss);
 ONB_API int32_t onb_mcts_select(onb_ctx* ctx);
 ONB_API int32_t onb_mcts_expand_backup(onb_ctx* ctx);
 ONB_API int32_t onb_mcts_eval(onb_ctx* ctx, int32_t evaluator); /* fills POLICY/VALUE from LEAF_PLANES on the device */
@@ -421,6 +454,9 @@ ONB_API int32_t onb_copy_to_host(onb_ctx* ctx, void* host, const void* device, i
 /* ONB_AGENT_GUMBEL_MUZERO: as ONB_AGENT_GUMBEL (the same fields and defaults) with interior = 1: Gumbel MuZero, interior selection
  * below the root instead of PUCT. ONB_AGENT_GUMBEL agents search with interior = 0 whatever the context's setting says. */
 #define ONB_AGENT_GUMBEL_MUZERO 6
+/* ONB_AGENT_PUCT_VL: as ONB_AGENT_PUCT with virtual loss (onb_mcts_set_virtual_loss): K = min_node_visits (2 .. 32, else
+ * ONB_E_INVALID) descents per round and vl = 1. Every other agent searches without virtual loss, whatever the switch says. */
+#define ONB_AGENT_PUCT_VL 7
 typedef struct onb_agent {
     int32_t kind;
     int32_t evaluator;

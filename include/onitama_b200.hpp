@@ -147,6 +147,7 @@ public:
     void check(int32_t rc) const { if (rc != ONB_OK) throw Error(rc, onb_last_error(ctx_)); }
     std::vector<uint8_t> last_fight_results;  ///< per-game MoveResult codes of the last fight_device (0 undecided, 1 RedWin, 2 BlueWin)
     onb_gumbel_config gumbel_applied{};       ///< the Gumbel setting last passed to onb_mcts_set_gumbel (enabled = 0: off)
+    std::pair<uint32_t, double> vl_applied{1, 1.0};  ///< (leaves, virtual_loss) last passed to onb_mcts_set_virtual_loss (leaves 1: off)
     /// one-game engine shared by the single-state methods of State / the agents (thread local: a context is single threaded)
     static Engine& single(uint32_t min_sims = 0) {
         thread_local std::unique_ptr<Engine> e;
@@ -423,6 +424,11 @@ struct AlphaZeroMctsConfig {  // alphazero_mcts/mod.rs:26-43
     // step0); every search takes the next step. Does not combine with train or reuse (ONB_E_STATE). interior = 1: Gumbel MuZero's
     // interior selection below the root instead of PUCT.
     onb_gumbel_config gumbel{};
+    // leaf parallelism with virtual loss (onb_mcts_set_virtual_loss, DESIGN.md §5h): leaves_per_round >= 2 runs every search in rounds
+    // of that many descents (round 0: one), each pending descent counting as a lost visit of virtual_loss; a HostEvaluator then
+    // evaluates n * leaves_per_round rows per round. Applied when it changes. Does not combine with train, reuse or gumbel (ONB_E_STATE).
+    uint32_t leaves_per_round = 1;
+    double virtual_loss = 1.0;
 };
 inline double reward(MoveResult r, PlayerColor c) {  // alphazero_mcts/mod.rs:45-53
     if (c == PlayerColor::Red) return r == MoveResult::RedWin ? 1. : r == MoveResult::BlueWin ? -1. : 0.;
@@ -446,18 +452,26 @@ inline void run_search(Engine& e, const AlphaZeroMctsConfig& cfg, int32_t device
         e.check(onb_mcts_set_gumbel(e.ctx(), &g));
         e.gumbel_applied = g;
     }
+    const uint32_t k = cfg.leaves_per_round > 1 ? cfg.leaves_per_round : 1u;
+    const std::pair<uint32_t, double> vl{k, k > 1 ? cfg.virtual_loss : 1.0};
+    if (vl != e.vl_applied) {
+        e.check(onb_mcts_set_virtual_loss(e.ctx(), vl.first, vl.second));
+        e.vl_applied = vl;
+    }
     e.check(onb_mcts_begin(e.ctx(), cfg.exploration_c, cfg.max_playouts));
     if (!net) {
         e.check(onb_mcts_run(e.ctx(), device_eval, cfg.max_playouts));
     } else {
-        const int64_t n = e.n();
-        std::vector<float> planes((size_t)n * 525), pol((size_t)n * 50), val((size_t)n);
-        for (uint32_t s = 0; s < cfg.max_playouts; ++s) {
+        // rounds of one select / evaluation / expand-backup: sims of them, or 1 + ceil((sims - 1) / K) over n K rows with virtual loss
+        const int64_t rows = e.n() * k;
+        const uint32_t s = cfg.max_playouts, rounds = k > 1 && s ? 1u + (s - 1u + k - 1u) / k : s;
+        std::vector<float> planes((size_t)rows * 525), pol((size_t)rows * 50), val((size_t)rows);
+        for (uint32_t r = 0; r < rounds; ++r) {
             e.check(onb_mcts_select(e.ctx()));
-            e.check(onb_read_buffer(e.ctx(), ONB_BUF_LEAF_PLANES, planes.data(), n * 2100));
-            net(planes.data(), n, pol.data(), val.data());
-            e.check(onb_write_buffer(e.ctx(), ONB_BUF_POLICY, pol.data(), n * 200));
-            e.check(onb_write_buffer(e.ctx(), ONB_BUF_VALUE, val.data(), n * 4));
+            e.check(onb_read_buffer(e.ctx(), k > 1 ? ONB_BUF_VL_PLANES : ONB_BUF_LEAF_PLANES, planes.data(), rows * 2100));
+            net(planes.data(), rows, pol.data(), val.data());
+            e.check(onb_write_buffer(e.ctx(), k > 1 ? ONB_BUF_VL_POLICY : ONB_BUF_POLICY, pol.data(), rows * 200));
+            e.check(onb_write_buffer(e.ctx(), k > 1 ? ONB_BUF_VL_VALUE : ONB_BUF_VALUE, val.data(), rows * 4));
             e.check(onb_mcts_expand_backup(e.ctx()));
         }
     }
@@ -489,19 +503,21 @@ struct AlphaZeroMcts : Agent {  // alphazero_mcts/mod.rs:81-161
     std::pair<DoneMove, double> generate_move(const GameState& gs) override {
         TrainingAlphaZeroMcts t{config, device_evaluator, model};
         auto r = t.generate_move_tensor(gs.state, gs.curr_player_color);
-        // the reference reports the network's value of the root position (mod.rs:136-142): one extra evaluation of the root
+        // the reference reports the network's value of the root position (mod.rs:136-142): one extra evaluation of the root (with
+        // virtual loss on, round 0's single descent: row 0 of the VL rows)
         Engine& e = Engine::single(config.max_playouts);
+        const bool vl = config.leaves_per_round > 1;
         double value = 0.;
         e.check(onb_mcts_begin(e.ctx(), config.exploration_c, config.max_playouts));
         e.check(onb_mcts_select(e.ctx()));
         float v = 0.f;
         if (model) {
             std::vector<float> planes(525), pol(50);
-            e.check(onb_read_buffer(e.ctx(), ONB_BUF_LEAF_PLANES, planes.data(), 2100));
+            e.check(onb_read_buffer(e.ctx(), vl ? ONB_BUF_VL_PLANES : ONB_BUF_LEAF_PLANES, planes.data(), 2100));
             model(planes.data(), 1, pol.data(), &v);
         } else {
             e.check(onb_mcts_eval(e.ctx(), device_evaluator));
-            e.check(onb_read_buffer(e.ctx(), ONB_BUF_VALUE, &v, 4));
+            e.check(onb_read_buffer(e.ctx(), vl ? ONB_BUF_VL_VALUE : ONB_BUF_VALUE, &v, 4));
         }
         value = (double)v;
         return {r.first, value};

@@ -14,7 +14,7 @@ POLICY_UNIFORM, POLICY_AGENT = 0, 1
 OUT_MASKS, OUT_PLANES, OUT_ACTIONS = 1, 2, 4
 EVAL_UNIFORM, EVAL_HASH, EVAL_NET = 0, 1, 2
 (BUF_STATES, BUF_MASKS, BUF_PLANES, BUF_ACTIONS, BUF_LEAF_PLANES, BUF_POLICY, BUF_VALUE, BUF_PI, BUF_BEST,
- BUF_STATS) = range(10)
+ BUF_STATS, BUF_VL_PLANES, BUF_VL_POLICY, BUF_VL_VALUE) = range(13)
 STAT_STEPS, STAT_RED_WINS, STAT_BLUE_WINS, STAT_PASSES, STAT_RESETS, STAT_BAD_ACTIONS, STAT_COUNT = 0, 1, 2, 3, 4, 5, 8
 HOST_MASKS, HOST_DONE, HOST_STATS = 1, 2, 4
 NET_F16, NET_TF32, NET_F32 = 0, 1, 2
@@ -84,6 +84,7 @@ SYMBOLS = {
     "onb_mcts_set_reuse": (C.c_int32, [_P, C.c_int32]),
     "onb_mcts_reuse_stats": (C.c_int32, [_P, _P, C.c_int32]),
     "onb_mcts_set_gumbel": (C.c_int32, [_P, _P]),
+    "onb_mcts_set_virtual_loss": (C.c_int32, [_P, C.c_uint32, C.c_double]),
     "onb_mcts_select": (C.c_int32, [_P]),
     "onb_mcts_expand_backup": (C.c_int32, [_P]),
     "onb_mcts_eval": (C.c_int32, [_P, C.c_int32]),
@@ -129,7 +130,7 @@ class SelfPlayConfig(C.Structure):
                 ("train", C.c_int32), ("noise_seed", C.c_uint64), ("sample_cap", C.c_int64)]
 
 
-AGENT_RANDOM, AGENT_PUCT, AGENT_UCT, AGENT_ALPHABETA, AGENT_GUMBEL, AGENT_TABLEBASE, AGENT_GUMBEL_MUZERO = 0, 1, 2, 3, 4, 5, 6
+AGENT_RANDOM, AGENT_PUCT, AGENT_UCT, AGENT_ALPHABETA, AGENT_GUMBEL, AGENT_TABLEBASE, AGENT_GUMBEL_MUZERO, AGENT_PUCT_VL = 0, 1, 2, 3, 4, 5, 6, 7
 ALPHABETA_MAX_DEPTH = 8
 ALPHABETA_WIN = 1000000
 TB_MAX_PAWNS = 4

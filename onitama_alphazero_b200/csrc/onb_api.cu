@@ -148,7 +148,8 @@ int32_t onb_destroy(onb_ctx* ctx) {
                     c->d_tree_size, c->d_tree_flags, c->d_roots, c->d_leaf_node, c->d_leaf_state, c->d_leaf_planes, c->d_policy, c->d_value,
                     c->d_pi, c->d_best, c->d_root_visits, c->d_root_q, c->d_child_visits, c->net[0].w, c->net[0].bias, c->net[0].head, c->net[1].w,
                     c->net[1].bias, c->net[1].head, c->d_ln_table, c->d_ab_score, c->d_ab_nodes, c->d_gb,
-                    c->d_gb_tab, c->d_gb_base, c->d_gb_p, c->d_gb_r0, c->d_gb_rx, c->d_tb_values};
+                    c->d_gb_tab, c->d_gb_base, c->d_gb_p, c->d_gb_r0, c->d_gb_rx, c->d_tb_values, c->d_vl_cnt,
+                    c->d_vl_leaf_node, c->d_vl_leaf_state, c->d_vl_planes, c->d_vl_policy, c->d_vl_value};
     reuse_free(c);
     tb_free(c);
     for (void* p : c->sp_buf)
@@ -193,8 +194,13 @@ int32_t onb_buffer(onb_ctx* ctx, int32_t which, void** dev_ptr, int64_t* bytes) 
         case ONB_BUF_PI: p = c->d_pi; b = n * 200; break;
         case ONB_BUF_BEST: p = c->d_best; b = n * 2; break;
         case ONB_BUF_STATS: p = c->d_stats; b = ONB_STAT_COUNT * 8; break;
+        case ONB_BUF_VL_PLANES: p = c->d_vl_planes; b = n * c->vl_cap * 2100; break;
+        case ONB_BUF_VL_POLICY: p = c->d_vl_policy; b = n * c->vl_cap * 200; break;
+        case ONB_BUF_VL_VALUE: p = c->d_vl_value; b = n * c->vl_cap * 4; break;
         default: return fail(c, ONB_E_INVALID, "onb_buffer: unknown buffer %d", which);
     }
+    if (!p && which >= ONB_BUF_VL_PLANES)
+        return fail(c, ONB_E_STATE, "onb_buffer: buffer %d exists after the first onb_mcts_set_virtual_loss with leaves >= 2", which);
     if (!p) return fail(c, ONB_E_STATE, "onb_buffer: buffer %d was not allocated by onb_create (see onb_config)", which);
     if (dev_ptr) *dev_ptr = p;
     if (bytes) *bytes = b;
@@ -461,6 +467,14 @@ static int32_t begin_search(Ctx* c, const SearchPlan& p, const char* who) {
     // the combinations a Gumbel search does not support (include/onb.h, onb_mcts_set_gumbel)
     if (p.gumbel && p.reuse) return fail(c, ONB_E_STATE, "%s: the Gumbel root search does not combine with tree reuse (onb_mcts_set_reuse)", who);
     if (p.gumbel && p.noise) return fail(c, ONB_E_STATE, "%s: the Gumbel root search does not combine with train-mode noise (onb_mcts_set_noise)", who);
+    // the combinations a search with virtual loss does not support (include/onb.h, onb_mcts_set_virtual_loss)
+    if (p.leaves >= 2 && (p.noise || p.gumbel || p.reuse))
+        return fail(c, ONB_E_STATE, "%s: virtual loss (onb_mcts_set_virtual_loss) does not combine with %s", who,
+                    p.noise ? "train-mode noise" : p.gumbel ? "the Gumbel root search" : "tree reuse");
+    if (c->vl_dirty) {  // a select with virtual loss whose round was never backed up left counts behind
+        ONB_CUDA(c, cudaMemsetAsync(c->d_vl_cnt, 0, (size_t)c->n * c->node_cap, c->stream));
+        c->vl_dirty = 0;
+    }
     c->search.plan = p;
     if (p.reuse) {
         ONB_CUDA(c, launch_reuse_begin(c, p.d_games, p.d_games ? p.m : c->n, p.sims));
@@ -528,8 +542,71 @@ static int32_t gumbel_alloc(Ctx* c, bool interior) {
     }
     return ONB_OK;
 }
+// the buffers of a search with virtual loss: the counts by the first call, the rows whenever K grows beyond vl_cap (the new rows are
+// allocated and zeroed before the old ones are freed, so a failure leaves everything as it was)
+static int32_t vl_alloc(Ctx* c, uint32_t leaves) {
+    const size_t n = (size_t)c->n;
+    if (!c->d_vl_cnt) {
+        cudaError_t e = dalloc(&c->d_vl_cnt, n * c->node_cap);
+        if (e == cudaSuccess) e = cudaMemsetAsync(c->d_vl_cnt, 0, n * c->node_cap, c->stream);
+        if (e != cudaSuccess) {
+            if (c->d_vl_cnt) cudaFree(c->d_vl_cnt);
+            c->d_vl_cnt = nullptr;
+            return e == cudaErrorMemoryAllocation ? fail(c, ONB_E_NOMEM, "onb_mcts_set_virtual_loss: out of device memory for the virtual counts")
+                                                  : cuda_fail(c, e, "onb_mcts_set_virtual_loss");
+        }
+    }
+    if (leaves <= c->vl_cap) return ONB_OK;
+    const size_t rows = n * leaves;
+    uint32_t* node = nullptr;
+    uint4* state = nullptr;
+    float *planes = nullptr, *policy = nullptr, *value = nullptr;
+    cudaError_t e = dalloc(&node, rows);
+    if (e == cudaSuccess) e = dalloc(&state, rows);
+    if (e == cudaSuccess) e = dalloc(&planes, rows * 525);
+    if (e == cudaSuccess) e = dalloc(&policy, rows * 50);
+    if (e == cudaSuccess) e = dalloc(&value, rows);
+    // zeroed: every row the network reads is finite, descents or not
+    if (e == cudaSuccess) e = cudaMemsetAsync(node, 0, rows * 4, c->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(state, 0, rows * 16, c->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(planes, 0, rows * 2100, c->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(policy, 0, rows * 200, c->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(value, 0, rows * 4, c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);  // the old rows may still be in use by queued work
+    if (e != cudaSuccess) {
+        for (void* p : {(void*)node, (void*)state, (void*)planes, (void*)policy, (void*)value})
+            if (p) cudaFree(p);
+        return e == cudaErrorMemoryAllocation ? fail(c, ONB_E_NOMEM, "onb_mcts_set_virtual_loss: out of device memory for %u rows per game", leaves)
+                                              : cuda_fail(c, e, "onb_mcts_set_virtual_loss");
+    }
+    for (void* p : {(void*)c->d_vl_leaf_node, (void*)c->d_vl_leaf_state, (void*)c->d_vl_planes, (void*)c->d_vl_policy, (void*)c->d_vl_value})
+        if (p) cudaFree(p);
+    c->d_vl_leaf_node = node;
+    c->d_vl_leaf_state = state;
+    c->d_vl_planes = planes;
+    c->d_vl_policy = policy;
+    c->d_vl_value = value;
+    c->vl_cap = leaves;
+    return ONB_OK;
+}
 }  // namespace onb
 extern "C" {
+int32_t onb_mcts_set_virtual_loss(onb_ctx* ctx, uint32_t leaves, double virtual_loss) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (leaves <= 1) {
+        c->vl_leaves = 0;
+        return ONB_OK;
+    }
+    if (leaves > 32 || !std::isfinite(virtual_loss) || !(virtual_loss >= 0.0))
+        return fail(c, ONB_E_INVALID, "onb_mcts_set_virtual_loss: need leaves <= 32 and a finite virtual_loss >= 0");
+    if (!c->d_nodes) return fail(c, ONB_E_STATE, "onb_mcts_set_virtual_loss: context created with mcts_max_sims = 0");
+    const int32_t rc = vl_alloc(c, leaves);
+    if (rc != ONB_OK) return rc;
+    c->vl_leaves = leaves;
+    c->vl_loss = virtual_loss;
+    return ONB_OK;
+}
 int32_t onb_mcts_begin(onb_ctx* ctx, double c_puct, uint32_t sims) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
@@ -544,6 +621,8 @@ int32_t onb_mcts_begin(onb_ctx* ctx, double c_puct, uint32_t sims) {
     p.gumbel = c->gb_on != 0;
     p.gb_cfg = c->gb_cfg;
     p.gb_step = c->gb_serial;
+    p.leaves = c->vl_leaves;
+    p.vloss = c->vl_loss;
     const int32_t rc = begin_search(c, p, "onb_mcts_begin");
     if (rc == ONB_OK && p.gumbel) c->gb_serial += 1;
     return rc;
@@ -612,6 +691,12 @@ int32_t onb_mcts_select(onb_ctx* ctx) {
     if (a.plan.reuse) return refuse_after_reuse(c, "onb_mcts_select");
     if (a.plan.gumbel && a.sims_done >= a.plan.sims)
         return fail(c, ONB_E_STATE, "onb_mcts_select: a Gumbel search runs at most the begin's %u simulations", a.plan.sims);
+    if (a.plan.leaves >= 2) {  // the split phase counts every round against the begin's sims
+        if (a.sims_done >= a.plan.sims)
+            return fail(c, ONB_E_STATE, "onb_mcts_select: a search with virtual loss runs at most the begin's %u simulations", a.plan.sims);
+        a.vl_target = a.plan.sims;
+        c->vl_dirty = 1;
+    }
     ONB_CUDA(c, launch_mcts_select(c));
     a.phase = 2;
     return ONB_OK;
@@ -623,7 +708,10 @@ int32_t onb_mcts_eval(onb_ctx* ctx, int32_t evaluator) {
     if (c->search.phase != 2) return fail(c, ONB_E_STATE, "onb_mcts_eval: no leaves selected");
     if (evaluator == ONB_EVAL_NET) {
         if (!c->net[c->net_cur].loaded) return fail(c, ONB_E_STATE, "onb_mcts_eval: no network loaded (onb_net_load)");
-        ONB_CUDA(c, launch_net_forward(c, c->d_leaf_planes, c->d_policy, c->d_value, trees(c)));
+        if (c->search.plan.leaves >= 2)
+            ONB_CUDA(c, launch_net_forward(c, c->d_vl_planes, c->d_vl_policy, c->d_vl_value, trees(c) * c->search.plan.leaves));
+        else
+            ONB_CUDA(c, launch_net_forward(c, c->d_leaf_planes, c->d_policy, c->d_value, trees(c)));
         return ONB_OK;
     }
     if (evaluator != ONB_EVAL_UNIFORM && evaluator != ONB_EVAL_HASH) return fail(c, ONB_E_INVALID, "onb_mcts_eval: unknown evaluator %d", evaluator);
@@ -636,8 +724,14 @@ int32_t onb_mcts_expand_backup(onb_ctx* ctx) {
     if (c->search.plan.reuse) return refuse_after_reuse(c, "onb_mcts_expand_backup");
     if (c->search.phase != 2) return fail(c, ONB_E_STATE, "onb_mcts_expand_backup: call onb_mcts_select first");
     ONB_CUDA(c, launch_mcts_expand_backup(c));
-    c->search.phase = 1;
-    c->search.sims_done += 1;
+    ActiveSearch& a = c->search;
+    a.phase = 1;
+    if (a.plan.leaves >= 2) {
+        a.sims_done += vl_descents(a.sims_done, a.plan.leaves, a.vl_target);
+        c->vl_dirty = 0;
+    } else {
+        a.sims_done += 1;
+    }
     return ONB_OK;
 }
 // onb_mcts_run after a reuse begin: slot t runs max(0, sims - N_root) simulations; the slots are ordered by that budget, so round r
@@ -682,6 +776,23 @@ int32_t onb_mcts_run(onb_ctx* ctx, int32_t evaluator, uint32_t sims) {
     if (a.plan.reuse) return reuse_run(c, evaluator, sims);
     if (a.plan.gumbel && a.sims_done + sims > a.plan.sims)
         return fail(c, ONB_E_STATE, "onb_mcts_run: a Gumbel search runs at most the begin's %u simulations", a.plan.sims);
+    if (a.plan.leaves >= 2) {  // rounds of K descents per tree (round 0: one), counted against this call's end
+        if (a.sims_done + sims > a.plan.sims)
+            return fail(c, ONB_E_STATE, "onb_mcts_run: a search with virtual loss runs at most the begin's %u simulations", a.plan.sims);
+        if (evaluator == ONB_EVAL_NET && !c->net[c->net_cur].loaded) return fail(c, ONB_E_STATE, "onb_mcts_run: no network loaded (onb_net_load)");
+        a.vl_target = a.sims_done + sims;
+        const int64_t rows = trees(c) * a.plan.leaves;
+        while (a.sims_done < a.vl_target) {
+            ONB_CUDA(c, launch_mcts_select(c));
+            if (evaluator == ONB_EVAL_NET)
+                ONB_CUDA(c, launch_net_forward(c, c->d_vl_planes, c->d_vl_policy, c->d_vl_value, rows));
+            else
+                ONB_CUDA(c, launch_mcts_eval(c, evaluator));
+            ONB_CUDA(c, launch_mcts_expand_backup(c));
+            a.sims_done += vl_descents(a.sims_done, a.plan.leaves, a.vl_target);
+        }
+        return ONB_OK;
+    }
     if (evaluator == ONB_EVAL_NET) {
         // the network sits between select and expand: three launches per simulation round, all on the context's stream
         // (one launch for expand_backup(s) + select(s + 1) was measured slower, DESIGN.md section 8)
@@ -730,6 +841,7 @@ int32_t onb_self_play(onb_ctx* ctx, const onb_selfplay_config* cfg, onb_selfplay
     if (cfg->n_games <= 0) return fail(c, ONB_E_INVALID, "onb_self_play: n_games must be positive");
     if (cfg->train && c->gb_on) return fail(c, ONB_E_INVALID, "onb_self_play: train-mode noise does not combine with the Gumbel root search");
     if (c->reuse_on && c->gb_on) return fail(c, ONB_E_STATE, "onb_self_play: tree reuse does not combine with the Gumbel root search");
+    if (c->vl_leaves >= 2) return fail(c, ONB_E_STATE, "onb_self_play: self-play searches without virtual loss; switch it off (onb_mcts_set_virtual_loss)");
     memset(out, 0, sizeof(*out));
     c->ru_live = 0;  // self-play starts from fresh deals: nothing is kept from earlier searches
     char err[400];
@@ -782,9 +894,13 @@ static int32_t fight_move(Ctx* c, const onb_agent* ag, uint32_t ply, const int32
         p.gb_cfg.interior = ag->kind == ONB_AGENT_GUMBEL_MUZERO ? 1u : 0u;
         p.gb_step = ply;
     }
+    if (ag->kind == ONB_AGENT_PUCT_VL) {  // PUCT with K = min_node_visits descents per round and vl = 1
+        p.leaves = ag->min_node_visits;
+        p.vloss = 1.0;
+    }
     int32_t rc = begin_search(c, p, "search");
     if (rc != ONB_OK) return rc;
-    if (ag->kind == ONB_AGENT_PUCT || p.gumbel) {
+    if (ag->kind == ONB_AGENT_PUCT || ag->kind == ONB_AGENT_PUCT_VL || p.gumbel) {
         if (ag->evaluator == ONB_EVAL_NET && (rc = onb_net_select(x, ag->net_slot)) != ONB_OK) return rc;
         rc = onb_mcts_run(x, ag->evaluator, ag->sims);
     } else {
@@ -803,7 +919,7 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
     if (!a || !b || !a_is_red_host || !out) return fail(c, ONB_E_INVALID, "onb_fight: null argument");
     for (const onb_agent* ag : {a, b}) {
         if (ag->kind != ONB_AGENT_RANDOM && ag->kind != ONB_AGENT_PUCT && ag->kind != ONB_AGENT_UCT && ag->kind != ONB_AGENT_ALPHABETA &&
-            ag->kind != ONB_AGENT_GUMBEL && ag->kind != ONB_AGENT_TABLEBASE && ag->kind != ONB_AGENT_GUMBEL_MUZERO)
+            ag->kind != ONB_AGENT_GUMBEL && ag->kind != ONB_AGENT_TABLEBASE && ag->kind != ONB_AGENT_GUMBEL_MUZERO && ag->kind != ONB_AGENT_PUCT_VL)
             return fail(c, ONB_E_INVALID, "onb_fight: unknown agent kind %d", ag->kind);
         if (ag->kind == ONB_AGENT_TABLEBASE) {
             if (!c->tb_live) return fail(c, ONB_E_STATE, "onb_fight: a tablebase agent needs a solved table (onb_tb_solve)");
@@ -811,6 +927,8 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
         }
         if ((ag->kind == ONB_AGENT_GUMBEL || ag->kind == ONB_AGENT_GUMBEL_MUZERO) && (ag->min_node_visits > 40 || !std::isfinite(ag->c) || !(ag->c >= 0.0)))
             return fail(c, ONB_E_INVALID, "onb_fight: a Gumbel agent needs min_node_visits (m) <= 40 and a finite c (c_scale) >= 0");
+        if (ag->kind == ONB_AGENT_PUCT_VL && (ag->min_node_visits < 2 || ag->min_node_visits > 32))
+            return fail(c, ONB_E_INVALID, "onb_fight: a virtual-loss agent needs 2 <= min_node_visits (leaves per round) <= 32");
         if (ag->kind == ONB_AGENT_ALPHABETA) {
             if (ag->sims < 1 || ag->sims > ONB_ALPHABETA_MAX_DEPTH)
                 return fail(c, ONB_E_INVALID, "onb_fight: an alpha-beta agent needs 1 <= depth (sims) <= %d", ONB_ALPHABETA_MAX_DEPTH);
@@ -837,6 +955,10 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
     const bool muzero = a->kind == ONB_AGENT_GUMBEL_MUZERO || b->kind == ONB_AGENT_GUMBEL_MUZERO;
     int32_t rc;
     if ((a->kind == ONB_AGENT_GUMBEL || b->kind == ONB_AGENT_GUMBEL || muzero) && (rc = gumbel_alloc(c, muzero)) != ONB_OK) return rc;
+    uint32_t vl_need = 0;  // the virtual-loss agents' buffers; the context's switch is left as it is
+    for (const onb_agent* ag : {a, b})
+        if (ag->kind == ONB_AGENT_PUCT_VL && ag->min_node_visits > vl_need) vl_need = ag->min_node_visits;
+    if (vl_need && (rc = vl_alloc(c, vl_need)) != ONB_OK) return rc;
     char err[400];
     err[0] = 0;
     rc = run_fight(c, a, b, a_is_red_host, max_plies, out, fight_move, err, sizeof(err));
@@ -876,6 +998,7 @@ int32_t onb_uct_run(onb_ctx* ctx, float exploration_c, uint32_t min_node_visits,
     if (a.phase != 1) return fail(c, ONB_E_STATE, "onb_uct_run: call onb_mcts_begin first");
     if (a.plan.reuse) return refuse_after_reuse(c, "onb_uct_run");
     if (a.plan.gumbel) return fail(c, ONB_E_STATE, "onb_uct_run: the search was begun with the Gumbel root search on (onb_mcts_set_gumbel)");
+    if (a.plan.leaves >= 2) return fail(c, ONB_E_STATE, "onb_uct_run: the search was begun with virtual loss on (onb_mcts_set_virtual_loss)");
     if (a.sims_done + playouts > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_uct_run: more playouts than mcts_max_sims");
     const uint32_t need = a.sims_done + playouts + 2;
     if (c->ln_cap < need) {  // ln(parent visits) as the reference computes it: f32 logf on the host

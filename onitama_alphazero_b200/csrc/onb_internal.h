@@ -57,7 +57,17 @@ struct SearchPlan {
     bool gumbel;             // the Gumbel root search (onb_mcts_set_gumbel); gb_cfg.interior: Gumbel MuZero below the root
     onb_gumbel_config gb_cfg;
     uint32_t gb_step;
+    uint32_t leaves;         // K >= 2: leaf parallelism with virtual loss (onb_mcts_set_virtual_loss), 0: one descent per round
+    double vloss;
 };
+// Descents of the next round of a search with virtual loss (DESIGN.md §5h), from the descents done so far (= the root's visits) and
+// the target the round counts against: 1 for round 0, then min(K, target - done). The kernels derive it from the root's visit count,
+// so a captured round (CUDA graph) runs the right number of descents on every replay.
+__host__ __device__ inline uint32_t vl_descents(uint32_t done, uint32_t leaves, uint32_t target) {
+    if (done >= target) return 0u;
+    if (done == 0u) return 1u;
+    return target - done < leaves ? target - done : leaves;
+}
 // the search begun last
 struct ActiveSearch {
     SearchPlan plan;
@@ -67,6 +77,7 @@ struct ActiveSearch {
     // tree of the same index. A subset plan sets them, launch_reuse_begin fills them for a reuse begin.
     int64_t n_act;
     const int32_t* d_tree_game;
+    uint32_t vl_target;  // with virtual loss: the descent count the current round is counted against (onb_mcts_run's end, or plan.sims)
 };
 
 struct Ctx {
@@ -158,6 +169,17 @@ struct Ctx {
     double* d_gb_r0;
     float* d_gb_rx;           // [n][node_cap], allocated by the first call that turns interior selection on
     uint32_t gb_tab_m, gb_tab_n;  // the table d_gb_tab holds (gb_tab_m = 0: none)
+    // leaf parallelism with virtual loss (onb_mcts_set_virtual_loss, DESIGN.md §5h); buffers allocated by the first enabling call
+    uint32_t vl_leaves;       // the switch: K (2..32), 0 off
+    double vl_loss;
+    uint32_t vl_cap;          // K the row buffers are sized for: n * vl_cap rows, row t * K + j = descent j of tree t
+    int vl_dirty;             // a select left virtual counts that no expand/backup has cleared (the next begin clears them)
+    uint8_t* d_vl_cnt;        // [n][node_cap] virtual visits of the current round (zero between rounds)
+    uint32_t* d_vl_leaf_node; // rows: leaf node, packed leaf state, planes [21][5][5], policy [50], value
+    uint4* d_vl_leaf_state;
+    float* d_vl_planes;
+    float* d_vl_policy;
+    float* d_vl_value;
     // endgame tablebase (onb_tablebase.cu, onb_tb_solve)
     int16_t* d_tb;            // every solved class, class 5 p + q at d_tb + tb_off[5 p + q]
     int64_t tb_off[25], tb_len[25];  // tb_len = 0: class not in the table
@@ -195,7 +217,8 @@ cudaError_t launch_mcts_finish(Ctx* c, float* pi, uint16_t* best, uint32_t* root
 cudaError_t launch_mcts_play_best(Ctx* c, uint32_t out_flags);
 cudaError_t launch_mcts_scatter_best(Ctx* c, uint16_t* dst_actions);  // dst[game of tree t] = best[t]
 // the search launchers take their kernel from c->search.plan: noise, Gumbel at the root (select, run, finish) and Gumbel MuZero
-// below it (select, run, expand_backup)
+// below it (select, run, expand_backup), virtual loss (select, eval, expand_backup over the K rows of every tree, round target
+// search.vl_target)
 
 // network (onb_net.cu)
 int32_t net_load(Ctx* c, int32_t n_tensors, const char* const* names, const float* const* data, const int64_t* numel, std::string& err);

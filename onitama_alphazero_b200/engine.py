@@ -82,8 +82,12 @@ class Context:
     def tensor(self, which):
         """Zero-copy torch view of a device buffer (the network reads LEAF_PLANES and writes POLICY / VALUE in place)."""
         import torch
-        p, _ = self.buffer(which)
+        p, nbytes = self.buffer(which)
         n = self.n
+        if which in (L.BUF_VL_PLANES, L.BUF_VL_POLICY, L.BUF_VL_VALUE):  # every allocated row (a search with K uses the first n K)
+            row = {L.BUF_VL_PLANES: (21, 5, 5), L.BUF_VL_POLICY: (2, 25), L.BUF_VL_VALUE: ()}[which]
+            rows = nbytes // (4 * int(np.prod(row, dtype=np.int64)))
+            return torch.as_tensor(_DevBuf(p, (rows,) + row, "<f4"), device="cuda:%d" % self.device)
         spec = {L.BUF_MASKS: ((n, 2), "<u4", torch.int32), L.BUF_PLANES: ((n, 21, 5, 5), "<f4", None),
                 L.BUF_ACTIONS: ((n,), "<i2", None), L.BUF_LEAF_PLANES: ((n, 21, 5, 5), "<f4", None),
                 L.BUF_POLICY: ((n, 2, 25), "<f4", None), L.BUF_VALUE: ((n,), "<f4", None), L.BUF_PI: ((n, 2, 25), "<f4", None),
@@ -218,6 +222,38 @@ class Context:
         self.gumbel = (int(m), float(c_visit), float(c_scale), float(gumbel_scale), int(seed)) + ((True,) if interior else ()) if enabled else None
         self.gumbel_step = int(step0)  # self_play_native and fight_native leave the library's serial as they found it
 
+    def set_virtual_loss(self, leaves, virtual_loss=1.0):
+        """onb_mcts_set_virtual_loss: leaf parallelism with virtual loss for the searches begun afterwards -- rounds of `leaves` (K, 2 ..
+        32) descents per tree, each pending descent counting as a lost visit of `virtual_loss` for the next; leaves <= 1 switches it
+        off. See include/onb.h and DESIGN.md §5h."""
+        self._ck(self._lib.onb_mcts_set_virtual_loss(self._h, int(leaves), float(virtual_loss)))
+        self.vl = (int(leaves), float(virtual_loss)) if leaves > 1 else None
+
+    def _use_vl(self, vl):
+        """the vl= argument of the search drivers: None leaves the switch, K (virtual loss 1) or (K, virtual_loss) sets it, K <= 1 or
+        False switches it off"""
+        if vl is None:
+            return
+        k, loss = (vl, 1.0) if not isinstance(vl, (tuple, list)) else vl
+        want = (int(k), float(loss)) if int(k) > 1 else None
+        if want != getattr(self, "vl", None):
+            self.set_virtual_loss(int(k), float(loss))
+
+    def _vl_rows(self):
+        """zero-copy views (planes, policy, value) of the n K rows of the switch as it is; None without virtual loss"""
+        k = getattr(self, "vl", None)
+        if k is None:
+            return None
+        rows = self.n * k[0]
+        return self.tensor(L.BUF_VL_PLANES)[:rows], self.tensor(L.BUF_VL_POLICY)[:rows], self.tensor(L.BUF_VL_VALUE)[:rows]
+
+    def vl_rounds(self, sims):
+        """rounds of a search of `sims` simulations begun with the switch as it is: 1 + ceil((sims - 1) / K) with virtual loss"""
+        k = getattr(self, "vl", None)
+        if k is None or sims == 0:
+            return sims
+        return 1 + (sims - 1 + k[0] - 1) // k[0]
+
     def _use_gumbel(self, gumbel):
         """the gumbel= argument of the search drivers: None leaves the switch, False switches it off, True (the defaults) or a dict of
         set_gumbel keywords switches it on unless that setting is already on (so consecutive searches keep advancing the step)"""
@@ -280,7 +316,10 @@ class Context:
         return L.Agent(L.AGENT_RANDOM, 0, 0, 0, 0.0, 0, 0)
 
     @staticmethod
-    def agent_puct(sims, c_puct=2.0, evaluator=L.EVAL_UNIFORM, net_slot=0):
+    def agent_puct(sims, c_puct=2.0, evaluator=L.EVAL_UNIFORM, net_slot=0, leaves=1):
+        """AlphaZeroMcts as an arena agent; leaves > 1: ONB_AGENT_PUCT_VL, rounds of `leaves` descents with virtual loss 1"""
+        if leaves > 1:
+            return L.Agent(L.AGENT_PUCT_VL, evaluator, net_slot, sims, c_puct, int(leaves), 0)
         return L.Agent(L.AGENT_PUCT, evaluator, net_slot, sims, c_puct, 0, 0)
 
     @staticmethod
@@ -450,22 +489,25 @@ class Context:
         self._ck(self._lib.onb_mcts_dump_tree(self._h, tree, cap, C.byref(td), C.byref(nn)))
         return {k: v[:nn.value].copy() for k, v in arrs.items()}
 
-    def search(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, fused=True, net=None):
+    def search(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, fused=True, net=None, vl=None):
         """MctsArena::search for every game at once. net: callable(leaf_planes tensor [n,21,5,5]) -> (policy [n,2,25], value [n])
-        running on this context's stream; it reads/writes the device buffers zero-copy."""
+        running on this context's stream; it reads/writes the device buffers zero-copy. vl: None leaves the virtual-loss switch, K or
+        (K, virtual_loss) sets it, 1 switches it off (set_virtual_loss); with it on, `net` gets the n K rows of ONB_BUF_VL_PLANES and
+        the split phase runs vl_rounds(sims) rounds."""
+        self._use_vl(vl)
         self.mcts_begin(c_puct, sims)
         if net is None and fused:
             self.mcts_run(evaluator, sims)
         elif net is None:
-            for _ in range(sims):
+            for _ in range(self.vl_rounds(sims)):
                 self.mcts_select()
                 self.mcts_eval(evaluator)
                 self.mcts_expand_backup()
         else:
             import torch
             with torch.cuda.stream(self.torch_stream()):
-                planes, pol, val = self.tensor(L.BUF_LEAF_PLANES), self.tensor(L.BUF_POLICY), self.tensor(L.BUF_VALUE)
-                for _ in range(sims):
+                planes, pol, val = self._vl_rows() or (self.tensor(L.BUF_LEAF_PLANES), self.tensor(L.BUF_POLICY), self.tensor(L.BUF_VALUE))
+                for _ in range(self.vl_rounds(sims)):
                     self.mcts_select()
                     p, v = net(planes)
                     pol.copy_(p.reshape(pol.shape))
@@ -544,17 +586,20 @@ class Actor:
             pass
 
 
-def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_graph=False, reuse=None, gumbel=None):
+def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_graph=False, reuse=None, gumbel=None, vl=None):
     """Context.search without copying the results to the host (PI / BEST stay in their device buffers).
     use_graph: capture one simulation round (select -> network -> expand/backup) in a CUDA graph on the context's stream and
     replay it; the round is launch-bound otherwise (~40 small network kernels per round).
     reuse: True / False sets the tree-reuse switch first (set_reuse), None leaves it. Reuse needs a device evaluator (a torch `net`
     drives the split phase, which a reuse search refuses).
     gumbel: None leaves the Gumbel switch as it is, False switches it off, True or a dict of set_gumbel keywords switches it on (only
-    when that setting is not on already, so that consecutive searches take consecutive steps)."""
+    when that setting is not on already, so that consecutive searches take consecutive steps).
+    vl: as for search. With virtual loss a torch `net` gets the n K rows, and use_graph runs round 0 eagerly and replays one captured
+    round for the others: the kernels take a round's descents from the root's visit count, so the short last round replays too."""
     if reuse is not None and bool(reuse) != getattr(self, "reuse", False):
         self.set_reuse(reuse)
     self._use_gumbel(gumbel)
+    self._use_vl(vl)
     if net is not None and getattr(self, "reuse", False):
         raise ValueError("search_device: tree reuse needs a device evaluator (EVAL_UNIFORM / EVAL_HASH / EVAL_NET), not a torch net")
     self.mcts_begin(c_puct, sims)
@@ -564,7 +609,9 @@ def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_g
         import torch
         ts = self.torch_stream()
         with torch.cuda.stream(ts):
-            planes, pol, val = self.tensor(L.BUF_LEAF_PLANES), self.tensor(L.BUF_POLICY), self.tensor(L.BUF_VALUE)
+            vl_rows = self._vl_rows()
+            planes, pol, val = vl_rows or (self.tensor(L.BUF_LEAF_PLANES), self.tensor(L.BUF_POLICY), self.tensor(L.BUF_VALUE))
+            rounds = self.vl_rounds(sims)
 
             def one_round():
                 self.mcts_select()
@@ -573,9 +620,23 @@ def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_g
                 val.copy_(v.reshape(val.shape))
                 self.mcts_expand_backup()
 
-            if not use_graph or sims < 3:
-                for _ in range(sims):
+            if not use_graph or rounds < 3:
+                for _ in range(rounds):
                     one_round()
+            elif vl_rows is not None:
+                # the captured round bakes in K, vl, the round target (the begin's sims) and the row buffers (reallocated by a larger K)
+                key = (id(net), float(c_puct), self.vl, int(sims), self.buffer(L.BUF_VL_PLANES)[0])
+                cache = self.__dict__.setdefault("_graphs", {})
+                one_round()  # round 0 (one descent), eagerly: also the warm-up before a capture
+                if key not in cache:
+                    ts.synchronize()
+                    g = torch.cuda.CUDAGraph()
+                    with torch.cuda.graph(g, stream=ts):
+                        one_round()  # captured, not executed
+                    cache[key] = (g, net)
+                g = cache[key][0]
+                for _ in range(rounds - 1):
+                    g.replay()
             else:
                 # a captured round bakes in everything the launches were given: the evaluator, c_puct AND the root-noise settings
                 # (ADVICE r01: switching train mode after a capture must not replay the old setting). The cache holds a strong
