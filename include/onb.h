@@ -616,6 +616,32 @@ ONB_API int32_t onb_tb_probe(onb_ctx* ctx, int16_t* values_host); /* [n] */
 ONB_API int32_t onb_tb_best(onb_ctx* ctx, onb_action* best_host); /* [n], also left in ONB_BUF_ACTIONS */
 ONB_API int32_t onb_tb_index(const uint8_t cards5[5], const onb_state* s, int64_t n, int32_t* cls, int64_t* idx);
 ONB_API int32_t onb_tb_state(const uint8_t cards5[5], int32_t cls, const int64_t* idx, int64_t n, onb_state* out);
+/* Tablebase leaves (DESIGN.md §5i): the PUCT search probes the resident table at its leaves. Off by default; enabled = 0 switches it
+ * off, and every entry point then computes what it computes without this call. enabled != 0 switches it on for the searches begun
+ * afterwards (ONB_E_STATE without a resident table); onb_tb_free and onb_tb_solve switch it off. A search begun with the switch on
+ * (exact to the bit) takes, at the leaf L a descent reaches, v = the resident table's value of L's position by onb_tb_probe's rule
+ * (ONB_TB_NONE for a decided position, another card set or a class the table does not hold):
+ *   v = ONB_TB_NONE: as without the switch.
+ *   v != ONB_TB_NONE, L not the root: L is NOT expanded (it stays an unexpanded node, n_child 0 and flags unchanged, on every later
+ *     visit) and the evaluator's policy and value of L are ignored. The reward backed up is that of a decided leaf whose winner is the
+ *     table's winner: reward colour = the colour of L's parent, so -1 if v > 0 (the side to move at L wins), +1 if v < 0, 0 if v = 0.
+ *   v != ONB_TB_NONE, L the root (its first descent): the root is expanded with the evaluator's policy as without the switch (a search
+ *     must have children) and backs up +1 / -1 / 0 by the sign of v, from the root mover's view.
+ *   The backup is unchanged. Material never increases, so below a root inside the table every leaf is in the table or decided.
+ * The rule holds in every search path: with virtual loss row j's leaf follows it (a table leaf is never expanded, so "an earlier
+ * descent of the round expanded it" never applies to it); the Gumbel root and interior selection are unchanged above the leaf (r_x
+ * is stored on expansion only); train-mode noise only touches the selection. onb_mcts_run with ONB_EVAL_UNIFORM / ONB_EVAL_HASH runs
+ * the split phase's rounds (select, evaluation, expand/backup: three launches per simulation) instead of the fused kernel, so such a
+ * search is launch-bound with few trees and slower than the fused one with many (DESIGN.md §5i has the measured cost); ONB_EVAL_NET
+ * rounds are unchanged apart from the expand/backup. Refused with ONB_E_STATE: a begin with the switch on together with tree reuse; onb_uct_run after such a
+ * begin; onb_self_play while the switch is on; onb_mcts_select / _run / _expand_backup of a search begun with the switch on after
+ * onb_tb_free or onb_tb_solve (the search never reads a freed table). onb_fight probes the table only for ONB_AGENT_PUCT_TB agents,
+ * whatever the switch says, and leaves the switch as it found it. */
+ONB_API int32_t onb_mcts_set_tablebase(onb_ctx* ctx, int32_t enabled);
+/* ONB_AGENT_PUCT_TB: as ONB_AGENT_PUCT (the same fields) with the table: in a game whose position is in the resident table it plays
+ * onb_tb_best's move, in every other game it plays an eval-mode PUCT search with tablebase leaves (so games of another card set get
+ * plain PUCT). It needs a resident table (ONB_E_STATE otherwise); unlike ONB_AGENT_TABLEBASE, games need not start in the table. */
+#define ONB_AGENT_PUCT_TB 8
 
 /* ---- policy/value network on the device ---------------------------------------------------------------------
  * ConvResNet::forward (alphazero-training/src/net.rs:215-232) for every position of a plane buffer, as one fused

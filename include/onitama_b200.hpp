@@ -148,6 +148,18 @@ public:
     std::vector<uint8_t> last_fight_results;  ///< per-game MoveResult codes of the last fight_device (0 undecided, 1 RedWin, 2 BlueWin)
     onb_gumbel_config gumbel_applied{};       ///< the Gumbel setting last passed to onb_mcts_set_gumbel (enabled = 0: off)
     std::pair<uint32_t, double> vl_applied{1, 1.0};  ///< (leaves, virtual_loss) last passed to onb_mcts_set_virtual_loss (leaves 1: off)
+    bool tb_applied = false;                  ///< the tablebase-leaf switch last passed to onb_mcts_set_tablebase
+    int32_t tb_max_pawns = -1;                ///< the table resident on this engine (solve_tablebase): max_pawns, -1 none
+    std::array<uint8_t, 5> tb_cards{};        ///< ... and its card set as given
+    /// onb_tb_solve on this engine's context: the table of one five-card set with at most max_pawns pawns, which tablebase leaves
+    /// (AlphaZeroMctsConfig::tablebase_leaves) and ONB_AGENT_PUCT_TB agents in fight_device read. A solve switches tablebase leaves off.
+    void solve_tablebase(const std::array<uint8_t, 5>& cards, int32_t max_pawns) {
+        tb_max_pawns = -1;
+        tb_applied = false;
+        check(onb_tb_solve(ctx_, cards.data(), max_pawns, nullptr));
+        tb_cards = cards;
+        tb_max_pawns = max_pawns;
+    }
     /// one-game engine shared by the single-state methods of State / the agents (thread local: a context is single threaded)
     static Engine& single(uint32_t min_sims = 0) {
         thread_local std::unique_ptr<Engine> e;
@@ -429,6 +441,14 @@ struct AlphaZeroMctsConfig {  // alphazero_mcts/mod.rs:26-43
     // evaluates n * leaves_per_round rows per round. Applied when it changes. Does not combine with train, reuse or gumbel (ONB_E_STATE).
     uint32_t leaves_per_round = 1;
     double virtual_loss = 1.0;
+    // tablebase leaves (onb_mcts_set_tablebase, DESIGN.md §5i): the search's engine holds the table of tablebase_cards with at most
+    // tablebase_max_pawns pawns (solved on first use and whenever these change) and every search probes it at its leaves: a leaf below
+    // the root that the table holds is not expanded and backs up the table's exact value. Does not combine with reuse (ONB_E_STATE).
+    // With a device evaluator the search runs one select, evaluation and expand/backup launch per simulation instead of the fused
+    // kernel (DESIGN.md §5i gives the cost).
+    bool tablebase_leaves = false;
+    std::array<uint8_t, 5> tablebase_cards{};
+    int32_t tablebase_max_pawns = 3;
 };
 inline double reward(MoveResult r, PlayerColor c) {  // alphazero_mcts/mod.rs:45-53
     if (c == PlayerColor::Red) return r == MoveResult::RedWin ? 1. : r == MoveResult::BlueWin ? -1. : 0.;
@@ -457,6 +477,12 @@ inline void run_search(Engine& e, const AlphaZeroMctsConfig& cfg, int32_t device
     if (vl != e.vl_applied) {
         e.check(onb_mcts_set_virtual_loss(e.ctx(), vl.first, vl.second));
         e.vl_applied = vl;
+    }
+    if (cfg.tablebase_leaves && (e.tb_max_pawns != cfg.tablebase_max_pawns || e.tb_cards != cfg.tablebase_cards))
+        e.solve_tablebase(cfg.tablebase_cards, cfg.tablebase_max_pawns);
+    if (cfg.tablebase_leaves != e.tb_applied) {
+        e.check(onb_mcts_set_tablebase(e.ctx(), cfg.tablebase_leaves ? 1 : 0));
+        e.tb_applied = cfg.tablebase_leaves;
     }
     e.check(onb_mcts_begin(e.ctx(), cfg.exploration_c, cfg.max_playouts));
     if (!net) {
@@ -712,6 +738,18 @@ inline FightStatistics fight(const EvaluatorConfig& config, std::unique_ptr<Agen
 /// evaluator.rs:393-397; the statistics incl. the Elo updates are folded in game order ON THE DEVICE (onb_fight_stats).
 /// Agents are described by onb_agent (ONB_AGENT_RANDOM / ONB_AGENT_PUCT / ONB_AGENT_UCT / ONB_AGENT_ALPHABETA with the depth in
 /// sims); the engine must have been created with n_games == config.game_amnt and enough mcts_max_sims for the searching agents.
+/// ONB_AGENT_PUCT_TB (PUCT with tablebase leaves that plays the table's move in the games of the table, DESIGN.md §5i) and
+/// ONB_AGENT_TABLEBASE read the table solved on the engine (Engine::solve_tablebase); without one onb_fight refuses them (ONB_E_STATE).
+/// puct_tablebase_agent builds the former.
+inline onb_agent puct_tablebase_agent(uint32_t sims, double c_puct = 2.0, int32_t evaluator = ONB_EVAL_UNIFORM, int32_t net_slot = 0) {
+    onb_agent a{};
+    a.kind = ONB_AGENT_PUCT_TB;
+    a.evaluator = evaluator;
+    a.net_slot = net_slot;
+    a.sims = sims;
+    a.c = c_puct;
+    return a;
+}
 inline FightStatistics fight_device(Engine& e, const EvaluatorConfig& config, const onb_agent& agent, const onb_agent& opponent, double rating_a = 800.,
                                     double rating_b = 800.) {
     if ((size_t)e.n() != config.game_amnt) throw Error(ONB_E_INVALID, "fight_device: the engine must hold game_amnt games");

@@ -85,6 +85,7 @@ SYMBOLS = {
     "onb_mcts_reuse_stats": (C.c_int32, [_P, _P, C.c_int32]),
     "onb_mcts_set_gumbel": (C.c_int32, [_P, _P]),
     "onb_mcts_set_virtual_loss": (C.c_int32, [_P, C.c_uint32, C.c_double]),
+    "onb_mcts_set_tablebase": (C.c_int32, [_P, C.c_int32]),
     "onb_mcts_select": (C.c_int32, [_P]),
     "onb_mcts_expand_backup": (C.c_int32, [_P]),
     "onb_mcts_eval": (C.c_int32, [_P, C.c_int32]),
@@ -131,6 +132,7 @@ class SelfPlayConfig(C.Structure):
 
 
 AGENT_RANDOM, AGENT_PUCT, AGENT_UCT, AGENT_ALPHABETA, AGENT_GUMBEL, AGENT_TABLEBASE, AGENT_GUMBEL_MUZERO, AGENT_PUCT_VL = 0, 1, 2, 3, 4, 5, 6, 7
+AGENT_PUCT_TB = 8
 ALPHABETA_MAX_DEPTH = 8
 ALPHABETA_WIN = 1000000
 TB_MAX_PAWNS = 4

@@ -471,11 +471,18 @@ static int32_t begin_search(Ctx* c, const SearchPlan& p, const char* who) {
     if (p.leaves >= 2 && (p.noise || p.gumbel || p.reuse))
         return fail(c, ONB_E_STATE, "%s: virtual loss (onb_mcts_set_virtual_loss) does not combine with %s", who,
                     p.noise ? "train-mode noise" : p.gumbel ? "the Gumbel root search" : "tree reuse");
+    // tablebase leaves (include/onb.h, onb_mcts_set_tablebase): the resident table, copied into the plan
+    if (p.tb && p.reuse) return fail(c, ONB_E_STATE, "%s: tablebase leaves (onb_mcts_set_tablebase) do not combine with tree reuse", who);
+    if (p.tb && !c->tb_live) return fail(c, ONB_E_STATE, "%s: tablebase leaves need a resident table (onb_tb_solve)", who);
     if (c->vl_dirty) {  // a select with virtual loss whose round was never backed up left counts behind
         ONB_CUDA(c, cudaMemsetAsync(c->d_vl_cnt, 0, (size_t)c->n * c->node_cap, c->stream));
         c->vl_dirty = 0;
     }
     c->search.plan = p;
+    if (p.tb) {
+        c->search.plan.tb_table = tb_table(c);
+        c->search.plan.tb_serial = c->tb_serial;
+    }
     if (p.reuse) {
         ONB_CUDA(c, launch_reuse_begin(c, p.d_games, p.d_games ? p.m : c->n, p.sims));
     } else {
@@ -607,6 +614,13 @@ int32_t onb_mcts_set_virtual_loss(onb_ctx* ctx, uint32_t leaves, double virtual_
     c->vl_loss = virtual_loss;
     return ONB_OK;
 }
+int32_t onb_mcts_set_tablebase(onb_ctx* ctx, int32_t enabled) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (enabled && !c->tb_live) return fail(c, ONB_E_STATE, "onb_mcts_set_tablebase: no tablebase is resident (onb_tb_solve)");
+    c->tb_search = enabled ? 1 : 0;
+    return ONB_OK;
+}
 int32_t onb_mcts_begin(onb_ctx* ctx, double c_puct, uint32_t sims) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
@@ -623,6 +637,7 @@ int32_t onb_mcts_begin(onb_ctx* ctx, double c_puct, uint32_t sims) {
     p.gb_step = c->gb_serial;
     p.leaves = c->vl_leaves;
     p.vloss = c->vl_loss;
+    p.tb = c->tb_search != 0;
     const int32_t rc = begin_search(c, p, "onb_mcts_begin");
     if (rc == ONB_OK && p.gumbel) c->gb_serial += 1;
     return rc;
@@ -669,6 +684,11 @@ int32_t onb_mcts_reuse_stats(onb_ctx* ctx, uint64_t out[4], int32_t clear) {
     if (clear) memset(c->ru_stats, 0, sizeof(c->ru_stats));
     return ONB_OK;
 }
+// a search begun with tablebase leaves whose table has been freed since (onb_tb_free, onb_tb_solve) must not read it
+static bool table_gone(const Ctx* c) { return c->search.plan.tb && c->search.plan.tb_serial != c->tb_serial; }
+static int32_t refuse_table_gone(Ctx* c, const char* what) {
+    return fail(c, ONB_E_STATE, "%s: the search was begun with tablebase leaves and that table has been freed (onb_tb_free / onb_tb_solve)", what);
+}
 static int32_t refuse_after_reuse(Ctx* c, const char* what) {
     return fail(c, ONB_E_STATE, "%s: the search was begun with tree reuse on (onb_mcts_set_reuse), which only onb_mcts_run can continue; "
                                 "switch reuse off before onb_mcts_begin for a caller-driven search", what);
@@ -689,6 +709,7 @@ int32_t onb_mcts_select(onb_ctx* ctx) {
     ActiveSearch& a = c->search;
     if (a.phase != 1) return fail(c, ONB_E_STATE, "onb_mcts_select: call onb_mcts_begin / onb_mcts_expand_backup first");
     if (a.plan.reuse) return refuse_after_reuse(c, "onb_mcts_select");
+    if (table_gone(c)) return refuse_table_gone(c, "onb_mcts_select");
     if (a.plan.gumbel && a.sims_done >= a.plan.sims)
         return fail(c, ONB_E_STATE, "onb_mcts_select: a Gumbel search runs at most the begin's %u simulations", a.plan.sims);
     if (a.plan.leaves >= 2) {  // the split phase counts every round against the begin's sims
@@ -723,6 +744,7 @@ int32_t onb_mcts_expand_backup(onb_ctx* ctx) {
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
     if (c->search.plan.reuse) return refuse_after_reuse(c, "onb_mcts_expand_backup");
     if (c->search.phase != 2) return fail(c, ONB_E_STATE, "onb_mcts_expand_backup: call onb_mcts_select first");
+    if (table_gone(c)) return refuse_table_gone(c, "onb_mcts_expand_backup");
     ONB_CUDA(c, launch_mcts_expand_backup(c));
     ActiveSearch& a = c->search;
     a.phase = 1;
@@ -774,6 +796,7 @@ int32_t onb_mcts_run(onb_ctx* ctx, int32_t evaluator, uint32_t sims) {
         return fail(c, ONB_E_INVALID, "onb_mcts_run: unknown evaluator %d", evaluator);
     if (a.sims_done + sims > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_mcts_run: more simulations than mcts_max_sims");
     if (a.plan.reuse) return reuse_run(c, evaluator, sims);
+    if (table_gone(c)) return refuse_table_gone(c, "onb_mcts_run");
     if (a.plan.gumbel && a.sims_done + sims > a.plan.sims)
         return fail(c, ONB_E_STATE, "onb_mcts_run: a Gumbel search runs at most the begin's %u simulations", a.plan.sims);
     if (a.plan.leaves >= 2) {  // rounds of K descents per tree (round 0: one), counted against this call's end
@@ -791,6 +814,16 @@ int32_t onb_mcts_run(onb_ctx* ctx, int32_t evaluator, uint32_t sims) {
             ONB_CUDA(c, launch_mcts_expand_backup(c));
             a.sims_done += vl_descents(a.sims_done, a.plan.leaves, a.vl_target);
         }
+        return ONB_OK;
+    }
+    if (a.plan.tb && evaluator != ONB_EVAL_NET) {
+        // tablebase leaves live in the split phase's expand/backup only: one select, evaluation and expand/backup per simulation
+        for (uint32_t s = 0; s < sims; ++s) {
+            ONB_CUDA(c, launch_mcts_select(c));
+            ONB_CUDA(c, launch_mcts_eval(c, evaluator));
+            ONB_CUDA(c, launch_mcts_expand_backup(c));
+        }
+        a.sims_done += sims;
         return ONB_OK;
     }
     if (evaluator == ONB_EVAL_NET) {
@@ -842,6 +875,9 @@ int32_t onb_self_play(onb_ctx* ctx, const onb_selfplay_config* cfg, onb_selfplay
     if (cfg->train && c->gb_on) return fail(c, ONB_E_INVALID, "onb_self_play: train-mode noise does not combine with the Gumbel root search");
     if (c->reuse_on && c->gb_on) return fail(c, ONB_E_STATE, "onb_self_play: tree reuse does not combine with the Gumbel root search");
     if (c->vl_leaves >= 2) return fail(c, ONB_E_STATE, "onb_self_play: self-play searches without virtual loss; switch it off (onb_mcts_set_virtual_loss)");
+    if (c->tb_search)
+        return fail(c, ONB_E_STATE, "onb_self_play: self-play deals every game from the RNG and searches without tablebase leaves; switch them off "
+                                    "(onb_mcts_set_tablebase)");
     memset(out, 0, sizeof(*out));
     c->ru_live = 0;  // self-play starts from fresh deals: nothing is kept from earlier searches
     char err[400];
@@ -876,6 +912,7 @@ static int32_t fight_move(Ctx* c, const onb_agent* ag, uint32_t ply, const int32
         ONB_CUDA(c, launch_tb_best(c, d_games, m, d_out));
         return ONB_OK;
     }
+    const bool tb = ag->kind == ONB_AGENT_PUCT_TB;
     // eval mode (AlphaZeroMcts, not TrainingAlphaZeroMcts) and no reuse; PUCT and UCT agents search without the Gumbel root step
     SearchPlan p = {};
     p.c_puct = ag->c;
@@ -898,9 +935,10 @@ static int32_t fight_move(Ctx* c, const onb_agent* ag, uint32_t ply, const int32
         p.leaves = ag->min_node_visits;
         p.vloss = 1.0;
     }
+    p.tb = tb;  // PUCT with tablebase leaves; the table's move replaces the search's in the games of the table (below)
     int32_t rc = begin_search(c, p, "search");
     if (rc != ONB_OK) return rc;
-    if (ag->kind == ONB_AGENT_PUCT || ag->kind == ONB_AGENT_PUCT_VL || p.gumbel) {
+    if (ag->kind == ONB_AGENT_PUCT || ag->kind == ONB_AGENT_PUCT_VL || tb || p.gumbel) {
         if (ag->evaluator == ONB_EVAL_NET && (rc = onb_net_select(x, ag->net_slot)) != ONB_OK) return rc;
         rc = onb_mcts_run(x, ag->evaluator, ag->sims);
     } else {
@@ -910,6 +948,7 @@ static int32_t fight_move(Ctx* c, const onb_agent* ag, uint32_t ply, const int32
     if (rc != ONB_OK) return rc;
     // the chosen moves become the agent's actions (ONB_ACTION_NONE for decided roots)
     ONB_CUDA(c, launch_mcts_scatter_best(c, d_out));
+    if (tb) ONB_CUDA(c, launch_tb_best_in_table(c, d_games, m, d_out, reinterpret_cast<uint16_t*>(c->d_tb_values)));
     return ONB_OK;
 }
 int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const uint8_t* a_is_red_host, uint32_t max_plies, onb_fight_result* out,
@@ -919,8 +958,11 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
     if (!a || !b || !a_is_red_host || !out) return fail(c, ONB_E_INVALID, "onb_fight: null argument");
     for (const onb_agent* ag : {a, b}) {
         if (ag->kind != ONB_AGENT_RANDOM && ag->kind != ONB_AGENT_PUCT && ag->kind != ONB_AGENT_UCT && ag->kind != ONB_AGENT_ALPHABETA &&
-            ag->kind != ONB_AGENT_GUMBEL && ag->kind != ONB_AGENT_TABLEBASE && ag->kind != ONB_AGENT_GUMBEL_MUZERO && ag->kind != ONB_AGENT_PUCT_VL)
+            ag->kind != ONB_AGENT_GUMBEL && ag->kind != ONB_AGENT_TABLEBASE && ag->kind != ONB_AGENT_GUMBEL_MUZERO && ag->kind != ONB_AGENT_PUCT_VL &&
+            ag->kind != ONB_AGENT_PUCT_TB)
             return fail(c, ONB_E_INVALID, "onb_fight: unknown agent kind %d", ag->kind);
+        if (ag->kind == ONB_AGENT_PUCT_TB && !c->tb_live)
+            return fail(c, ONB_E_STATE, "onb_fight: a PUCT agent with tablebase leaves needs a solved table (onb_tb_solve)");
         if (ag->kind == ONB_AGENT_TABLEBASE) {
             if (!c->tb_live) return fail(c, ONB_E_STATE, "onb_fight: a tablebase agent needs a solved table (onb_tb_solve)");
             continue;
@@ -955,6 +997,7 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
     const bool muzero = a->kind == ONB_AGENT_GUMBEL_MUZERO || b->kind == ONB_AGENT_GUMBEL_MUZERO;
     int32_t rc;
     if ((a->kind == ONB_AGENT_GUMBEL || b->kind == ONB_AGENT_GUMBEL || muzero) && (rc = gumbel_alloc(c, muzero)) != ONB_OK) return rc;
+    if ((a->kind == ONB_AGENT_PUCT_TB || b->kind == ONB_AGENT_PUCT_TB) && !c->d_tb_values) ONB_CUDA(c, dalloc(&c->d_tb_values, (size_t)c->n));
     uint32_t vl_need = 0;  // the virtual-loss agents' buffers; the context's switch is left as it is
     for (const onb_agent* ag : {a, b})
         if (ag->kind == ONB_AGENT_PUCT_VL && ag->min_node_visits > vl_need) vl_need = ag->min_node_visits;
@@ -999,6 +1042,7 @@ int32_t onb_uct_run(onb_ctx* ctx, float exploration_c, uint32_t min_node_visits,
     if (a.plan.reuse) return refuse_after_reuse(c, "onb_uct_run");
     if (a.plan.gumbel) return fail(c, ONB_E_STATE, "onb_uct_run: the search was begun with the Gumbel root search on (onb_mcts_set_gumbel)");
     if (a.plan.leaves >= 2) return fail(c, ONB_E_STATE, "onb_uct_run: the search was begun with virtual loss on (onb_mcts_set_virtual_loss)");
+    if (a.plan.tb) return fail(c, ONB_E_STATE, "onb_uct_run: the search was begun with tablebase leaves on (onb_mcts_set_tablebase)");
     if (a.sims_done + playouts > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_uct_run: more playouts than mcts_max_sims");
     const uint32_t need = a.sims_done + playouts + 2;
     if (c->ln_cap < need) {  // ln(parent visits) as the reference computes it: f32 logf on the host
@@ -1037,6 +1081,7 @@ int32_t onb_alphabeta_run(onb_ctx* ctx, int32_t depth, onb_action* best_host, in
 int32_t onb_tb_solve(onb_ctx* ctx, const uint8_t cards5[5], int32_t max_pawns, onb_tb_class out[25]) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    c->tb_search = 0;  // every solve switches tablebase leaves off, also one refused before it replaces the table
     char err[400];
     err[0] = 0;
     const int32_t rc = tb_solve(c, cards5, max_pawns, out, err, sizeof(err));

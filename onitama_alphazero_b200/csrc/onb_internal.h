@@ -41,6 +41,13 @@ struct GumbelDev {
     float* rx;                          // [n][node_cap] r_x: the reward the expanding simulation backed up into node x (interior only)
 };
 
+// The resident endgame tablebase as the kernels that probe it take it (by value): class 5 p + q at tab[5 p + q] (nullptr: not in the
+// table), the set's cards (bit id) and the largest p + q solved. onb_tablebase.cuh holds the index and the lookup.
+struct TbTable {
+    int16_t* tab[25];
+    uint32_t setmask, max_pawns;
+};
+
 // Everything a search is begun with (begin_search). onb_mcts_begin builds it from the context's switches, onb_self_play from its
 // config, onb_fight from the agent; the launchers read only the copy in Ctx::search, so a switch changed after the begin does not
 // reach the search already running.
@@ -59,6 +66,9 @@ struct SearchPlan {
     uint32_t gb_step;
     uint32_t leaves;         // K >= 2: leaf parallelism with virtual loss (onb_mcts_set_virtual_loss), 0: one descent per round
     double vloss;
+    bool tb;                 // tablebase leaves (onb_mcts_set_tablebase, DESIGN.md §5i): begin_search copies the table into tb_table
+    TbTable tb_table;
+    uint32_t tb_serial;      // Ctx::tb_serial at the begin: the search continues only while that table is resident
 };
 // Descents of the next round of a search with virtual loss (DESIGN.md §5h), from the descents done so far (= the root's visits) and
 // the target the round counts against: 1 for round 0, then min(K, target - done). The kernels derive it from the root's visit count,
@@ -186,7 +196,9 @@ struct Ctx {
     uint32_t tb_setmask;      // bit id set for the five cards of the set
     int32_t tb_max_pawns;
     int tb_live;              // a solved table is resident
-    int16_t* d_tb_values;     // [n] onb_tb_probe's output (allocated on first use)
+    int tb_search;            // the switch of onb_mcts_set_tablebase (tablebase leaves); tb_free switches it off
+    uint32_t tb_serial;       // raised by every tb_free, so a search begun with an earlier table knows it is gone
+    int16_t* d_tb_values;     // [n] onb_tb_probe's output, and ONB_AGENT_PUCT_TB's table moves (allocated on first use)
     char err[512];
 };
 
@@ -218,7 +230,7 @@ cudaError_t launch_mcts_play_best(Ctx* c, uint32_t out_flags);
 cudaError_t launch_mcts_scatter_best(Ctx* c, uint16_t* dst_actions);  // dst[game of tree t] = best[t]
 // the search launchers take their kernel from c->search.plan: noise, Gumbel at the root (select, run, finish) and Gumbel MuZero
 // below it (select, run, expand_backup), virtual loss (select, eval, expand_backup over the K rows of every tree, round target
-// search.vl_target)
+// search.vl_target), tablebase leaves (expand_backup)
 
 // network (onb_net.cu)
 int32_t net_load(Ctx* c, int32_t n_tensors, const char* const* names, const float* const* data, const int64_t* numel, std::string& err);
@@ -235,6 +247,9 @@ void tb_free(Ctx* c);
 cudaError_t launch_tb_probe(Ctx* c, int16_t* d_values, unsigned long long* d_missing);
 // d_out[game] = onb_tb_best's move for the games d_games[0 .. m) (nullptr: games 0 .. m)
 cudaError_t launch_tb_best(Ctx* c, const int32_t* d_games, int64_t m, uint16_t* d_out);
+// the same for the listed games in the table only (the others keep d_out[game]), through d_tmp [n]
+cudaError_t launch_tb_best_in_table(Ctx* c, const int32_t* d_games, int64_t m, uint16_t* d_out, uint16_t* d_tmp);
+TbTable tb_table(const Ctx* c);  // the resident table as the search kernels take it
 
 // tree reuse (onb_reuse.cu)
 cudaError_t reuse_alloc(Ctx* c);

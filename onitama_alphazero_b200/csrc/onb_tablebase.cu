@@ -8,52 +8,13 @@
 // whose every child is a win. During the solve 0 means "unresolved"; the entries still unresolved at the end are the draws.
 #include <cstring>
 
-#include "onb_internal.h"
-#include "onb_rules.cuh"
+#include "onb_tablebase.cuh"
 
 namespace onb {
 
 constexpr int kTbThreads = 256;
-constexpr uint32_t kTbPairs = 600;      // ordered king pairs on distinct squares
-constexpr uint32_t kTbDecided = 47;     // of them with the red king on square 2 or the blue king on square 22
+constexpr uint32_t kTbDecided = 47;     // ordered king pairs (kTbPairs) with the red king on square 2 or the blue king on square 22
 
-// C(n, k) for n <= 24, k <= 4 at [5 n + k]
-struct BinomTable {
-    uint32_t b[25 * 5];
-};
-constexpr BinomTable make_binom() {
-    BinomTable t{};
-    for (int n = 0; n < 25; ++n)
-        for (int k = 0; k < 5; ++k) {
-            uint64_t v = 1;
-            for (int i = 0; i < k && i < n; ++i) v = v * (uint64_t)(n - i) / (uint64_t)(i + 1);
-            t.b[n * 5 + k] = k > n ? 0u : (uint32_t)v;
-        }
-    return t;
-}
-constexpr BinomTable kBinomHost = make_binom();
-static __device__ BinomTable g_binom = make_binom();
-
-__host__ __device__ __forceinline__ uint32_t low_bit(uint32_t x) {
-#ifdef __CUDA_ARCH__
-    return (uint32_t)(__ffs(x) - 1);
-#else
-    return (uint32_t)__builtin_ctz(x);
-#endif
-}
-__host__ __device__ __forceinline__ uint32_t below(uint32_t s) { return (1u << s) - 1u; }
-
-// colex rank of the squares of `set` among the squares not in `occ` (a square's position there is s - popc(occ below s))
-__host__ __device__ __forceinline__ uint32_t colex_rank(const uint32_t* B, uint32_t set, uint32_t occ) {
-    uint32_t r = 0, i = 1;
-    while (set) {
-        const uint32_t s = low_bit(set);
-        set &= set - 1;
-        r += B[(s - popc32(occ & below(s))) * 5 + i];
-        ++i;
-    }
-    return r;
-}
 // the k squares outside `occ` whose colex rank is r
 __host__ __device__ __forceinline__ uint32_t colex_unrank(const uint32_t* B, uint32_t r, uint32_t k, uint32_t occ) {
     uint32_t set = 0;
@@ -68,27 +29,6 @@ __host__ __device__ __forceinline__ uint32_t colex_unrank(const uint32_t* B, uin
     return set;
 }
 
-// card configuration 6 j + r of a neutral card and a red hand (ids) within the set `setmask`
-__host__ __device__ __forceinline__ uint32_t card_cfg(uint32_t setmask, uint32_t neutral, uint32_t ra, uint32_t rb) {
-    const uint32_t j = popc32(setmask & below(neutral));
-    uint32_t a = popc32(setmask & below(ra)), b = popc32(setmask & below(rb));
-    a -= a > j;
-    b -= b > j;
-    const uint32_t lo = a < b ? a : b, hi = a < b ? b : a;
-    return 6u * j + lo + hi * (hi - 1u) / 2u;
-}
-
-__host__ __device__ __forceinline__ uint64_t class_subsets(const uint32_t* B, uint32_t p, uint32_t q) {
-    return (uint64_t)B[23 * 5 + p] * B[(23 - p) * 5 + q];
-}
-// entry of a position within its class (p, q); pr, pb internal-layout pawn boards, kr, kb king squares
-__host__ __device__ __forceinline__ uint64_t tb_entry(const uint32_t* B, uint32_t pr, uint32_t pb, uint32_t kr, uint32_t kb, uint32_t cfg,
-                                                      uint32_t side, uint32_t p, uint32_t q) {
-    const uint32_t kings = (1u << kr) | (1u << kb);
-    const uint64_t sb = B[(23 - p) * 5 + q];
-    const uint64_t pair = (uint64_t)(cfg * 2u + side) * kTbPairs + 24u * kr + kb - (kb > kr ? 1u : 0u);
-    return pair * ((uint64_t)B[23 * 5 + p] * sb) + (uint64_t)colex_rank(B, pr, kings) * sb + colex_rank(B, pb, kings | pr);
-}
 struct TbPos {
     uint32_t pr, pb, kr, kb, cfg, side;
 };
@@ -110,14 +50,6 @@ __host__ __device__ __forceinline__ TbPos tb_unrank(const uint32_t* B, uint32_t 
     x.pb = colex_unrank(B, sub % sb, q, kings | x.pr);
     return x;
 }
-
-// Kernel parameters (by value): the class tables and the card configurations of the set
-struct TbParams {
-    int16_t* tab[25];       // class 5 p + q; nullptr: not in the table
-    uint32_t setmask, max_pawns;
-    uint8_t cards[30][4];   // hand cards of configuration cfg in slots red lo, red hi, blue lo, blue hi
-    uint8_t child[30][4];   // configuration after the mover plays hand card u (it becomes the neutral card)
-};
 
 __device__ __forceinline__ void tb_load_smem(uint32_t* s_att, uint32_t* s_b) {
     load_attack_table_to_smem(s_att);
@@ -247,21 +179,6 @@ __global__ void __launch_bounds__(kTbThreads) k_tb_compact(const int16_t* __rest
     warp_append(i < m && T[e] == 0, e, out, cnt);
 }
 
-// value of a game, ONB_TB_NONE when it is decided or not a position of the table
-__device__ __forceinline__ int32_t tb_lookup(const TbParams& P, const uint32_t* B, const Game& g) {
-    if (g.result != 0 || current_state(g) != 0) return ONB_TB_NONE;
-    uint32_t seen = 0;
-    for (uint32_t s = 0; s < 5; ++s) seen |= 1u << card_at(g.cards, s);
-    if (seen != P.setmask) return ONB_TB_NONE;
-    if (popc32(g.king_r) != 1 || popc32(g.king_b) != 1 || (g.king_r & g.king_b) || (g.pawn_r & g.pawn_b) ||
-        ((g.pawn_r | g.pawn_b) & (g.king_r | g.king_b)))
-        return ONB_TB_NONE;
-    const uint32_t p = popc32(g.pawn_r), q = popc32(g.pawn_b);
-    if (p + q > P.max_pawns) return ONB_TB_NONE;
-    const uint32_t cfg = card_cfg(P.setmask, card_at(g.cards, 4), card_at(g.cards, 0), card_at(g.cards, 1));
-    return P.tab[5 * p + q][tb_entry(B, g.pawn_r, g.pawn_b, low_bit(g.king_r), low_bit(g.king_b), cfg, g.side, p, q)];
-}
-
 // values [n] (optional) and the number of undecided games outside the table (optional)
 __global__ void __launch_bounds__(kTbThreads) k_tb_probe(const TbParams P, const uint4* __restrict__ states, int64_t n, int16_t* values,
                                                          unsigned long long* missing) {
@@ -324,6 +241,15 @@ __global__ void __launch_bounds__(kTbThreads) k_tb_best(const TbParams P, const 
     out[game] = (uint16_t)best;
 }
 
+// out[games[i]] = moves[games[i]] where that is a move (the game is in the table); the other games keep out[game]
+__global__ void __launch_bounds__(kTbThreads) k_tb_keep_moves(const uint16_t* __restrict__ moves, const int32_t* __restrict__ games, int64_t m,
+                                                              uint16_t* __restrict__ out) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= m) return;
+    const int64_t game = games ? (int64_t)games[i] : i;
+    if (moves[game] != 0xFFFFu) out[game] = moves[game];
+}
+
 // ------------------------------------------------------------------------------------------------ host side
 static bool tb_cards_ok(const uint8_t cards5[5], uint32_t* setmask) {
     uint32_t m = 0;
@@ -374,6 +300,8 @@ void tb_free(Ctx* c) {
     if (c->d_tb) cudaFree(c->d_tb);
     c->d_tb = nullptr;
     c->tb_live = 0;
+    c->tb_search = 0;  // the table's searches end with it (onb_mcts_set_tablebase)
+    c->tb_serial += 1;
     memset(c->tb_off, 0, sizeof(c->tb_off));
     memset(c->tb_len, 0, sizeof(c->tb_len));
 }
@@ -516,6 +444,14 @@ cudaError_t launch_tb_best(Ctx* c, const int32_t* d_games, int64_t m, uint16_t* 
     k_tb_best<<<(unsigned)((m + kTbThreads - 1) / kTbThreads), kTbThreads, 0, c->stream>>>(P, c->d_states, d_games, m, d_out);
     return cudaGetLastError();
 }
+cudaError_t launch_tb_best_in_table(Ctx* c, const int32_t* d_games, int64_t m, uint16_t* d_out, uint16_t* d_tmp) {
+    if (m <= 0) return cudaSuccess;
+    const cudaError_t e = launch_tb_best(c, d_games, m, d_tmp);
+    if (e != cudaSuccess) return e;
+    k_tb_keep_moves<<<(unsigned)((m + kTbThreads - 1) / kTbThreads), kTbThreads, 0, c->stream>>>(d_tmp, d_games, m, d_out);
+    return cudaGetLastError();
+}
+TbTable tb_table(const Ctx* c) { return tb_params(c); }
 
 }  // namespace onb
 

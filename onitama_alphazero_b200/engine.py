@@ -34,6 +34,8 @@ class Context:
         self.seed = seed
         self.game_id_base = game_id_base
         self.mcts_max_sims = mcts_max_sims
+        self.tb_leaves = False  # the tablebase-leaf switch (set_tablebase)
+        self._tb_serial = 0     # raised by every tb_solve / tb_free: the table a captured search round was given
 
     # ------------------------------------------------------------------ plumbing
     def _ck(self, rc):
@@ -229,6 +231,22 @@ class Context:
         self._ck(self._lib.onb_mcts_set_virtual_loss(self._h, int(leaves), float(virtual_loss)))
         self.vl = (int(leaves), float(virtual_loss)) if leaves > 1 else None
 
+    def set_tablebase(self, enabled):
+        """onb_mcts_set_tablebase: tablebase leaves for the searches begun afterwards -- a leaf below the root whose position the
+        resident table holds is not expanded and backs up the table's exact value (needs tb_solve first; tb_free and tb_solve switch it
+        off). See include/onb.h and DESIGN.md §5i."""
+        self._ck(self._lib.onb_mcts_set_tablebase(self._h, int(bool(enabled))))
+        self.tb_leaves = bool(enabled)
+
+    def _use_tb(self, tb):
+        """the tb= argument of the search drivers: None leaves the tablebase-leaf switch, True / False sets it"""
+        if tb is not None and bool(tb) != self.tb_leaves:
+            self.set_tablebase(tb)
+
+    def _tb_graph_key(self):
+        """what a captured round with tablebase leaves bakes in: the table the expand/backup launch was given"""
+        return self._tb_serial if self.tb_leaves else None
+
     def _use_vl(self, vl):
         """the vl= argument of the search drivers: None leaves the switch, K (virtual loss 1) or (K, virtual_loss) sets it, K <= 1 or
         False switches it off"""
@@ -316,8 +334,14 @@ class Context:
         return L.Agent(L.AGENT_RANDOM, 0, 0, 0, 0.0, 0, 0)
 
     @staticmethod
-    def agent_puct(sims, c_puct=2.0, evaluator=L.EVAL_UNIFORM, net_slot=0, leaves=1):
-        """AlphaZeroMcts as an arena agent; leaves > 1: ONB_AGENT_PUCT_VL, rounds of `leaves` descents with virtual loss 1"""
+    def agent_puct(sims, c_puct=2.0, evaluator=L.EVAL_UNIFORM, net_slot=0, leaves=1, tablebase=False):
+        """AlphaZeroMcts as an arena agent; leaves > 1: ONB_AGENT_PUCT_VL, rounds of `leaves` descents with virtual loss 1;
+        tablebase=True: ONB_AGENT_PUCT_TB, the table's move in the games of the resident table and a search with tablebase leaves in
+        the others (no agent kind combines it with leaves > 1)"""
+        if tablebase and leaves > 1:
+            raise ValueError("agent_puct: tablebase=True does not combine with leaves > 1 (no agent kind covers both)")
+        if tablebase:
+            return L.Agent(L.AGENT_PUCT_TB, evaluator, net_slot, sims, c_puct, 0, 0)
         if leaves > 1:
             return L.Agent(L.AGENT_PUCT_VL, evaluator, net_slot, sims, c_puct, int(leaves), 0)
         return L.Agent(L.AGENT_PUCT, evaluator, net_slot, sims, c_puct, 0, 0)
@@ -393,12 +417,16 @@ class Context:
         context. Returns {(p, q): dict(entries, wins, losses, draws, invalid, max_win, max_loss, iterations, examined)}."""
         c = np.ascontiguousarray(cards, dtype=np.uint8).reshape(5)
         out = (L.TbClass * 25)()
+        self.tb_leaves = False  # the solve switches tablebase leaves off, whether it succeeds or not
+        self._tb_serial += 1
         self._ck(self._lib.onb_tb_solve(self._h, L.ptr(c), int(max_pawns), out))
         return {(k // 5, k % 5): {f: int(getattr(out[k], f)) for f, _ in L.TbClass._fields_ if f != "solved"}
                 for k in range(25) if out[k].solved}
 
     def tb_free(self):
         self._ck(self._lib.onb_tb_free(self._h))
+        self.tb_leaves = False
+        self._tb_serial += 1
 
     def tb_table(self, p, q):
         """zero-copy torch int16 view of the solved class (p, q) on the device (valid until the next solve / tb_free)"""
@@ -489,12 +517,13 @@ class Context:
         self._ck(self._lib.onb_mcts_dump_tree(self._h, tree, cap, C.byref(td), C.byref(nn)))
         return {k: v[:nn.value].copy() for k, v in arrs.items()}
 
-    def search(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, fused=True, net=None, vl=None):
+    def search(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, fused=True, net=None, vl=None, tb=None):
         """MctsArena::search for every game at once. net: callable(leaf_planes tensor [n,21,5,5]) -> (policy [n,2,25], value [n])
         running on this context's stream; it reads/writes the device buffers zero-copy. vl: None leaves the virtual-loss switch, K or
         (K, virtual_loss) sets it, 1 switches it off (set_virtual_loss); with it on, `net` gets the n K rows of ONB_BUF_VL_PLANES and
-        the split phase runs vl_rounds(sims) rounds."""
+        the split phase runs vl_rounds(sims) rounds. tb: None leaves the tablebase-leaf switch, True / False sets it (set_tablebase)."""
         self._use_vl(vl)
+        self._use_tb(tb)
         self.mcts_begin(c_puct, sims)
         if net is None and fused:
             self.mcts_run(evaluator, sims)
@@ -586,7 +615,7 @@ class Actor:
             pass
 
 
-def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_graph=False, reuse=None, gumbel=None, vl=None):
+def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_graph=False, reuse=None, gumbel=None, vl=None, tb=None):
     """Context.search without copying the results to the host (PI / BEST stay in their device buffers).
     use_graph: capture one simulation round (select -> network -> expand/backup) in a CUDA graph on the context's stream and
     replay it; the round is launch-bound otherwise (~40 small network kernels per round).
@@ -595,11 +624,13 @@ def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_g
     gumbel: None leaves the Gumbel switch as it is, False switches it off, True or a dict of set_gumbel keywords switches it on (only
     when that setting is not on already, so that consecutive searches take consecutive steps).
     vl: as for search. With virtual loss a torch `net` gets the n K rows, and use_graph runs round 0 eagerly and replays one captured
-    round for the others: the kernels take a round's descents from the root's visit count, so the short last round replays too."""
+    round for the others: the kernels take a round's descents from the root's visit count, so the short last round replays too.
+    tb: as for search. A captured round with tablebase leaves bakes in the table, so a new tb_solve captures anew."""
     if reuse is not None and bool(reuse) != getattr(self, "reuse", False):
         self.set_reuse(reuse)
     self._use_gumbel(gumbel)
     self._use_vl(vl)
+    self._use_tb(tb)
     if net is not None and getattr(self, "reuse", False):
         raise ValueError("search_device: tree reuse needs a device evaluator (EVAL_UNIFORM / EVAL_HASH / EVAL_NET), not a torch net")
     self.mcts_begin(c_puct, sims)
@@ -625,7 +656,7 @@ def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_g
                     one_round()
             elif vl_rows is not None:
                 # the captured round bakes in K, vl, the round target (the begin's sims) and the row buffers (reallocated by a larger K)
-                key = (id(net), float(c_puct), self.vl, int(sims), self.buffer(L.BUF_VL_PLANES)[0])
+                key = (id(net), float(c_puct), self.vl, int(sims), self.buffer(L.BUF_VL_PLANES)[0], self._tb_graph_key())
                 cache = self.__dict__.setdefault("_graphs", {})
                 one_round()  # round 0 (one descent), eagerly: also the warm-up before a capture
                 if key not in cache:
@@ -641,7 +672,7 @@ def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_g
                 # a captured round bakes in everything the launches were given: the evaluator, c_puct AND the root-noise settings
                 # (ADVICE r01: switching train mode after a capture must not replay the old setting). The cache holds a strong
                 # reference to `net`, so its id cannot be recycled for another module while the graph lives; close() drops it.
-                key = (id(net), float(c_puct), getattr(self, "_noise", (False,)), getattr(self, "gumbel", None))
+                key = (id(net), float(c_puct), getattr(self, "_noise", (False,)), getattr(self, "gumbel", None), self._tb_graph_key())
                 cache = self.__dict__.setdefault("_graphs", {})
                 done = 0
                 if key not in cache:

@@ -247,6 +247,20 @@ def _fight(ctx, move_fn_a, move_fn_b, a_is_red, max_plies):
     return a_wins, b_wins, int(n - a_wins - b_wins)
 
 
+def puct_tb_move(sims, c_puct=2.0, evaluator=L.EVAL_UNIFORM):
+    """ONB_AGENT_PUCT_TB as a move function of fight(): an eval-mode PUCT search with tablebase leaves (tb=True) over every game,
+    then the table's move (tb_best) in the games of the resident table. The context's tablebase-leaf switch is left as it was."""
+    def move(ctx):
+        was = ctx.tb_leaves
+        ctx.search_device(c_puct, sims, evaluator=evaluator, tb=True)
+        ctx._use_tb(was)
+        best = ctx.tensor(L.BUF_BEST).clone()
+        ctx.tb_best(to_host=False)  # the table's moves into ACTIONS, ACTION_NONE (-1 as int16) outside the table
+        acts = ctx.tensor(L.BUF_ACTIONS)
+        acts.copy_(torch.where(acts != -1, acts, best))
+    return move
+
+
 class ReplayBuffer:
     """Fixed-capacity ring buffer of self-play samples on one device (train.rs:213,241-245 keeps `data_buffer =
     Vec::with_capacity(buffer_size)` and only ever extends it; the ring bounds it: the newest samples overwrite the oldest).
