@@ -8,6 +8,7 @@ Everything game-, search- and inference-related runs in libonb.so: the current w
 onb_net_load after every update and evaluated by the tensor-core kernel between select and expand. The optimiser, the
 backward pass and the bookkeeping are plain PyTorch / Python (out of scope of the hot path).
 Usage: python examples/selfplay_train_loop.py [--slots 256] [--games 512] [--sims 64] [--iters 2] [--hidden {64,128}] [--torch-net]
+       [--temp-plies 30 --temperature 1 --resign-fp 0.05]
 """
 import argparse
 import os
@@ -41,6 +42,12 @@ def main(argv=None):
                          "policy instead of PUCT with root noise; the arena adds Gumbel(--sims) against PUCT(--sims)")
     ap.add_argument("--gumbel-interior", action="store_true",
                     help="with --gumbel: Gumbel MuZero, interior selection below the root instead of PUCT (onb_gumbel_config.interior)")
+    ap.add_argument("--temp-plies", type=int, default=0, help="AlphaZero's opening temperature: the first N plies of a self-play game sample "
+                                                               "their move in proportion to N^(1/temperature) (onb_self_play_set_protocol)")
+    ap.add_argument("--temperature", type=float, default=1.0)
+    ap.add_argument("--resign-fp", type=float, default=None, metavar="F",
+                    help="AlphaGo Zero's resignation: the first iteration holds out every game, each later one resigns below the threshold "
+                         "calibrated on the previous iteration's held-out games for a false-positive rate F, holding out 10%% of its games")
     ap.add_argument("--seed", type=int, default=0)
     ap.add_argument("--out", default=None, help="directory for the reference's on-disk artefacts: loss_stats JSON (stats.rs) and .ot checkpoints (train.rs:414-430)")
     ap.add_argument("--hidden", type=int, default=64, choices=[64, 128], help="hidden channels of the ConvResNet (both run on the tensor cores)")
@@ -69,16 +76,29 @@ def main(argv=None):
     gumbel = dict(m=args.gumbel, seed=args.seed, interior=args.gumbel_interior) if args.gumbel else None
     if args.reuse and args.torch_net:
         ap.error("--reuse needs the on-device network (a PyTorch module drives the split phase, which tree reuse does not support)")
+    if args.temp_plies and args.gumbel:
+        ap.error("--temp-plies does not combine with --gumbel (Gumbel plays its sequential-halving winner)")
+    resign_below = None   # the threshold calibrated on the previous iteration's held-out games
     for it in range(args.iters):
+        protocol = None
+        if args.temp_plies or args.resign_fp is not None:
+            protocol = dict(temp_plies=args.temp_plies, temperature=args.temperature, seed=args.seed + 7 * it)
+            if args.resign_fp is not None:   # the first iteration (no threshold yet) holds out every game
+                protocol.update(resign=True, resign_below=resign_below if resign_below is not None else -1.0,
+                                resign_holdout=0.1 if resign_below is not None else 1.0)
         # ---- self-play (train.rs:218-245): train-mode root noise, the current network as evaluator, finished slots restart at once
         with onb.Context(args.slots, seed=args.seed + it, mcts_max_sims=args.sims) as ctx:
             ev, net = evaluator_for(ctx)
             if net is None:   # the whole loop inside the library (onb_self_play)
                 data = ctx.self_play_native(2.0, args.sims, args.games, max_plies=args.max_plies, evaluator=ev, train=not gumbel,
-                                            noise_seed=args.seed + 1000 * it, reuse=args.reuse, gumbel=gumbel)
+                                            noise_seed=args.seed + 1000 * it, reuse=args.reuse, gumbel=gumbel, protocol=protocol or False)
             else:             # the same loop driven from Python, the PyTorch module between select and expand
                 data = onb.self_play_continuous(ctx, 2.0, args.sims, n_games=args.games, max_plies=args.max_plies, evaluator=ev, net=net,
-                                                train=not gumbel, noise_seed=args.seed + 1000 * it, gumbel=gumbel)
+                                                train=not gumbel, noise_seed=args.seed + 1000 * it, gumbel=gumbel, protocol=protocol)
+        if args.resign_fp is not None:
+            v = onb.resign_threshold(data["held_out"], args.resign_fp)
+            if np.isfinite(v):   # +inf: too few held-out games to bound the false positives; keep holding out every game
+                resign_below = v
         replay.add(data["planes"], data["pi"], data["z"])
         # ---- training (train.rs:264-339)
         model.train()
@@ -152,7 +172,9 @@ def main(argv=None):
                         value_loss=losses[-1][0], policy_loss=losses[-1][1], wins=results["random"]["wins"],
                         losses=results["random"]["losses"], draws=results["random"]["draws"], elo=results["random"]["elo"],
                         vs_mcts=results["mcts"], vs_alphabeta=results["alphabeta"],
-                        **({"gumbel_vs_puct": results["gumbel_vs_puct"]} if args.gumbel else {})))
+                        **({"gumbel_vs_puct": results["gumbel_vs_puct"]} if args.gumbel else {}),
+                        **({"resigned": data["resigned"], "held_out": int(data["held_out"]["result"].shape[0]), "resign_below": resign_below}
+                           if args.resign_fp is not None else {})))
         print(log[-1], flush=True)
     return log
 

@@ -102,6 +102,7 @@ typedef struct onb_state {
 #define ONB_BUF_VL_PLANES 10  /* float[n K'][21][5][5] written by onb_mcts_select */
 #define ONB_BUF_VL_POLICY 11  /* float[n K'][2][25]    read by onb_mcts_expand_backup */
 #define ONB_BUF_VL_VALUE 12   /* float[n K']           read by onb_mcts_expand_backup */
+#define ONB_BUF_ROOT_M 13     /* double[n]            written by onb_mcts_choose: max(v_root, q_best) */
 
 #define ONB_STAT_STEPS 0     /* transitions applied */
 #define ONB_STAT_RED_WINS 1
@@ -430,6 +431,50 @@ typedef struct onb_selfplay_result {
     int64_t* valid_idx; /* [n_valid] */
 } onb_selfplay_result;
 ONB_API int32_t onb_self_play(onb_ctx* ctx, const onb_selfplay_config* cfg, onb_selfplay_result* out);
+
+/* ---- AlphaZero's self-play move protocol: opening temperature and resignation (DESIGN.md §5j) -------------------------------
+ * A context setting read by every later onb_self_play; NULL or an all-zero struct switches it off, and with it off onb_self_play
+ * computes exactly what it computes without this call. Per searched tree of game slot s, with p = plies already played in the slot's
+ * current game, tick = the loop's ply, gen = the slot's generation, g = game_id_base + s, N(c) / W(c) = the root children's visits
+ * and reward sums in child order (pass children included), best = onb_mcts_finish's best child:
+ *   move: p >= temp_plies: best. p < temp_plies: w(c) = onb_exp(onb_log(N(c)) / temperature) for N(c) > 0, else 0; S = the sum of
+ *     w in child order; u = (r + 0.5) 2^-32 with r = onb_rand_u32(seed, g, tick, 0x20000); the move is the first child whose
+ *     inclusive running sum exceeds u S, else (rounding) the last child with N > 0, else (no visited child) best. All f64, IEEE basic
+ *     operations, no FMA contraction, the same onb_log / onb_exp on the CPU and the GPU. pi stays the visit distribution.
+ *   value: m = max(v_root, q_best) with v_root = -W_root / N_root (the root's value from the side to move's view; W_root is stored
+ *     from the other side's) and q_best = W(best) / N(best); m = v_root when N(best) = 0.
+ *   held out: onb_rand_u32(seed, g, gen, 0x20001) < floor(resign_holdout 2^32), compared as uint64 (h = 1 holds out every game).
+ *   resignation (resign = 1): a game that is not held out ends at the first search with m < resign_below (strict). That ply's sample
+ *     is recorded, no move is played, the side to move loses (z = -1 on its samples, +1 on the opponent's) and the slot restarts or
+ *     goes idle exactly as after a win. Held-out games play to their end.
+ * For every completed held-out game the run keeps (in the order the games end, slot order within a ply) its serial, its result (0 a
+ * draw at the ply cap, 1 Red, 2 Blue) and min m over Red's and over Blue's searches (+inf for a side that never searched).
+ * Checks: temperature finite and > 0 when temp_plies > 0, resign 0 or 1, resign_below finite and resign_holdout in [0, 1] when
+ * resign = 1; otherwise ONB_E_INVALID and the setting stays as it was. onb_self_play with temp_plies > 0 while the Gumbel root
+ * search is on: ONB_E_STATE (Gumbel plays its sequential-halving winner); resignation combines with every search. */
+typedef struct onb_selfplay_protocol {
+    uint32_t temp_plies; /* T: plies of a game that sample their move, 0 = off (AlphaGo Zero: 30) */
+    uint32_t resign;     /* 1: resignation on */
+    double temperature;  /* tau */
+    double resign_below; /* v_resign */
+    double resign_holdout; /* h: fraction of games that never resign */
+    uint64_t seed;
+} onb_selfplay_protocol;
+ONB_API int32_t onb_self_play_set_protocol(onb_ctx* ctx, const onb_selfplay_protocol* protocol);
+/* after an onb_self_play: games that ended by resignation, completed held-out games and their records (device pointers, valid until
+ * the next onb_self_play, like onb_selfplay_result). ONB_E_STATE before the first onb_self_play. */
+typedef struct onb_selfplay_protocol_stats {
+    int64_t resigned, held_out;
+    int64_t* serial;  /* [held_out] */
+    uint8_t* result;  /* [held_out] 0 draw, 1 Red, 2 Blue */
+    double* min_m;    /* [held_out][2] min m over Red's, Blue's searches */
+} onb_selfplay_protocol_stats;
+ONB_API int32_t onb_self_play_protocol_stats(onb_ctx* ctx, onb_selfplay_protocol_stats* out);
+/* the protocol's move and value for the trees of the last search, after its onb_mcts_finish: tree of game i samples its move at
+ * temperature `temperature` with r = onb_rand_u32(seed, game_id_base + i, step, 0x20000) when sample_mask_host[i] != 0 (NULL: no
+ * game samples) and plays best otherwise. The moves go to ONB_BUF_ACTIONS, m to ONB_BUF_ROOT_M (game order). Games no tree searched
+ * keep both. ONB_E_STATE without a finished search, ONB_E_INVALID for a temperature that is not finite and > 0. */
+ONB_API int32_t onb_mcts_choose(onb_ctx* ctx, uint64_t seed, uint32_t step, double temperature, const uint8_t* sample_mask_host);
 /* host copy of a borrowed device pointer (onb_buffer, onb_selfplay_result), ordered after the work queued on the context's stream */
 ONB_API int32_t onb_copy_to_host(onb_ctx* ctx, void* host, const void* device, int64_t bytes);
 

@@ -582,6 +582,14 @@ struct TrainConfig {  // the self-play fields of train.rs:100-154
     long max_plies = 150;
     std::optional<Deck> deck;
     uint64_t seed = 0;
+    // AlphaZero's self-play move protocol (onb_self_play_set_protocol, DESIGN.md §5j; self_play_continuous only, the project's own
+    // setting: the reference plays the best move and never resigns). The first temp_plies plies of a game sample their move in
+    // proportion to N^(1/temperature); with resign_below set, the side to move resigns when max(v_root, q_best) < *resign_below,
+    // except in a resign_holdout fraction of games. Draws are keyed by `seed`.
+    uint32_t temp_plies = 0;
+    double temperature = 1.0;
+    std::optional<double> resign_below;
+    double resign_holdout = 0.1;
 };
 /// All `self_play_game_amnt` games are played in lockstep on one engine (the reference plays them one after another on one
 /// thread); samples are returned game-major, ply-minor like the reference's play_buffer.
@@ -634,9 +642,19 @@ inline std::vector<SelfPlayData> self_play(const TrainingAlphaZeroMcts& mcts, co
 /// games remain to be started, and EVERY started game is played to its end: exactly max(config.self_play_game_amnt, slots) complete
 /// games come back (onb_self_play: the loop runs inside the library, the samples are copied to the host once at the end). Needs a
 /// device evaluator: mcts.device_evaluator = ONB_EVAL_NET after Engine::load_network, or ONB_EVAL_UNIFORM / ONB_EVAL_HASH. Samples
-/// come ply-major.
+/// come ply-major. The move protocol of config (temp_plies, temperature, resign_below, resign_holdout; all default: off) becomes the
+/// engine's setting: it replaces whatever protocol the caller set on e through onb_self_play_set_protocol and stays in force for
+/// later onb_self_play calls on e (the C ABI has no getter to restore an earlier setting from; TrainConfig is the source of truth).
 inline std::vector<SelfPlayData> self_play_continuous(Engine& e, const TrainingAlphaZeroMcts& mcts, const TrainConfig& config) {
     if (mcts.model) throw Error(ONB_E_INVALID, "self_play_continuous: a host evaluator cannot run inside the library; load the network instead");
+    onb_selfplay_protocol proto{};
+    proto.temp_plies = config.temp_plies;
+    proto.temperature = config.temperature;
+    proto.resign = config.resign_below ? 1u : 0u;
+    proto.resign_below = config.resign_below.value_or(0.0);
+    proto.resign_holdout = config.resign_holdout;
+    proto.seed = config.seed;
+    e.check(onb_self_play_set_protocol(e.ctx(), &proto));
     onb_selfplay_config cfg{};
     cfg.c_puct = mcts.config.exploration_c; cfg.sims = mcts.config.max_playouts; cfg.evaluator = mcts.device_evaluator;
     cfg.n_games = (int64_t)config.self_play_game_amnt; cfg.max_plies = (uint32_t)config.max_plies; cfg.train = mcts.config.train ? 1 : 0;

@@ -14,7 +14,7 @@ POLICY_UNIFORM, POLICY_AGENT = 0, 1
 OUT_MASKS, OUT_PLANES, OUT_ACTIONS = 1, 2, 4
 EVAL_UNIFORM, EVAL_HASH, EVAL_NET = 0, 1, 2
 (BUF_STATES, BUF_MASKS, BUF_PLANES, BUF_ACTIONS, BUF_LEAF_PLANES, BUF_POLICY, BUF_VALUE, BUF_PI, BUF_BEST,
- BUF_STATS, BUF_VL_PLANES, BUF_VL_POLICY, BUF_VL_VALUE) = range(13)
+ BUF_STATS, BUF_VL_PLANES, BUF_VL_POLICY, BUF_VL_VALUE, BUF_ROOT_M) = range(14)
 STAT_STEPS, STAT_RED_WINS, STAT_BLUE_WINS, STAT_PASSES, STAT_RESETS, STAT_BAD_ACTIONS, STAT_COUNT = 0, 1, 2, 3, 4, 5, 8
 HOST_MASKS, HOST_DONE, HOST_STATS = 1, 2, 4
 NET_F16, NET_TF32, NET_F32 = 0, 1, 2
@@ -96,6 +96,9 @@ SYMBOLS = {
     "onb_mcts_tree_info": (C.c_int32, [_P, _P, _P]),
     "onb_selftest": (C.c_int32, [_P, C.c_int32, _P]),
     "onb_self_play": (C.c_int32, [_P, _P, _P]),
+    "onb_self_play_set_protocol": (C.c_int32, [_P, _P]),
+    "onb_self_play_protocol_stats": (C.c_int32, [_P, _P]),
+    "onb_mcts_choose": (C.c_int32, [_P, C.c_uint64, C.c_uint32, C.c_double, _P]),
     "onb_copy_to_host": (C.c_int32, [_P, _P, _P, C.c_int64]),
     "onb_fight": (C.c_int32, [_P, _P, _P, _P, C.c_uint32, _P, _P]),
     "onb_fight_stats": (C.c_int32, [_P, C.c_double, C.c_double, _P, _P]),
@@ -129,6 +132,17 @@ SYMBOLS = {
 class SelfPlayConfig(C.Structure):
     _fields_ = [("c_puct", C.c_double), ("sims", C.c_uint32), ("evaluator", C.c_int32), ("n_games", C.c_int64), ("max_plies", C.c_uint32),
                 ("train", C.c_int32), ("noise_seed", C.c_uint64), ("sample_cap", C.c_int64)]
+
+
+class SelfPlayProtocol(C.Structure):
+    """onb_selfplay_protocol (onb_self_play_set_protocol)"""
+    _fields_ = [("temp_plies", C.c_uint32), ("resign", C.c_uint32), ("temperature", C.c_double), ("resign_below", C.c_double),
+                ("resign_holdout", C.c_double), ("seed", C.c_uint64)]
+
+
+class SelfPlayProtocolStats(C.Structure):
+    """onb_selfplay_protocol_stats (onb_self_play_protocol_stats)"""
+    _fields_ = [("resigned", C.c_int64), ("held_out", C.c_int64), ("serial", C.c_void_p), ("result", C.c_void_p), ("min_m", C.c_void_p)]
 
 
 AGENT_RANDOM, AGENT_PUCT, AGENT_UCT, AGENT_ALPHABETA, AGENT_GUMBEL, AGENT_TABLEBASE, AGENT_GUMBEL_MUZERO, AGENT_PUCT_VL = 0, 1, 2, 3, 4, 5, 6, 7

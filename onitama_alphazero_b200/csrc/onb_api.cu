@@ -132,6 +132,8 @@ int32_t onb_create(const onb_config* cfg, onb_ctx** out) {
         ONB_CREATE_CUDA(dalloc(&c->d_root_visits, n));
         ONB_CREATE_CUDA(dalloc(&c->d_root_q, n));
         ONB_CREATE_CUDA(dalloc(&c->d_child_visits, n * 40));
+        ONB_CREATE_CUDA(dalloc(&c->d_root_m, n));
+        ONB_CREATE_CUDA(dalloc(&c->d_choose_mask, n));
     }
     ONB_CREATE_CUDA(cudaStreamSynchronize(c->stream));
 #undef ONB_CREATE_CUDA
@@ -149,7 +151,7 @@ int32_t onb_destroy(onb_ctx* ctx) {
                     c->d_pi, c->d_best, c->d_root_visits, c->d_root_q, c->d_child_visits, c->net[0].w, c->net[0].bias, c->net[0].head, c->net[1].w,
                     c->net[1].bias, c->net[1].head, c->d_ln_table, c->d_ab_score, c->d_ab_nodes, c->d_gb,
                     c->d_gb_tab, c->d_gb_base, c->d_gb_p, c->d_gb_r0, c->d_gb_rx, c->d_tb_values, c->d_vl_cnt,
-                    c->d_vl_leaf_node, c->d_vl_leaf_state, c->d_vl_planes, c->d_vl_policy, c->d_vl_value};
+                    c->d_vl_leaf_node, c->d_vl_leaf_state, c->d_vl_planes, c->d_vl_policy, c->d_vl_value, c->d_root_m, c->d_choose_mask};
     reuse_free(c);
     tb_free(c);
     for (void* p : c->sp_buf)
@@ -197,9 +199,10 @@ int32_t onb_buffer(onb_ctx* ctx, int32_t which, void** dev_ptr, int64_t* bytes) 
         case ONB_BUF_VL_PLANES: p = c->d_vl_planes; b = n * c->vl_cap * 2100; break;
         case ONB_BUF_VL_POLICY: p = c->d_vl_policy; b = n * c->vl_cap * 200; break;
         case ONB_BUF_VL_VALUE: p = c->d_vl_value; b = n * c->vl_cap * 4; break;
+        case ONB_BUF_ROOT_M: p = c->d_root_m; b = n * 8; break;
         default: return fail(c, ONB_E_INVALID, "onb_buffer: unknown buffer %d", which);
     }
-    if (!p && which >= ONB_BUF_VL_PLANES)
+    if (!p && which >= ONB_BUF_VL_PLANES && which <= ONB_BUF_VL_VALUE)
         return fail(c, ONB_E_STATE, "onb_buffer: buffer %d exists after the first onb_mcts_set_virtual_loss with leaves >= 2", which);
     if (!p) return fail(c, ONB_E_STATE, "onb_buffer: buffer %d was not allocated by onb_create (see onb_config)", which);
     if (dev_ptr) *dev_ptr = p;
@@ -748,6 +751,7 @@ int32_t onb_mcts_expand_backup(onb_ctx* ctx) {
     ONB_CUDA(c, launch_mcts_expand_backup(c));
     ActiveSearch& a = c->search;
     a.phase = 1;
+    a.finished = false;
     if (a.plan.leaves >= 2) {
         a.sims_done += vl_descents(a.sims_done, a.plan.leaves, a.vl_target);
         c->vl_dirty = 0;
@@ -792,6 +796,7 @@ int32_t onb_mcts_run(onb_ctx* ctx, int32_t evaluator, uint32_t sims) {
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
     ActiveSearch& a = c->search;
     if (a.phase != 1) return fail(c, ONB_E_STATE, "onb_mcts_run: call onb_mcts_begin first");
+    a.finished = false;
     if (evaluator != ONB_EVAL_UNIFORM && evaluator != ONB_EVAL_HASH && evaluator != ONB_EVAL_NET)
         return fail(c, ONB_E_INVALID, "onb_mcts_run: unknown evaluator %d", evaluator);
     if (a.sims_done + sims > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_mcts_run: more simulations than mcts_max_sims");
@@ -875,6 +880,8 @@ int32_t onb_self_play(onb_ctx* ctx, const onb_selfplay_config* cfg, onb_selfplay
     if (cfg->train && c->gb_on) return fail(c, ONB_E_INVALID, "onb_self_play: train-mode noise does not combine with the Gumbel root search");
     if (c->reuse_on && c->gb_on) return fail(c, ONB_E_STATE, "onb_self_play: tree reuse does not combine with the Gumbel root search");
     if (c->vl_leaves >= 2) return fail(c, ONB_E_STATE, "onb_self_play: self-play searches without virtual loss; switch it off (onb_mcts_set_virtual_loss)");
+    if (c->sp_proto.temp_plies && c->gb_on)
+        return fail(c, ONB_E_STATE, "onb_self_play: the Gumbel root search plays its sequential-halving winner; the protocol's temp_plies must be 0");
     if (c->tb_search)
         return fail(c, ONB_E_STATE, "onb_self_play: self-play deals every game from the RNG and searches without tablebase leaves; switch them off "
                                     "(onb_mcts_set_tablebase)");
@@ -893,6 +900,41 @@ int32_t onb_self_play(onb_ctx* ctx, const onb_selfplay_config* cfg, onb_selfplay
     c->search.d_tree_game = nullptr;
     onb_mcts_set_noise(ctx, 0, 0.25, 0.03, 0);  // onb_self_play has always left train-mode noise off; its searches take noise from cfg
     if (rc != ONB_OK) return fail(c, rc, "%s", err);
+    return ONB_OK;
+}
+int32_t onb_self_play_set_protocol(onb_ctx* ctx, const onb_selfplay_protocol* protocol) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    onb_selfplay_protocol p;
+    memset(&p, 0, sizeof(p));
+    if (protocol) p = *protocol;
+    if ((p.temp_plies && !(std::isfinite(p.temperature) && p.temperature > 0.0)) || p.resign > 1 ||
+        (p.resign && !(std::isfinite(p.resign_below) && p.resign_holdout >= 0.0 && p.resign_holdout <= 1.0)))
+        return fail(c, ONB_E_INVALID, "onb_self_play_set_protocol: need a finite temperature > 0 with temp_plies > 0, resign 0 or 1, and with resign a "
+                                      "finite resign_below and 0 <= resign_holdout <= 1");
+    c->sp_proto = p;
+    return ONB_OK;
+}
+int32_t onb_self_play_protocol_stats(onb_ctx* ctx, onb_selfplay_protocol_stats* out) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (!out) return fail(c, ONB_E_INVALID, "onb_self_play_protocol_stats: null argument");
+    if (!c->sp_ran) return fail(c, ONB_E_STATE, "onb_self_play_protocol_stats: no onb_self_play has run on this context");
+    *out = c->sp_stats;
+    return ONB_OK;
+}
+int32_t onb_mcts_choose(onb_ctx* ctx, uint64_t seed, uint32_t step, double temperature, const uint8_t* sample_mask_host) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (!c->d_nodes || c->search.phase != 1 || !c->search.finished) return fail(c, ONB_E_STATE, "onb_mcts_choose: no search to choose from (onb_mcts_begin / _run / _finish)");
+    if (!(std::isfinite(temperature) && temperature > 0.0)) return fail(c, ONB_E_INVALID, "onb_mcts_choose: need a finite temperature > 0");
+    if (sample_mask_host)
+        ONB_CUDA(c, cudaMemcpyAsync(c->d_choose_mask, sample_mask_host, (size_t)c->n, cudaMemcpyHostToDevice, c->stream));
+    else
+        ONB_CUDA(c, cudaMemsetAsync(c->d_choose_mask, 0, (size_t)c->n, c->stream));
+    const bool slot_order = c->search.plan.reuse && c->search.plan.game_order;  // onb_mcts_finish left the tree-order best in d_ru_best
+    ONB_CUDA(c, launch_mcts_choose(c, slot_order ? c->d_ru_best : c->d_best, seed, step, temperature, c->d_choose_mask, nullptr, 0,
+                                   c->d_actions));
     return ONB_OK;
 }
 // one agent chooses for the m games in which it is to move (d_games) and leaves the actions in d_out[game]
@@ -1139,6 +1181,7 @@ int32_t onb_mcts_finish(onb_ctx* ctx, onb_action* best_host, float* pi_host, uin
     } else {
         ONB_CUDA(c, launch_mcts_finish(c, c->d_pi, c->d_best, c->d_root_visits, c->d_root_q, c->d_child_visits));
     }
+    c->search.finished = true;
     const size_t n = (size_t)c->n;
     bool any = false;
     if (best_host) { ONB_CUDA(c, cudaMemcpyAsync(best_host, c->d_best, n * 2, cudaMemcpyDeviceToHost, c->stream)); any = true; }

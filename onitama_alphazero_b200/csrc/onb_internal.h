@@ -87,6 +87,7 @@ struct ActiveSearch {
     // tree of the same index. A subset plan sets them, launch_reuse_begin fills them for a reuse begin.
     int64_t n_act;
     const int32_t* d_tree_game;
+    bool finished;       // onb_mcts_finish has run since the last simulation (onb_mcts_choose reads its best)
     uint32_t vl_target;  // with virtual loss: the descent count the current round is counted against (onb_mcts_run's end, or plan.sims)
 };
 
@@ -199,6 +200,12 @@ struct Ctx {
     int tb_search;            // the switch of onb_mcts_set_tablebase (tablebase leaves); tb_free switches it off
     uint32_t tb_serial;       // raised by every tb_free, so a search begun with an earlier table knows it is gone
     int16_t* d_tb_values;     // [n] onb_tb_probe's output, and ONB_AGENT_PUCT_TB's table moves (allocated on first use)
+    // self-play move protocol (onb_self_play_set_protocol, DESIGN.md §5j)
+    onb_selfplay_protocol sp_proto;  // all zero: off
+    double* d_root_m;         // [n] ONB_BUF_ROOT_M, written by k_mcts_choose
+    uint8_t* d_choose_mask;   // [n] onb_mcts_choose's sample mask
+    int sp_ran;               // an onb_self_play has run (its protocol stats are readable)
+    onb_selfplay_protocol_stats sp_stats;
     char err[512];
 };
 
@@ -228,6 +235,11 @@ cudaError_t launch_uct_run(Ctx* c, float exploration_c, uint32_t min_node_visits
 cudaError_t launch_mcts_finish(Ctx* c, float* pi, uint16_t* best, uint32_t* root_visits, double* root_q, uint32_t* child_visits);
 cudaError_t launch_mcts_play_best(Ctx* c, uint32_t out_flags);
 cudaError_t launch_mcts_scatter_best(Ctx* c, uint16_t* dst_actions);  // dst[game of tree t] = best[t]
+// the self-play protocol's move and m (include/onb.h onb_self_play_set_protocol) of every tree after launch_mcts_finish, into
+// dst_actions / d_root_m [game of tree t]. best: the finish's best in tree order. The tree of game i samples iff mask[i] != 0 (mask)
+// or plies[i] < temp_plies (plies); both nullptr: no tree samples.
+cudaError_t launch_mcts_choose(Ctx* c, const uint16_t* best, uint64_t seed, uint32_t step, double temperature, const uint8_t* mask,
+                               const int32_t* plies, uint32_t temp_plies, uint16_t* dst_actions);
 // the search launchers take their kernel from c->search.plan: noise, Gumbel at the root (select, run, finish) and Gumbel MuZero
 // below it (select, run, expand_backup), virtual loss (select, eval, expand_backup over the K rows of every tree, round target
 // search.vl_target), tablebase leaves (expand_backup)

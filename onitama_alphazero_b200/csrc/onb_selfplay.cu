@@ -8,6 +8,7 @@
 // slot). When a game ends, z = reward(final result, sample colour) (train.rs:83-85, alphazero_mcts/mod.rs:45-53; 0 for a game cut
 // at the ply cap) is written to the game's samples (the last `plies` samples of the slot: i, i - n, i - 2n, ...) and they become
 // valid; samples of games still running when the quota is reached stay invalid.
+#include <cmath>
 #include <cstring>
 #include <vector>
 
@@ -130,6 +131,98 @@ __global__ void __launch_bounds__(256) k_sp_finish(uint4* __restrict__ states, i
     }
 }
 
+// ---- the self-play move protocol (include/onb.h onb_self_play_set_protocol, DESIGN.md §5j) ------------------------------------------
+struct SpProto {       // per slot, for the game in progress
+    double mmin[2];    // min m over Red's / Blue's searches
+    uint32_t held;     // the game is held out: it never resigns
+    uint32_t resigned; // the game ended by resignation at this ply
+};
+__device__ __forceinline__ SpProto sp_fresh(uint64_t seed, uint64_t g, uint32_t gen, uint64_t held_below) {
+    SpProto p;
+    p.mmin[0] = p.mmin[1] = __longlong_as_double(0x7FF0000000000000ll);
+    p.held = (uint64_t)rand_from_key(game_key(seed, g), gen, 0x20001u) < held_below ? 1u : 0u;
+    p.resigned = 0;
+    return p;
+}
+__global__ void __launch_bounds__(256) k_sp_proto_init(SpProto* __restrict__ st, int64_t n, uint64_t seed, uint64_t game0, uint64_t held_below) {
+    const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (s < n) st[s] = sp_fresh(seed, game0 + (uint64_t)s, 0u, held_below);
+}
+// after the move choice, before the step: the side to move's minimum of m, and resignation (no move: ONB_ACTION_NONE; n_resigned
+// counts the run's resignations)
+__global__ void __launch_bounds__(256) k_sp_resign(SpProto* __restrict__ st, int64_t n, const uint8_t* __restrict__ idle, const uint8_t* __restrict__ color,
+                                                   const double* __restrict__ root_m, int32_t resign, double below, uint16_t* __restrict__ actions,
+                                                   unsigned long long* __restrict__ n_resigned) {
+    const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= n || idle[s]) return;
+    const double m = root_m[s];
+    const uint32_t side = color[s];
+    if (m < st[s].mmin[side]) st[s].mmin[side] = m;
+    if (resign && !st[s].held && m < below) {
+        st[s].resigned = 1;
+        actions[s] = 0xFFFFu;
+        atomicAdd(n_resigned, 1ull);
+    }
+}
+// k_sp_over with resignation: a resigned game is over too; held_over flags the over games that were held out
+__global__ void __launch_bounds__(256) k_sp_over_pr(const uint4* __restrict__ states, int64_t n, const uint8_t* __restrict__ idle, int32_t* __restrict__ plies,
+                                                    uint32_t max_plies, const SpProto* __restrict__ st, uint8_t* __restrict__ over,
+                                                    uint8_t* __restrict__ held_over) {
+    const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= n) return;
+    uint8_t o = 0;
+    if (!idle[s]) {
+        const int32_t p = plies[s] + 1;
+        plies[s] = p;
+        o = (st[s].resigned || unpack(states[s]).result != 0 || (uint32_t)p >= max_plies + 2u) ? 1 : 0;
+    }
+    over[s] = o;
+    held_over[s] = o && st[s].held;
+}
+// the result of slot s's finished game: the opponent of the side to move (color of this ply's sample) wins a resigned game
+__device__ __forceinline__ uint32_t sp_result(const SpProto& p, const Game& g, uint8_t mover) { return p.resigned ? (mover ^ 1u) + 1u : g.result; }
+// the held-out records of the finished games list[0 .. *m) (slot order), appended at record first + j
+__global__ void __launch_bounds__(256) k_sp_records(const int32_t* __restrict__ list, const unsigned long long* __restrict__ m, const uint4* __restrict__ states,
+                                                    int64_t n, const int32_t* __restrict__ generation, const SpProto* __restrict__ st,
+                                                    const uint8_t* __restrict__ color, int64_t first, int64_t* __restrict__ serial,
+                                                    uint8_t* __restrict__ result, double* __restrict__ min_m) {
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= (int64_t)*m) return;
+    const int64_t s = list[j], r = first + j;
+    serial[r] = s + n * (int64_t)generation[s];
+    result[r] = (uint8_t)sp_result(st[s], unpack(states[s]), color[s]);
+    min_m[2 * r] = st[s].mmin[0];
+    min_m[2 * r + 1] = st[s].mmin[1];
+}
+// k_sp_finish with resignation: the game's result from sp_result, and the restarted slot's protocol state for its next game
+__global__ void __launch_bounds__(256) k_sp_finish_pr(uint4* __restrict__ states, int64_t n, const int32_t* __restrict__ over_list,
+                                                      const unsigned long long* __restrict__ n_over, int32_t* __restrict__ generation,
+                                                      int32_t* __restrict__ plies, uint8_t* __restrict__ idle, uint8_t* __restrict__ live, int64_t base,
+                                                      const uint8_t* __restrict__ color, uint8_t* __restrict__ valid, float* __restrict__ z, int64_t started,
+                                                      int64_t target, int32_t fixed_cards, uint64_t seed, uint64_t game0, uint32_t epoch,
+                                                      SpProto* __restrict__ st, uint64_t proto_seed, uint64_t held_below) {
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= (int64_t)*n_over) return;
+    const int64_t s = over_list[j];
+    const uint32_t res = sp_result(st[s], unpack(states[s]), color[base + s]);
+    const int32_t p = plies[s];
+    for (int32_t k = 0; k < p; ++k) {
+        const int64_t i = base + s - (int64_t)k * n;
+        z[i] = res == 0 ? 0.f : ((res - 1u) == (uint32_t)color[i] ? 1.f : -1.f);
+        valid[i] = 1;
+    }
+    plies[s] = 0;
+    st[s].resigned = 0;
+    if (started + j < target) {
+        states[s] = pack(start_game(fixed_cards >= 0 ? (uint32_t)fixed_cards : deal_cards(game_key(seed, game0 + (uint64_t)s), epoch)));
+        generation[s] += 1;
+        st[s] = sp_fresh(proto_seed, game0 + (uint64_t)s, (uint32_t)generation[s], held_below);
+    } else {
+        idle[s] = 1;
+        live[s] = 0;
+    }
+}
+
 // arena: who moves where. fa[i] / fb[i] = game i is undecided and agent A / B is to move (A moves when the side to move is its colour)
 __global__ void __launch_bounds__(256) k_fight_plan(const uint4* __restrict__ states, int64_t n, const uint8_t* __restrict__ a_is_red,
                                                     uint8_t* __restrict__ fa, uint8_t* __restrict__ fb) {
@@ -207,9 +300,10 @@ cudaError_t grow(Ctx* c, int slot, size_t bytes, void** out) {
 enum : int {
     kSpPlanes = 0, kSpPi, kSpZ, kSpColor, kSpValid, kSpSerial, kSpGeneration, kSpPlies, kSpCounters, kSpValidIdx, kSpIdle, kSpLive, kSpOver,
     kSpLiveList, kSpOverList, kSpBlocks,
-    kFtMask = 16, kFtResults, kFtActA, kFtActB, kFtCounters, kFtFlagA, kFtFlagB, kFtListA, kFtListB, kFtBlocks, kFtElo, kFtHistory
+    kFtMask = 16, kFtResults, kFtActA, kFtActB, kFtCounters, kFtFlagA, kFtFlagB, kFtListA, kFtListB, kFtBlocks, kFtElo, kFtHistory,
+    kSpProto = 28, kSpHeldOver, kSpHeldList, kSpRecords  // onb_self_play with the move protocol
 };
-static_assert(kFtHistory < 32, "Ctx::sp_buf has 32 slots");
+static_assert(kSpRecords < 32, "Ctx::sp_buf has 32 slots");
 
 // Returns ONB_OK, or an ONB_E_* code with `err` filled. `search` runs one search (begin / run / finish) for ply `ply` over the m games
 // listed in d_games (device, ascending; nullptr = all games of the context).
@@ -227,7 +321,21 @@ int32_t run_self_play(Ctx* c, const onb_selfplay_config* cfg, onb_selfplay_resul
     int64_t *serial = nullptr, *idx = nullptr;
     int32_t *generation = nullptr, *plies = nullptr, *live_list = nullptr, *over_list = nullptr;
     uint32_t* blocks = nullptr;
-    unsigned long long* counters = nullptr;  // [0] games over in this ply, [1] live slots after it
+    unsigned long long* counters = nullptr;  // [0] games over in this ply, [1] live slots after it; protocol: [2] held-out games over in
+                                             // this ply, [3] resignations so far
+    // the move protocol: per-slot state, the held-out games over in this ply (flags, list) and the records (serial, min m, result)
+    const onb_selfplay_protocol& pr = c->sp_proto;
+    const bool proto = pr.temp_plies > 0 || pr.resign;
+    const uint64_t held_below = pr.resign ? (uint64_t)floor(pr.resign_holdout * 4294967296.0) : 0;
+    SpProto* st = nullptr;
+    uint8_t* held_over = nullptr;
+    int32_t* held_list = nullptr;
+    int64_t* rec_serial = nullptr;
+    double* rec_min = nullptr;
+    uint8_t* rec_result = nullptr;
+    int64_t n_rec = 0;
+    c->sp_ran = 1;
+    memset(&c->sp_stats, 0, sizeof(c->sp_stats));
     cudaError_t e;
 #define SP(call)                                                                       \
     do {                                                                               \
@@ -245,7 +353,7 @@ int32_t run_self_play(Ctx* c, const onb_selfplay_config* cfg, onb_selfplay_resul
     SP(grow(c, kSpSerial, cap * 8, (void**)&serial));
     SP(grow(c, kSpGeneration, (size_t)n * 4, (void**)&generation));
     SP(grow(c, kSpPlies, (size_t)n * 4, (void**)&plies));
-    SP(grow(c, kSpCounters, 16, (void**)&counters));
+    SP(grow(c, kSpCounters, 32, (void**)&counters));
     SP(grow(c, kSpIdle, (size_t)n, (void**)&idle));
     SP(grow(c, kSpLive, (size_t)n, (void**)&live));
     SP(grow(c, kSpOver, (size_t)n, (void**)&over));
@@ -264,6 +372,20 @@ int32_t run_self_play(Ctx* c, const onb_selfplay_config* cfg, onb_selfplay_resul
     // i.e. preferentially the long ones, and bias z / pi towards short games (the reference's workers each play their
     // self_play_game_amnt games to completion, train.rs:44-98).
     const int64_t target = cfg->n_games > n ? cfg->n_games : n;
+    if (proto) {
+        void* rec = nullptr;
+        SP(grow(c, kSpProto, (size_t)n * sizeof(SpProto), (void**)&st));
+        SP(grow(c, kSpHeldOver, (size_t)n, (void**)&held_over));
+        SP(grow(c, kSpHeldList, (size_t)n * 4, (void**)&held_list));
+        SP(grow(c, kSpRecords, (size_t)target * 25, &rec));  // every started game ends once: at most `target` records
+        rec_serial = (int64_t*)rec;
+        rec_min = (double*)((char*)rec + (size_t)target * 8);
+        rec_result = (uint8_t*)rec + (size_t)target * 24;
+        SP(cudaMemsetAsync(counters, 0, 32, c->stream));
+        k_sp_proto_init<<<grid, 256, 0, c->stream>>>(st, n, pr.seed, c->cfg.game_id_base, held_below);
+        SP(cudaGetLastError());
+    }
+    unsigned long long h[4] = {0, 0, 0, 0};
     int64_t started = n, finished = 0, n_live = n, tick = 0;
     int truncated = 0;
     while (n_live > 0) {
@@ -290,18 +412,37 @@ int32_t run_self_play(Ctx* c, const onb_selfplay_config* cfg, onb_selfplay_resul
             SP(cudaGetLastError());
         }
         SP(cudaMemsetAsync(c->d_actions, 0xFF, (size_t)n * 2, c->stream));   // ONB_ACTION_NONE: idle slots are not stepped
-        SP(launch_mcts_scatter_best(c, c->d_actions));
+        if (proto) {
+            SP(launch_mcts_choose(c, c->d_best, pr.seed, (uint32_t)tick, pr.temperature, nullptr, plies, pr.temp_plies, c->d_actions));
+            k_sp_resign<<<grid, 256, 0, c->stream>>>(st, n, idle, color + base, c->d_root_m, (int32_t)pr.resign, pr.resign_below, c->d_actions, counters + 3);
+            SP(cudaGetLastError());
+        } else {
+            SP(launch_mcts_scatter_best(c, c->d_actions));
+        }
         SP(launch_env_step(c, kModeActions, 0, 0, 0));
-        k_sp_over<<<grid, 256, 0, c->stream>>>(c->d_states, n, idle, plies, cfg->max_plies, over);
+        if (proto)
+            k_sp_over_pr<<<grid, 256, 0, c->stream>>>(c->d_states, n, idle, plies, cfg->max_plies, st, over, held_over);
+        else
+            k_sp_over<<<grid, 256, 0, c->stream>>>(c->d_states, n, idle, plies, cfg->max_plies, over);
         SP(cudaGetLastError());
         SP(compact(c, over, n, blocks, over_list, counters));
-        k_sp_finish<<<grid, 256, 0, c->stream>>>(c->d_states, n, over_list, counters, generation, plies, idle, live, base, color, valid, z, started, target,
-                                                 c->fixed_cards, c->cfg.seed, c->cfg.game_id_base, (uint32_t)(tick + 1));
+        if (proto) {
+            SP(compact(c, held_over, n, blocks, held_list, counters + 2));
+            k_sp_records<<<grid, 256, 0, c->stream>>>(held_list, counters + 2, c->d_states, n, generation, st, color + base, n_rec, rec_serial, rec_result,
+                                                      rec_min);
+            SP(cudaGetLastError());
+            k_sp_finish_pr<<<grid, 256, 0, c->stream>>>(c->d_states, n, over_list, counters, generation, plies, idle, live, base, color, valid, z, started,
+                                                        target, c->fixed_cards, c->cfg.seed, c->cfg.game_id_base, (uint32_t)(tick + 1), st, pr.seed,
+                                                        held_below);
+        } else {
+            k_sp_finish<<<grid, 256, 0, c->stream>>>(c->d_states, n, over_list, counters, generation, plies, idle, live, base, color, valid, z, started,
+                                                     target, c->fixed_cards, c->cfg.seed, c->cfg.game_id_base, (uint32_t)(tick + 1));
+        }
         SP(cudaGetLastError());
         SP(compact(c, live, n, blocks, live_list, counters + 1));
-        unsigned long long h[2] = {0, 0};
-        SP(cudaMemcpyAsync(h, counters, 16, cudaMemcpyDeviceToHost, c->stream));
+        SP(cudaMemcpyAsync(h, counters, proto ? 32 : 16, cudaMemcpyDeviceToHost, c->stream));
         SP(cudaStreamSynchronize(c->stream));
+        n_rec += (int64_t)h[2];
         finished += (int64_t)h[0];
         started += (int64_t)h[0] < target - started ? (int64_t)h[0] : target - started;
         n_live = (int64_t)h[1];
@@ -329,6 +470,13 @@ int32_t run_self_play(Ctx* c, const onb_selfplay_config* cfg, onb_selfplay_resul
     out->color = color;
     out->serial = serial;
     out->valid_idx = idx;
+    if (proto) {
+        c->sp_stats.resigned = (int64_t)h[3];
+        c->sp_stats.held_out = n_rec;
+        c->sp_stats.serial = rec_serial;
+        c->sp_stats.result = rec_result;
+        c->sp_stats.min_m = rec_min;
+    }
     c->search.phase = 0;
     return ONB_OK;
 }

@@ -93,7 +93,8 @@ class Context:
         spec = {L.BUF_MASKS: ((n, 2), "<u4", torch.int32), L.BUF_PLANES: ((n, 21, 5, 5), "<f4", None),
                 L.BUF_ACTIONS: ((n,), "<i2", None), L.BUF_LEAF_PLANES: ((n, 21, 5, 5), "<f4", None),
                 L.BUF_POLICY: ((n, 2, 25), "<f4", None), L.BUF_VALUE: ((n,), "<f4", None), L.BUF_PI: ((n, 2, 25), "<f4", None),
-                L.BUF_BEST: ((n,), "<i2", None), L.BUF_STATES: ((n, 4), "<i4", None), L.BUF_STATS: ((L.STAT_COUNT,), "<i8", None)}[which]
+                L.BUF_BEST: ((n,), "<i2", None), L.BUF_STATES: ((n, 4), "<i4", None), L.BUF_STATS: ((L.STAT_COUNT,), "<i8", None),
+                L.BUF_ROOT_M: ((n,), "<f8", None)}[which]
         shape, typestr, _ = spec
         if typestr == "<u4":
             typestr = "<i4"
@@ -287,6 +288,41 @@ class Context:
         if getattr(self, "gumbel", None) != want or "step0" in kw:
             self.set_gumbel(True, **kw)
 
+    def set_selfplay_protocol(self, protocol):
+        """onb_self_play_set_protocol: AlphaZero's self-play move protocol for the onb_self_play runs started afterwards. protocol: None /
+        False / {} switches it off, else a dict with the keys of selfplay_protocol() -- temp_plies (T: the first T plies of a game
+        sample their move in proportion to N^(1/temperature)), temperature, resign (the side to move resigns when max(v_root, q_best) <
+        resign_below), resign_below, resign_holdout (fraction of games that never resign and are recorded for calibration) and seed.
+        See include/onb.h and DESIGN.md §5j."""
+        p = selfplay_protocol(**protocol) if protocol else None
+        cfg = L.SelfPlayProtocol(p["temp_plies"], int(p["resign"]), p["temperature"], p["resign_below"], p["resign_holdout"], p["seed"]) if p else None
+        self._ck(self._lib.onb_self_play_set_protocol(self._h, C.byref(cfg) if p else None))
+        self.selfplay_protocol = p
+
+    def selfplay_protocol_stats(self):
+        """onb_self_play_protocol_stats after self_play_native: dict(resigned, held_out=dict(serial, result, min_m)) with torch copies of
+        the held-out records (result 0 draw, 1 Red, 2 Blue; min_m [G, 2] over Red's and Blue's searches)"""
+        import torch
+        st = L.SelfPlayProtocolStats()
+        self._ck(self._lib.onb_self_play_protocol_stats(self._h, C.byref(st)))
+        g, dev = int(st.held_out), "cuda:%d" % self.device
+        with torch.cuda.stream(self.torch_stream()):
+            if g == 0:
+                rec = dict(serial=torch.zeros(0, dtype=torch.int64, device=dev), result=torch.zeros(0, dtype=torch.uint8, device=dev),
+                           min_m=torch.zeros((0, 2), dtype=torch.float64, device=dev))
+            else:
+                rec = dict(serial=torch.as_tensor(_DevBuf(st.serial, (g,), "<i8"), device=dev).clone(),
+                           result=torch.as_tensor(_DevBuf(st.result, (g,), "|u1"), device=dev).clone(),
+                           min_m=torch.as_tensor(_DevBuf(st.min_m, (g, 2), "<f8"), device=dev).clone())
+        return dict(resigned=int(st.resigned), held_out=rec)
+
+    def mcts_choose(self, seed, step, temperature=1.0, sample_mask=None):
+        """onb_mcts_choose after mcts_finish: the self-play protocol's move of every searched game into BUF_ACTIONS and m = max(v_root,
+        q_best) into BUF_ROOT_M; games with sample_mask[i] != 0 sample at `temperature` (draw onb_rand_u32(seed, game_id_base + i,
+        step, 0x20000)), the others play best"""
+        m = None if sample_mask is None else np.ascontiguousarray(sample_mask, dtype=np.uint8).reshape(self.n)
+        self._ck(self._lib.onb_mcts_choose(self._h, int(seed), int(step), float(temperature), L.ptr(m)))
+
     def mcts_select(self):
         self._ck(self._lib.onb_mcts_select(self._h))
 
@@ -300,15 +336,19 @@ class Context:
         self._ck(self._lib.onb_mcts_run(self._h, evaluator, sims))
 
     def self_play_native(self, c_puct, sims, n_games, max_plies=150, evaluator=L.EVAL_UNIFORM, train=False, noise_seed=0, sample_cap=None,
-                         reuse=None, gumbel=None):
+                         reuse=None, gumbel=None, protocol=None):
         """onb_self_play: the whole self-play loop inside the library (search, recording, moves, z, restart of finished slots).
         Returns torch tensors of the completed games' samples (gathered from the context's device buffers) like
         selfplay.self_play_continuous. reuse: True / False sets the tree-reuse switch first (set_reuse), None leaves it. gumbel: as for
-        search_device (the Gumbel step of ply p is p; pi is then the improved policy)."""
+        search_device (the Gumbel step of ply p is p; pi is then the improved policy). protocol: None leaves the self-play protocol as
+        it is, False switches it off, a dict sets it (set_selfplay_protocol); with it on the result also has `resigned` and `held_out`
+        (selfplay_protocol_stats)."""
         import torch
         if reuse is not None:
             self.set_reuse(reuse)
         self._use_gumbel(gumbel)
+        if protocol is not None:
+            self.set_selfplay_protocol(protocol)
         if sample_cap is None:
             sample_cap = self.n * (max_plies + 2) * max(2, 2 * (n_games + self.n - 1) // self.n)
         cfg = L.SelfPlayConfig(c_puct, sims, evaluator, n_games, max_plies, int(bool(train)), noise_seed, sample_cap)
@@ -327,6 +367,8 @@ class Context:
                        z=view(res.z, (m,), "<f4", torch.float32)[idx], color=view(res.color, (m,), "|u1", torch.uint8)[idx].to(torch.int8),
                        serial=view(res.serial, (m,), "<i8", torch.int64)[idx], games=int(res.n_games), plies_run=int(res.plies_run),
                        truncated=bool(res.truncated))
+        if getattr(self, "selfplay_protocol", None):
+            out.update(self.selfplay_protocol_stats())
         return out
 
     @staticmethod
@@ -690,6 +732,12 @@ def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_g
 
 
 Context.search_device = _search_device
+
+
+def selfplay_protocol(temp_plies=0, temperature=1.0, resign=False, resign_below=-1.0, resign_holdout=0.1, seed=0):
+    """the self-play protocol setting (onb_selfplay_protocol) as a dict with every key; see Context.set_selfplay_protocol"""
+    return dict(temp_plies=int(temp_plies), temperature=float(temperature), resign=bool(resign), resign_below=float(resign_below),
+                resign_holdout=float(resign_holdout), seed=int(seed))
 
 
 def tb_index(cards, states):

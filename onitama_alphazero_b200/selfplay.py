@@ -108,7 +108,7 @@ def _self_play(ctx, c_puct, sims, max_plies, evaluator, net, decks):
 
 
 def self_play_continuous(ctx, c_puct, sims, n_games, max_plies=150, evaluator=L.EVAL_UNIFORM, net=None, train=False, noise_seed=0, reuse=False,
-                         gumbel=None):
+                         gumbel=None, protocol=None):
     """self_play for at least n_games games with every slot of the context kept busy: a slot whose game ends (or hits the ply cap)
     is re-dealt at once (onb_env_reset_games), the way a worker thread of the reference starts its next game as soon as one is over
     (train.rs:218-245 around :44-98). Lockstep self_play instead searches finished slots until the longest game ends -- with game
@@ -117,9 +117,18 @@ def self_play_continuous(ctx, c_puct, sims, n_games, max_plies=150, evaluator=L.
     reuse=True keeps the played child's subtree between plies (Context.set_reuse; device evaluators only), as
     onb_self_play does with the switch on; the switch is left as it was.
     gumbel=True or a dict of Context.set_gumbel keywords: the Gumbel root search with step = ply (set_gumbel(step0=0) at the start, one
-    search per ply), pi = its improved policy, as onb_self_play does with the switch on; the switch is left as it was."""
+    search per ply), pi = its improved policy, as onb_self_play does with the switch on; the switch is left as it was.
+    protocol: a dict of Context.set_selfplay_protocol keys -- the self-play move protocol as onb_self_play plays it with that setting
+    (DESIGN.md §5j): Context.mcts_choose picks the moves and m, resignation and the held-out records are restated here. The result then
+    also has `resigned`, `held_out` (dict(serial, result, min_m), as Context.selfplay_protocol_stats) and `m` (each sample's search's
+    max(v_root, q_best)). The context's own protocol
+    setting is not used and left as it was."""
     if reuse and net is not None:
         raise ValueError("self_play_continuous: reuse=True needs a device evaluator, not a torch net")
+    from .engine import selfplay_protocol
+    protocol = selfplay_protocol(**protocol) if protocol else None
+    if protocol and protocol["temp_plies"] and gumbel:
+        raise ValueError("self_play_continuous: the Gumbel root search plays its sequential-halving winner; temp_plies must be 0")
     was = getattr(ctx, "reuse", False)
     gb_was, step_was = getattr(ctx, "gumbel", None), getattr(ctx, "gumbel_step", 0)
     if reuse:
@@ -128,7 +137,7 @@ def self_play_continuous(ctx, c_puct, sims, n_games, max_plies=150, evaluator=L.
     if gumbel:
         ctx.set_gumbel(True, **dict(dict(gumbel) if isinstance(gumbel, dict) else {}, step0=0))
     try:
-        return _self_play_continuous(ctx, c_puct, sims, n_games, max_plies, evaluator, net, train, noise_seed, bool(reuse))
+        return _self_play_continuous(ctx, c_puct, sims, n_games, max_plies, evaluator, net, train, noise_seed, bool(reuse), protocol)
     finally:
         if getattr(ctx, "reuse", False) != was:
             ctx.set_reuse(was)
@@ -140,7 +149,13 @@ def self_play_continuous(ctx, c_puct, sims, n_games, max_plies=150, evaluator=L.
                 ctx.set_gumbel(True, m, c_visit, c_scale, scale, seed, step0=step_was, interior=len(gb_was) > 5)  # the setting and its step as they were
 
 
-def _self_play_continuous(ctx, c_puct, sims, n_games, max_plies, evaluator, net, train, noise_seed, reuse):
+def _held_out(ctx, protocol, slots, generation):
+    """onb_rand_u32(seed, g, gen, 0x20001) < floor(h 2^32) for the games (slot, generation): the held-out games never resign"""
+    lib, below = L.load(), int(np.floor(protocol["resign_holdout"] * 4294967296.0)) if protocol["resign"] else 0
+    return [lib.onb_rand_u32(protocol["seed"], ctx.game_id_base + s, g, 0x20001) < below for s, g in zip(slots, generation)]
+
+
+def _self_play_continuous(ctx, c_puct, sims, n_games, max_plies, evaluator, net, train, noise_seed, reuse, protocol):
     with torch.cuda.stream(ctx.torch_stream()):
         n = ctx.n
         dev = "cuda:%d" % ctx.device
@@ -160,27 +175,56 @@ def _self_play_continuous(ctx, c_puct, sims, n_games, max_plies, evaluator, net,
         idle = torch.zeros(n, dtype=torch.bool, device=dev)
         acts_t, best_t = ctx.tensor(L.BUF_ACTIONS), ctx.tensor(L.BUF_BEST)
         rec["live"] = []
+        if protocol:   # per slot: held out, min m over Red's / Blue's searches; the records of the completed held-out games
+            held = torch.tensor(_held_out(ctx, protocol, range(n), [0] * n), dtype=torch.bool, device=dev)
+            mmin = torch.full((n, 2), float("inf"), dtype=torch.float64, device=dev)
+            records = {"serial": [], "result": [], "min_m": []}
+            n_resigned = 0
+            m_t = ctx.tensor(L.BUF_ROOT_M)
+            rec["m"] = []
         while not bool(idle.all()):
             st = states_t.clone()
             ctx.encode(to_host=False)                       # create_tensor_from_state of the searched position (train.rs:58)
             ctx.search_device(c_puct, sims, evaluator=evaluator, net=net, reuse=reuse)   # (this driver searches idle slots too and ignores them)
+            side = ((st[:, 1] >> 30) & 1).long()
             rec["planes"].append(ctx.tensor(L.BUF_PLANES).clone())
             rec["pi"].append(ctx.tensor(L.BUF_PI).clone())
-            rec["color"].append(((st[:, 1] >> 30) & 1).to(torch.int8))
+            rec["color"].append(side.to(torch.int8))
             rec["serial"].append(slots + n * generation)
             rec["live"].append(~idle)
-            acts_t.copy_(best_t)
+            resigned = torch.zeros(n, dtype=torch.bool, device=dev)
+            if protocol:
+                t_plies = protocol["temp_plies"]
+                mask = ((~idle) & (plies < t_plies)).to(torch.uint8).cpu().numpy() if t_plies else None
+                ctx.mcts_choose(protocol["seed"], tick, protocol["temperature"] if t_plies else 1.0, mask)   # the move into ACTIONS, m
+                m = m_t.clone()
+                rec["m"].append(m)
+                live_ = ~idle
+                cur = mmin[slots, side]
+                mmin[slots, side] = torch.where(live_ & (m < cur), m, cur)
+                if protocol["resign"]:
+                    resigned = live_ & ~held & (m < protocol["resign_below"])
+                    n_resigned += int(resigned.sum())
+                    acts_t[resigned] = -1                    # a resigning side plays no move
+            else:
+                acts_t.copy_(best_t)
             acts_t[idle] = -1                                # ONB_ACTION_NONE: an idle slot (e.g. a game cut at the ply cap) is not stepped
             ctx.step(None)
             plies += (~idle).to(plies.dtype)
             result = (states_t.clone()[:, 2] >> 29) & 3
+            result = torch.where(resigned, (side ^ 1) + 1, result.long())   # the side to move resigned: the opponent wins
             # train.rs:74-79: the cap is checked after the move with max_plies counting down from 150 -> a game has at most max_plies + 2 plies
-            over = ~idle & ((result != 0) | (plies >= max_plies + 2))
+            over = ~idle & (resigned | (result != 0) | (plies >= max_plies + 2))
             if bool(over.any()):
                 idx = over.nonzero(as_tuple=True)[0]
                 ser = (idx + n * generation[idx]).tolist()
                 for s_, r_ in zip(ser, result[idx].tolist()):
                     winners[s_] = r_
+                if protocol:
+                    h = idx[held[idx]]
+                    records["serial"].append(h + n * generation[h])
+                    records["result"].append(result[h].to(torch.uint8))
+                    records["min_m"].append(mmin[h].clone())
                 done += len(ser)
                 k = min(len(ser), target - started)
                 again, stop = idx[:k], idx[k:]
@@ -190,6 +234,9 @@ def _self_play_continuous(ctx, c_puct, sims, n_games, max_plies, evaluator, net,
                     ctx.reset_games(mask.cpu().numpy(), epoch=tick + 1)
                     generation[again] += 1
                     started += k
+                    if protocol:
+                        held[again] = torch.tensor(_held_out(ctx, protocol, again.tolist(), generation[again].tolist()), dtype=torch.bool, device=dev)
+                        mmin[again] = float("inf")
                 idle[stop] = True
                 plies[idx] = 0
             tick += 1
@@ -206,7 +253,27 @@ def _self_play_continuous(ctx, c_puct, sims, n_games, max_plies, evaluator, net,
         r, color_k = r[keep], color[keep]
         z = torch.where(r == 0, 0.0, torch.where((r - 1) == color_k.to(r.dtype), 1.0, -1.0)).to(torch.float32)
         ctx.mcts_set_noise(False)
-        return dict(planes=planes[keep], pi=pi[keep], z=z, color=color_k, serial=serial[keep], games=done)
+        out = dict(planes=planes[keep], pi=pi[keep], z=z, color=color_k, serial=serial[keep], games=done)
+        if protocol:
+            out["m"] = torch.cat(rec["m"])[keep]   # the m of each sample's search
+            out["resigned"] = n_resigned
+            out["held_out"] = {k: (torch.cat(v) if v else torch.zeros((0, 2) if k == "min_m" else (0,), dtype=torch.float64 if k == "min_m" else
+                                                                        (torch.int64 if k == "serial" else torch.uint8), device=dev))
+                               for k, v in records.items()}
+        return out
+
+
+def resign_threshold(records, fp=0.05):
+    """AlphaGo Zero's resignation threshold from the held-out games of a self-play run (records: the `held_out` dict of self_play_native /
+    self_play_continuous, or any dict with `result` [G] (0 draw, 1 Red, 2 Blue) and `min_m` [G, 2]). A held-out game would have been a
+    false positive at v if a side that did not lose (the winner, either side of a draw) has min m < v. Returns the (floor(fp G) + 1)-th
+    smallest such non-loser minimum (+inf when there are fewer): resigning below it, at most floor(fp G) of the G held-out games would
+    have been false positives."""
+    result = np.asarray(records["result"].cpu() if hasattr(records["result"], "cpu") else records["result"]).astype(np.int64).reshape(-1)
+    min_m = np.asarray(records["min_m"].cpu() if hasattr(records["min_m"], "cpu") else records["min_m"], dtype=np.float64).reshape(-1, 2)
+    k = int(np.floor(fp * len(result)))
+    vals = np.sort(np.concatenate([min_m[result != 2, 0], min_m[result != 1, 1]]))   # Red did not lose, Blue did not lose
+    return float(vals[k]) if k < len(vals) else float("inf")
 
 
 def fight(ctx, move_fn_a, move_fn_b, a_is_red, max_plies=150):

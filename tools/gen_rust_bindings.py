@@ -11,7 +11,8 @@ TMAP = {'int32_t': 'i32', 'uint32_t': 'u32', 'int64_t': 'i64', 'uint64_t': 'u64'
         'onb_state': 'onb_state', 'onb_tree_dump': 'onb_tree_dump', 'onb_selfplay_config': 'onb_selfplay_config',
         'onb_selfplay_result': 'onb_selfplay_result', 'onb_agent': 'onb_agent', 'onb_fight_result': 'onb_fight_result',
         'onb_actor': 'onb_actor', 'onb_actor_view': 'onb_actor_view', 'onb_fight_statistics': 'onb_fight_statistics', 'onb_comm': 'onb_comm', 'onb_replay': 'onb_replay',
-        'onb_gumbel_config': 'onb_gumbel_config', 'int16_t': 'i16', 'onb_tb_class': 'onb_tb_class'}
+        'onb_gumbel_config': 'onb_gumbel_config', 'int16_t': 'i16', 'onb_tb_class': 'onb_tb_class',
+        'onb_selfplay_protocol': 'onb_selfplay_protocol', 'onb_selfplay_protocol_stats': 'onb_selfplay_protocol_stats'}
 I32_PREFIXES = ('ONB_E_', 'ONB_BUF', 'ONB_STAT', 'ONB_RESULT', 'ONB_POLICY', 'ONB_EVAL', 'ONB_AGENT', 'ONB_NET_', 'ONB_SELFTEST', 'ONB_ALPHABETA', 'ONB_TB_MAX')
 I32_NAMES = ('ONB_VERSION', 'ONB_OK', 'ONB_RED', 'ONB_BLUE', 'ONB_PAWN', 'ONB_KING')
 STRUCTS = '''#[repr(C)]
@@ -93,6 +94,26 @@ pub struct onb_gumbel_config {
     pub seed: u64,
     pub step0: u32,
     pub interior: u32,
+}
+
+#[repr(C)]
+#[derive(Clone, Copy, Default, Debug)]
+pub struct onb_selfplay_protocol {
+    pub temp_plies: u32,
+    pub resign: u32,
+    pub temperature: f64,
+    pub resign_below: f64,
+    pub resign_holdout: f64,
+    pub seed: u64,
+}
+
+#[repr(C)]
+pub struct onb_selfplay_protocol_stats {
+    pub resigned: i64,
+    pub held_out: i64,
+    pub serial: *mut i64,
+    pub result: *mut u8,
+    pub min_m: *mut f64,
 }
 
 #[repr(C)]
