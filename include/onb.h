@@ -103,6 +103,7 @@ typedef struct onb_state {
 #define ONB_BUF_VL_POLICY 11  /* float[n K'][2][25]    read by onb_mcts_expand_backup */
 #define ONB_BUF_VL_VALUE 12   /* float[n K']           read by onb_mcts_expand_backup */
 #define ONB_BUF_ROOT_M 13     /* double[n]            written by onb_mcts_choose: max(v_root, q_best) */
+#define ONB_BUF_ROOT_PROOF 14 /* int8[n]              written by onb_mcts_finish of a solver search (onb_mcts_set_solver) */
 
 #define ONB_STAT_STEPS 0     /* transitions applied */
 #define ONB_STAT_RED_WINS 1
@@ -389,7 +390,7 @@ typedef struct onb_tree_dump { /* host arrays of length cap */
     int32_t* parent;
     uint32_t* first_child;
     uint32_t* n_child;
-    uint8_t* flags; /* bit0 expanded, bit1 terminal, bit2 pass child */
+    uint8_t* flags; /* bit0 expanded, bit1 terminal, bit2 pass child, ONB_NODE_WIN, ONB_NODE_LOSS (onb_mcts_set_solver) */
 } onb_tree_dump;
 /* copies tree `tree` (arena order == reference arena order); *n_nodes receives the node count */
 ONB_API int32_t onb_mcts_dump_tree(onb_ctx* ctx, int64_t tree, int64_t cap, onb_tree_dump* out, int64_t* n_nodes);
@@ -687,6 +688,39 @@ ONB_API int32_t onb_mcts_set_tablebase(onb_ctx* ctx, int32_t enabled);
  * onb_tb_best's move, in every other game it plays an eval-mode PUCT search with tablebase leaves (so games of another card set get
  * plain PUCT). It needs a resident table (ONB_E_STATE otherwise); unlike ONB_AGENT_TABLEBASE, games need not start in the table. */
 #define ONB_AGENT_PUCT_TB 8
+
+/* MCTS solver (DESIGN.md §5k; Winands, Bjornsson & Saito 2008): the PUCT search proves wins and losses and propagates the proofs to the
+ * root. Off by default; enabled = 0 switches it off, and every entry point then computes what it computes without this call. enabled
+ * != 0 switches it on for the searches begun afterwards and allocates ONB_BUF_ROOT_PROOF (reading that buffer before the first enabling
+ * call gives ONB_E_STATE). A search begun with the switch on computes, exact to the bit:
+ *   Flags (onb_tree_dump.flags): ONB_NODE_WIN = the side that moved into the node wins with best play, ONB_NODE_LOSS = it loses. A node
+ *     never carries both; "proven" = either. The root follows the same convention: a root proven LOSS means its side to move wins.
+ *   Sources of proof: (1) a child that a descent finds terminal gets TERMINAL | WIN (in Onitama a move only ends the game in the
+ *     mover's favour); (2) at every successful expansion each child whose action captures on the enemy king's square, or moves the own
+ *     king onto the enemy temple, is born TERMINAL | WIN; (3) with tablebase leaves (onb_mcts_set_tablebase) a table leaf below the
+ *     root of value v gets LOSS if v > 0, WIN if v < 0, and no proof if v = 0 (draws are not proven).
+ *   Propagation: after each descent's expansion and backup, from the deepest node that became proven up the descent's path: the parent
+ *     of a node proven WIN becomes LOSS; the parent of a node proven LOSS becomes WIN if every child of it (pass pseudo-children
+ *     included) is LOSS; it stops at the first level that does not change, or at the root.
+ *   Selection: a descent stops at a proven node (the root included: once the root is proven every later descent ends there). At an
+ *     unproven expanded node the PUCT argmax (last maximal child) skips children flagged LOSS; such a node has no WIN child and not
+ *     every child is LOSS, so the choice is always defined.
+ *   Reward: a descent that ends at a proven node, or whose expansion proves its leaf, backs up the reward of a decided leaf whose
+ *     winner is the proven winner (the side that moved into the leaf for WIN, the side to move at it for LOSS) in place of the
+ *     evaluator's value; N and W are otherwise backed up as without the switch.
+ *   onb_mcts_finish / onb_mcts_play_best: best = the first terminal WIN root child in child order, else the WIN child with the most
+ *     visits (last maximal); without WIN children the visit rule over the children without LOSS; if every child is LOSS, the visit
+ *     rule over all. pi stays the visit distribution. ONB_BUF_ROOT_PROOF [game] = +1 (the side to move at the root wins: root LOSS),
+ *     -1 (it loses: root WIN) or 0.
+ * onb_mcts_run with ONB_EVAL_UNIFORM / ONB_EVAL_HASH runs a fused solver kernel (split rounds with tablebase leaves, as §5i), with
+ * ONB_EVAL_NET the split phase's solver kernels. Refused with ONB_E_STATE: a begin with the switch on together with train-mode noise,
+ * the Gumbel root search, virtual loss or tree reuse; onb_uct_run after such a begin; onb_self_play while the switch is on.
+ * onb_fight searches with the solver only for ONB_AGENT_PUCT_SOLVER agents, whatever the switch says, and leaves it as it found it. */
+#define ONB_NODE_WIN 8
+#define ONB_NODE_LOSS 16
+ONB_API int32_t onb_mcts_set_solver(onb_ctx* ctx, int32_t enabled);
+/* ONB_AGENT_PUCT_SOLVER: as ONB_AGENT_PUCT (the same fields), searching with the solver and playing the solver's best move. */
+#define ONB_AGENT_PUCT_SOLVER 9
 
 /* ---- policy/value network on the device ---------------------------------------------------------------------
  * ConvResNet::forward (alphazero-training/src/net.rs:215-232) for every position of a plane buffer, as one fused

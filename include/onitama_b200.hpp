@@ -149,6 +149,7 @@ public:
     onb_gumbel_config gumbel_applied{};       ///< the Gumbel setting last passed to onb_mcts_set_gumbel (enabled = 0: off)
     std::pair<uint32_t, double> vl_applied{1, 1.0};  ///< (leaves, virtual_loss) last passed to onb_mcts_set_virtual_loss (leaves 1: off)
     bool tb_applied = false;                  ///< the tablebase-leaf switch last passed to onb_mcts_set_tablebase
+    bool solver_applied = false;              ///< the MCTS-solver switch last passed to onb_mcts_set_solver
     int32_t tb_max_pawns = -1;                ///< the table resident on this engine (solve_tablebase): max_pawns, -1 none
     std::array<uint8_t, 5> tb_cards{};        ///< ... and its card set as given
     /// onb_tb_solve on this engine's context: the table of one five-card set with at most max_pawns pawns, which tablebase leaves
@@ -449,6 +450,10 @@ struct AlphaZeroMctsConfig {  // alphazero_mcts/mod.rs:26-43
     bool tablebase_leaves = false;
     std::array<uint8_t, 5> tablebase_cards{};
     int32_t tablebase_max_pawns = 3;
+    // the MCTS solver (onb_mcts_set_solver, DESIGN.md §5k): every search proves wins and losses, propagates them to the root and
+    // plays a proven win (the first terminal winning child, else the most visited proven win, else the visit rule over the children
+    // not proven lost). Applied when it changes. Does not combine with train, reuse, gumbel or leaves_per_round >= 2 (ONB_E_STATE).
+    bool solver = false;
 };
 inline double reward(MoveResult r, PlayerColor c) {  // alphazero_mcts/mod.rs:45-53
     if (c == PlayerColor::Red) return r == MoveResult::RedWin ? 1. : r == MoveResult::BlueWin ? -1. : 0.;
@@ -483,6 +488,10 @@ inline void run_search(Engine& e, const AlphaZeroMctsConfig& cfg, int32_t device
     if (cfg.tablebase_leaves != e.tb_applied) {
         e.check(onb_mcts_set_tablebase(e.ctx(), cfg.tablebase_leaves ? 1 : 0));
         e.tb_applied = cfg.tablebase_leaves;
+    }
+    if (cfg.solver != e.solver_applied) {
+        e.check(onb_mcts_set_solver(e.ctx(), cfg.solver ? 1 : 0));
+        e.solver_applied = cfg.solver;
     }
     e.check(onb_mcts_begin(e.ctx(), cfg.exploration_c, cfg.max_playouts));
     if (!net) {
@@ -762,6 +771,17 @@ inline FightStatistics fight(const EvaluatorConfig& config, std::unique_ptr<Agen
 inline onb_agent puct_tablebase_agent(uint32_t sims, double c_puct = 2.0, int32_t evaluator = ONB_EVAL_UNIFORM, int32_t net_slot = 0) {
     onb_agent a{};
     a.kind = ONB_AGENT_PUCT_TB;
+    a.evaluator = evaluator;
+    a.net_slot = net_slot;
+    a.sims = sims;
+    a.c = c_puct;
+    return a;
+}
+/// ONB_AGENT_PUCT_SOLVER: PUCT with the MCTS solver (DESIGN.md §5k), playing the solver's best move. onb_fight searches with the
+/// solver for this agent only and leaves the engine's switch (AlphaZeroMctsConfig::solver) as it found it.
+inline onb_agent puct_solver_agent(uint32_t sims, double c_puct = 2.0, int32_t evaluator = ONB_EVAL_UNIFORM, int32_t net_slot = 0) {
+    onb_agent a{};
+    a.kind = ONB_AGENT_PUCT_SOLVER;
     a.evaluator = evaluator;
     a.net_slot = net_slot;
     a.sims = sims;

@@ -6,7 +6,7 @@ from . import _lib
 from ._lib import (ACTION_NONE, BUF_ACTIONS, BUF_BEST, BUF_LEAF_PLANES, BUF_MASKS, BUF_PI, BUF_PLANES, BUF_POLICY, BUF_STATES,
                    BUF_STATS, BUF_VALUE, EVAL_HASH, EVAL_NET, EVAL_UNIFORM, OUT_ACTIONS, OUT_MASKS, OUT_PLANES, POLICY_AGENT, POLICY_UNIFORM,
                    STAT_BLUE_WINS, STAT_PASSES, STAT_RED_WINS, STAT_RESETS, STAT_STEPS, STATE_DTYPE, TB_NONE, BUF_VL_PLANES, BUF_VL_POLICY,
-                   BUF_VL_VALUE, BUF_ROOT_M, OnbError)
+                   BUF_VL_VALUE, BUF_ROOT_M, BUF_ROOT_PROOF, NODE_LOSS, NODE_WIN, OnbError)
 from .engine import Context, selfplay_protocol, start_states, tb_index, tb_states
 from .selfplay import (EloRating, FightStatistics, NativeReplayBuffer, ReplayBuffer, fight, fight_statistics, resign_threshold, self_play,
                        self_play_continuous)

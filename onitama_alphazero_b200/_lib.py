@@ -14,7 +14,8 @@ POLICY_UNIFORM, POLICY_AGENT = 0, 1
 OUT_MASKS, OUT_PLANES, OUT_ACTIONS = 1, 2, 4
 EVAL_UNIFORM, EVAL_HASH, EVAL_NET = 0, 1, 2
 (BUF_STATES, BUF_MASKS, BUF_PLANES, BUF_ACTIONS, BUF_LEAF_PLANES, BUF_POLICY, BUF_VALUE, BUF_PI, BUF_BEST,
- BUF_STATS, BUF_VL_PLANES, BUF_VL_POLICY, BUF_VL_VALUE, BUF_ROOT_M) = range(14)
+ BUF_STATS, BUF_VL_PLANES, BUF_VL_POLICY, BUF_VL_VALUE, BUF_ROOT_M, BUF_ROOT_PROOF) = range(15)
+NODE_WIN, NODE_LOSS = 8, 16  # tree-dump flags of the MCTS solver (onb_mcts_set_solver)
 STAT_STEPS, STAT_RED_WINS, STAT_BLUE_WINS, STAT_PASSES, STAT_RESETS, STAT_BAD_ACTIONS, STAT_COUNT = 0, 1, 2, 3, 4, 5, 8
 HOST_MASKS, HOST_DONE, HOST_STATS = 1, 2, 4
 NET_F16, NET_TF32, NET_F32 = 0, 1, 2
@@ -86,6 +87,7 @@ SYMBOLS = {
     "onb_mcts_set_gumbel": (C.c_int32, [_P, _P]),
     "onb_mcts_set_virtual_loss": (C.c_int32, [_P, C.c_uint32, C.c_double]),
     "onb_mcts_set_tablebase": (C.c_int32, [_P, C.c_int32]),
+    "onb_mcts_set_solver": (C.c_int32, [_P, C.c_int32]),
     "onb_mcts_select": (C.c_int32, [_P]),
     "onb_mcts_expand_backup": (C.c_int32, [_P]),
     "onb_mcts_eval": (C.c_int32, [_P, C.c_int32]),
@@ -147,6 +149,7 @@ class SelfPlayProtocolStats(C.Structure):
 
 AGENT_RANDOM, AGENT_PUCT, AGENT_UCT, AGENT_ALPHABETA, AGENT_GUMBEL, AGENT_TABLEBASE, AGENT_GUMBEL_MUZERO, AGENT_PUCT_VL = 0, 1, 2, 3, 4, 5, 6, 7
 AGENT_PUCT_TB = 8
+AGENT_PUCT_SOLVER = 9
 ALPHABETA_MAX_DEPTH = 8
 ALPHABETA_WIN = 1000000
 TB_MAX_PAWNS = 4

@@ -151,7 +151,7 @@ int32_t onb_destroy(onb_ctx* ctx) {
                     c->d_pi, c->d_best, c->d_root_visits, c->d_root_q, c->d_child_visits, c->net[0].w, c->net[0].bias, c->net[0].head, c->net[1].w,
                     c->net[1].bias, c->net[1].head, c->d_ln_table, c->d_ab_score, c->d_ab_nodes, c->d_gb,
                     c->d_gb_tab, c->d_gb_base, c->d_gb_p, c->d_gb_r0, c->d_gb_rx, c->d_tb_values, c->d_vl_cnt,
-                    c->d_vl_leaf_node, c->d_vl_leaf_state, c->d_vl_planes, c->d_vl_policy, c->d_vl_value, c->d_root_m, c->d_choose_mask};
+                    c->d_vl_leaf_node, c->d_vl_leaf_state, c->d_vl_planes, c->d_vl_policy, c->d_vl_value, c->d_root_m, c->d_choose_mask, c->d_root_proof};
     reuse_free(c);
     tb_free(c);
     for (void* p : c->sp_buf)
@@ -200,10 +200,12 @@ int32_t onb_buffer(onb_ctx* ctx, int32_t which, void** dev_ptr, int64_t* bytes) 
         case ONB_BUF_VL_POLICY: p = c->d_vl_policy; b = n * c->vl_cap * 200; break;
         case ONB_BUF_VL_VALUE: p = c->d_vl_value; b = n * c->vl_cap * 4; break;
         case ONB_BUF_ROOT_M: p = c->d_root_m; b = n * 8; break;
+        case ONB_BUF_ROOT_PROOF: p = c->d_root_proof; b = n; break;
         default: return fail(c, ONB_E_INVALID, "onb_buffer: unknown buffer %d", which);
     }
     if (!p && which >= ONB_BUF_VL_PLANES && which <= ONB_BUF_VL_VALUE)
         return fail(c, ONB_E_STATE, "onb_buffer: buffer %d exists after the first onb_mcts_set_virtual_loss with leaves >= 2", which);
+    if (!p && which == ONB_BUF_ROOT_PROOF) return fail(c, ONB_E_STATE, "onb_buffer: buffer %d exists after the first onb_mcts_set_solver with enabled != 0", which);
     if (!p) return fail(c, ONB_E_STATE, "onb_buffer: buffer %d was not allocated by onb_create (see onb_config)", which);
     if (dev_ptr) *dev_ptr = p;
     if (bytes) *bytes = b;
@@ -477,6 +479,11 @@ static int32_t begin_search(Ctx* c, const SearchPlan& p, const char* who) {
     // tablebase leaves (include/onb.h, onb_mcts_set_tablebase): the resident table, copied into the plan
     if (p.tb && p.reuse) return fail(c, ONB_E_STATE, "%s: tablebase leaves (onb_mcts_set_tablebase) do not combine with tree reuse", who);
     if (p.tb && !c->tb_live) return fail(c, ONB_E_STATE, "%s: tablebase leaves need a resident table (onb_tb_solve)", who);
+    // the combinations the MCTS solver does not support (include/onb.h, onb_mcts_set_solver)
+    if (p.solver && (p.noise || p.gumbel || p.leaves >= 2 || p.reuse))
+        return fail(c, ONB_E_STATE, "%s: the MCTS solver (onb_mcts_set_solver) does not combine with %s", who,
+                    p.noise ? "train-mode noise" : p.gumbel ? "the Gumbel root search" : p.leaves >= 2 ? "virtual loss" : "tree reuse");
+    if (p.solver && !c->d_root_proof) return fail(c, ONB_E_STATE, "%s: the solver's buffers are not allocated (onb_mcts_set_solver)", who);
     if (c->vl_dirty) {  // a select with virtual loss whose round was never backed up left counts behind
         ONB_CUDA(c, cudaMemsetAsync(c->d_vl_cnt, 0, (size_t)c->n * c->node_cap, c->stream));
         c->vl_dirty = 0;
@@ -624,6 +631,31 @@ int32_t onb_mcts_set_tablebase(onb_ctx* ctx, int32_t enabled) {
     c->tb_search = enabled ? 1 : 0;
     return ONB_OK;
 }
+// the solver's root-proof buffer, allocated (and zeroed) by the first call: onb_mcts_set_solver and onb_fight's solver agents
+static int32_t solver_alloc(Ctx* c) {
+    if (c->d_root_proof) return ONB_OK;
+    cudaError_t e = dalloc(&c->d_root_proof, (size_t)c->n);
+    if (e == cudaSuccess) e = cudaMemsetAsync(c->d_root_proof, 0, (size_t)c->n, c->stream);
+    if (e != cudaSuccess) {
+        if (c->d_root_proof) cudaFree(c->d_root_proof);
+        c->d_root_proof = nullptr;
+        return e == cudaErrorMemoryAllocation ? fail(c, ONB_E_NOMEM, "onb_mcts_set_solver: out of device memory") : cuda_fail(c, e, "onb_mcts_set_solver");
+    }
+    return ONB_OK;
+}
+int32_t onb_mcts_set_solver(onb_ctx* ctx, int32_t enabled) {
+    ONB_CHECK_CTX(ctx);
+    Ctx* c = reinterpret_cast<Ctx*>(ctx);
+    if (!enabled) {
+        c->solver_on = 0;
+        return ONB_OK;
+    }
+    if (!c->d_nodes) return fail(c, ONB_E_STATE, "onb_mcts_set_solver: context created with mcts_max_sims = 0");
+    const int32_t rc = solver_alloc(c);
+    if (rc != ONB_OK) return rc;
+    c->solver_on = 1;
+    return ONB_OK;
+}
 int32_t onb_mcts_begin(onb_ctx* ctx, double c_puct, uint32_t sims) {
     ONB_CHECK_CTX(ctx);
     Ctx* c = reinterpret_cast<Ctx*>(ctx);
@@ -641,6 +673,7 @@ int32_t onb_mcts_begin(onb_ctx* ctx, double c_puct, uint32_t sims) {
     p.leaves = c->vl_leaves;
     p.vloss = c->vl_loss;
     p.tb = c->tb_search != 0;
+    p.solver = c->solver_on != 0;
     const int32_t rc = begin_search(c, p, "onb_mcts_begin");
     if (rc == ONB_OK && p.gumbel) c->gb_serial += 1;
     return rc;
@@ -882,6 +915,8 @@ int32_t onb_self_play(onb_ctx* ctx, const onb_selfplay_config* cfg, onb_selfplay
     if (c->vl_leaves >= 2) return fail(c, ONB_E_STATE, "onb_self_play: self-play searches without virtual loss; switch it off (onb_mcts_set_virtual_loss)");
     if (c->sp_proto.temp_plies && c->gb_on)
         return fail(c, ONB_E_STATE, "onb_self_play: the Gumbel root search plays its sequential-halving winner; the protocol's temp_plies must be 0");
+    if (c->solver_on)
+        return fail(c, ONB_E_STATE, "onb_self_play: self-play searches without the MCTS solver; switch it off (onb_mcts_set_solver)");
     if (c->tb_search)
         return fail(c, ONB_E_STATE, "onb_self_play: self-play deals every game from the RNG and searches without tablebase leaves; switch them off "
                                     "(onb_mcts_set_tablebase)");
@@ -978,9 +1013,10 @@ static int32_t fight_move(Ctx* c, const onb_agent* ag, uint32_t ply, const int32
         p.vloss = 1.0;
     }
     p.tb = tb;  // PUCT with tablebase leaves; the table's move replaces the search's in the games of the table (below)
+    p.solver = ag->kind == ONB_AGENT_PUCT_SOLVER;  // PUCT with the solver, playing its best move
     int32_t rc = begin_search(c, p, "search");
     if (rc != ONB_OK) return rc;
-    if (ag->kind == ONB_AGENT_PUCT || ag->kind == ONB_AGENT_PUCT_VL || tb || p.gumbel) {
+    if (ag->kind == ONB_AGENT_PUCT || ag->kind == ONB_AGENT_PUCT_VL || tb || p.gumbel || p.solver) {
         if (ag->evaluator == ONB_EVAL_NET && (rc = onb_net_select(x, ag->net_slot)) != ONB_OK) return rc;
         rc = onb_mcts_run(x, ag->evaluator, ag->sims);
     } else {
@@ -1001,7 +1037,7 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
     for (const onb_agent* ag : {a, b}) {
         if (ag->kind != ONB_AGENT_RANDOM && ag->kind != ONB_AGENT_PUCT && ag->kind != ONB_AGENT_UCT && ag->kind != ONB_AGENT_ALPHABETA &&
             ag->kind != ONB_AGENT_GUMBEL && ag->kind != ONB_AGENT_TABLEBASE && ag->kind != ONB_AGENT_GUMBEL_MUZERO && ag->kind != ONB_AGENT_PUCT_VL &&
-            ag->kind != ONB_AGENT_PUCT_TB)
+            ag->kind != ONB_AGENT_PUCT_TB && ag->kind != ONB_AGENT_PUCT_SOLVER)
             return fail(c, ONB_E_INVALID, "onb_fight: unknown agent kind %d", ag->kind);
         if (ag->kind == ONB_AGENT_PUCT_TB && !c->tb_live)
             return fail(c, ONB_E_STATE, "onb_fight: a PUCT agent with tablebase leaves needs a solved table (onb_tb_solve)");
@@ -1044,6 +1080,7 @@ int32_t onb_fight(onb_ctx* ctx, const onb_agent* a, const onb_agent* b, const ui
     for (const onb_agent* ag : {a, b})
         if (ag->kind == ONB_AGENT_PUCT_VL && ag->min_node_visits > vl_need) vl_need = ag->min_node_visits;
     if (vl_need && (rc = vl_alloc(c, vl_need)) != ONB_OK) return rc;
+    if ((a->kind == ONB_AGENT_PUCT_SOLVER || b->kind == ONB_AGENT_PUCT_SOLVER) && c->d_nodes && (rc = solver_alloc(c)) != ONB_OK) return rc;
     char err[400];
     err[0] = 0;
     rc = run_fight(c, a, b, a_is_red_host, max_plies, out, fight_move, err, sizeof(err));
@@ -1085,6 +1122,7 @@ int32_t onb_uct_run(onb_ctx* ctx, float exploration_c, uint32_t min_node_visits,
     if (a.plan.gumbel) return fail(c, ONB_E_STATE, "onb_uct_run: the search was begun with the Gumbel root search on (onb_mcts_set_gumbel)");
     if (a.plan.leaves >= 2) return fail(c, ONB_E_STATE, "onb_uct_run: the search was begun with virtual loss on (onb_mcts_set_virtual_loss)");
     if (a.plan.tb) return fail(c, ONB_E_STATE, "onb_uct_run: the search was begun with tablebase leaves on (onb_mcts_set_tablebase)");
+    if (a.plan.solver) return fail(c, ONB_E_STATE, "onb_uct_run: the search was begun with the MCTS solver on (onb_mcts_set_solver)");
     if (a.sims_done + playouts > c->cfg.mcts_max_sims) return fail(c, ONB_E_INVALID, "onb_uct_run: more playouts than mcts_max_sims");
     const uint32_t need = a.sims_done + playouts + 2;
     if (c->ln_cap < need) {  // ln(parent visits) as the reference computes it: f32 logf on the host

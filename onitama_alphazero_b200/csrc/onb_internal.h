@@ -20,10 +20,12 @@ struct __align__(32) Node {
     uint32_t parent;       // 0xFFFFFFFF for the root
     uint16_t action;       // move that leads here (onb_action)
     uint8_t n_child;
-    uint8_t flags;         // bit0 expanded, bit1 terminal, bit2 pass pseudo-child
+    uint8_t flags;         // bit0 expanded, bit1 terminal, bit2 pass pseudo-child, bit3 proven win, bit4 proven loss (DESIGN.md §5k)
 };
 static_assert(sizeof(Node) == 32, "node must be one sector");
 constexpr uint8_t kNodeExpanded = 1, kNodeTerminal = 2, kNodePass = 4;
+// MCTS solver (onb_mcts_set_solver, DESIGN.md §5k): the side that moved into the node wins / loses with best play
+constexpr uint8_t kNodeWin = ONB_NODE_WIN, kNodeLoss = ONB_NODE_LOSS, kNodeProven = ONB_NODE_WIN | ONB_NODE_LOSS;
 constexpr uint8_t kTreePassSeen = 1, kTreeOverflow = 2;
 constexpr int kMaxDepth = 32;  // path entries kept in registers (lane l <-> level l); deeper paths spill to the parent chain
 
@@ -69,6 +71,7 @@ struct SearchPlan {
     bool tb;                 // tablebase leaves (onb_mcts_set_tablebase, DESIGN.md §5i): begin_search copies the table into tb_table
     TbTable tb_table;
     uint32_t tb_serial;      // Ctx::tb_serial at the begin: the search continues only while that table is resident
+    bool solver;             // the MCTS solver (onb_mcts_set_solver, DESIGN.md §5k)
 };
 // Descents of the next round of a search with virtual loss (DESIGN.md §5h), from the descents done so far (= the root's visits) and
 // the target the round counts against: 1 for round 0, then min(K, target - done). The kernels derive it from the root's visit count,
@@ -206,6 +209,9 @@ struct Ctx {
     uint8_t* d_choose_mask;   // [n] onb_mcts_choose's sample mask
     int sp_ran;               // an onb_self_play has run (its protocol stats are readable)
     onb_selfplay_protocol_stats sp_stats;
+    // MCTS solver (onb_mcts_set_solver, DESIGN.md §5k)
+    int solver_on;            // the switch
+    int8_t* d_root_proof;     // [n] ONB_BUF_ROOT_PROOF, written by the solver's finish; allocated by the first enabling call
     char err[512];
 };
 
@@ -242,7 +248,7 @@ cudaError_t launch_mcts_choose(Ctx* c, const uint16_t* best, uint64_t seed, uint
                                const int32_t* plies, uint32_t temp_plies, uint16_t* dst_actions);
 // the search launchers take their kernel from c->search.plan: noise, Gumbel at the root (select, run, finish) and Gumbel MuZero
 // below it (select, run, expand_backup), virtual loss (select, eval, expand_backup over the K rows of every tree, round target
-// search.vl_target), tablebase leaves (expand_backup)
+// search.vl_target), tablebase leaves (expand_backup), the solver (select, run, expand_backup, finish; finish also writes d_root_proof)
 
 // network (onb_net.cu)
 int32_t net_load(Ctx* c, int32_t n_tensors, const char* const* names, const float* const* data, const int64_t* numel, std::string& err);

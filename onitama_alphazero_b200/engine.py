@@ -35,6 +35,7 @@ class Context:
         self.game_id_base = game_id_base
         self.mcts_max_sims = mcts_max_sims
         self.tb_leaves = False  # the tablebase-leaf switch (set_tablebase)
+        self.solver = False     # the MCTS solver switch (set_solver)
         self._tb_serial = 0     # raised by every tb_solve / tb_free: the table a captured search round was given
 
     # ------------------------------------------------------------------ plumbing
@@ -94,7 +95,7 @@ class Context:
                 L.BUF_ACTIONS: ((n,), "<i2", None), L.BUF_LEAF_PLANES: ((n, 21, 5, 5), "<f4", None),
                 L.BUF_POLICY: ((n, 2, 25), "<f4", None), L.BUF_VALUE: ((n,), "<f4", None), L.BUF_PI: ((n, 2, 25), "<f4", None),
                 L.BUF_BEST: ((n,), "<i2", None), L.BUF_STATES: ((n, 4), "<i4", None), L.BUF_STATS: ((L.STAT_COUNT,), "<i8", None),
-                L.BUF_ROOT_M: ((n,), "<f8", None)}[which]
+                L.BUF_ROOT_M: ((n,), "<f8", None), L.BUF_ROOT_PROOF: ((n,), "|i1", None)}[which]
         shape, typestr, _ = spec
         if typestr == "<u4":
             typestr = "<i4"
@@ -239,6 +240,23 @@ class Context:
         self._ck(self._lib.onb_mcts_set_tablebase(self._h, int(bool(enabled))))
         self.tb_leaves = bool(enabled)
 
+    def set_solver(self, enabled):
+        """onb_mcts_set_solver: the MCTS solver for the searches begun afterwards -- immediate wins are marked at expansion, proofs
+        (ONB_NODE_WIN / ONB_NODE_LOSS in the tree dump) are propagated to the root, descents stop at proven nodes and skip children
+        proven lost, and mcts_finish plays a proven win. See include/onb.h and DESIGN.md §5k."""
+        self._ck(self._lib.onb_mcts_set_solver(self._h, int(bool(enabled))))
+        self.solver = bool(enabled)
+
+    def _use_solver(self, solver):
+        """the solver= argument of the search drivers: None leaves the solver switch, True / False sets it"""
+        if solver is not None and bool(solver) != self.solver:
+            self.set_solver(solver)
+
+    def root_proof(self):
+        """ONB_BUF_ROOT_PROOF after mcts_finish of a solver search: int8 [n], +1 the side to move wins with best play, -1 it loses,
+        0 unproven (game order)"""
+        return self.read(L.BUF_ROOT_PROOF, np.int8, (self.n,))
+
     def _use_tb(self, tb):
         """the tb= argument of the search drivers: None leaves the tablebase-leaf switch, True / False sets it"""
         if tb is not None and bool(tb) != self.tb_leaves:
@@ -376,12 +394,17 @@ class Context:
         return L.Agent(L.AGENT_RANDOM, 0, 0, 0, 0.0, 0, 0)
 
     @staticmethod
-    def agent_puct(sims, c_puct=2.0, evaluator=L.EVAL_UNIFORM, net_slot=0, leaves=1, tablebase=False):
+    def agent_puct(sims, c_puct=2.0, evaluator=L.EVAL_UNIFORM, net_slot=0, leaves=1, tablebase=False, solver=False):
         """AlphaZeroMcts as an arena agent; leaves > 1: ONB_AGENT_PUCT_VL, rounds of `leaves` descents with virtual loss 1;
         tablebase=True: ONB_AGENT_PUCT_TB, the table's move in the games of the resident table and a search with tablebase leaves in
-        the others (no agent kind combines it with leaves > 1)"""
+        the others (no agent kind combines it with leaves > 1); solver=True: ONB_AGENT_PUCT_SOLVER, a search with the MCTS solver
+        playing its best move (no agent kind combines it with leaves > 1 or tablebase=True)"""
         if tablebase and leaves > 1:
             raise ValueError("agent_puct: tablebase=True does not combine with leaves > 1 (no agent kind covers both)")
+        if solver and (leaves > 1 or tablebase):
+            raise ValueError("agent_puct: solver=True does not combine with leaves > 1 or tablebase=True (no agent kind covers both)")
+        if solver:
+            return L.Agent(L.AGENT_PUCT_SOLVER, evaluator, net_slot, sims, c_puct, 0, 0)
         if tablebase:
             return L.Agent(L.AGENT_PUCT_TB, evaluator, net_slot, sims, c_puct, 0, 0)
         if leaves > 1:
@@ -559,13 +582,15 @@ class Context:
         self._ck(self._lib.onb_mcts_dump_tree(self._h, tree, cap, C.byref(td), C.byref(nn)))
         return {k: v[:nn.value].copy() for k, v in arrs.items()}
 
-    def search(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, fused=True, net=None, vl=None, tb=None):
+    def search(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, fused=True, net=None, vl=None, tb=None, solver=None):
         """MctsArena::search for every game at once. net: callable(leaf_planes tensor [n,21,5,5]) -> (policy [n,2,25], value [n])
         running on this context's stream; it reads/writes the device buffers zero-copy. vl: None leaves the virtual-loss switch, K or
         (K, virtual_loss) sets it, 1 switches it off (set_virtual_loss); with it on, `net` gets the n K rows of ONB_BUF_VL_PLANES and
-        the split phase runs vl_rounds(sims) rounds. tb: None leaves the tablebase-leaf switch, True / False sets it (set_tablebase)."""
+        the split phase runs vl_rounds(sims) rounds. tb: None leaves the tablebase-leaf switch, True / False sets it (set_tablebase).
+        solver: None leaves the MCTS solver switch, True / False sets it (set_solver); root_proof() reads the proofs afterwards."""
         self._use_vl(vl)
         self._use_tb(tb)
+        self._use_solver(solver)
         self.mcts_begin(c_puct, sims)
         if net is None and fused:
             self.mcts_run(evaluator, sims)
@@ -657,7 +682,8 @@ class Actor:
             pass
 
 
-def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_graph=False, reuse=None, gumbel=None, vl=None, tb=None):
+def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_graph=False, reuse=None, gumbel=None, vl=None, tb=None,
+                   solver=None):
     """Context.search without copying the results to the host (PI / BEST stay in their device buffers).
     use_graph: capture one simulation round (select -> network -> expand/backup) in a CUDA graph on the context's stream and
     replay it; the round is launch-bound otherwise (~40 small network kernels per round).
@@ -667,12 +693,14 @@ def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_g
     when that setting is not on already, so that consecutive searches take consecutive steps).
     vl: as for search. With virtual loss a torch `net` gets the n K rows, and use_graph runs round 0 eagerly and replays one captured
     round for the others: the kernels take a round's descents from the root's visit count, so the short last round replays too.
-    tb: as for search. A captured round with tablebase leaves bakes in the table, so a new tb_solve captures anew."""
+    tb: as for search. A captured round with tablebase leaves bakes in the table, so a new tb_solve captures anew.
+    solver: as for search; a captured round bakes in the solver's kernels, so the switch is part of the graph key."""
     if reuse is not None and bool(reuse) != getattr(self, "reuse", False):
         self.set_reuse(reuse)
     self._use_gumbel(gumbel)
     self._use_vl(vl)
     self._use_tb(tb)
+    self._use_solver(solver)
     if net is not None and getattr(self, "reuse", False):
         raise ValueError("search_device: tree reuse needs a device evaluator (EVAL_UNIFORM / EVAL_HASH / EVAL_NET), not a torch net")
     self.mcts_begin(c_puct, sims)
@@ -714,7 +742,7 @@ def _search_device(self, c_puct, sims, evaluator=L.EVAL_UNIFORM, net=None, use_g
                 # a captured round bakes in everything the launches were given: the evaluator, c_puct AND the root-noise settings
                 # (ADVICE r01: switching train mode after a capture must not replay the old setting). The cache holds a strong
                 # reference to `net`, so its id cannot be recycled for another module while the graph lives; close() drops it.
-                key = (id(net), float(c_puct), getattr(self, "_noise", (False,)), getattr(self, "gumbel", None), self._tb_graph_key())
+                key = (id(net), float(c_puct), getattr(self, "_noise", (False,)), getattr(self, "gumbel", None), self._tb_graph_key(), self.solver)
                 cache = self.__dict__.setdefault("_graphs", {})
                 done = 0
                 if key not in cache:

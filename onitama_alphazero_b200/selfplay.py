@@ -328,6 +328,18 @@ def puct_tb_move(sims, c_puct=2.0, evaluator=L.EVAL_UNIFORM):
     return move
 
 
+def puct_solver_move(sims, c_puct=2.0, evaluator=L.EVAL_UNIFORM):
+    """ONB_AGENT_PUCT_SOLVER as a move function of fight(): an eval-mode PUCT search with the MCTS solver (solver=True) over every game,
+    playing the solver's best move. The context's solver switch is left as it was; ctx.last_root_proof keeps the root proofs."""
+    def move(ctx):
+        was = ctx.solver
+        ctx.search_device(c_puct, sims, evaluator=evaluator, solver=True)
+        ctx.last_root_proof = ctx.root_proof()
+        ctx._use_solver(was)
+        ctx.tensor(L.BUF_ACTIONS).copy_(ctx.tensor(L.BUF_BEST))
+    return move
+
+
 class ReplayBuffer:
     """Fixed-capacity ring buffer of self-play samples on one device (train.rs:213,241-245 keeps `data_buffer =
     Vec::with_capacity(buffer_size)` and only ever extends it; the ring bounds it: the newest samples overwrite the oldest).
